@@ -10,6 +10,7 @@ collective).  One JSON line is printed by rank 0 — see the keys below.
     python bench.py --gpus 1 --steps 10 --warmup 3
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference          # the CPU port of the reference path (oracle/)
+    python bench.py --dump-outputs DIR        # also write the last timed step's y, dq, dk, dv to DIR/<name>.npy
 
 value    : tokens/s, inputs resident in HBM, CUDA-event timed, max over ranks
 e2e      : tokens/s through the public layer API with HOST (pinned) buffers: H2D of q,k,v,dO and
@@ -164,7 +165,7 @@ def run_reference(args):
     cores = os.cpu_count() or 1
     torch.set_num_threads(cores)
     heads = args.ref_heads
-    steps, warmup = max(1, min(args.steps, 40)), max(0, min(args.warmup, 10))
+    steps, warmup = args.steps, args.warmup
     for _ in range(warmup):
         cpu_reference_step(heads)
     times = [cpu_reference_step(heads) for _ in range(steps)]
@@ -464,6 +465,24 @@ def sweep_bench(dev, rank, world, barrier, iters=3):
     return rows
 
 
+DUMP_BYTES = 32 << 20       # float32 bytes over all dumped arrays; at the bench shape every output is sampled
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """Writes every array as out_dir/<name>.npy in float32.  One larger than its share of DUMP_BYTES is reduced to
+    the elements at a fixed sample of flat positions (seeded, ascending, the same on every run), so the files of two
+    builds can be compared element for element."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    n_max = DUMP_BYTES // 4 // len(arrays)
+    for name, t in arrays.items():
+        t = t.detach()
+        if t.numel() > n_max:
+            pos = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))[:n_max].sort().values
+            t = t.reshape(-1)[pos.to(t.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
+
+
 # ---------------------------------------------------------------------------------------------------
 # main arm
 # ---------------------------------------------------------------------------------------------------
@@ -525,11 +544,13 @@ def run_ours(args):
     torch.cuda._sleep(1_000_000)
     a.record()
     for _ in range(args.steps):
-        step()
+        y = step()
     b.record()
     barrier()
     elapsed = a.elapsed_time(b) * 1e-3
     launches = ext.launch_count() - launches0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"y": y, "dq": q.grad, "dk": k.grad, "dv": v.grad})
 
     # ---- e2e: host (pinned) buffers in, host buffers out, through the public layer API ---------------
     # chunk-major pinned buffers: the four operands of a sequence are contiguous, one copy per chunk and direction
@@ -734,7 +755,14 @@ def main():
     ap.add_argument("--stage-path", action="store_true", help="run the reference-style stage kernels, not the fused path")
     ap.add_argument("--no-finetune", action="store_true", help="skip the configs[3] fine-tuning-step section")
     ap.add_argument("--no-sweep", action="store_true", help="skip the configs[4] sweep section")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write y, dq, dk, dv of the last timed step (rank 0) as DIR/<name>.npy, float32, a fixed "
+                         "seeded sample of each (32 MiB in all); GPU path only, refused with --impl reference")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     if args.impl == "reference":
         run_reference(args)
     else:

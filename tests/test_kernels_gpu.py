@@ -3,6 +3,8 @@ the CPU oracle (oracle/spt_oracle.py) — shape families follow the reference's 
 with fixed seeds.  Tolerances: PQ codes / lookup indices / CSC structure bit-exact; fp32 values
 atol 1e-3 (the reference tests' own tolerance, test_cdist.py:48-52, test_sddmm.py:79-85, ...);
 bf16 operands: compared after identical upcast, atol 2e-2 on bf16 outputs."""
+import os
+
 import pytest
 import torch
 
@@ -10,6 +12,10 @@ from oracle import spt_oracle as O
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda"
+
+
+def _gold(name):
+    return torch.load(os.path.join(os.path.dirname(__file__), "golden", name + ".pt"))
 
 
 def _ext():
@@ -171,6 +177,16 @@ def test_lookup_vs_reference_kernel(ref_ext):
         # conflict) as "lowest lane wins", which is what B200 does: all three must agree bit for bit
         assert torch.equal(ref.cpu(), emu), f"emulator vs reference kernel: {(ref.cpu() != emu).sum().item()} mismatches"
         assert torch.equal(got.cpu(), ref.cpu())
+
+
+def test_lookup_vs_recorded_reference_kernel():
+    """Without the reference extension: outputs of the unmodified reference lookup kernel recorded on a B200
+    (golden/lookup_ref_kernel_b200.pt, written by golden/make_lookup_golden_gpu.py; S 256 and 512)."""
+    for case in _gold("lookup_ref_kernel_b200"):
+        q, k, ref, coeff = case["q"].int(), case["k"].int(), case["ref"].int(), case["sparse_coeff"]
+        got = _kernels().lookup(q.to(DEV), k.to(DEV), sparse_coeff=coeff)
+        assert torch.equal(O.lookup_forward(q, k, coeff), ref)
+        assert torch.equal(got.cpu(), ref)
 
 
 # ---------------------------------------------------------------------------------- sddmm / softmax / spmm
@@ -353,6 +369,49 @@ def test_stage_kernels_vs_reference_extension(ref_ext):
     gq_got, gt_got = _ext().cdist_backward_cuda(qq, tt, go)
     assert torch.allclose(gq_ref, gq_got, atol=1e-4)
     assert torch.allclose(gt_ref, gt_got, atol=2e-2, rtol=1e-3)
+
+
+def test_stage_kernels_vs_reference_test_formulas():
+    """fp32 stage kernels, forward and backward, against the dense torch formulas the reference's kernel tests use as
+    oracles (test_sddmm.py:58-62, test_softmax.py:70, test_spmm.py:56), evaluated on a seeded pattern by
+    golden/make_golden.py (stage_formulas.pt), and cdist against the codes of the reference's PQV1 encoder (pq_v1.pt).
+    Every kernel reads the formulas' output of the stage before it, so a mismatch names one kernel."""
+    gd = _gold("stage_formulas")
+    B, S, d = gd["q"].shape
+    indptr = O.fixed_indptr(S, gd["k_per"]).to(DEV)
+    indices = gd["indices"].to(DEV)
+    rows = torch.arange(S).repeat_interleave(gd["k_per"])
+
+    def at(dense):            # [B, S, S] -> the CSR values of the pattern, on the device
+        return dense[torch.arange(B).view(-1, 1), rows.view(1, -1), gd["indices"].long()].to(DEV)
+
+    q, kk, v, w = (gd[n].to(DEV) for n in ("q", "k", "v", "w"))
+    f, t = torch.scalar_tensor(False), torch.scalar_tensor(True)
+    vals = _ext().sddmm_forward_cuda(f, t, indptr, indices, q, kk)
+    assert torch.allclose(vals, at(gd["scores"]), atol=1e-3)
+    s_raw = at(gd["scores"]) * d ** -0.5
+    p_gold = at(gd["probs"])
+    p = _ext().softmax_forward_cuda(indptr, indices, torch.clamp(s_raw, -10, 10))
+    assert torch.allclose(p, p_gold, atol=1e-5)
+    y = _ext().spmm_forward_cuda(f, f, indptr, indices, p_gold, v)
+    assert torch.allclose(y.cpu(), gd["y"], atol=1e-4)
+    dv = _ext().spmm_forward_cuda(t, f, indptr, indices, p_gold, w)
+    assert torch.allclose(dv.cpu(), gd["dv"], atol=1e-3)
+    # dQ, dK of sum(y * w): dP on the pattern, softmax backward, scale backward, direct and transposed product.  No score
+    # of these vectors reaches the clamp at +-10 (max |s| 3.5), so its backward is the identity here and not tested.
+    assert s_raw.abs().max() < 10
+    dp = _ext().sddmm_forward_cuda(f, t, indptr, indices, w, v)
+    ds = _ext().softmax_backward_cuda(indptr, indices, p_gold, dp) * d ** -0.5
+    dq = _ext().spmm_forward_cuda(f, f, indptr, indices, ds, kk)
+    dk = _ext().spmm_forward_cuda(t, f, indptr, indices, ds, q)
+    assert torch.allclose(dq.cpu(), gd["dq"], atol=1e-3)
+    assert torch.allclose(dk.cpu(), gd["dk"], atol=1e-3)
+    # cdist: the reference encoder's codes (torch.cdist(p=1) + argmin, quantizer.py:53-62), ties included
+    for case in _gold("pq_v1"):
+        m, c, dc = case["weight"].shape
+        z = case["z"].reshape(-1, m, dc).transpose(0, 1).contiguous()           # [m, n, dc], quantizer.py:43-48
+        _, codes = _ext().cdist_forward_cuda(z.to(DEV), case["weight"].to(DEV))
+        assert torch.equal(codes.t().cpu().long(), case["codes"].reshape(-1, m).long())
 
 
 # ---------------------------------------------------------------------------------- error behaviour
