@@ -217,7 +217,9 @@ int spt_softmax_clamp_bwd(const int32_t *indptr, const int32_t *indices, const f
  *
  * spt_sparse_attn_fwd: q, k, v [B, S, d] bf16 ->
  *   y [B, S, d] bf16 = sum_j p_rj v_j,  p = w * exp(clamp(scale * q.k, -clamp, clamp)) / Z,
- *   zsum [B, S] fp32 = Z (row sums, >= 1e-9) saved for the backward.  d = 64, S % 128 == 0.
+ *   zsum [B, S] fp32 = Z (row sums, >= 1e-9) saved for the backward.  d = 64, 80 or 128 (others
+ *   return SPT_ERR_UNSUPPORTED), S % 128 == 0.  d = 80 (OPT-2.7B) is padded to 128 in shared
+ *   memory and tensor memory only: every global read and write is exactly d columns wide.
  * spt_sparse_attn_bwd: grad_y -> grad_q, grad_k, grad_v [B, S, d] bf16.  Recomputes p from q, k
  *   (nothing of size S x k is read or written); deterministic (no atomics).
  *   workspace: spt_sparse_attn_bwd_workspace_bytes(B, S).

@@ -4,6 +4,7 @@
 #pragma once
 #include <cstdlib>
 #include <cstring>
+#include <type_traits>
 
 #include "tc.cuh"
 
@@ -17,13 +18,18 @@ constexpr int BN = 64;         // other tile rows per iteration
 constexpr int STAGES = 3;
 constexpr int N_MATH = 256;      // warps 0-7
 constexpr int THREADS = 320;
-// Head dim D in {64, 128}.  Operand tiles are stored as D / 64 sub-tiles of [rows][64] bf16 (one TMA box
-// each, 128-byte swizzled): an owner tile is [D/64][128 rows][64], an "other" tile [D/64][64 rows][64].
-// D = 64 needs 256 TMEM columns (two CTAs per SM), D = 128 takes the whole TMEM (one CTA per SM).
+// Head dim D in {64, 80, 128}.  Operand tiles are stored as NSUB = ceil(D / 64) sub-tiles of [rows][64] bf16 (one TMA
+// box each, 128-byte swizzled): an owner tile is [NSUB][128 rows][64], an "other" tile [NSUB][64 rows][64].
+// D = 80 is padded to DP = 128 in shared memory and TMEM only: the second box starts at column 64 and the TMA fills
+// its 48 columns past the row end with zeros, so Q K^T is unchanged and O, dQ, dK, dV get zero columns 80 .. 127,
+// which the epilogues never store.  The MMA shapes, TMEM columns and pipeline are those of D = 128.
+// D = 64 needs 256 TMEM columns (two CTAs per SM), D = 80 and 128 take the whole TMEM (one CTA per SM).
 template <int D>
 struct Dim {
-    static_assert(D == 64 || D == 128, "head dim must be 64 or 128");
-    static constexpr int NSUB = D / 64;
+    static_assert(D == 64 || D == 80 || D == 128, "head dim must be 64, 80 or 128");
+    static constexpr int NSUB = (D + 63) / 64;
+    static constexpr int DP = NSUB * 64;                                       // padded width in shared memory / TMEM
+    static constexpr int PREP_LANES = D / 8 <= 8 ? 8 : 16;                     // lanes per row of attn_bwd_prep_kernel
     static constexpr int OWN_SUB = BM * 64 * 2, T_SUB = BN * 64 * 2;          // 16 KB, 8 KB
     static constexpr int OWN_BYTES = NSUB * OWN_SUB, T_BYTES = NSUB * T_SUB;
     static constexpr int TMEM_COLS = D == 64 ? 256 : 512;
@@ -338,6 +344,39 @@ __device__ __forceinline__ void store_row32(__nv_bfloat16 *dst, const uint32_t (
 #pragma unroll
         for (int u = 0; u < 8; ++u) t[u] = __uint_as_float(r[i + u]) * s;
         Vec16<__nv_bfloat16>::store(dst + i, t);
+    }
+}
+// the same for the first W (16 or 32) of the 32 values
+template <int W>
+__device__ __forceinline__ void store_row_n(__nv_bfloat16 *dst, const uint32_t (&r)[32], float s) {
+    static_assert(W % 8 == 0 && W <= 32, "W must be a multiple of 8, at most 32");
+#pragma unroll
+    for (int i = 0; i < W; i += 8) {
+        float t[8];
+#pragma unroll
+        for (int u = 0; u < 8; ++u) t[u] = __uint_as_float(r[i + u]) * s;
+        Vec16<__nv_bfloat16>::store(dst + i, t);
+    }
+}
+template <int W>
+using Width = std::integral_constant<int, W>;
+// The epilogues read a row's D output columns from TMEM in 32-column chunks shared by the two warpgroups (`half`):
+// f(col, Width<W>) stores columns [col, col + W).  D = 64, 128: warpgroup h takes [h D/2, (h + 1) D/2).  D = 80:
+// warpgroup 0 takes [0, 32) and [64, 80), warpgroup 1 [32, 64); the padding columns 80 .. 127 are never stored (in the
+// [N, S, H, 80] layout they would overwrite the next head's row).
+template <int D, typename F>
+__device__ __forceinline__ void out_chunks(int half, F &&f) {
+    if constexpr (D % 64 == 0) {
+#pragma unroll
+        for (int c = 0; c < D / 64; ++c) f(half * (D / 2) + c * 32, Width<32>{});
+    } else {
+        static_assert(D == 80, "odd head dims other than 80 need their own column split");
+        if (half == 0) {
+            f(0, Width<32>{});
+            f(64, Width<16>{});
+        } else {
+            f(32, Width<32>{});
+        }
     }
 }
 

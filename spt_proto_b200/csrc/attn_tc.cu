@@ -52,7 +52,7 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_const
                    const int32_t *__restrict__ extra0, __nv_bfloat16 *__restrict__ y, float *__restrict__ zsum, int S,
                    int H, float scale_log2, float clamp_log2, int y_transposed) {
     constexpr int OWN_BYTES = Dim<D>::OWN_BYTES, T_BYTES = Dim<D>::T_BYTES, OWN_SUB = Dim<D>::OWN_SUB, T_SUB = Dim<D>::T_SUB,
-                  TMEM_COLS = Dim<D>::TMEM_COLS;
+                  TMEM_COLS = Dim<D>::TMEM_COLS, DP = Dim<D>::DP;
     constexpr int NBUF = 3;                            // score buffers
     extern __shared__ unsigned char smem_raw[];
     const Smem sm = align_smem(smem_raw);
@@ -121,7 +121,7 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_const
     } else if (warp == 9) {
         // ===== MMA issuer: the whole warp runs the (uniform) loop, one elected lane issues =====
         constexpr uint32_t id_s = idesc_bf16(BM, BN, 0, 0);   // S = Q K^T   (both K-major)
-        constexpr uint32_t id_o = idesc_bf16(BM, D, 0, 1);    // O += P V    (A from TMEM, V MN-major)
+        constexpr uint32_t id_o = idesc_bf16(BM, DP, 0, 1);    // O += P V    (A from TMEM, V MN-major)
         const uint64_t dq0 = desc_kmajor(s_q, 0), dk0 = desc_kmajor(s_k, 0), dv0 = desc_mnmajor(s_v, 0, T_SUB);
         // S = Q K^T runs two tiles ahead of O += P V, into the third (free) buffer, so the k-steps of S(j + 2) and of
         // PV(j) touch different TMEM columns and are interleaved: two accumulator chains in flight (consecutive MMAs into
@@ -135,7 +135,7 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_const
             if (elect_one()) {
                 const uint64_t dk = dk0 + (uint64_t)(st * (T_BYTES >> 4));
 #pragma unroll
-                for (int k = 0; k < D / 16; ++k)
+                for (int k = 0; k < DP / 16; ++k)
                     umma_bf16(tmem_base + COL_S + (j % NBUF) * BN, dq0 + kslice<OWN_SUB>(k), dk + kslice<T_SUB>(k), id_s, k != 0);
                 umma_commit(s_full(j % NBUF));
                 umma_commit(k_empty(st));
@@ -160,7 +160,7 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_const
                 const uint64_t dv = dv0 + (uint64_t)(st * (T_BYTES >> 4));
                 const uint64_t dk = dk0 + (uint64_t)(stn * (T_BYTES >> 4));
                 const uint32_t s_next = tmem_base + COL_S + ((j + 2) % NBUF) * BN, p_cur = tmem_base + COL_S + (j % NBUF) * BN;
-                constexpr int KS = D / 16, KP = BN / 16;
+                constexpr int KS = DP / 16, KP = BN / 16;
 #pragma unroll
                 for (int k = 0; k < (KS > KP ? KS : KP); ++k) {
                     if (k < KS && has_next) umma_bf16(s_next, dq0 + kslice<OWN_SUB>(k), dk + kslice<T_SUB>(k), id_s, k != 0);
@@ -242,24 +242,22 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_const
         mbar_wait(o_full, 0);
         fence_after_sync();
         if (!y_transposed) {
-            __nv_bfloat16 *dst = y + (((size_t)hn * S + row) * H + hh) * D + half * (D / 2);
-#pragma unroll
-            for (int c = 0; c < D / 64; ++c) {
+            __nv_bfloat16 *dst = y + (((size_t)hn * S + row) * H + hh) * D;
+            out_chunks<D>(half, [&](int col, auto w) {
                 uint32_t r[32];
-                tmem_ld32(lane_base + COL_O + half * (D / 2) + c * 32, r);
-                store_row32(dst + c * 32, r, inv);
-            }
+                tmem_ld32(lane_base + COL_O + col, r);
+                store_row_n<decltype(w)::value>(dst + col, r, inv);
+            });
         } else {
             // the shipped reference layer's output layout (attention.py:139-142): y^T [B, D, S] memory; a warp's 32
             // consecutive rows of one feature are 64 contiguous bytes
-            __nv_bfloat16 *dst = y + ((size_t)b * D + half * (D / 2)) * S + row;
-#pragma unroll
-            for (int c = 0; c < D / 64; ++c) {
+            out_chunks<D>(half, [&](int col, auto w) {
+                __nv_bfloat16 *dst = y + ((size_t)b * D + col) * S + row;
                 uint32_t r[32];
-                tmem_ld32(lane_base + COL_O + half * (D / 2) + c * 32, r);
+                tmem_ld32(lane_base + COL_O + col, r);
 #pragma unroll
-                for (int i = 0; i < 32; ++i) dst[(size_t)(c * 32 + i) * S] = __float2bfloat16(__uint_as_float(r[i]) * inv);
-            }
+                for (int i = 0; i < decltype(w)::value; ++i) dst[(size_t)i * S] = __float2bfloat16(__uint_as_float(r[i]) * inv);
+            });
         }
         PROF(pf.t[7] = clock64() - t_loop_end; pf.flush(0, 0, threadIdx.x == 0);)
     }
@@ -277,30 +275,37 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_const
 
 // ---------------------------------------------------------------------------------------------------
 // Backward prologue: -delta'_r = -(dO_r . y_r) / Z_r (stored negated)  and  dO'_r = dO_r / Z_r (bf16, same layout as dO).
-// 8 lanes per row (8 x 16 B = one 128-byte row).
+// D / 8 lanes per row (16 B each) in an aligned group of PREP_LANES lanes (a power of two for the butterfly sum; at
+// D = 80, 10 of 16 lanes carry data).
 // ---------------------------------------------------------------------------------------------------
 template <int D>
 __global__ void __launch_bounds__(256)
 attn_bwd_prep_kernel(const __nv_bfloat16 *__restrict__ dy, const __nv_bfloat16 *__restrict__ y,
                      const float *__restrict__ zsum, float *__restrict__ delta, __nv_bfloat16 *__restrict__ dys,
                      int64_t rows, int S, int H) {
-    constexpr int LPR = D / 8;                                             // lanes per row (16 B each)
-    const int64_t row = (int64_t)blockIdx.x * (256 / LPR) + (threadIdx.x / LPR);
+    constexpr int LPR = D / 8, G = Dim<D>::PREP_LANES;                    // data lanes per row, lanes per row
+    const int64_t row = (int64_t)blockIdx.x * (256 / G) + (threadIdx.x / G);
     if (row >= rows) return;
-    const int sub = threadIdx.x % LPR;
+    const int sub = threadIdx.x % G;
+    const bool active = sub < LPR;
     const int64_t b = row / S, r = row % S;                               // delta, zsum are head-major [B, S]
     const int64_t off = (((b / H) * S + r) * H + (b % H)) * D + sub * 8;
     float a[8], c[8];
-    Vec16<__nv_bfloat16>::load(dy + off, a);
-    Vec16<__nv_bfloat16>::load(y + off, c);
+    if (active) {
+        Vec16<__nv_bfloat16>::load(dy + off, a);
+        Vec16<__nv_bfloat16>::load(y + off, c);
+    } else {
+#pragma unroll
+        for (int i = 0; i < 8; ++i) a[i] = c[i] = 0.0f;
+    }
     float acc = 0.0f;
 #pragma unroll
     for (int i = 0; i < 8; ++i) acc = fmaf(a[i], c[i], acc);
-    acc = group_sum<LPR>(acc);
+    acc = group_sum<G>(acc);
     const float inv = 1.0f / zsum[row];
 #pragma unroll
     for (int i = 0; i < 8; ++i) a[i] *= inv;
-    Vec16<__nv_bfloat16>::store(dys + off, a);
+    if (active) Vec16<__nv_bfloat16>::store(dys + off, a);
     if (sub == 0) delta[row] = -acc * inv;        // stored negated: the kernels add it (dp - delta')
 }
 
@@ -340,12 +345,20 @@ attn_bwd_prep_t_kernel(const __nv_bfloat16 *__restrict__ dyt, const __nv_bfloat1
     const float inv = 1.0f / zsum[grow];
     const int hn = b / H, hh = b % H;
     __nv_bfloat16 *dst = dys + (((size_t)hn * S + r0 + r) * H + hh) * D + qd * EPT;
+    if constexpr (EPT % 8 == 0) {
 #pragma unroll
-    for (int i = 0; i < EPT; i += 8) {
-        float t[8];
+        for (int i = 0; i < EPT; i += 8) {
+            float t[8];
 #pragma unroll
-        for (int u = 0; u < 8; ++u) t[u] = a[i + u] * inv;
-        Vec16<__nv_bfloat16>::store(dst + i, t);
+            for (int u = 0; u < 8; ++u) t[u] = a[i + u] * inv;
+            Vec16<__nv_bfloat16>::store(dst + i, t);
+        }
+    } else {
+        // D = 80: a thread's 20 features start 40 bytes apart, so 8-byte stores
+        static_assert(EPT % 4 == 0, "features per thread must be a multiple of 4");
+#pragma unroll
+        for (int i = 0; i < EPT; i += 4)
+            *reinterpret_cast<uint2 *>(dst + i) = make_uint2(pack_bf16(a[i] * inv, a[i + 1] * inv), pack_bf16(a[i + 2] * inv, a[i + 3] * inv));
     }
     if (qd == 0) delta[grow] = -acc * inv;
 }
@@ -365,7 +378,7 @@ attn_bwd_q_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
                      const float *__restrict__ delta, __nv_bfloat16 *__restrict__ dq, int S, int H, float scale,
                      float scale_log2, float clamp_log2) {
     constexpr int OWN_BYTES = Dim<D>::OWN_BYTES, T_BYTES = Dim<D>::T_BYTES, OWN_SUB = Dim<D>::OWN_SUB, T_SUB = Dim<D>::T_SUB,
-                  TMEM_COLS = Dim<D>::TMEM_COLS;
+                  TMEM_COLS = Dim<D>::TMEM_COLS, DP = Dim<D>::DP;
     extern __shared__ unsigned char smem_raw[];
     const Smem sm = align_smem(smem_raw);
     const uint32_t s_q = sm.base, s_dy = s_q + OWN_BYTES, s_k = s_dy + OWN_BYTES, s_v = s_k + STAGES * T_BYTES;
@@ -423,7 +436,7 @@ attn_bwd_q_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
         }
     } else if (warp == 9) {
         constexpr uint32_t id_s = idesc_bf16(BM, BN, 0, 0);   // S = Q K^T, dP' = dO' V^T
-        constexpr uint32_t id_a = idesc_bf16(BM, D, 0, 1);    // dQ += dS K   (A from TMEM, K MN-major)
+        constexpr uint32_t id_a = idesc_bf16(BM, DP, 0, 1);    // dQ += dS K   (A from TMEM, K MN-major)
         const uint64_t dq0 = desc_kmajor(s_q, 0), ddy0 = desc_kmajor(s_dy, 0), dk0 = desc_kmajor(s_k, 0),
                        dv0 = desc_kmajor(s_v, 0), dkt0 = desc_mnmajor(s_k, 0, T_SUB);
         // The score MMAs of tile j are issued as soon as tile j-1's scores are in the math warps' registers (s_read): they are
@@ -459,7 +472,7 @@ attn_bwd_q_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
                 // S and dP' are independent accumulators: alternating their k-steps keeps consecutive MMAs independent
                 // (back-to-back MMAs into one accumulator are serialised by the accumulate dependency, ~93 clk each)
 #pragma unroll
-                for (int k = 0; k < D / 16; ++k) {
+                for (int k = 0; k < DP / 16; ++k) {
                     umma_bf16(tmem_base + COL_S, dq0 + kslice<OWN_SUB>(k), dk0 + off + kslice<T_SUB>(k), id_s, k != 0);
                     umma_bf16(tmem_base + COL_DP, ddy0 + kslice<OWN_SUB>(k), dv0 + off + kslice<T_SUB>(k), id_s, k != 0);
                 }
@@ -524,13 +537,12 @@ attn_bwd_q_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
         PROF(pf.t[5] = clock64() - t0; pf.t[4] = n_tiles / 2; pf.flush(1, 0, threadIdx.x == 0);)
         mbar_wait(acc_full, 0);
         fence_after_sync();
-        __nv_bfloat16 *dst = dq + (((size_t)hn * S + row) * H + hh) * D + half * (D / 2);
-#pragma unroll
-        for (int c = 0; c < D / 64; ++c) {
+        __nv_bfloat16 *dst = dq + (((size_t)hn * S + row) * H + hh) * D;
+        out_chunks<D>(half, [&](int col, auto w) {
             uint32_t r[32];
-            tmem_ld32(lane_base + COL_DQ + half * (D / 2) + c * 32, r);
-            store_row32(dst + c * 32, r, scale);
-        }
+            tmem_ld32(lane_base + COL_DQ + col, r);
+            store_row_n<decltype(w)::value>(dst + col, r, scale);
+        });
     }
     fence_before_sync();
     __syncthreads();
@@ -556,7 +568,7 @@ attn_bwd_kv_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_co
                       const float *__restrict__ delta, __nv_bfloat16 *__restrict__ dk, __nv_bfloat16 *__restrict__ dv,
                       int S, int H, float scale, float scale_log2, float clamp_log2) {
     constexpr int OWN_BYTES = Dim<D>::OWN_BYTES, T_BYTES = Dim<D>::T_BYTES, OWN_SUB = Dim<D>::OWN_SUB, T_SUB = Dim<D>::T_SUB,
-                  TMEM_COLS = Dim<D>::TMEM_COLS;
+                  TMEM_COLS = Dim<D>::TMEM_COLS, DP = Dim<D>::DP;
     extern __shared__ unsigned char smem_raw[];
     const Smem sm = align_smem(smem_raw);
     const uint32_t s_k = sm.base, s_v = s_k + OWN_BYTES, s_q = s_v + OWN_BYTES, s_dy = s_q + STAGES * T_BYTES;
@@ -601,7 +613,7 @@ attn_bwd_kv_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_co
     fence_after_sync();
     const uint32_t tmem_base = *tmem_slot;
     // score buffers b = 0, 1 (one per 32-row sub-tile in flight): S^T at 64 b, dP'^T at 64 b + 32
-    constexpr uint32_t COL_SC = 0, COL_DV = 128, COL_DK = 128 + D;
+    constexpr uint32_t COL_SC = 0, COL_DV = 128, COL_DK = 128 + DP;
     constexpr int SUBN = 32;
 
     if (warp == 8) {
@@ -639,7 +651,7 @@ attn_bwd_kv_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_co
         // Sub-tiles t = 2 j + h of 32 query rows: scores of sub-tile t+1 are issued before the math warps have
         // finished sub-tile t (two score buffers), the accumulating MMAs of t follow once its E^T / dS^T are written.
         constexpr uint32_t id_s = idesc_bf16(BM, SUBN, 0, 0); // S^T = K Q^T, dP'^T = V dO'^T   (N = 32 query rows)
-        constexpr uint32_t id_a = idesc_bf16(BM, D, 0, 1);    // dV += E^T dO', dK += dS^T Q (B MN-major, K = 32)
+        constexpr uint32_t id_a = idesc_bf16(BM, DP, 0, 1);    // dV += E^T dO', dK += dS^T Q (B MN-major, K = 32)
         const uint64_t dk0 = desc_kmajor(s_k, 0), dv0 = desc_kmajor(s_v, 0), dq0 = desc_kmajor(s_q, 0),
                        ddy0 = desc_kmajor(s_dy, 0), dqt0 = desc_mnmajor(s_q, 0, T_SUB),
                        ddyt0 = desc_mnmajor(s_dy, 0, T_SUB);
@@ -654,7 +666,7 @@ attn_bwd_kv_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_co
                 const uint32_t col = tmem_base + COL_SC + (t & 1) * 64;
                 // S^T and dP'^T are independent accumulators: alternate their k-steps (see the dQ kernel)
 #pragma unroll
-                for (int k = 0; k < D / 16; ++k) {
+                for (int k = 0; k < DP / 16; ++k) {
                     umma_bf16(col, dk0 + kslice<OWN_SUB>(k), dq0 + off + kslice<T_SUB>(k), id_s, k != 0);
                     umma_bf16(col + 32, dv0 + kslice<OWN_SUB>(k), ddy0 + off + kslice<T_SUB>(k), id_s, k != 0);
                 }
@@ -741,15 +753,14 @@ attn_bwd_kv_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_co
         PROF(pf.t[5] = clock64() - t0; pf.t[4] = n_tiles; pf.flush(2, 0, threadIdx.x == 0);)
         mbar_wait(acc_full, 0);
         fence_after_sync();
-        const size_t off = (((size_t)hn * S + n0 + kk) * H + hh) * D + half * (D / 2);
-#pragma unroll
-        for (int c = 0; c < D / 64; ++c) {
+        const size_t off = (((size_t)hn * S + n0 + kk) * H + hh) * D;
+        out_chunks<D>(half, [&](int col, auto w) {
             uint32_t r[32];
-            tmem_ld32(lane_base + COL_DV + half * (D / 2) + c * 32, r);
-            store_row32(dv + off + c * 32, r, 1.0f);
-            tmem_ld32(lane_base + COL_DK + half * (D / 2) + c * 32, r);
-            store_row32(dk + off + c * 32, r, scale);
-        }
+            tmem_ld32(lane_base + COL_DV + col, r);
+            store_row_n<decltype(w)::value>(dv + off + col, r, 1.0f);
+            tmem_ld32(lane_base + COL_DK + col, r);
+            store_row_n<decltype(w)::value>(dk + off + col, r, scale);
+        });
     }
     fence_before_sync();
     __syncthreads();
@@ -757,7 +768,8 @@ attn_bwd_kv_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_co
 }
 
 // ---- host -----------------------------------------------------------------------------------------
-// 4-D bf16 tensor map over a [N, S, H, D] tensor (H = 1: head-major [B, S, D]); box = 64 rows x 64 elements of one head
+// 4-D bf16 tensor map over a [N, S, H, D] tensor (H = 1: head-major [B, S, D]); box = 64 rows x 64 elements of one head.
+// D = 80: the box at column 64 holds the row's last 16 elements; the 48 out-of-bounds columns are filled with zeros.
 static int make_map(CUtensorMap *map, const void *base, int N, int S, int H, int D) {
     EncodeTiledFn fn = encode_fn();
     if (!fn) return fail(SPT_ERR_CUDA, "sparse_attn: cuTensorMapEncodeTiled entry point not available");
@@ -839,7 +851,7 @@ static int launch_prep(const __nv_bfloat16 *y, const __nv_bfloat16 *grad_y, cons
         return after_launch("attn_bwd_prep_t_kernel");
     }
     const int64_t rows = (int64_t)B * S;
-    constexpr int RPB = 256 / (D / 8);
+    constexpr int RPB = 256 / Dim<D>::PREP_LANES;
     attn_bwd_prep_kernel<D><<<(unsigned)((rows + RPB - 1) / RPB), 256, 0, st>>>(grad_y, y, zsum, delta, dys, rows, S, H);
     return after_launch("attn_bwd_prep_kernel");
 }
@@ -892,7 +904,8 @@ using namespace spt;
 
 static int check_attn_args(const char *what, int B, int S, int d, int H, int dtype) {
     if (dtype != SPT_BF16) return fail(SPT_ERR_UNSUPPORTED, "%s: only bf16 is supported on the fused path", what);
-    if (d != 64 && d != 128) return fail(SPT_ERR_UNSUPPORTED, "%s: head dim %d not supported (64 or 128)", what, d);
+    if (d != 64 && d != 80 && d != 128)
+        return fail(SPT_ERR_UNSUPPORTED, "%s: head dim %d not supported (64, 80 or 128)", what, d);
     if (B < 1 || B > 65535 || S < 128 || S % 128 != 0)
         return fail(SPT_ERR_INVALID_ARGUMENT, "%s: need 1 <= B <= 65535 and S a positive multiple of 128 (B=%d S=%d)", what, B, S);
     if (H < 1 || B % H != 0)
@@ -920,6 +933,7 @@ extern "C" int spt_sparse_attn_fwd_ex(const void *q, const void *k, const void *
     if ((rc = attn_tc::make_map(&mk, k, B / H, S, H, d)) != SPT_OK) return rc;
     if ((rc = attn_tc::make_map(&mv, v, B / H, S, H, d)) != SPT_OK) return rc;
     if (d == 64) return attn_tc::launch_fwd<64>(mq, mk, mv, mask, extra0, (bf *)y, zsum, B, S, H, scale, clamp, yt, as_stream(stream));
+    if (d == 80) return attn_tc::launch_fwd<80>(mq, mk, mv, mask, extra0, (bf *)y, zsum, B, S, H, scale, clamp, yt, as_stream(stream));
     return attn_tc::launch_fwd<128>(mq, mk, mv, mask, extra0, (bf *)y, zsum, B, S, H, scale, clamp, yt, as_stream(stream));
 }
 
@@ -972,8 +986,9 @@ extern "C" int spt_sparse_attn_bwd_ex(const void *q, const void *k, const void *
     float *dq_acc = (float *)((char *)workspace + (size_t)B * S * sizeof(float) + (size_t)B * S * 128 * 2);
     // the row kernel goes first: besides producing dO' and delta' it is a runtime-API launch, which binds the
     // device's primary context to this (autograd worker) thread before the driver-API tensor-map encoder runs
-    rc = d == 64 ? attn_tc::launch_prep<64>((const bf *)y, (const bf *)grad_y, zsum, delta, dys, B, S, H, yt, as_stream(stream))
-                 : attn_tc::launch_prep<128>((const bf *)y, (const bf *)grad_y, zsum, delta, dys, B, S, H, yt, as_stream(stream));
+    rc = d == 64   ? attn_tc::launch_prep<64>((const bf *)y, (const bf *)grad_y, zsum, delta, dys, B, S, H, yt, as_stream(stream))
+         : d == 80 ? attn_tc::launch_prep<80>((const bf *)y, (const bf *)grad_y, zsum, delta, dys, B, S, H, yt, as_stream(stream))
+                   : attn_tc::launch_prep<128>((const bf *)y, (const bf *)grad_y, zsum, delta, dys, B, S, H, yt, as_stream(stream));
     if (rc != SPT_OK) return rc;
     CUtensorMap mq, mk, mv, md;
     if ((rc = attn_tc::make_map(&mq, q, B / H, S, H, d)) != SPT_OK) return rc;
@@ -982,6 +997,9 @@ extern "C" int spt_sparse_attn_bwd_ex(const void *q, const void *k, const void *
     if ((rc = attn_tc::make_map(&md, dys, B / H, S, H, d)) != SPT_OK) return rc;
     if (d == 64)
         return attn_tc::launch_bwd<64>(mq, mk, mv, md, mask, extra0, delta, dq_acc, (bf *)grad_q, (bf *)grad_k, (bf *)grad_v,
+                                       B, S, H, scale, clamp, as_stream(stream));
+    if (d == 80)
+        return attn_tc::launch_bwd<80>(mq, mk, mv, md, mask, extra0, delta, dq_acc, (bf *)grad_q, (bf *)grad_k, (bf *)grad_v,
                                        B, S, H, scale, clamp, as_stream(stream));
     return attn_tc::launch_bwd<128>(mq, mk, mv, md, mask, extra0, delta, dq_acc, (bf *)grad_q, (bf *)grad_k, (bf *)grad_v, B,
                                     S, H, scale, clamp, as_stream(stream));

@@ -991,10 +991,10 @@ static int lookup_impl(const int32_t *query_codes, const int32_t *key_codes, int
     if (chunk_words > W) chunk_words = W;
     const size_t smem = img + per_word * chunk_words;
     const size_t msmem = (per_word + 2 * LKM_THREADS * 4) * (size_t)W;
-    if (mask_out && !output && (m == 8 || m == 16) && msmem <= 200 * 1024) {
+    if (mask_out && !output && (m == 8 || m == 10 || m == 16) && msmem <= 200 * 1024) {
         const dim3 mgrid(B, S / LKM_ROWS);
         static const bool v1 = [] { const char *e = getenv("SPT_LOOKUP_MASK_V1"); return e && atoi(e) == 1; }();   // A/B switch
-        if (v1) {
+        if (v1 && m != 10) {
             if (m == 8) {
                 cudaFuncSetAttribute(lookup_maskonly_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)msmem);
                 lookup_maskonly_kernel<8><<<mgrid, LKM_THREADS, msmem, st>>>(query_codes, kb, flag, mask_out, extra0_out, S, nnz, W, H);
@@ -1005,6 +1005,9 @@ static int lookup_impl(const int32_t *query_codes, const int32_t *key_codes, int
         } else if (m == 8) {
             cudaFuncSetAttribute(lookup_maskonly2_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)msmem);
             lookup_maskonly2_kernel<8><<<mgrid, LKM_THREADS, msmem, st>>>(query_codes, kb, flag, mask_out, extra0_out, S, nnz, W, H);
+        } else if (m == 10) {       // head dim 80 (OPT-2.7B) at d_codeword 8
+            cudaFuncSetAttribute(lookup_maskonly2_kernel<10>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)msmem);
+            lookup_maskonly2_kernel<10><<<mgrid, LKM_THREADS, msmem, st>>>(query_codes, kb, flag, mask_out, extra0_out, S, nnz, W, H);
         } else {
             cudaFuncSetAttribute(lookup_maskonly2_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)msmem);
             lookup_maskonly2_kernel<16><<<mgrid, LKM_THREADS, msmem, st>>>(query_codes, kb, flag, mask_out, extra0_out, S, nnz, W, H);
@@ -1016,12 +1019,15 @@ static int lookup_impl(const int32_t *query_codes, const int32_t *key_codes, int
         return SPT_OK;
     }
     const size_t bsmem = per_word * (size_t)W + (size_t)LKB_CHUNK * LKM_THREADS * 4;
-    if (mask_out && !output && (m == 8 || m == 16) && bsmem <= 200 * 1024) {
+    if (mask_out && !output && (m == 8 || m == 10 || m == 16) && bsmem <= 200 * 1024) {
         // long sequences: the plane-free mask-only kernel (S 8192 at m 8)
         const dim3 mgrid(B, S / LKM_ROWS);
         if (m == 8) {
             cudaFuncSetAttribute(lookup_maskonly_big_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bsmem);
             lookup_maskonly_big_kernel<8><<<mgrid, LKM_THREADS, bsmem, st>>>(query_codes, kb, flag, mask_out, extra0_out, S, nnz, W, H);
+        } else if (m == 10) {
+            cudaFuncSetAttribute(lookup_maskonly_big_kernel<10>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bsmem);
+            lookup_maskonly_big_kernel<10><<<mgrid, LKM_THREADS, bsmem, st>>>(query_codes, kb, flag, mask_out, extra0_out, S, nnz, W, H);
         } else {
             cudaFuncSetAttribute(lookup_maskonly_big_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bsmem);
             lookup_maskonly_big_kernel<16><<<mgrid, LKM_THREADS, bsmem, st>>>(query_codes, kb, flag, mask_out, extra0_out, S, nnz, W, H);

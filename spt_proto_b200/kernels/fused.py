@@ -1,4 +1,5 @@
-"""Fused sparse attention autograd Function: the fast path of the V2 layers (bf16, d_head 64).
+"""Fused sparse attention autograd Function: the fast path of the V2 layers (bf16, d_head 64, 80
+or 128).
 Equivalent to  spmm(softmax(clamp_(scale * sddmm(q, k), -10, 10)), v)  on the lookup's pattern
 (reference layers/sparse/attention.py:122-141 + the three backward passes), computed as masked dense
 tiles on the tensor cores from the lookup's bitmask output."""

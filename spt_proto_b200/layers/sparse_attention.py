@@ -62,8 +62,9 @@ class _SparseV2Mixin:
     # False is the opt-in corrected layout (identical to the reference's dense VanillaAttention on
     # the same pattern).  Also a constructor keyword.  INTEGRATION.md, "Output layout".
     reference_output_layout: bool = True
-    # bf16, d_head 64 or 128, S % 128 == 0 on CUDA: run lookup -> bitmask -> fused masked-dense attention on
+    # bf16, d_head 64, 80 or 128, S % 128 == 0 on CUDA: run lookup -> bitmask -> fused masked-dense attention on
     # the tensor cores instead of the stage chain (same result up to bf16 rounding; DESIGN.md sec. 5).
+    # False keeps the stage chain for every shape.
     use_fused: bool = True
     # The reference reads its device-side `trigger` buffer with `is_nonzero()` on every forward
     # (attention.py:98) — a device->host synchronisation per layer call.  None (default) keeps that
@@ -102,7 +103,7 @@ class _SparseV2Mixin:
         return x.view(-1, x.size(-2), x.size(-1))
 
     def _fused_ok(self, q) -> bool:
-        return (self.use_fused and q.is_cuda and q.dtype == torch.bfloat16 and q.size(-1) in (64, 128)
+        return (self.use_fused and q.is_cuda and q.dtype == torch.bfloat16 and q.size(-1) in (64, 80, 128)
                 and q.size(1) % 128 == 0 and q.size(1) % self.sparse_coeff == 0
                 and (q.size(1) // self.sparse_coeff) % 4 == 0 and q.size(1) // self.sparse_coeff >= 8)
 
