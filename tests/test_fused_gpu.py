@@ -29,7 +29,12 @@ def _mask_from_indices(indices, S):
                                             (2, 384, 16, 4, 8), (1, 128, 8, 16, 4),
                                             # long sequences: the plane-free mask-only kernel (configs[4]: S 8192, top-k 256 / 16;
                                             # c = 1, 2 overflow the bucket capacities and exercise the clobber fix-up)
-                                            (1, 8192, 8, 16, 32), (1, 8192, 8, 16, 512), (1, 8192, 8, 2, 64), (1, 4224, 8, 1, 8)])
+                                            (1, 8192, 8, 16, 32), (1, 8192, 8, 16, 512), (1, 8192, 8, 2, 64), (1, 4224, 8, 1, 8),
+                                            # m = 16 (d 128, LLaMA-7B) at long S: S 2048 runs lookup_maskonly2_kernel<16>, S 4096
+                                            # lookup_maskonly_big_kernel<16>; S 8192 exceeds both kernels' shared memory at m 16
+                                            # and takes the index-emitting bitmap kernel with mask output
+                                            (1, 2048, 16, 16, 8), (1, 4096, 16, 16, 8), (1, 4096, 16, 2, 16),
+                                            (1, 8192, 16, 16, 32), (1, 8192, 16, 2, 64)])
 def test_lookup_mask_matches_index_output(B, S, m, c, coeff):
     from spt_proto_b200 import ext
     g = torch.Generator().manual_seed(S + c)
