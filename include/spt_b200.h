@@ -13,7 +13,8 @@
  *   - every pointer is a DEVICE pointer unless the name ends in `_host`;
  *   - tensors are dense, row-major, contiguous (the reference's CHECK_DIM requires contiguity,
  *     extension/common.h:13-18);
- *   - `dtype` selects the element type of q/k/v-like operands: SPT_F32 or SPT_BF16.  Indices are
+ *   - `dtype` selects the element type of q/k/v-like operands: SPT_F32 or SPT_BF16 (SPT_F16 where
+ *     stated, see spt_dtype).  Indices are
  *     int32, CSR values / probabilities / distances are always fp32, accumulation is fp32;
  *   - `stream` is a cudaStream_t passed as void* (0 = legacy default stream).  Every kernel is
  *     launched on it; nothing synchronises the device;
@@ -40,7 +41,9 @@ typedef enum {
     SPT_ERR_CUDA = 3              /* launch or runtime error (cudaGetLastError)                    */
 } spt_status;
 
-typedef enum { SPT_F32 = 0, SPT_BF16 = 1 } spt_dtype;
+/* SPT_F16 is accepted by spt_pq_encode, spt_pq_encode_pair, spt_pq_train_fwd / _bwd and the fused attention
+ * (spt_sparse_attn_fwd / _bwd and their _ex variants); every other entry point takes SPT_F32 / SPT_BF16 only. */
+typedef enum { SPT_F32 = 0, SPT_BF16 = 1, SPT_F16 = 2 } spt_dtype;
 
 #define SPT_ABI_VERSION 1
 
@@ -215,12 +218,14 @@ int spt_softmax_clamp_bwd(const int32_t *indptr, const int32_t *indices, const f
  *   extra0 [B, S] int32 = number of zero-padding slots of the row (multiplicity of key 0 beyond its
  *   own bit).  `output` (the int32 index tensor) may be NULL on this path.  Needs S % 128 == 0.
  *
- * spt_sparse_attn_fwd: q, k, v [B, S, d] bf16 ->
- *   y [B, S, d] bf16 = sum_j p_rj v_j,  p = w * exp(clamp(scale * q.k, -clamp, clamp)) / Z,
+ * spt_sparse_attn_fwd: q, k, v [B, S, d] bf16 or fp16 (dtype SPT_BF16 / SPT_F16) ->
+ *   y [B, S, d] (same type) = sum_j p_rj v_j,  p = w * exp(clamp(scale * q.k, -clamp, clamp)) / Z,
  *   zsum [B, S] fp32 = Z (row sums, >= 1e-9) saved for the backward.  d = 64, 80 or 128 (others
  *   return SPT_ERR_UNSUPPORTED), S % 128 == 0.  d = 80 (OPT-2.7B) is padded to 128 in shared
  *   memory and tensor memory only: every global read and write is exactly d columns wide.
- * spt_sparse_attn_bwd: grad_y -> grad_q, grad_k, grad_v [B, S, d] bf16.  Recomputes p from q, k
+ *   fp16 keeps every packed probability in range with a power-of-two scale per row that cancels in
+ *   y and in the gradients (DESIGN.md section 4.1); it needs clamp <= 10 (SPT_ERR_UNSUPPORTED beyond).
+ * spt_sparse_attn_bwd: grad_y -> grad_q, grad_k, grad_v [B, S, d] (dtype).  Recomputes p from q, k
  *   (nothing of size S x k is read or written); deterministic (no atomics).
  *   workspace: spt_sparse_attn_bwd_workspace_bytes(B, S).
  * Layout: H = 1 means head-major [B, S, *] operands (the reference's layout after its transposes);

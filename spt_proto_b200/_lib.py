@@ -11,6 +11,7 @@ LIB_PATH = os.path.join(_HERE, "lib", "libspt_b200.so")
 SPT_OK = 0
 SPT_F32 = 0
 SPT_BF16 = 1
+SPT_F16 = 2          # PQ encode / train and the fused attention only (include/spt_b200.h)
 SPT_ATTN_Y_TRANSPOSED = 1
 
 

@@ -18,7 +18,7 @@ constexpr int BN = 64;         // other tile rows per iteration
 constexpr int STAGES = 3;
 constexpr int N_MATH = 256;      // warps 0-7
 constexpr int THREADS = 320;
-// Head dim D in {64, 80, 128}.  Operand tiles are stored as NSUB = ceil(D / 64) sub-tiles of [rows][64] bf16 (one TMA
+// Head dim D in {64, 80, 128}.  Operand tiles are stored as NSUB = ceil(D / 64) sub-tiles of [rows][64] bf16 or fp16 (one TMA
 // box each, 128-byte swizzled): an owner tile is [NSUB][128 rows][64], an "other" tile [NSUB][64 rows][64].
 // D = 80 is padded to DP = 128 in shared memory and TMEM only: the second box starts at column 64 and the TMA fills
 // its 48 columns past the row end with zeros, so Q K^T is unchanged and O, dQ, dK, dV get zero columns 80 .. 127,
@@ -65,6 +65,32 @@ __device__ __forceinline__ uint32_t pack_bf16(float lo, float hi) {
     __nv_bfloat162 h = __floats2bfloat162_rn(lo, hi);
     return *reinterpret_cast<uint32_t *>(&h);
 }
+// ---- element type ---------------------------------------------------------------------------------
+// The operands are bf16 or fp16 (T = __nv_bfloat16 / __half): kind::f16 MMAs take either at the same rate.  fp16 has
+// 3 more mantissa bits but a largest value of 65504, so the fp16 kernels scale every score row by a power of two
+// 2^-o_r (DESIGN.md section 4.1): the exponent argument becomes  scale s log2(e) - o_r, which cancels exactly in
+// y = sum e v / Z, in E / Z and in dO / Z.
+template <typename T>
+constexpr bool is_f16 = std::is_same<T, __half>::value;
+template <typename T>
+__device__ __forceinline__ constexpr uint32_t idesc_of(int M, int N, int a_mn_major, int b_mn_major) {
+    return is_f16<T> ? idesc_fp16(M, N, a_mn_major, b_mn_major) : idesc_bf16(M, N, a_mn_major, b_mn_major);
+}
+template <typename T>
+__device__ __forceinline__ uint32_t pack2(float lo, float hi) {
+    if constexpr (is_f16<T>) {
+        __half2 h = __floats2half2_rn(lo, hi);
+        return *reinterpret_cast<uint32_t *>(&h);
+    } else {
+        return pack_bf16(lo, hi);
+    }
+}
+// largest clamp the fp16 row scaling covers: the smallest element e^-c of a row scaled by 2^-o_min stays a normal fp16
+constexpr float F16_MAX_CLAMP = 10.0f;
+// Backward row scale of fp16: o_r = floor(log2 Z_r), so Z_r 2^-o_r is in [1, 2).  Returns -o_r (exact, as a float).
+__device__ __forceinline__ float f16_bwd_nofs(float z) { return (float)(127 - (int)((__float_as_uint(z) >> 23) & 0xff)); }
+// Z 2^-o in [1, 2): the mantissa of Z (Z >= 1e-9 is a normal float)
+__device__ __forceinline__ float f16_bwd_zs(float z) { return __uint_as_float((__float_as_uint(z) & 0x007fffffu) | 0x3f800000u); }
 // ---- element math --------------------------------------------------------------------------------
 // Per score element the three kernels need  e = w * exp(clamp(scale s, -10, 10))  (and, in the backward,
 // ds = e (dp - delta') [|scale s| <= 10]).  The first version spent ~11-15 instructions per element on it and was
@@ -157,16 +183,19 @@ __device__ __forceinline__ constexpr bool poly_pair(int p) {
     return SPT_ATTN_POLY_MOD > 0 && (p % mod) == mod - 1;
 }
 
-// e of one pair of raw scores: exp2(clamp(s c)); CLAMP: exact path, also returns the per-element gradient indicators
-template <bool CLAMP, bool POLY>
-__device__ __forceinline__ void exp_pair(float s0, float s1, const MathK mk, float &e0, float &e1, bool &in0, bool &in1) {
-    uint64_t a = mul2(pk2(s0, s1), pk2(mk.c, mk.c));
+// e of one pair of raw scores: exp2(clamp(s c)); CLAMP: exact path, also returns the per-element gradient indicators.
+// OFS (fp16): exp2(clamp(s c) + nofs), nofs = -o of the pair's rows (one FFMA2 instead of the FMUL2 when unclamped).
+template <bool CLAMP, bool POLY, bool OFS = false>
+__device__ __forceinline__ void exp_pair(float s0, float s1, const MathK mk, float &e0, float &e1, bool &in0, bool &in1,
+                                         uint64_t nofs = 0) {
+    uint64_t a = (OFS && !CLAMP) ? fma2(pk2(s0, s1), pk2(mk.c, mk.c), nofs) : mul2(pk2(s0, s1), pk2(mk.c, mk.c));
     if constexpr (CLAMP) {
         float a0, a1;
         up2(a, a0, a1);
         in0 = fabsf(s0) <= mk.thr;
         in1 = fabsf(s1) <= mk.thr;
         a = pk2(fminf(fmaxf(a0, -mk.L), mk.L), fminf(fmaxf(a1, -mk.L), mk.L));
+        if constexpr (OFS) a = add2(a, nofs);
     }
     ex2_pair<POLY>(a, e0, e1);
 }
@@ -185,13 +214,24 @@ __device__ __forceinline__ void pair_masks(uint32_t X, int n, uint32_t &m01, uin
     m23 = prmt(Y, 0u, 0xBBAAu);
 }
 __device__ __forceinline__ uint64_t unpack_bf16x2(uint32_t p) { return pk2(__uint_as_float(p << 16), __uint_as_float(p & 0xffff0000u)); }
+template <typename T>
+__device__ __forceinline__ uint64_t unpack2(uint32_t p) {
+    if constexpr (is_f16<T>) {
+        const float2 f = __half22float2(*reinterpret_cast<const __half2 *>(&p));
+        return pk2(f.x, f.y);
+    } else {
+        return unpack_bf16x2(p);
+    }
+}
 
 // Forward: 32 score columns of one row -> 16 masked packed bf16 pairs of e = w * exp(clamp(scale s)); the row sum
 // accumulates the bf16-rounded values (exactly the weights the P V product uses).  FIRST: column 0 is key 0, which also
-// carries the row's zero-padding multiplicity ex0 (mult0 = bit + ex0 when > 0).
-template <bool FIRST, bool CLAMP>
+// carries the row's zero-padding multiplicity ex0 (mult0 = bit + ex0 when > 0).  fp16: e 2^-o, nofs = -o of the row.
+template <bool FIRST, bool CLAMP, typename T = __nv_bfloat16>
 __device__ __forceinline__ void fwd_chunk32(const uint32_t (&r)[32], uint32_t X, const MathK mk, float ex0, uint64_t &sum2,
-                                            uint32_t (&pk)[16]) {
+                                            uint32_t (&pk)[16], float nofs = 0.0f) {
+    constexpr bool OFS = is_f16<T>;
+    const uint64_t no2 = pk2(nofs, nofs);
     float mult0 = 1.0f;
     if (FIRST) {
         mult0 = (float)(X & 1u) + ex0;
@@ -207,20 +247,23 @@ __device__ __forceinline__ void fwd_chunk32(const uint32_t (&r)[32], uint32_t X,
             const int i = 4 * n + 2 * h;
             float e0, e1;
             bool in0, in1;
-            if (poly_pair(i >> 1)) exp_pair<CLAMP, true>(__uint_as_float(r[i]), __uint_as_float(r[i + 1]), mk, e0, e1, in0, in1);
-            else exp_pair<CLAMP, false>(__uint_as_float(r[i]), __uint_as_float(r[i + 1]), mk, e0, e1, in0, in1);
+            if (poly_pair(i >> 1)) exp_pair<CLAMP, true, OFS>(__uint_as_float(r[i]), __uint_as_float(r[i + 1]), mk, e0, e1, in0, in1, no2);
+            else exp_pair<CLAMP, false, OFS>(__uint_as_float(r[i]), __uint_as_float(r[i + 1]), mk, e0, e1, in0, in1, no2);
             if (FIRST && i == 0) e0 *= mult0;
-            const uint32_t p = pack_bf16(e0, e1) & (h ? m23 : m01);
-            sum2 = add2(sum2, unpack_bf16x2(p));
+            const uint32_t p = pack2<T>(e0, e1) & (h ? m23 : m01);
+            sum2 = add2(sum2, unpack2<T>(p));
             pk[i >> 1] = p;
         }
     }
 }
 
 // dQ kernel: 32 columns (keys) of one query row -> 16 masked packed pairs of ds = e (dp - delta') [unclamped]; ndelta = -delta'.
-template <bool FIRST, bool CLAMP>
+// fp16: e 2^-o, nofs = -o of the row.
+template <bool FIRST, bool CLAMP, typename T = __nv_bfloat16>
 __device__ __forceinline__ void bwdq_chunk32(const uint32_t (&r)[32], const uint32_t (&g)[32], uint32_t X, const MathK mk,
-                                             float ndelta, float ex0, uint32_t (&pk)[16]) {
+                                             float ndelta, float ex0, uint32_t (&pk)[16], float nofs = 0.0f) {
+    constexpr bool OFS = is_f16<T>;
+    const uint64_t no2 = pk2(nofs, nofs);
     float mult0 = 1.0f;
     if (FIRST) {
         mult0 = (float)(X & 1u) + ex0;
@@ -237,8 +280,8 @@ __device__ __forceinline__ void bwdq_chunk32(const uint32_t (&r)[32], const uint
             const int i = 4 * n + 2 * h;
             float e0, e1;
             bool in0 = true, in1 = true;
-            if (poly_pair(i >> 1)) exp_pair<CLAMP, true>(__uint_as_float(r[i]), __uint_as_float(r[i + 1]), mk, e0, e1, in0, in1);
-            else exp_pair<CLAMP, false>(__uint_as_float(r[i]), __uint_as_float(r[i + 1]), mk, e0, e1, in0, in1);
+            if (poly_pair(i >> 1)) exp_pair<CLAMP, true, OFS>(__uint_as_float(r[i]), __uint_as_float(r[i + 1]), mk, e0, e1, in0, in1, no2);
+            else exp_pair<CLAMP, false, OFS>(__uint_as_float(r[i]), __uint_as_float(r[i + 1]), mk, e0, e1, in0, in1, no2);
             if (FIRST && i == 0) e0 *= mult0;
             float d0, d1;
             up2(mul2(pk2(e0, e1), add2(pk2(__uint_as_float(g[i]), __uint_as_float(g[i + 1])), nd2)), d0, d1);
@@ -246,7 +289,7 @@ __device__ __forceinline__ void bwdq_chunk32(const uint32_t (&r)[32], const uint
                 d0 = in0 ? d0 : 0.0f;
                 d1 = in1 ? d1 : 0.0f;
             }
-            pk[i >> 1] = pack_bf16(d0, d1) & (h ? m23 : m01);
+            pk[i >> 1] = pack2<T>(d0, d1) & (h ? m23 : m01);
         }
     }
 }
@@ -255,10 +298,12 @@ __device__ __forceinline__ void bwdq_chunk32(const uint32_t (&r)[32], const uint
 // stage ([64] in shared memory), shl moves the key's bit to bit 31; s_ndelta = -delta' of the rows.
 // KEY0: this thread is key 0 (adds the rows' zero-padding multiplicity s_ex0).
 // r / g hold NR values of which [OFF, OFF + 16) are processed; c0 = tile row of r[OFF].
-template <bool KEY0, bool CLAMP, int OFF = 0, int NR = 16, typename EX0 = float>
+// fp16: s_nofs = -o of the rows (the row scale of each column).
+template <bool KEY0, bool CLAMP, int OFF = 0, int NR = 16, typename EX0 = float, typename T = __nv_bfloat16>
 __device__ __forceinline__ void bwdkv_chunk16(const uint32_t (&rr)[NR], const uint32_t (&gg)[NR], const uint32_t *mrow,
                                               const float *s_ndelta, const EX0 *s_ex0, int c0, int shl, const MathK mk,
-                                              uint32_t (&pe)[8], uint32_t (&pd)[8]) {
+                                              uint32_t (&pe)[8], uint32_t (&pd)[8], const float *s_nofs = nullptr) {
+    constexpr bool OFS = is_f16<T>;
     uint32_t r[16], g[16];
 #pragma unroll
     for (int i = 0; i < 16; ++i) {
@@ -271,13 +316,16 @@ __device__ __forceinline__ void bwdkv_chunk16(const uint32_t (&rr)[NR], const ui
         const float4 nd = *reinterpret_cast<const float4 *>(s_ndelta + c0 + q4);
         const uint32_t mwv[4] = {mw.x << shl, mw.y << shl, mw.z << shl, mw.w << shl};
         const float ndv[4] = {nd.x, nd.y, nd.z, nd.w};
+        float4 no = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+        if constexpr (OFS) no = *reinterpret_cast<const float4 *>(s_nofs + c0 + q4);
+        const uint64_t nov[2] = {pk2(no.x, no.y), pk2(no.z, no.w)};
 #pragma unroll
         for (int h = 0; h < 2; ++h) {
             const int i = q4 + 2 * h;
             float e0, e1;
             bool in0 = true, in1 = true;
-            if (poly_pair(i >> 1)) exp_pair<CLAMP, true>(__uint_as_float(r[i]), __uint_as_float(r[i + 1]), mk, e0, e1, in0, in1);
-            else exp_pair<CLAMP, false>(__uint_as_float(r[i]), __uint_as_float(r[i + 1]), mk, e0, e1, in0, in1);
+            if (poly_pair(i >> 1)) exp_pair<CLAMP, true, OFS>(__uint_as_float(r[i]), __uint_as_float(r[i + 1]), mk, e0, e1, in0, in1, nov[h]);
+            else exp_pair<CLAMP, false, OFS>(__uint_as_float(r[i]), __uint_as_float(r[i + 1]), mk, e0, e1, in0, in1, nov[h]);
             uint32_t ma = mwv[2 * h], mb = mwv[2 * h + 1];
             if (KEY0) {     // key 0: weight = bit + zero-padding multiplicity of the row
                 const float w0 = (float)(ma >> 31) + (float)s_ex0[c0 + i], w1 = (float)(mb >> 31) + (float)s_ex0[c0 + i + 1];
@@ -294,8 +342,8 @@ __device__ __forceinline__ void bwdkv_chunk16(const uint32_t (&rr)[NR], const ui
                 d0 = in0 ? d0 : 0.0f;
                 d1 = in1 ? d1 : 0.0f;
             }
-            pe[i >> 1] = pack_bf16(e0, e1) & m;
-            pd[i >> 1] = pack_bf16(d0, d1) & m;
+            pe[i >> 1] = pack2<T>(e0, e1) & m;
+            pd[i >> 1] = pack2<T>(d0, d1) & m;
         }
     }
 }
@@ -336,28 +384,32 @@ __device__ __forceinline__ Smem align_smem(unsigned char *raw) {
 }
 __device__ __forceinline__ void math_warps_sync() { asm volatile("bar.sync 1, %0;" ::"n"(N_MATH) : "memory"); }
 
-// store 32 fp32 accumulator values (scaled) as 32 bf16 = 64 contiguous bytes
-__device__ __forceinline__ void store_row32(__nv_bfloat16 *dst, const uint32_t (&r)[32], float s) {
+// store 32 fp32 accumulator values (scaled) as 32 bf16 / fp16 = 64 contiguous bytes
+template <typename T>
+__device__ __forceinline__ void store_row32(T *dst, const uint32_t (&r)[32], float s) {
 #pragma unroll
     for (int i = 0; i < 32; i += 8) {
         float t[8];
 #pragma unroll
         for (int u = 0; u < 8; ++u) t[u] = __uint_as_float(r[i + u]) * s;
-        Vec16<__nv_bfloat16>::store(dst + i, t);
+        Vec16<T>::store(dst + i, t);
     }
 }
 // the same for the first W (16 or 32) of the 32 values
-template <int W>
-__device__ __forceinline__ void store_row_n(__nv_bfloat16 *dst, const uint32_t (&r)[32], float s) {
+template <int W, typename T>
+__device__ __forceinline__ void store_row_n(T *dst, const uint32_t (&r)[32], float s) {
     static_assert(W % 8 == 0 && W <= 32, "W must be a multiple of 8, at most 32");
 #pragma unroll
     for (int i = 0; i < W; i += 8) {
         float t[8];
 #pragma unroll
         for (int u = 0; u < 8; ++u) t[u] = __uint_as_float(r[i + u]) * s;
-        Vec16<__nv_bfloat16>::store(dst + i, t);
+        Vec16<T>::store(dst + i, t);
     }
 }
+// one output element (the y^T epilogue)
+__device__ __forceinline__ __nv_bfloat16 out_elem(float v, __nv_bfloat16 *) { return __float2bfloat16(v); }
+__device__ __forceinline__ __half out_elem(float v, __half *) { return __float2half_rn(v); }
 template <int W>
 using Width = std::integral_constant<int, W>;
 // The epilogues read a row's D output columns from TMEM in 32-column chunks shared by the two warpgroups (`half`):
@@ -384,12 +436,15 @@ __device__ __forceinline__ void out_chunks(int half, F &&f) {
 
 // 128 x 128-tile kernels (attn_tc128.cu), head dim 64
 namespace attn_tc128 {
+// T = __nv_bfloat16 or __half; zsum is read by the fp16 kernels only (row scales)
+template <typename T>
 int launch_bwd_kv128(const CUtensorMap &mq, const CUtensorMap &mk, const CUtensorMap &mv, const CUtensorMap &md,
-                     const uint32_t *mask, const int32_t *extra0, const float *ndelta, __nv_bfloat16 *gk,
-                     __nv_bfloat16 *gv, int B, int S, int H, float scale, float clamp, cudaStream_t st);
+                     const uint32_t *mask, const int32_t *extra0, const float *ndelta, const float *zsum, T *gk, T *gv,
+                     int B, int S, int H, float scale, float clamp, cudaStream_t st);
+template <typename T>
 int launch_bwd_q128(const CUtensorMap &mq, const CUtensorMap &mk, const CUtensorMap &mv, const CUtensorMap &md,
-                    const uint32_t *mask, const int32_t *extra0, const float *ndelta, __nv_bfloat16 *gq, int B, int S,
-                    int H, float scale, float clamp, cudaStream_t st);
+                    const uint32_t *mask, const int32_t *extra0, const float *ndelta, const float *zsum, T *gq, int B,
+                    int S, int H, float scale, float clamp, cudaStream_t st);
 int launch_bwd_fused128(const CUtensorMap &mq, const CUtensorMap &mk, const CUtensorMap &mv, const CUtensorMap &md,
                         const uint32_t *mask, const int32_t *extra0, const float *ndelta, float *dq_acc,
                         __nv_bfloat16 *gq, __nv_bfloat16 *gk, __nv_bfloat16 *gv, int B, int S, int H, float scale,

@@ -45,12 +45,13 @@ namespace attn_tc {
 // Forward.  TMEM columns: S[2] 0/64 (fp32 128x64), P[2] 128/160 (bf16 pairs, 32 cols), O 192 (128x64).
 // ---------------------------------------------------------------------------------------------------
 
-template <int D>
+// fp16 (T = __half): kg is the key tensor itself (the row scale reads key row 0 of the head); unused in bf16.
+template <int D, typename T>
 __global__ void __launch_bounds__(THREADS, Dim<D>::CTAS)
 attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_k,
                    const __grid_constant__ CUtensorMap map_v, const uint32_t *__restrict__ mask,
-                   const int32_t *__restrict__ extra0, __nv_bfloat16 *__restrict__ y, float *__restrict__ zsum, int S,
-                   int H, float scale_log2, float clamp_log2, int y_transposed) {
+                   const int32_t *__restrict__ extra0, T *__restrict__ y, float *__restrict__ zsum, int S,
+                   int H, float scale_log2, float clamp_log2, int y_transposed, const T *__restrict__ kg) {
     constexpr int OWN_BYTES = Dim<D>::OWN_BYTES, T_BYTES = Dim<D>::T_BYTES, OWN_SUB = Dim<D>::OWN_SUB, T_SUB = Dim<D>::T_SUB,
                   TMEM_COLS = Dim<D>::TMEM_COLS, DP = Dim<D>::DP;
     constexpr int NBUF = 3;                            // score buffers
@@ -120,8 +121,8 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_const
         }
     } else if (warp == 9) {
         // ===== MMA issuer: the whole warp runs the (uniform) loop, one elected lane issues =====
-        constexpr uint32_t id_s = idesc_bf16(BM, BN, 0, 0);   // S = Q K^T   (both K-major)
-        constexpr uint32_t id_o = idesc_bf16(BM, DP, 0, 1);    // O += P V    (A from TMEM, V MN-major)
+        constexpr uint32_t id_s = idesc_of<T>(BM, BN, 0, 0);   // S = Q K^T   (both K-major)
+        constexpr uint32_t id_o = idesc_of<T>(BM, DP, 0, 1);    // O += P V    (A from TMEM, V MN-major)
         const uint64_t dq0 = desc_kmajor(s_q, 0), dk0 = desc_kmajor(s_k, 0), dv0 = desc_mnmajor(s_v, 0, T_SUB);
         // S = Q K^T runs two tiles ahead of O += P V, into the third (free) buffer, so the k-steps of S(j + 2) and of
         // PV(j) touch different TMEM columns and are interleaved: two accumulator chains in flight (consecutive MMAs into
@@ -195,6 +196,30 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_const
         uint64_t sum2 = pk2(0.0f, 0.0f);
         const MathK mk = make_math(scale_log2, clamp_log2);
         uint4 mw = __ldg(mrow);
+        float nofs = 0.0f;                                // fp16: -o of this row
+        if constexpr (is_f16<T>) {
+            // o = max(floor(c log2 e) - 15, floor(log2 t0) - 14), t0 = (1 + ex0) exp(clamp(scale q.k_0)) the key-0 term:
+            // t0 2^-o < 2^15 and e^c 2^-o < 2^16, so no element can overflow, and a row whose scores are all low keeps
+            // normal fp16 values.  q.k_0 in fp32 from the row's Q in shared memory and key row 0 of the head.
+            mbar_wait(q_full, 0);
+            const T *k0 = kg + ((size_t)hn * S * H + hh) * D;
+            float dot = 0.0f;
+#pragma unroll
+            for (int c = 0; c < D / 8; ++c) {              // 16-byte chunk c: sub-tile c / 8, 128-byte swizzled by the row
+                const uint4 qa = *reinterpret_cast<const uint4 *>(sm.ptr + (c / 8) * OWN_SUB + rt * 128 + (((c % 8) ^ (rt & 7)) * 16));
+                const uint4 ka = __ldg(reinterpret_cast<const uint4 *>(k0) + c);
+                const uint32_t qw[4] = {qa.x, qa.y, qa.z, qa.w}, kw[4] = {ka.x, ka.y, ka.z, ka.w};
+#pragma unroll
+                for (int i = 0; i < 4; ++i) {
+                    float q0, q1, k0f, k1f;
+                    up2(unpack2<T>(qw[i]), q0, q1);
+                    up2(unpack2<T>(kw[i]), k0f, k1f);
+                    dot = fmaf(q1, k1f, fmaf(q0, k0f, dot));
+                }
+            }
+            const float l0 = __log2f(1.0f + ex0) + fminf(fmaxf(dot * mk.c, -mk.L), mk.L);
+            nofs = -fmaxf(floorf(mk.L) - 15.0f, floorf(l0) - 14.0f);
+        }
         PROF(Prof pf; pf.start(); const long long t0 = pf.last; pf.t[6] = t0 - t_entry;)
         for (int j = half, it = 0; j < n_tiles; j += 2, ++it) {
             // tile j = keys 64 j .. 64 j + 63 = bits 16 half .. 16 half + 15 of the lane-major words of key group it = j >> 1
@@ -212,11 +237,11 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_const
                 uint32_t pk[16];
                 const bool first = (j == 0 && c == 0);
                 if (!warp_needs_clamp(r, mk.thr)) {
-                    if (first) fwd_chunk32<true, false>(r, X, mk, ex0, sum2, pk);
-                    else fwd_chunk32<false, false>(r, X, mk, ex0, sum2, pk);
+                    if (first) fwd_chunk32<true, false, T>(r, X, mk, ex0, sum2, pk, nofs);
+                    else fwd_chunk32<false, false, T>(r, X, mk, ex0, sum2, pk, nofs);
                 } else {
-                    if (first) fwd_chunk32<true, true>(r, X, mk, ex0, sum2, pk);
-                    else fwd_chunk32<false, true>(r, X, mk, ex0, sum2, pk);
+                    if (first) fwd_chunk32<true, true, T>(r, X, mk, ex0, sum2, pk, nofs);
+                    else fwd_chunk32<false, true, T>(r, X, mk, ex0, sum2, pk, nofs);
                 }
                 PROF(pf.lap(2);)
                 tmem_st16(buf + c * 16, pk);             // in place: these columns were consumed by this thread's chunk 0
@@ -236,13 +261,21 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_const
         }
         s_part[half * BM + rt] = sum;
         math_warps_sync();
-        sum = fmaxf(s_part[rt] + s_part[BM + rt], 1e-9f);
-        if (half == 0) zsum[grow] = sum;
-        const float inv = 1.0f / sum;
+        float inv;
+        if constexpr (is_f16<T>) {                        // sum of e 2^-o; Z = sum 2^o (exact)
+            const float rs = __uint_as_float((uint32_t)(127 + (int)nofs) << 23);     // 2^-o
+            sum = fmaxf(s_part[rt] + s_part[BM + rt], 1e-9f * rs);
+            if (half == 0) zsum[grow] = sum * __uint_as_float((uint32_t)(127 - (int)nofs) << 23);
+            inv = 1.0f / sum;
+        } else {
+            sum = fmaxf(s_part[rt] + s_part[BM + rt], 1e-9f);
+            if (half == 0) zsum[grow] = sum;
+            inv = 1.0f / sum;
+        }
         mbar_wait(o_full, 0);
         fence_after_sync();
         if (!y_transposed) {
-            __nv_bfloat16 *dst = y + (((size_t)hn * S + row) * H + hh) * D;
+            T *dst = y + (((size_t)hn * S + row) * H + hh) * D;
             out_chunks<D>(half, [&](int col, auto w) {
                 uint32_t r[32];
                 tmem_ld32(lane_base + COL_O + col, r);
@@ -252,11 +285,11 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_const
             // the shipped reference layer's output layout (attention.py:139-142): y^T [B, D, S] memory; a warp's 32
             // consecutive rows of one feature are 64 contiguous bytes
             out_chunks<D>(half, [&](int col, auto w) {
-                __nv_bfloat16 *dst = y + ((size_t)b * D + col) * S + row;
+                T *dst = y + ((size_t)b * D + col) * S + row;
                 uint32_t r[32];
                 tmem_ld32(lane_base + COL_O + col, r);
 #pragma unroll
-                for (int i = 0; i < decltype(w)::value; ++i) dst[(size_t)i * S] = __float2bfloat16(__uint_as_float(r[i]) * inv);
+                for (int i = 0; i < decltype(w)::value; ++i) dst[(size_t)i * S] = out_elem(__uint_as_float(r[i]) * inv, dst);
             });
         }
         PROF(pf.t[7] = clock64() - t_loop_end; pf.flush(0, 0, threadIdx.x == 0);)
@@ -276,12 +309,15 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_const
 // ---------------------------------------------------------------------------------------------------
 // Backward prologue: -delta'_r = -(dO_r . y_r) / Z_r (stored negated)  and  dO'_r = dO_r / Z_r (bf16, same layout as dO).
 // D / 8 lanes per row (16 B each) in an aligned group of PREP_LANES lanes (a power of two for the butterfly sum; at
-// D = 80, 10 of 16 lanes carry data).
+// D = 80, 10 of 16 lanes carry data).  fp16: Z_r 2^-o_r in [1, 2) takes the place of Z_r (the kernels scale e by 2^-o_r),
+// so dO' stays within the range of dO.
 // ---------------------------------------------------------------------------------------------------
-template <int D>
+__device__ __forceinline__ float prep_inv(float z, bool f16) { return 1.0f / (f16 ? f16_bwd_zs(z) : z); }
+
+template <int D, typename T>
 __global__ void __launch_bounds__(256)
-attn_bwd_prep_kernel(const __nv_bfloat16 *__restrict__ dy, const __nv_bfloat16 *__restrict__ y,
-                     const float *__restrict__ zsum, float *__restrict__ delta, __nv_bfloat16 *__restrict__ dys,
+attn_bwd_prep_kernel(const T *__restrict__ dy, const T *__restrict__ y,
+                     const float *__restrict__ zsum, float *__restrict__ delta, T *__restrict__ dys,
                      int64_t rows, int S, int H) {
     constexpr int LPR = D / 8, G = Dim<D>::PREP_LANES;                    // data lanes per row, lanes per row
     const int64_t row = (int64_t)blockIdx.x * (256 / G) + (threadIdx.x / G);
@@ -292,8 +328,8 @@ attn_bwd_prep_kernel(const __nv_bfloat16 *__restrict__ dy, const __nv_bfloat16 *
     const int64_t off = (((b / H) * S + r) * H + (b % H)) * D + sub * 8;
     float a[8], c[8];
     if (active) {
-        Vec16<__nv_bfloat16>::load(dy + off, a);
-        Vec16<__nv_bfloat16>::load(y + off, c);
+        Vec16<T>::load(dy + off, a);
+        Vec16<T>::load(y + off, c);
     } else {
 #pragma unroll
         for (int i = 0; i < 8; ++i) a[i] = c[i] = 0.0f;
@@ -302,23 +338,23 @@ attn_bwd_prep_kernel(const __nv_bfloat16 *__restrict__ dy, const __nv_bfloat16 *
 #pragma unroll
     for (int i = 0; i < 8; ++i) acc = fmaf(a[i], c[i], acc);
     acc = group_sum<G>(acc);
-    const float inv = 1.0f / zsum[row];
+    const float inv = prep_inv(zsum[row], is_f16<T>);
 #pragma unroll
     for (int i = 0; i < 8; ++i) a[i] *= inv;
-    if (active) Vec16<__nv_bfloat16>::store(dys + off, a);
+    if (active) Vec16<T>::store(dys + off, a);
     if (sub == 0) delta[row] = -acc * inv;        // stored negated: the kernels add it (dp - delta')
 }
 
 // The same for dO and y in the reference layer's output layout (y^T, dO^T: [B, D, S] memory): a block transposes a
 // [D] x [64 rows] tile of each through shared memory; dO' is written in the standard [N, S, H, D] layout the TMA maps read.
-template <int D>
+template <int D, typename T>
 __global__ void __launch_bounds__(256)
-attn_bwd_prep_t_kernel(const __nv_bfloat16 *__restrict__ dyt, const __nv_bfloat16 *__restrict__ yt,
-                       const float *__restrict__ zsum, float *__restrict__ delta, __nv_bfloat16 *__restrict__ dys, int S,
+attn_bwd_prep_t_kernel(const T *__restrict__ dyt, const T *__restrict__ yt,
+                       const float *__restrict__ zsum, float *__restrict__ delta, T *__restrict__ dys, int S,
                        int H) {
     constexpr int TR = 64, LD = TR + 8;
-    __shared__ __align__(16) __nv_bfloat16 s_dy[D][LD];
-    __shared__ __align__(16) __nv_bfloat16 s_y[D][LD];
+    __shared__ __align__(16) T s_dy[D][LD];
+    __shared__ __align__(16) T s_y[D][LD];
     const int b = blockIdx.y, r0 = blockIdx.x * TR;
     const size_t base = (size_t)b * D * S + r0;
     constexpr int EPT = D / 4;                       // features per thread
@@ -337,28 +373,28 @@ attn_bwd_prep_t_kernel(const __nv_bfloat16 *__restrict__ dyt, const __nv_bfloat1
     float acc = 0.0f;
 #pragma unroll
     for (int i = 0; i < EPT; ++i) {
-        a[i] = __bfloat162float(s_dy[qd * EPT + i][rs]);
-        acc = fmaf(a[i], __bfloat162float(s_y[qd * EPT + i][rs]), acc);
+        a[i] = to_f32(s_dy[qd * EPT + i][rs]);
+        acc = fmaf(a[i], to_f32(s_y[qd * EPT + i][rs]), acc);
     }
     acc = group_sum<4>(acc);
     const size_t grow = (size_t)b * S + r0 + r;
-    const float inv = 1.0f / zsum[grow];
+    const float inv = prep_inv(zsum[grow], is_f16<T>);
     const int hn = b / H, hh = b % H;
-    __nv_bfloat16 *dst = dys + (((size_t)hn * S + r0 + r) * H + hh) * D + qd * EPT;
+    T *dst = dys + (((size_t)hn * S + r0 + r) * H + hh) * D + qd * EPT;
     if constexpr (EPT % 8 == 0) {
 #pragma unroll
         for (int i = 0; i < EPT; i += 8) {
             float t[8];
 #pragma unroll
             for (int u = 0; u < 8; ++u) t[u] = a[i + u] * inv;
-            Vec16<__nv_bfloat16>::store(dst + i, t);
+            Vec16<T>::store(dst + i, t);
         }
     } else {
         // D = 80: a thread's 20 features start 40 bytes apart, so 8-byte stores
         static_assert(EPT % 4 == 0, "features per thread must be a multiple of 4");
 #pragma unroll
         for (int i = 0; i < EPT; i += 4)
-            *reinterpret_cast<uint2 *>(dst + i) = make_uint2(pack_bf16(a[i] * inv, a[i + 1] * inv), pack_bf16(a[i + 2] * inv, a[i + 3] * inv));
+            *reinterpret_cast<uint2 *>(dst + i) = make_uint2(pack2<T>(a[i] * inv, a[i + 1] * inv), pack2<T>(a[i + 2] * inv, a[i + 3] * inv));
     }
     if (qd == 0) delta[grow] = -acc * inv;
 }
@@ -370,13 +406,14 @@ attn_bwd_prep_t_kernel(const __nv_bfloat16 *__restrict__ dyt, const __nv_bfloat1
 // registers, so the tensor core computes the next tile's scores under this tile's exp math.
 // ---------------------------------------------------------------------------------------------------
 
-template <int D>
+// fp16: zsum gives the row scales (read by the fp16 instantiations only)
+template <int D, typename T>
 __global__ void __launch_bounds__(THREADS, Dim<D>::CTAS)
 attn_bwd_q_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_k,
                      const __grid_constant__ CUtensorMap map_v, const __grid_constant__ CUtensorMap map_dys,
                      const uint32_t *__restrict__ mask, const int32_t *__restrict__ extra0,
-                     const float *__restrict__ delta, __nv_bfloat16 *__restrict__ dq, int S, int H, float scale,
-                     float scale_log2, float clamp_log2) {
+                     const float *__restrict__ delta, T *__restrict__ dq, int S, int H, float scale,
+                     float scale_log2, float clamp_log2, const float *__restrict__ zsum) {
     constexpr int OWN_BYTES = Dim<D>::OWN_BYTES, T_BYTES = Dim<D>::T_BYTES, OWN_SUB = Dim<D>::OWN_SUB, T_SUB = Dim<D>::T_SUB,
                   TMEM_COLS = Dim<D>::TMEM_COLS, DP = Dim<D>::DP;
     extern __shared__ unsigned char smem_raw[];
@@ -435,8 +472,8 @@ attn_bwd_q_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
             }
         }
     } else if (warp == 9) {
-        constexpr uint32_t id_s = idesc_bf16(BM, BN, 0, 0);   // S = Q K^T, dP' = dO' V^T
-        constexpr uint32_t id_a = idesc_bf16(BM, DP, 0, 1);    // dQ += dS K   (A from TMEM, K MN-major)
+        constexpr uint32_t id_s = idesc_of<T>(BM, BN, 0, 0);   // S = Q K^T, dP' = dO' V^T
+        constexpr uint32_t id_a = idesc_of<T>(BM, DP, 0, 1);    // dQ += dS K   (A from TMEM, K MN-major)
         const uint64_t dq0 = desc_kmajor(s_q, 0), ddy0 = desc_kmajor(s_dy, 0), dk0 = desc_kmajor(s_k, 0),
                        dv0 = desc_kmajor(s_v, 0), dkt0 = desc_mnmajor(s_k, 0, T_SUB);
         // The score MMAs of tile j are issued as soon as tile j-1's scores are in the math warps' registers (s_read): they are
@@ -492,6 +529,7 @@ attn_bwd_q_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
         const uint4 *mrow = reinterpret_cast<const uint4 *>(mask + grow * (S / 32));
         const float ex0 = (float)extra0[grow];
         const float dl = delta[grow];
+        const float nofs = is_f16<T> ? f16_bwd_nofs(zsum[grow]) : 0.0f;
         const uint32_t lane_base = tmem_base + ((uint32_t)(quarter * 32) << 16);
         const MathK mk = make_math(scale_log2, clamp_log2);
         uint4 mw = __ldg(mrow);
@@ -519,11 +557,11 @@ attn_bwd_q_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
                 uint32_t pk[16];
                 const bool first = (j == 0 && c == 0);
                 if (!warp_needs_clamp(r, mk.thr)) {
-                    if (first) bwdq_chunk32<true, false>(r, g, X, mk, dl, ex0, pk);
-                    else bwdq_chunk32<false, false>(r, g, X, mk, dl, ex0, pk);
+                    if (first) bwdq_chunk32<true, false, T>(r, g, X, mk, dl, ex0, pk, nofs);
+                    else bwdq_chunk32<false, false, T>(r, g, X, mk, dl, ex0, pk, nofs);
                 } else {
-                    if (first) bwdq_chunk32<true, true>(r, g, X, mk, dl, ex0, pk);
-                    else bwdq_chunk32<false, true>(r, g, X, mk, dl, ex0, pk);
+                    if (first) bwdq_chunk32<true, true, T>(r, g, X, mk, dl, ex0, pk, nofs);
+                    else bwdq_chunk32<false, true, T>(r, g, X, mk, dl, ex0, pk, nofs);
                 }
                 PROF(pf.lap(2);)
                 tmem_st16(lane_base + COL_DS + half * 32 + c * 16, pk);
@@ -537,7 +575,7 @@ attn_bwd_q_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
         PROF(pf.t[5] = clock64() - t0; pf.t[4] = n_tiles / 2; pf.flush(1, 0, threadIdx.x == 0);)
         mbar_wait(acc_full, 0);
         fence_after_sync();
-        __nv_bfloat16 *dst = dq + (((size_t)hn * S + row) * H + hh) * D;
+        T *dst = dq + (((size_t)hn * S + row) * H + hh) * D;
         out_chunks<D>(half, [&](int col, auto w) {
             uint32_t r[32];
             tmem_ld32(lane_base + COL_DQ + col, r);
@@ -558,23 +596,23 @@ attn_bwd_q_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
 // columns each, then dV, dK): the tensor core computes the next sub-tile's scores under this one's exp math.
 // E^T / dS^T (bf16 pairs) are written back over score columns the same thread has already consumed.
 // Per-row quantities of the 64 query rows (mask words of this key group, delta', extra0) are staged in
-// shared memory by the producer warp, one slot per pipeline stage.
+// shared memory by the producer warp, one slot per pipeline stage (fp16: also the rows' -o, from zsum).
 // ---------------------------------------------------------------------------------------------------
-template <int D>
+template <int D, typename T>
 __global__ void __launch_bounds__(THREADS, Dim<D>::CTAS)
 attn_bwd_kv_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_k,
                       const __grid_constant__ CUtensorMap map_v, const __grid_constant__ CUtensorMap map_dys,
                       const uint32_t *__restrict__ mask, const int32_t *__restrict__ extra0,
-                      const float *__restrict__ delta, __nv_bfloat16 *__restrict__ dk, __nv_bfloat16 *__restrict__ dv,
-                      int S, int H, float scale, float scale_log2, float clamp_log2) {
+                      const float *__restrict__ delta, T *__restrict__ dk, T *__restrict__ dv,
+                      int S, int H, float scale, float scale_log2, float clamp_log2, const float *__restrict__ zsum) {
     constexpr int OWN_BYTES = Dim<D>::OWN_BYTES, T_BYTES = Dim<D>::T_BYTES, OWN_SUB = Dim<D>::OWN_SUB, T_SUB = Dim<D>::T_SUB,
                   TMEM_COLS = Dim<D>::TMEM_COLS, DP = Dim<D>::DP;
     extern __shared__ unsigned char smem_raw[];
     const Smem sm = align_smem(smem_raw);
     const uint32_t s_k = sm.base, s_v = s_k + OWN_BYTES, s_q = s_v + OWN_BYTES, s_dy = s_q + STAGES * T_BYTES;
-    unsigned char *rowq = sm.ptr + 2 * OWN_BYTES + 2 * STAGES * T_BYTES;   // per stage: mask^T [4][64 + 4], delta[64], ex0[64]
+    unsigned char *rowq = sm.ptr + 2 * OWN_BYTES + 2 * STAGES * T_BYTES;   // per stage: mask^T [4][64 + 4], delta[64], ex0[64] (, -o[64])
     constexpr int MT = BN + 4;                         // padded row of the transposed mask: the 4 words hit distinct banks
-    constexpr int ROWQ_BYTES = MT * 16 + BN * 4 + BN * 4;
+    constexpr int ROWQ_BYTES = MT * 16 + BN * 4 + BN * 4 + (is_f16<T> ? BN * 4 : 0);
     uint64_t *bars = reinterpret_cast<uint64_t *>(rowq + STAGES * ROWQ_BYTES);
     const uint32_t bar0 = smem_u32(bars);
     const uint32_t own_full = bar0, acc_full = bar0 + 8;
@@ -644,14 +682,15 @@ attn_bwd_kv_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_co
                 mt[3 * MT + rr] = mw.w;
                 reinterpret_cast<float *>(slot + MT * 16)[rr] = delta[gr];      // -delta' (the math adds it: dp - delta')
                 reinterpret_cast<float *>(slot + MT * 16 + BN * 4)[rr] = (float)extra0[gr];
+                if constexpr (is_f16<T>) reinterpret_cast<float *>(slot + MT * 16 + 2 * BN * 4)[rr] = f16_bwd_nofs(zsum[gr]);
             }
             mbar_arrive(qd_full(st));
         }
     } else if (warp == 9) {
         // Sub-tiles t = 2 j + h of 32 query rows: scores of sub-tile t+1 are issued before the math warps have
         // finished sub-tile t (two score buffers), the accumulating MMAs of t follow once its E^T / dS^T are written.
-        constexpr uint32_t id_s = idesc_bf16(BM, SUBN, 0, 0); // S^T = K Q^T, dP'^T = V dO'^T   (N = 32 query rows)
-        constexpr uint32_t id_a = idesc_bf16(BM, DP, 0, 1);    // dV += E^T dO', dK += dS^T Q (B MN-major, K = 32)
+        constexpr uint32_t id_s = idesc_of<T>(BM, SUBN, 0, 0); // S^T = K Q^T, dP'^T = V dO'^T   (N = 32 query rows)
+        constexpr uint32_t id_a = idesc_of<T>(BM, DP, 0, 1);    // dV += E^T dO', dK += dS^T Q (B MN-major, K = 32)
         const uint64_t dk0 = desc_kmajor(s_k, 0), dv0 = desc_kmajor(s_v, 0), dq0 = desc_kmajor(s_q, 0),
                        ddy0 = desc_kmajor(s_dy, 0), dqt0 = desc_mnmajor(s_q, 0, T_SUB),
                        ddyt0 = desc_mnmajor(s_dy, 0, T_SUB);
@@ -718,6 +757,7 @@ attn_bwd_kv_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_co
             const uint32_t *mrow = reinterpret_cast<const uint32_t *>(slot) + wsel * MT;   // this key's word of every row
             const float *s_ndelta = reinterpret_cast<const float *>(slot + MT * 16);
             const float *s_ex0 = s_ndelta + BN;
+            const float *s_nofs = s_ndelta + 2 * BN;
             mbar_wait(qd_full(st), (j / STAGES) & 1);   // the producer lanes' row data of this stage
             mbar_wait(sc_full(h), j & 1);
             PROF(pf.lap(0);)
@@ -733,11 +773,11 @@ attn_bwd_kv_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_co
             uint32_t pe[8], pd[8];
 #define SPT_KV_HALF(OFF)                                                                                                   \
             if (key0) {                                                                                                    \
-                if (clamp) bwdkv_chunk16<true, true, OFF, 32>(r, g, mrow, s_ndelta, s_ex0, c0 + OFF, shl, mk, pe, pd);     \
-                else bwdkv_chunk16<true, false, OFF, 32>(r, g, mrow, s_ndelta, s_ex0, c0 + OFF, shl, mk, pe, pd);          \
+                if (clamp) bwdkv_chunk16<true, true, OFF, 32, float, T>(r, g, mrow, s_ndelta, s_ex0, c0 + OFF, shl, mk, pe, pd, s_nofs); \
+                else bwdkv_chunk16<true, false, OFF, 32, float, T>(r, g, mrow, s_ndelta, s_ex0, c0 + OFF, shl, mk, pe, pd, s_nofs);      \
             } else {                                                                                                       \
-                if (clamp) bwdkv_chunk16<false, true, OFF, 32>(r, g, mrow, s_ndelta, s_ex0, c0 + OFF, shl, mk, pe, pd);    \
-                else bwdkv_chunk16<false, false, OFF, 32>(r, g, mrow, s_ndelta, s_ex0, c0 + OFF, shl, mk, pe, pd);         \
+                if (clamp) bwdkv_chunk16<false, true, OFF, 32, float, T>(r, g, mrow, s_ndelta, s_ex0, c0 + OFF, shl, mk, pe, pd, s_nofs); \
+                else bwdkv_chunk16<false, false, OFF, 32, float, T>(r, g, mrow, s_ndelta, s_ex0, c0 + OFF, shl, mk, pe, pd, s_nofs);     \
             }                                                                                                              \
             tmem_st8(col + (OFF) / 2, pe);      /* E^T over the S^T columns this thread has consumed */                    \
             tmem_st8(col + 32 + (OFF) / 2, pd); /* dS^T over its dP'^T columns */
@@ -768,16 +808,16 @@ attn_bwd_kv_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_co
 }
 
 // ---- host -----------------------------------------------------------------------------------------
-// 4-D bf16 tensor map over a [N, S, H, D] tensor (H = 1: head-major [B, S, D]); box = 64 rows x 64 elements of one head.
-// D = 80: the box at column 64 holds the row's last 16 elements; the 48 out-of-bounds columns are filled with zeros.
-static int make_map(CUtensorMap *map, const void *base, int N, int S, int H, int D) {
+// 4-D bf16 / fp16 tensor map over a [N, S, H, D] tensor (H = 1: head-major [B, S, D]); box = 64 rows x 64 elements of one
+// head.  D = 80: the box at column 64 holds the row's last 16 elements; the 48 out-of-bounds columns are filled with zeros.
+static int make_map(CUtensorMap *map, const void *base, int N, int S, int H, int D, bool f16) {
     EncodeTiledFn fn = encode_fn();
     if (!fn) return fail(SPT_ERR_CUDA, "sparse_attn: cuTensorMapEncodeTiled entry point not available");
     cuuint64_t dims[4] = {(cuuint64_t)D, (cuuint64_t)H, (cuuint64_t)S, (cuuint64_t)N};
     cuuint64_t strides[3] = {(cuuint64_t)D * 2, (cuuint64_t)H * D * 2, (cuuint64_t)S * H * D * 2};
     cuuint32_t box[4] = {64, 1, (cuuint32_t)BN, 1};
     cuuint32_t estr[4] = {1, 1, 1, 1};
-    CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void *>(base), dims, strides, box, estr,
+    CUresult r = fn(map, f16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void *>(base), dims, strides, box, estr,
                     CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) return fail(SPT_ERR_CUDA, "sparse_attn: cuTensorMapEncodeTiled failed (%d)", (int)r);
@@ -831,37 +871,41 @@ static bool fwd128() {
     return on;
 }
 
-template <int D>
+// k: the key tensor (read by the fp16 forward only, for its row scales).  fp16 always runs the 128 x 64 forward.
+template <int D, typename T>
 static int launch_fwd(const CUtensorMap &mq, const CUtensorMap &mk, const CUtensorMap &mv, const uint32_t *mask,
-                      const int32_t *extra0, __nv_bfloat16 *y, float *zsum, int B, int S, int H, float scale, float clamp,
-                      int y_transposed, cudaStream_t st) {
-    if (D == 64 && fwd128()) return attn_tc128::launch_fwd128(mq, mk, mv, mask, extra0, y, zsum, B, S, H, scale, clamp, y_transposed, st);
+                      const int32_t *extra0, T *y, float *zsum, int B, int S, int H, float scale, float clamp,
+                      int y_transposed, const T *k, cudaStream_t st) {
+    if constexpr (!is_f16<T>)
+        if (D == 64 && fwd128()) return attn_tc128::launch_fwd128(mq, mk, mv, mask, extra0, y, zsum, B, S, H, scale, clamp, y_transposed, st);
     static const int extra_smem = [] { const char *e = getenv("SPT_ATTN_EXTRA_SMEM"); return e ? atoi(e) : 0; }();   // diagnostics: forces 1 CTA / SM
-    cudaFuncSetAttribute(attn_fwd_tc_kernel<D>, cudaFuncAttributeMaxDynamicSharedMemorySize, Dim<D>::FWD_SMEM + extra_smem);
-    attn_fwd_tc_kernel<D><<<dim3(B, S / BM), THREADS, Dim<D>::FWD_SMEM + extra_smem, st>>>(mq, mk, mv, mask, extra0, y, zsum, S, H,
-                                                                              scale * LOG2E, clamp * LOG2E, y_transposed);
+    cudaFuncSetAttribute(attn_fwd_tc_kernel<D, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, Dim<D>::FWD_SMEM + extra_smem);
+    attn_fwd_tc_kernel<D, T><<<dim3(B, S / BM), THREADS, Dim<D>::FWD_SMEM + extra_smem, st>>>(mq, mk, mv, mask, extra0, y, zsum, S, H,
+                                                                                 scale * LOG2E, clamp * LOG2E, y_transposed, k);
     return after_launch("attn_fwd_tc_kernel");
 }
 
-template <int D>
-static int launch_prep(const __nv_bfloat16 *y, const __nv_bfloat16 *grad_y, const float *zsum, float *delta,
-                       __nv_bfloat16 *dys, int B, int S, int H, int y_transposed, cudaStream_t st) {
+template <int D, typename T>
+static int launch_prep(const T *y, const T *grad_y, const float *zsum, float *delta, T *dys, int B, int S, int H,
+                       int y_transposed, cudaStream_t st) {
     if (y_transposed) {
-        attn_bwd_prep_t_kernel<D><<<dim3(S / 64, B), 256, 0, st>>>(grad_y, y, zsum, delta, dys, S, H);
+        attn_bwd_prep_t_kernel<D, T><<<dim3(S / 64, B), 256, 0, st>>>(grad_y, y, zsum, delta, dys, S, H);
         return after_launch("attn_bwd_prep_t_kernel");
     }
     const int64_t rows = (int64_t)B * S;
     constexpr int RPB = 256 / Dim<D>::PREP_LANES;
-    attn_bwd_prep_kernel<D><<<(unsigned)((rows + RPB - 1) / RPB), 256, 0, st>>>(grad_y, y, zsum, delta, dys, rows, S, H);
+    attn_bwd_prep_kernel<D, T><<<(unsigned)((rows + RPB - 1) / RPB), 256, 0, st>>>(grad_y, y, zsum, delta, dys, rows, S, H);
     return after_launch("attn_bwd_prep_kernel");
 }
 
-template <int D>
+// fp16 never takes the one-pass backward (SPT_ATTN_BWD_FUSED=1 leaves it on the dK/dV + dQ kernels)
+template <int D, typename T>
 static int launch_bwd(const CUtensorMap &mq, const CUtensorMap &mk, const CUtensorMap &mv, const CUtensorMap &md,
-                      const uint32_t *mask, const int32_t *extra0, const float *delta, float *dq_acc, __nv_bfloat16 *gq,
-                      __nv_bfloat16 *gk, __nv_bfloat16 *gv, int B, int S, int H, float scale, float clamp, cudaStream_t st) {
-    if (D == 64 && tile128() && bwd_fused())
-        return attn_tc128::launch_bwd_fused128(mq, mk, mv, md, mask, extra0, delta, dq_acc, gq, gk, gv, B, S, H, scale, clamp, st);
+                      const uint32_t *mask, const int32_t *extra0, const float *delta, const float *zsum, float *dq_acc,
+                      T *gq, T *gk, T *gv, int B, int S, int H, float scale, float clamp, cudaStream_t st) {
+    if constexpr (!is_f16<T>)
+        if (D == 64 && tile128() && bwd_fused())
+            return attn_tc128::launch_bwd_fused128(mq, mk, mv, md, mask, extra0, delta, dq_acc, gq, gk, gv, B, S, H, scale, clamp, st);
     if (D == 64 && tile128() && bwd_two_streams()) {
         // The dK/dV and the dQ kernel are independent: the dQ kernel goes to a side stream (fork / join with events, which
         // a stream capture records as graph edges), so its CTAs start on each SM as that SM's dK/dV CTA retires instead of
@@ -871,9 +915,9 @@ static int launch_bwd(const CUtensorMap &mq, const CUtensorMap &mk, const CUtens
         if (ss) {
             if (cudaEventRecord(ss->fork, st) != cudaSuccess || cudaStreamWaitEvent(ss->stream, ss->fork, 0) != cudaSuccess)
                 return fail(SPT_ERR_CUDA, "sparse_attn_bwd: fork to the side stream failed");
-            int rc = attn_tc128::launch_bwd_kv128(mq, mk, mv, md, mask, extra0, delta, gk, gv, B, S, H, scale, clamp, st);
+            int rc = attn_tc128::launch_bwd_kv128(mq, mk, mv, md, mask, extra0, delta, zsum, gk, gv, B, S, H, scale, clamp, st);
             if (rc != SPT_OK) return rc;
-            rc = attn_tc128::launch_bwd_q128(mq, mk, mv, md, mask, extra0, delta, gq, B, S, H, scale, clamp, ss->stream);
+            rc = attn_tc128::launch_bwd_q128(mq, mk, mv, md, mask, extra0, delta, zsum, gq, B, S, H, scale, clamp, ss->stream);
             if (rc != SPT_OK) return rc;
             if (cudaEventRecord(ss->join, ss->stream) != cudaSuccess || cudaStreamWaitEvent(st, ss->join, 0) != cudaSuccess)
                 return fail(SPT_ERR_CUDA, "sparse_attn_bwd: join of the side stream failed");
@@ -881,18 +925,19 @@ static int launch_bwd(const CUtensorMap &mq, const CUtensorMap &mk, const CUtens
         }
     }
     if (D == 64 && tile128()) {
-        const int rc = attn_tc128::launch_bwd_kv128(mq, mk, mv, md, mask, extra0, delta, gk, gv, B, S, H, scale, clamp, st);
+        const int rc = attn_tc128::launch_bwd_kv128(mq, mk, mv, md, mask, extra0, delta, zsum, gk, gv, B, S, H, scale, clamp, st);
         if (rc != SPT_OK) return rc;
     } else {
-        cudaFuncSetAttribute(attn_bwd_kv_tc_kernel<D>, cudaFuncAttributeMaxDynamicSharedMemorySize, Dim<D>::BWD_SMEM);
-        attn_bwd_kv_tc_kernel<D><<<dim3(B, S / BM), THREADS, Dim<D>::BWD_SMEM, st>>>(
-            mq, mk, mv, md, mask, extra0, delta, gk, gv, S, H, scale, scale * LOG2E, clamp * LOG2E);
+        constexpr int kv_smem = Dim<D>::BWD_SMEM + (is_f16<T> ? STAGES * BN * 4 : 0);      // fp16: the rows' -o per stage
+        cudaFuncSetAttribute(attn_bwd_kv_tc_kernel<D, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, kv_smem);
+        attn_bwd_kv_tc_kernel<D, T><<<dim3(B, S / BM), THREADS, kv_smem, st>>>(
+            mq, mk, mv, md, mask, extra0, delta, gk, gv, S, H, scale, scale * LOG2E, clamp * LOG2E, zsum);
         SPT_LAUNCH_CHECK("attn_bwd_kv_tc_kernel");
     }
-    if (D == 64 && tile128()) return attn_tc128::launch_bwd_q128(mq, mk, mv, md, mask, extra0, delta, gq, B, S, H, scale, clamp, st);
-    cudaFuncSetAttribute(attn_bwd_q_tc_kernel<D>, cudaFuncAttributeMaxDynamicSharedMemorySize, Dim<D>::BWD_SMEM);
-    attn_bwd_q_tc_kernel<D><<<dim3(B, S / BM), THREADS, Dim<D>::BWD_SMEM, st>>>(
-        mq, mk, mv, md, mask, extra0, delta, gq, S, H, scale, scale * LOG2E, clamp * LOG2E);
+    if (D == 64 && tile128()) return attn_tc128::launch_bwd_q128(mq, mk, mv, md, mask, extra0, delta, zsum, gq, B, S, H, scale, clamp, st);
+    cudaFuncSetAttribute(attn_bwd_q_tc_kernel<D, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, Dim<D>::BWD_SMEM);
+    attn_bwd_q_tc_kernel<D, T><<<dim3(B, S / BM), THREADS, Dim<D>::BWD_SMEM, st>>>(
+        mq, mk, mv, md, mask, extra0, delta, gq, S, H, scale, scale * LOG2E, clamp * LOG2E, zsum);
     SPT_LAUNCH_CHECK("attn_bwd_q_tc_kernel");
     return SPT_OK;
 }
@@ -902,8 +947,11 @@ static int launch_bwd(const CUtensorMap &mq, const CUtensorMap &mk, const CUtens
 
 using namespace spt;
 
-static int check_attn_args(const char *what, int B, int S, int d, int H, int dtype) {
-    if (dtype != SPT_BF16) return fail(SPT_ERR_UNSUPPORTED, "%s: only bf16 is supported on the fused path", what);
+static int check_attn_args(const char *what, int B, int S, int d, int H, int dtype, float clamp) {
+    if (dtype != SPT_BF16 && dtype != SPT_F16)
+        return fail(SPT_ERR_UNSUPPORTED, "%s: only bf16 and fp16 are supported on the fused path", what);
+    if (dtype == SPT_F16 && !(clamp >= 0.0f && clamp <= attn_tc::F16_MAX_CLAMP))
+        return fail(SPT_ERR_UNSUPPORTED, "%s: fp16 needs 0 <= clamp <= %g (got %g)", what, (double)attn_tc::F16_MAX_CLAMP, (double)clamp);
     if (d != 64 && d != 80 && d != 128)
         return fail(SPT_ERR_UNSUPPORTED, "%s: head dim %d not supported (64, 80 or 128)", what, d);
     if (B < 1 || B > 65535 || S < 128 || S % 128 != 0)
@@ -911,6 +959,46 @@ static int check_attn_args(const char *what, int B, int S, int d, int H, int dty
     if (H < 1 || B % H != 0)
         return fail(SPT_ERR_INVALID_ARGUMENT, "%s: B=%d must be a multiple of the interleaved head count H=%d", what, B, H);
     return SPT_OK;
+}
+
+template <typename T>
+static int attn_fwd_typed(const CUtensorMap &mq, const CUtensorMap &mk, const CUtensorMap &mv, const uint32_t *mask,
+                          const int32_t *extra0, void *y, float *zsum, int B, int S, int d, int H, float scale, float clamp,
+                          int yt, const void *k, cudaStream_t st) {
+    T *yy = (T *)y;
+    const T *kk = (const T *)k;
+    if (d == 64) return attn_tc::launch_fwd<64, T>(mq, mk, mv, mask, extra0, yy, zsum, B, S, H, scale, clamp, yt, kk, st);
+    if (d == 80) return attn_tc::launch_fwd<80, T>(mq, mk, mv, mask, extra0, yy, zsum, B, S, H, scale, clamp, yt, kk, st);
+    return attn_tc::launch_fwd<128, T>(mq, mk, mv, mask, extra0, yy, zsum, B, S, H, scale, clamp, yt, kk, st);
+}
+
+// the backward after the argument checks: row kernel, tensor maps, dK/dV + dQ kernels
+template <typename T>
+static int attn_bwd_typed(const void *q, const void *k, const void *v, const void *y, const void *grad_y,
+                          const uint32_t *mask, const int32_t *extra0, const float *zsum, void *grad_q, void *grad_k,
+                          void *grad_v, void *workspace, int B, int S, int d, int H, float scale, float clamp, int yt,
+                          cudaStream_t st) {
+    constexpr bool f16 = attn_tc::is_f16<T>;
+    float *delta = (float *)workspace;
+    T *dys = (T *)((char *)workspace + (size_t)B * S * sizeof(float));
+    float *dq_acc = (float *)((char *)workspace + (size_t)B * S * sizeof(float) + (size_t)B * S * 128 * 2);
+    // the row kernel goes first: besides producing dO' and delta' it is a runtime-API launch, which binds the
+    // device's primary context to this (autograd worker) thread before the driver-API tensor-map encoder runs
+    int rc = d == 64   ? attn_tc::launch_prep<64, T>((const T *)y, (const T *)grad_y, zsum, delta, dys, B, S, H, yt, st)
+             : d == 80 ? attn_tc::launch_prep<80, T>((const T *)y, (const T *)grad_y, zsum, delta, dys, B, S, H, yt, st)
+                       : attn_tc::launch_prep<128, T>((const T *)y, (const T *)grad_y, zsum, delta, dys, B, S, H, yt, st);
+    if (rc != SPT_OK) return rc;
+    CUtensorMap mq, mk, mv, md;
+    if ((rc = attn_tc::make_map(&mq, q, B / H, S, H, d, f16)) != SPT_OK) return rc;
+    if ((rc = attn_tc::make_map(&mk, k, B / H, S, H, d, f16)) != SPT_OK) return rc;
+    if ((rc = attn_tc::make_map(&mv, v, B / H, S, H, d, f16)) != SPT_OK) return rc;
+    if ((rc = attn_tc::make_map(&md, dys, B / H, S, H, d, f16)) != SPT_OK) return rc;
+    T *gq = (T *)grad_q, *gk = (T *)grad_k, *gv = (T *)grad_v;
+    if (d == 64)
+        return attn_tc::launch_bwd<64, T>(mq, mk, mv, md, mask, extra0, delta, zsum, dq_acc, gq, gk, gv, B, S, H, scale, clamp, st);
+    if (d == 80)
+        return attn_tc::launch_bwd<80, T>(mq, mk, mv, md, mask, extra0, delta, zsum, dq_acc, gq, gk, gv, B, S, H, scale, clamp, st);
+    return attn_tc::launch_bwd<128, T>(mq, mk, mv, md, mask, extra0, delta, zsum, dq_acc, gq, gk, gv, B, S, H, scale, clamp, st);
 }
 
 extern "C" int spt_sparse_attn_fwd(const void *q, const void *k, const void *v, const uint32_t *mask,
@@ -924,17 +1012,16 @@ extern "C" int spt_sparse_attn_fwd_ex(const void *q, const void *k, const void *
                                       float scale, float clamp, int dtype, int flags, spt_stream_t stream) {
     SPT_REQUIRE(q && k && v && mask && extra0 && y && zsum, "sparse_attn_fwd: null pointer");
     const int yt = (flags & SPT_ATTN_Y_TRANSPOSED) ? 1 : 0;
-    int rc = check_attn_args("sparse_attn_fwd", B, S, d, H, dtype);
+    int rc = check_attn_args("sparse_attn_fwd", B, S, d, H, dtype, clamp);
     if (rc != SPT_OK) return rc;
     SPT_REQUIRE(((uintptr_t)q | (uintptr_t)k | (uintptr_t)v | (uintptr_t)y) % 16 == 0, "sparse_attn_fwd: operands must be 16-byte aligned");
-    using bf = __nv_bfloat16;
+    const bool f16 = dtype == SPT_F16;
     CUtensorMap mq, mk, mv;
-    if ((rc = attn_tc::make_map(&mq, q, B / H, S, H, d)) != SPT_OK) return rc;
-    if ((rc = attn_tc::make_map(&mk, k, B / H, S, H, d)) != SPT_OK) return rc;
-    if ((rc = attn_tc::make_map(&mv, v, B / H, S, H, d)) != SPT_OK) return rc;
-    if (d == 64) return attn_tc::launch_fwd<64>(mq, mk, mv, mask, extra0, (bf *)y, zsum, B, S, H, scale, clamp, yt, as_stream(stream));
-    if (d == 80) return attn_tc::launch_fwd<80>(mq, mk, mv, mask, extra0, (bf *)y, zsum, B, S, H, scale, clamp, yt, as_stream(stream));
-    return attn_tc::launch_fwd<128>(mq, mk, mv, mask, extra0, (bf *)y, zsum, B, S, H, scale, clamp, yt, as_stream(stream));
+    if ((rc = attn_tc::make_map(&mq, q, B / H, S, H, d, f16)) != SPT_OK) return rc;
+    if ((rc = attn_tc::make_map(&mk, k, B / H, S, H, d, f16)) != SPT_OK) return rc;
+    if ((rc = attn_tc::make_map(&mv, v, B / H, S, H, d, f16)) != SPT_OK) return rc;
+    return f16 ? attn_fwd_typed<__half>(mq, mk, mv, mask, extra0, y, zsum, B, S, d, H, scale, clamp, yt, k, as_stream(stream))
+               : attn_fwd_typed<__nv_bfloat16>(mq, mk, mv, mask, extra0, y, zsum, B, S, d, H, scale, clamp, yt, k, as_stream(stream));
 }
 
 // diagnostics: phase timers of the attention kernels (all zeros unless built with -DSPT_ATTN_PROF); reset != 0 clears them
@@ -976,31 +1063,13 @@ extern "C" int spt_sparse_attn_bwd_ex(const void *q, const void *k, const void *
     const int yt = (flags & SPT_ATTN_Y_TRANSPOSED) ? 1 : 0;
     SPT_REQUIRE(q && k && v && y && grad_y && mask && extra0 && zsum && grad_q && grad_k && grad_v && workspace,
                 "sparse_attn_bwd: null pointer");
-    int rc = check_attn_args("sparse_attn_bwd", B, S, d, H, dtype);
+    int rc = check_attn_args("sparse_attn_bwd", B, S, d, H, dtype, clamp);
     if (rc != SPT_OK) return rc;
     SPT_REQUIRE(((uintptr_t)q | (uintptr_t)k | (uintptr_t)v | (uintptr_t)grad_y | (uintptr_t)workspace) % 16 == 0,
                 "sparse_attn_bwd: operands must be 16-byte aligned");
-    using bf = __nv_bfloat16;
-    float *delta = (float *)workspace;
-    bf *dys = (bf *)((char *)workspace + (size_t)B * S * sizeof(float));
-    float *dq_acc = (float *)((char *)workspace + (size_t)B * S * sizeof(float) + (size_t)B * S * 128 * 2);
-    // the row kernel goes first: besides producing dO' and delta' it is a runtime-API launch, which binds the
-    // device's primary context to this (autograd worker) thread before the driver-API tensor-map encoder runs
-    rc = d == 64   ? attn_tc::launch_prep<64>((const bf *)y, (const bf *)grad_y, zsum, delta, dys, B, S, H, yt, as_stream(stream))
-         : d == 80 ? attn_tc::launch_prep<80>((const bf *)y, (const bf *)grad_y, zsum, delta, dys, B, S, H, yt, as_stream(stream))
-                   : attn_tc::launch_prep<128>((const bf *)y, (const bf *)grad_y, zsum, delta, dys, B, S, H, yt, as_stream(stream));
-    if (rc != SPT_OK) return rc;
-    CUtensorMap mq, mk, mv, md;
-    if ((rc = attn_tc::make_map(&mq, q, B / H, S, H, d)) != SPT_OK) return rc;
-    if ((rc = attn_tc::make_map(&mk, k, B / H, S, H, d)) != SPT_OK) return rc;
-    if ((rc = attn_tc::make_map(&mv, v, B / H, S, H, d)) != SPT_OK) return rc;
-    if ((rc = attn_tc::make_map(&md, dys, B / H, S, H, d)) != SPT_OK) return rc;
-    if (d == 64)
-        return attn_tc::launch_bwd<64>(mq, mk, mv, md, mask, extra0, delta, dq_acc, (bf *)grad_q, (bf *)grad_k, (bf *)grad_v,
-                                       B, S, H, scale, clamp, as_stream(stream));
-    if (d == 80)
-        return attn_tc::launch_bwd<80>(mq, mk, mv, md, mask, extra0, delta, dq_acc, (bf *)grad_q, (bf *)grad_k, (bf *)grad_v,
-                                       B, S, H, scale, clamp, as_stream(stream));
-    return attn_tc::launch_bwd<128>(mq, mk, mv, md, mask, extra0, delta, dq_acc, (bf *)grad_q, (bf *)grad_k, (bf *)grad_v, B,
-                                    S, H, scale, clamp, as_stream(stream));
+    if (dtype == SPT_F16)
+        return attn_bwd_typed<__half>(q, k, v, y, grad_y, mask, extra0, zsum, grad_q, grad_k, grad_v, workspace, B, S, d, H,
+                                      scale, clamp, yt, as_stream(stream));
+    return attn_bwd_typed<__nv_bfloat16>(q, k, v, y, grad_y, mask, extra0, zsum, grad_q, grad_k, grad_v, workspace, B, S, d,
+                                         H, scale, clamp, yt, as_stream(stream));
 }

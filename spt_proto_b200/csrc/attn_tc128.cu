@@ -60,13 +60,21 @@ __device__ __forceinline__ void warp_arrive(uint32_t bar, int lane) {
 constexpr int MT = T + 4;                              // padded row of the transposed mask: the 4 words hit distinct banks
 constexpr int ROWQ = MT * 16 + T * 4 + T * 4;          // bytes per stage
 constexpr int KV_SMEM = 4 * TILE + 2 * ST * TILE + ST * ROWQ + 256 + 1024;
+// fp16 adds the rows' -o (row scale, from zsum) to every stage: T * 4 bytes after extra0
+template <typename E>
+constexpr int rowq_bytes = ROWQ + (is_f16<E> ? T * 4 : 0);
+template <typename E>
+constexpr int kv_smem = KV_SMEM + ST * (rowq_bytes<E> - ROWQ);
 
+// E: element type (__nv_bfloat16 or __half); zsum is read by the fp16 instantiation only
+template <typename E>
 __global__ void __launch_bounds__(THREADS, 1)
 attn_bwd_kv128_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_k,
                       const __grid_constant__ CUtensorMap map_v, const __grid_constant__ CUtensorMap map_dys,
                       const uint32_t *__restrict__ mask, const int32_t *__restrict__ extra0,
-                      const float *__restrict__ ndelta, __nv_bfloat16 *__restrict__ dk, __nv_bfloat16 *__restrict__ dv,
-                      int S, int H, int B, float scale, float scale_log2, float clamp_log2) {
+                      const float *__restrict__ ndelta, E *__restrict__ dk, E *__restrict__ dv,
+                      int S, int H, int B, float scale, float scale_log2, float clamp_log2, const float *__restrict__ zsum) {
+    constexpr int ROWQ = rowq_bytes<E>;
     extern __shared__ unsigned char smem_raw[];
     const Smem sm = align_smem(smem_raw);
     const uint32_t s_k = sm.base, s_v = s_k + 2 * TILE, s_q = s_v + 2 * TILE, s_dy = s_q + ST * TILE;
@@ -148,6 +156,7 @@ attn_bwd_kv128_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_co
                     mt[MT + rr] = mw[u].y;
                     mt[2 * MT + rr] = mw[u].z;
                     mt[3 * MT + rr] = mw[u].w;
+                    if constexpr (is_f16<E>) reinterpret_cast<float *>(slot + MT * 16 + 2 * T * 4)[rr] = f16_bwd_nofs(zsum[head + r0 + rr]);
                 }
                 if (j + 1 < n_tiles) {                                    // the next tile's words travel under this wait
 #pragma unroll
@@ -160,8 +169,8 @@ attn_bwd_kv128_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_co
         }
     } else if (warp == W_MMA) {
         // ===== MMA issuer (warp-uniform loop, one elected lane) =====
-        constexpr uint32_t id_s = idesc_bf16(T, T, 0, 0);     // S^T = K Q^T, dP'^T = V dO'^T
-        constexpr uint32_t id_a = idesc_bf16(T, D, 0, 1);     // dV += E^T dO', dK += dS^T Q   (A in TMEM, B MN-major)
+        constexpr uint32_t id_s = idesc_of<E>(T, T, 0, 0);     // S^T = K Q^T, dP'^T = V dO'^T
+        constexpr uint32_t id_a = idesc_of<E>(T, D, 0, 1);     // dV += E^T dO', dK += dS^T Q   (A in TMEM, B MN-major)
         const uint64_t dk0 = desc_kmajor(s_k, 0), dv0 = desc_kmajor(s_v, 0), dq0 = desc_kmajor(s_q, 0),
                        ddy0 = desc_kmajor(s_dy, 0), dqt0 = desc_mnmajor(s_q, 0, TILE), ddyt0 = desc_mnmajor(s_dy, 0, TILE);
         int g = 0, w = 0;
@@ -236,6 +245,7 @@ attn_bwd_kv128_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_co
                 const uint32_t *mrow = reinterpret_cast<const uint32_t *>(slot) + wsel * MT;   // this key's word of every row
                 const float *s_nd = reinterpret_cast<const float *>(slot + MT * 16);
                 const int32_t *s_ex0 = reinterpret_cast<const int32_t *>(slot + MT * 16 + T * 4);
+                const float *s_nofs = reinterpret_cast<const float *>(slot + MT * 16 + 2 * T * 4);
                 mbar_wait(qd_full(st), (g / ST) & 1);
                 mbar_wait(sc_full, g & 1);
                 PROF(pf.lap(0);)
@@ -260,11 +270,11 @@ attn_bwd_kv128_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_co
                 uint32_t pe0[8], pd0[8], pe1[8], pd1[8];
 #define SPT_KV_HALF(OFF, PE, PD)                                                                                           \
                 if (pad) {                                                                                                \
-                    if (clamp) bwdkv_chunk16<true, true, OFF, 32>(r, gr, mrow, s_nd, s_ex0, c0 + OFF, shl, mk, PE, PD);    \
-                    else bwdkv_chunk16<true, false, OFF, 32>(r, gr, mrow, s_nd, s_ex0, c0 + OFF, shl, mk, PE, PD);         \
+                    if (clamp) bwdkv_chunk16<true, true, OFF, 32, int32_t, E>(r, gr, mrow, s_nd, s_ex0, c0 + OFF, shl, mk, PE, PD, s_nofs);  \
+                    else bwdkv_chunk16<true, false, OFF, 32, int32_t, E>(r, gr, mrow, s_nd, s_ex0, c0 + OFF, shl, mk, PE, PD, s_nofs);       \
                 } else {                                                                                                   \
-                    if (clamp) bwdkv_chunk16<false, true, OFF, 32>(r, gr, mrow, s_nd, s_ex0, c0 + OFF, shl, mk, PE, PD);   \
-                    else bwdkv_chunk16<false, false, OFF, 32>(r, gr, mrow, s_nd, s_ex0, c0 + OFF, shl, mk, PE, PD);        \
+                    if (clamp) bwdkv_chunk16<false, true, OFF, 32, int32_t, E>(r, gr, mrow, s_nd, s_ex0, c0 + OFF, shl, mk, PE, PD, s_nofs); \
+                    else bwdkv_chunk16<false, false, OFF, 32, int32_t, E>(r, gr, mrow, s_nd, s_ex0, c0 + OFF, shl, mk, PE, PD, s_nofs);      \
                 }
                 SPT_KV_HALF(0, pe0, pd0)
                 SPT_KV_HALF(16, pe1, pd1)
@@ -301,26 +311,35 @@ attn_bwd_kv128_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_co
     if (warp == W_MMA) tmem_dealloc<512>(tmem_base);
 }
 
+template <typename E>
 int launch_bwd_kv128(const CUtensorMap &mq, const CUtensorMap &mk, const CUtensorMap &mv, const CUtensorMap &md,
-                     const uint32_t *mask, const int32_t *extra0, const float *ndelta, __nv_bfloat16 *gk,
-                     __nv_bfloat16 *gv, int B, int S, int H, float scale, float clamp, cudaStream_t st) {
-    cudaFuncSetAttribute(attn_bwd_kv128_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, KV_SMEM);
+                     const uint32_t *mask, const int32_t *extra0, const float *ndelta, const float *zsum, E *gk, E *gv,
+                     int B, int S, int H, float scale, float clamp, cudaStream_t st) {
+    cudaFuncSetAttribute(attn_bwd_kv128_kernel<E>, cudaFuncAttributeMaxDynamicSharedMemorySize, kv_smem<E>);
     const int n_items = (S / T) * B;
     const int grid = n_items < num_sms() ? n_items : num_sms();
-    attn_bwd_kv128_kernel<<<grid, THREADS, KV_SMEM, st>>>(mq, mk, mv, md, mask, extra0, ndelta, gk, gv, S, H, B, scale,
-                                                        scale * LOG2E, clamp * LOG2E);
+    attn_bwd_kv128_kernel<E><<<grid, THREADS, kv_smem<E>, st>>>(mq, mk, mv, md, mask, extra0, ndelta, gk, gv, S, H, B, scale,
+                                                              scale * LOG2E, clamp * LOG2E, zsum);
     return after_launch("attn_bwd_kv128_kernel");
 }
+template int launch_bwd_kv128<__nv_bfloat16>(const CUtensorMap &, const CUtensorMap &, const CUtensorMap &,
+                                             const CUtensorMap &, const uint32_t *, const int32_t *, const float *,
+                                             const float *, __nv_bfloat16 *, __nv_bfloat16 *, int, int, int, float, float,
+                                             cudaStream_t);
+template int launch_bwd_kv128<__half>(const CUtensorMap &, const CUtensorMap &, const CUtensorMap &, const CUtensorMap &,
+                                      const uint32_t *, const int32_t *, const float *, const float *, __half *, __half *,
+                                      int, int, int, float, float, cudaStream_t);
 
 
-// 16 fp32 accumulator values (scaled) -> 16 bf16 = 32 contiguous bytes
-__device__ __forceinline__ void store_row16(__nv_bfloat16 *dst, const uint32_t (&r)[16], float s) {
+// 16 fp32 accumulator values (scaled) -> 16 bf16 / fp16 = 32 contiguous bytes
+template <typename E>
+__device__ __forceinline__ void store_row16(E *dst, const uint32_t (&r)[16], float s) {
 #pragma unroll
     for (int i = 0; i < 16; i += 8) {
         float t[8];
 #pragma unroll
         for (int u = 0; u < 8; ++u) t[u] = __uint_as_float(r[i + u]) * s;
-        Vec16<__nv_bfloat16>::store(dst + i, t);
+        Vec16<E>::store(dst + i, t);
     }
 }
 __device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&r)[16]) {
@@ -696,12 +715,14 @@ int launch_bwd_fused128(const CUtensorMap &mq, const CUtensorMap &mk, const CUte
 // ---------------------------------------------------------------------------------------------------------------------
 constexpr int Q_SMEM = 4 * TILE + 2 * ST * TILE + 256 + 1024;
 
+// E: element type; zsum is read by the fp16 instantiation only (row scales)
+template <typename E>
 __global__ void __launch_bounds__(THREADS, 1)
 attn_bwd_q128_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_k,
                      const __grid_constant__ CUtensorMap map_v, const __grid_constant__ CUtensorMap map_dys,
                      const uint32_t *__restrict__ mask, const int32_t *__restrict__ extra0,
-                     const float *__restrict__ ndelta, __nv_bfloat16 *__restrict__ dq, int S, int H, int B, float scale,
-                     float scale_log2, float clamp_log2) {
+                     const float *__restrict__ ndelta, E *__restrict__ dq, int S, int H, int B, float scale,
+                     float scale_log2, float clamp_log2, const float *__restrict__ zsum) {
     extern __shared__ unsigned char smem_raw[];
     const Smem sm = align_smem(smem_raw);
     const uint32_t s_q = sm.base, s_dy = s_q + 2 * TILE, s_k = s_dy + 2 * TILE, s_v = s_k + ST * TILE;
@@ -765,8 +786,8 @@ attn_bwd_q128_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
             }
         }
     } else if (warp == W_MMA) {
-        constexpr uint32_t id_s = idesc_bf16(T, T, 0, 0);     // S = Q K^T, dP' = dO' V^T
-        constexpr uint32_t id_a = idesc_bf16(T, D, 0, 1);     // dQ += dS K   (A in TMEM, K MN-major)
+        constexpr uint32_t id_s = idesc_of<E>(T, T, 0, 0);     // S = Q K^T, dP' = dO' V^T
+        constexpr uint32_t id_a = idesc_of<E>(T, D, 0, 1);     // dQ += dS K   (A in TMEM, K MN-major)
         const uint64_t dq0 = desc_kmajor(s_q, 0), ddy0 = desc_kmajor(s_dy, 0), dk0 = desc_kmajor(s_k, 0),
                        dv0 = desc_kmajor(s_v, 0), dkt0 = desc_mnmajor(s_k, 0, TILE);
         int g = 0, w = 0;
@@ -835,6 +856,7 @@ attn_bwd_q128_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
             const uint4 *mrow = reinterpret_cast<const uint4 *>(mask + grow * (S / 32));
             const float ex0 = (float)extra0[grow];
             const float nd = ndelta[grow];
+            const float nofs = is_f16<E> ? f16_bwd_nofs(zsum[grow]) : 0.0f;
             uint4 mw = __ldg(mrow);
             for (int j = 0; j < n_tiles; ++j, ++g) {
                 const uint4 mw_next = (j + 1 < n_tiles) ? __ldg(mrow + j + 1) : mw;
@@ -851,11 +873,11 @@ attn_bwd_q128_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
                 uint32_t pk[16];
                 const bool first = (j == 0 && cg == 0);
                 if (!warp_needs_clamp(r, mk.thr)) {
-                    if (first) bwdq_chunk32<true, false>(r, gr, X, mk, nd, ex0, pk);
-                    else bwdq_chunk32<false, false>(r, gr, X, mk, nd, ex0, pk);
+                    if (first) bwdq_chunk32<true, false, E>(r, gr, X, mk, nd, ex0, pk, nofs);
+                    else bwdq_chunk32<false, false, E>(r, gr, X, mk, nd, ex0, pk, nofs);
                 } else {
-                    if (first) bwdq_chunk32<true, true>(r, gr, X, mk, nd, ex0, pk);
-                    else bwdq_chunk32<false, true>(r, gr, X, mk, nd, ex0, pk);
+                    if (first) bwdq_chunk32<true, true, E>(r, gr, X, mk, nd, ex0, pk, nofs);
+                    else bwdq_chunk32<false, true, E>(r, gr, X, mk, nd, ex0, pk, nofs);
                 }
                 PROF(pf.lap(2);)
                 if (g >= 2) {                           // this dS buffer's previous tile has been consumed
@@ -1102,14 +1124,21 @@ attn_fwd128_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_const
 
 static int grid_for(int n_items) { return n_items < num_sms() ? n_items : num_sms(); }
 
+template <typename E>
 int launch_bwd_q128(const CUtensorMap &mq, const CUtensorMap &mk, const CUtensorMap &mv, const CUtensorMap &md,
-                    const uint32_t *mask, const int32_t *extra0, const float *ndelta, __nv_bfloat16 *gq, int B, int S,
-                    int H, float scale, float clamp, cudaStream_t st) {
-    cudaFuncSetAttribute(attn_bwd_q128_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, Q_SMEM);
-    attn_bwd_q128_kernel<<<grid_for((S / T) * B), THREADS, Q_SMEM, st>>>(mq, mk, mv, md, mask, extra0, ndelta, gq, S, H, B,
-                                                                        scale, scale * LOG2E, clamp * LOG2E);
+                    const uint32_t *mask, const int32_t *extra0, const float *ndelta, const float *zsum, E *gq, int B,
+                    int S, int H, float scale, float clamp, cudaStream_t st) {
+    cudaFuncSetAttribute(attn_bwd_q128_kernel<E>, cudaFuncAttributeMaxDynamicSharedMemorySize, Q_SMEM);
+    attn_bwd_q128_kernel<E><<<grid_for((S / T) * B), THREADS, Q_SMEM, st>>>(mq, mk, mv, md, mask, extra0, ndelta, gq, S, H, B,
+                                                                           scale, scale * LOG2E, clamp * LOG2E, zsum);
     return after_launch("attn_bwd_q128_kernel");
 }
+template int launch_bwd_q128<__nv_bfloat16>(const CUtensorMap &, const CUtensorMap &, const CUtensorMap &,
+                                            const CUtensorMap &, const uint32_t *, const int32_t *, const float *,
+                                            const float *, __nv_bfloat16 *, int, int, int, float, float, cudaStream_t);
+template int launch_bwd_q128<__half>(const CUtensorMap &, const CUtensorMap &, const CUtensorMap &, const CUtensorMap &,
+                                     const uint32_t *, const int32_t *, const float *, const float *, __half *, int, int,
+                                     int, float, float, cudaStream_t);
 
 int launch_fwd128(const CUtensorMap &mq, const CUtensorMap &mk, const CUtensorMap &mv, const uint32_t *mask,
                   const int32_t *extra0, __nv_bfloat16 *y, float *zsum, int B, int S, int H, float scale, float clamp,

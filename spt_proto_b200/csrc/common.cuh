@@ -1,6 +1,7 @@
 // Shared device/host helpers for libspt_b200 (sm_100a).  No torch headers anywhere in csrc/.
 #pragma once
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 
@@ -135,13 +136,40 @@ struct Vec16<__nv_bfloat16> {
     }
 };
 
+template <>
+struct Vec16<__half> {
+    static constexpr int N = 8;
+    __device__ __forceinline__ static void load(const __half *p, float (&o)[8]) {
+        uint4 v = *reinterpret_cast<const uint4 *>(p);
+        const uint32_t w[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+        for (int i = 0; i < 4; ++i) {  // fp16 -> fp32: exact
+            const float2 f = __half22float2(*reinterpret_cast<const __half2 *>(&w[i]));
+            o[2 * i] = f.x;
+            o[2 * i + 1] = f.y;
+        }
+    }
+    __device__ __forceinline__ static void store(__half *p, const float (&o)[8]) {
+        uint32_t w[4];
+#pragma unroll
+        for (int i = 0; i < 4; ++i) {
+            __half2 h = __floats2half2_rn(o[2 * i], o[2 * i + 1]);
+            w[i] = *reinterpret_cast<uint32_t *>(&h);
+        }
+        *reinterpret_cast<uint4 *>(p) = make_uint4(w[0], w[1], w[2], w[3]);
+    }
+};
+
 __device__ __forceinline__ float to_f32(float v) { return v; }
 __device__ __forceinline__ float to_f32(__nv_bfloat16 v) { return __bfloat162float(v); }
+__device__ __forceinline__ float to_f32(__half v) { return __half2float(v); }
 template <typename T>
 __device__ __forceinline__ T from_f32(float v);
 template <>
 __device__ __forceinline__ float from_f32<float>(float v) { return v; }
 template <>
 __device__ __forceinline__ __nv_bfloat16 from_f32<__nv_bfloat16>(float v) { return __float2bfloat16_rn(v); }
+template <>
+__device__ __forceinline__ __half from_f32<__half>(float v) { return __float2half_rn(v); }
 
 }  // namespace spt

@@ -273,6 +273,10 @@ __device__ __forceinline__ constexpr uint32_t idesc_bf16(int M, int N, int a_mn_
     return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)a_mn_major << 15) | ((uint32_t)b_mn_major << 16) |
            ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
 }
+// The same with A = B = fp16: the A / B format fields (bits 7-9, 10-12) are 0 for fp16
+__device__ __forceinline__ constexpr uint32_t idesc_fp16(int M, int N, int a_mn_major, int b_mn_major) {
+    return idesc_bf16(M, N, a_mn_major, b_mn_major) & ~((7u << 7) | (7u << 10));
+}
 
 // ---- host: tensor maps -----------------------------------------------------------------------------
 typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *,

@@ -19,9 +19,12 @@ from typing import List, Tuple
 
 import torch
 
-from ._lib import SPT_ATTN_Y_TRANSPOSED, SPT_BF16, SPT_F32, check, lib
+from ._lib import SPT_ATTN_Y_TRANSPOSED, SPT_BF16, SPT_F16, SPT_F32, check, lib
 
 _DTYPES = {torch.float32: SPT_F32, torch.bfloat16: SPT_BF16}
+# fp16 is taken by the PQ encode / train kernels and the fused attention only (not by the stage entry points)
+_PQ_DTYPES = {**_DTYPES, torch.float16: SPT_F16}
+_ATTN_DTYPES = {torch.bfloat16: SPT_BF16, torch.float16: SPT_F16}
 
 # softmax_backward_cuda computes the TRUE softmax gradient.  The shipped reference kernel clamps the row
 # dot product sum(y * dy) to >= 1e-9 (extension/softmax.cu:69), which is wrong whenever that sum is
@@ -54,6 +57,13 @@ def _float_code(x: torch.Tensor, name: str) -> int:
     code = _DTYPES.get(x.dtype)
     if code is None:
         raise RuntimeError(f"{name} must be type of torch.float32 or torch.bfloat16")
+    return code
+
+
+def _pq_code(x: torch.Tensor, name: str) -> int:
+    code = _PQ_DTYPES.get(x.dtype)
+    if code is None:
+        raise RuntimeError(f"{name} must be type of torch.float32, torch.bfloat16 or torch.float16")
     return code
 
 
@@ -135,7 +145,7 @@ def pq_encode(z: torch.Tensor, table: torch.Tensor) -> torch.Tensor:
     if not z.is_cuda or not z.is_contiguous():
         raise RuntimeError("z must be a contiguous CUDA tensor")
     _check_dim(table, 3, "table")
-    code = _float_code(z, "z")
+    code = _pq_code(z, "z")
     m, c, dc = table.shape
     if z.size(-1) != m * dc:
         raise RuntimeError("z last dim must equal n_subspaces * d_codeword")
@@ -155,7 +165,7 @@ def pq_encode_pair(z0: torch.Tensor, z1: torch.Tensor, table: torch.Tensor):
     if z0.shape != z1.shape or z0.dtype != z1.dtype:
         raise RuntimeError("z0 and z1 must have the same shape and dtype")
     _check_dim(table, 3, "table")
-    code = _float_code(z0, "z0")
+    code = _pq_code(z0, "z0")
     m, c, dc = table.shape
     if z0.size(-1) != m * dc:
         raise RuntimeError("z last dim must equal n_subspaces * d_codeword")
@@ -171,7 +181,7 @@ def pq_encode_pair(z0: torch.Tensor, z1: torch.Tensor, table: torch.Tensor):
 
 
 def pq_train_supported(z: torch.Tensor, table: torch.Tensor) -> bool:
-    return (z.is_cuda and z.dtype in _DTYPES and table.dim() == 3 and table.size(1) == 16 and table.size(2) == 8
+    return (z.is_cuda and z.dtype in _PQ_DTYPES and table.dim() == 3 and table.size(1) == 16 and table.size(2) == 8
             and table.size(0) <= 64 and z.size(-1) == table.size(0) * 8 and z.numel() > 0)
 
 
@@ -182,7 +192,7 @@ def pq_train_fwd(z: torch.Tensor, table32: torch.Tensor):
     zq = torch.empty((rows, m * dc), dtype=torch.float32, device=z.device)
     partial = torch.empty((lib.spt_pq_train_blocks(rows, m),), dtype=torch.float32, device=z.device)
     with _on_device(z):
-        check(lib.spt_pq_train_fwd(_p(z), _p(table32), _p(zq), _p(partial), rows, m, c, dc, _float_code(z, "z"), _stream(z)))
+        check(lib.spt_pq_train_fwd(_p(z), _p(table32), _p(zq), _p(partial), rows, m, c, dc, _pq_code(z, "z"), _stream(z)))
     return zq, partial.sum() / float(rows * m * dc)
 
 
@@ -195,7 +205,7 @@ def pq_train_bwd(z: torch.Tensor, table32: torch.Tensor, grad_zq, grad_loss: tor
     gl = grad_loss.reshape(1).float().contiguous()
     with _on_device(z):
         check(lib.spt_pq_train_bwd(_p(z), _p(table32), _p(grad_zq), _p(gl), _p(grad_z), _p(partial), rows, m, c, dc,
-                                   _float_code(z, "z"), _stream(z)))
+                                   _pq_code(z, "z"), _stream(z)))
     return grad_z, partial.sum(0)
 
 
@@ -493,41 +503,45 @@ def lookup_mask(query: torch.Tensor, key: torch.Tensor, sparse_coeff: int, want_
 
 
 def _check_attn(q, k, v):
+    """-> (B, S, d, H, dtype code): q, k, v of one shape and one dtype, bf16 or fp16."""
+    if q.dtype not in _ATTN_DTYPES:
+        raise RuntimeError("q must be type of torch.bfloat16 or torch.float16")
     for name, t in (("q", q), ("k", k), ("v", v)):
         _check_dim(t, q.dim(), name)
-        _check_type(t, torch.bfloat16, name)
+        _check_type(t, q.dtype, name)
     if q.shape != k.shape or q.shape != v.shape:
         raise RuntimeError("q, k, v must have the same shape")
     B, S, H = _heads(q, "q")
-    return B, S, q.size(-1), H
+    return B, S, q.size(-1), H, _ATTN_DTYPES[q.dtype]
 
 
 def sparse_attn_fwd(q, k, v, mask, extra0, scale: float, clamp: float = 10.0, reference_layout: bool = False):
-    """q, k, v: [B,S,d] head-major or [N,S,H,d] (native layer layout, no transposes) bf16
-    -> (y, same shape as q; zsum [B,S] fp32).  reference_layout: y's MEMORY is the shipped layer's y^T [B, d, S]
+    """q, k, v: [B,S,d] head-major or [N,S,H,d] (native layer layout, no transposes), all bf16 or all fp16
+    -> (y, same shape and dtype as q; zsum [B,S] fp32).  fp16 needs 0 <= clamp <= 10.  reference_layout: y's MEMORY is the shipped layer's y^T [B, d, S]
     (attention.py:139-142), returned viewed with q's shape.  See include/spt_b200.h."""
-    B, S, d, H = _check_attn(q, k, v)
+    B, S, d, H, code = _check_attn(q, k, v)
     y = torch.empty_like(q)
     zsum = torch.empty((B, S), dtype=torch.float32, device=q.device)
     with _on_device(q):
         check(lib.spt_sparse_attn_fwd_ex(_p(q), _p(k), _p(v), _p(mask), _p(extra0), _p(y), _p(zsum), B, S, d, H,
-                                         float(scale), float(clamp), SPT_BF16,
+                                         float(scale), float(clamp), code,
                                          SPT_ATTN_Y_TRANSPOSED if reference_layout else 0, _stream(q)))
     return y, zsum
 
 
 def sparse_attn_bwd(q, k, v, y, grad_y, mask, extra0, zsum, scale: float, clamp: float = 10.0,
                     reference_layout: bool = False):
-    """-> (grad_q, grad_k, grad_v) bf16.  reference_layout: y and grad_y are in the layout sparse_attn_fwd(...,
-    reference_layout=True) returned."""
-    B, S, d, H = _check_attn(q, k, v)
+    """-> (grad_q, grad_k, grad_v) in q's dtype.  reference_layout: y and grad_y are in the layout
+    sparse_attn_fwd(..., reference_layout=True) returned."""
+    B, S, d, H, code = _check_attn(q, k, v)
     _check_dim(grad_y, q.dim(), "grad_y")
-    _check_type(grad_y, torch.bfloat16, "grad_y")
+    _check_type(grad_y, q.dtype, "grad_y")
+    _check_type(y, q.dtype, "y")
     gq, gk, gv = torch.empty_like(q), torch.empty_like(k), torch.empty_like(v)
     ws = _workspace(lib.spt_sparse_attn_bwd_workspace_bytes(B, S), q)
     with _on_device(q):
         check(lib.spt_sparse_attn_bwd_ex(_p(q), _p(k), _p(v), _p(y), _p(grad_y), _p(mask), _p(extra0), _p(zsum),
-                                         _p(gq), _p(gk), _p(gv), _p(ws), B, S, d, H, float(scale), float(clamp), SPT_BF16,
+                                         _p(gq), _p(gk), _p(gv), _p(ws), B, S, d, H, float(scale), float(clamp), code,
                                          SPT_ATTN_Y_TRANSPOSED if reference_layout else 0, _stream(q)))
     return gq, gk, gv
 

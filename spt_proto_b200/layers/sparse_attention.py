@@ -62,9 +62,9 @@ class _SparseV2Mixin:
     # False is the opt-in corrected layout (identical to the reference's dense VanillaAttention on
     # the same pattern).  Also a constructor keyword.  INTEGRATION.md, "Output layout".
     reference_output_layout: bool = True
-    # bf16, d_head 64, 80 or 128, S % 128 == 0 on CUDA: run lookup -> bitmask -> fused masked-dense attention on
-    # the tensor cores instead of the stage chain (same result up to bf16 rounding; DESIGN.md sec. 5).
-    # False keeps the stage chain for every shape.
+    # bf16 or fp16, d_head 64, 80 or 128, S % 128 == 0 on CUDA: run lookup -> bitmask -> fused masked-dense attention
+    # on the tensor cores instead of the stage chain (same result up to bf16 / fp16 rounding; DESIGN.md sec. 5).
+    # False keeps the stage chain for every shape (fp16 operands run it in fp32 and the result is returned in fp16).
     use_fused: bool = True
     # The reference reads its device-side `trigger` buffer with `is_nonzero()` on every forward
     # (attention.py:98) — a device->host synchronisation per layer call.  None (default) keeps that
@@ -103,7 +103,7 @@ class _SparseV2Mixin:
         return x.view(-1, x.size(-2), x.size(-1))
 
     def _fused_ok(self, q) -> bool:
-        return (self.use_fused and q.is_cuda and q.dtype == torch.bfloat16 and q.size(-1) in (64, 80, 128)
+        return (self.use_fused and q.is_cuda and q.dtype in (torch.bfloat16, torch.float16) and q.size(-1) in (64, 80, 128)
                 and q.size(1) % 128 == 0 and q.size(1) % self.sparse_coeff == 0
                 and (q.size(1) // self.sparse_coeff) % 4 == 0 and q.size(1) // self.sparse_coeff >= 8)
 
@@ -147,6 +147,12 @@ class _SparseV2Mixin:
         values = kernels.sddmm_softmax(indptr, csr_indices, q, k, self.scaling, 10.0)
         return indptr, csr_indices, values
 
+    def _stage_forward(self, q, k, v, attn_mask):
+        # the stage kernels take fp32 / bf16: fp16 operands run the chain in fp32 and the result goes back to fp16
+        if q.dtype == torch.float16:
+            return VanillaAttention.forward(self, q.float(), k.float(), v.float(), attn_mask).to(q.dtype)
+        return VanillaAttention.forward(self, q, k, v, attn_mask)
+
     def _apply_attn(self, attn, v):
         v_size = v.size()
         indptr, indices, values = attn
@@ -175,7 +181,7 @@ class SparseVanillaAttentionV2(_SparseV2Mixin, VanillaAttention):
             self.last_path = "fused"
             return self._fused_forward(q, k, v)
         self.last_path = "stage"
-        return VanillaAttention.forward(self, q, k, v, attn_mask)
+        return self._stage_forward(q, k, v, attn_mask)
 
 
 class SparseRotaryAttentionV2(_SparseV2Mixin, RotaryAttention):
@@ -199,4 +205,4 @@ class SparseRotaryAttentionV2(_SparseV2Mixin, RotaryAttention):
             # operands in the input's own dtype
             return self._fused_forward(self._rotate(q).to(q.dtype), self._rotate(k).to(k.dtype), v)
         self.last_path = "stage"
-        return VanillaAttention.forward(self, q, k, v, attn_mask)
+        return self._stage_forward(q, k, v, attn_mask)
