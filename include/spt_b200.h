@@ -254,6 +254,48 @@ int spt_sparse_attn_bwd(const void *q, const void *k, const void *v, const void 
                         const uint32_t *mask, const int32_t *extra0, const float *zsum, void *grad_q,
                         void *grad_k, void *grad_v, void *workspace, int B, int S, int d, int H,
                         float scale, float clamp, int dtype, spt_stream_t stream);
+/* ------------------------------------------------------------------------------------------
+ * Packed variable-length sequences (DESIGN.md section 4.5).  n_seq sequences of lengths S_i are
+ * concatenated along the token axis, T = sum S_i; cu_seqlens int32 [n_seq + 1] (device) holds the
+ * offsets, cu[0] = 0, cu[n_seq] = T.  Sequence i (rows cu[i] .. cu[i+1]) gets exactly what the
+ * fixed-length calls give for it alone as a batch of one: keys are relative to its first token
+ * (key 0 = that token, which zero padding aliases), attention is causal from there.  Needs
+ * S_i % 32 == 0, S_i % (4 sparse_coeff) == 0, S_i >= 8 sparse_coeff, S_i <= max_seqlen; S_i and
+ * cu[i] need not be multiples of 128.  Nothing synchronises with the host (graph-capturable).
+ *
+ * spt_varlen_worklist: cu_seqlens -> work list `work` (spt_varlen_worklist_bytes(n_seq, T), 16-byte
+ *   aligned): one item per (sequence, 128-row tile), heaviest tiles first.  Built once and passed
+ *   to the lookup, the forward and the backward.  Every sequence is clamped to [0, T] and to
+ *   max_seqlen on the device, so a bad device-side cu_seqlens cannot send a kernel outside its
+ *   tensors (validate host-side offsets before the copy).
+ * spt_lookup_mask_varlen_fwd: codes [T, H, m] (m = 8, 10 or 16) -> mask [H, T, Wm] uint32,
+ *   Wm = 4 ceil(max_seqlen / 128), lane-major words relative to the sequence start (words past a
+ *   row's sequence are zero), extra0 [H, T]; nnz_i = S_i / sparse_coeff.  workspace:
+ *   spt_lookup_mask_varlen_workspace_bytes.  spt_lookup_mask_varlen_max_seqlen(m) is the longest
+ *   max_seqlen the mask-only kernels take at m (0: m not supported).
+ * spt_sparse_attn_varlen_fwd / _bwd: as the _ex calls on q, k, v [T, H, d]; zsum [H, T].
+ *   SPT_ATTN_Y_TRANSPOSED: sequence i's y (and grad_y) memory is its own y_i^T [H, d, S_i] at
+ *   token offset cu[i] — the reference layer's layout for that sequence alone.
+ * ------------------------------------------------------------------------------------------ */
+size_t spt_varlen_worklist_bytes(int n_seq, int T);
+int spt_varlen_worklist(const int32_t *cu_seqlens, int n_seq, int T, int max_seqlen, void *work,
+                        spt_stream_t stream);
+size_t spt_lookup_mask_varlen_workspace_bytes(int n_seq, int T, int H, int m);
+int spt_lookup_mask_varlen_max_seqlen(int m);
+int spt_lookup_mask_varlen_fwd(const int32_t *query_codes, const int32_t *key_codes, const void *work,
+                               uint32_t *mask, int32_t *extra0, void *workspace, int n_seq, int T,
+                               int max_seqlen, int H, int m, int sparse_coeff, spt_stream_t stream);
+int spt_sparse_attn_varlen_fwd(const void *q, const void *k, const void *v, const uint32_t *mask,
+                               const int32_t *extra0, void *y, float *zsum, const void *work, int n_seq,
+                               int T, int max_seqlen, int d, int H, float scale, float clamp, int dtype,
+                               int flags, spt_stream_t stream);
+size_t spt_sparse_attn_varlen_bwd_workspace_bytes(int T, int H);
+int spt_sparse_attn_varlen_bwd(const void *q, const void *k, const void *v, const void *y,
+                               const void *grad_y, const uint32_t *mask, const int32_t *extra0,
+                               const float *zsum, void *grad_q, void *grad_k, void *grad_v,
+                               void *workspace, const void *work, int n_seq, int T, int max_seqlen,
+                               int d, int H, float scale, float clamp, int dtype, int flags,
+                               spt_stream_t stream);
 /* diagnostics: in-kernel phase timers of the attention kernels, 3 kernels x 16 slots of summed clock64() deltas
  * (zeros and return value 0 unless the library was built with -DSPT_ATTN_PROF); reset != 0 clears them */
 int spt_debug_attn_prof(unsigned long long *out48, int reset);

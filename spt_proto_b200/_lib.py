@@ -88,6 +88,15 @@ def _load() -> ctypes.CDLL:
     sig["spt_softmax_clamp_bwd"] = (i32, [vp] * 6 + [i32, i32, i64, f32, f32, i32, vp])
     sig["spt_swap_dims12"] = (i32, [vp, vp, i64, i64, i64, i64, vp])
     sig["spt_transpose_last2"] = (i32, [vp, vp, i64, i32, i32, i32, vp])
+    # packed variable-length sequences
+    sig["spt_varlen_worklist_bytes"] = (sz, [i32, i32])
+    sig["spt_varlen_worklist"] = (i32, [vp, i32, i32, i32, vp, vp])
+    sig["spt_lookup_mask_varlen_workspace_bytes"] = (sz, [i32, i32, i32, i32])
+    sig["spt_lookup_mask_varlen_max_seqlen"] = (i32, [i32])
+    sig["spt_lookup_mask_varlen_fwd"] = (i32, [vp] * 6 + [i32] * 6 + [vp])
+    sig["spt_sparse_attn_varlen_fwd"] = (i32, [vp] * 8 + [i32, i32, i32, i32, i32, f32, f32, i32, i32, vp])
+    sig["spt_sparse_attn_varlen_bwd_workspace_bytes"] = (sz, [i32, i32])
+    sig["spt_sparse_attn_varlen_bwd"] = (i32, [vp] * 13 + [i32, i32, i32, i32, i32, f32, f32, i32, i32, vp])
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)  # AttributeError => header/library mismatch, fail loudly
         fn.restype = res

@@ -56,6 +56,16 @@ __device__ __forceinline__ void tma_other(uint32_t dst, const CUtensorMap *map, 
 }
 constexpr float LOG2E = 1.4426950408889634f;
 
+// Packed variable-length batches (the VARLEN instantiations): q, k, v are [1, T, H, D] and every CTA takes one item of
+// the work list built by spt_varlen_worklist, {first token of its sequence, sequence length (a multiple of 32), 128-row
+// tile index, word offset of the sequence's key bitmaps}.  Items [0, *count) are in descending tile order; CTAs past
+// *count exit.  Mask rows are `mwords` 32-bit words wide; per-row data is head-major [H, T].
+struct Varlen {
+    const int4 *items;
+    const int *count;
+    int mwords;
+};
+
 __device__ __forceinline__ float ex2(float x) {
     float y;
     asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));

@@ -46,12 +46,15 @@ namespace attn_tc {
 // ---------------------------------------------------------------------------------------------------
 
 // fp16 (T = __half): kg is the key tensor itself (the row scale reads key row 0 of the head); unused in bf16.
-template <int D, typename T>
+// VARLEN: packed sequences (S = T, H heads, grid (H, work-list capacity)); rows at or past the sequence end read
+// neutral per-row data and store nothing.
+template <int D, typename T, bool VARLEN = false>
 __global__ void __launch_bounds__(THREADS, Dim<D>::CTAS)
 attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_k,
                    const __grid_constant__ CUtensorMap map_v, const uint32_t *__restrict__ mask,
                    const int32_t *__restrict__ extra0, T *__restrict__ y, float *__restrict__ zsum, int S,
-                   int H, float scale_log2, float clamp_log2, int y_transposed, const T *__restrict__ kg) {
+                   int H, float scale_log2, float clamp_log2, int y_transposed, const T *__restrict__ kg,
+                   const Varlen vl = {}) {
     constexpr int OWN_BYTES = Dim<D>::OWN_BYTES, T_BYTES = Dim<D>::T_BYTES, OWN_SUB = Dim<D>::OWN_SUB, T_SUB = Dim<D>::T_SUB,
                   TMEM_COLS = Dim<D>::TMEM_COLS, DP = Dim<D>::DP;
     constexpr int NBUF = 3;                            // score buffers
@@ -74,11 +77,16 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_const
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     // grid (heads, query tiles): blockIdx.x (fastest) = head, so the heaviest (last) query tile of EVERY head is scheduled
     // before any lighter tile — the launch ends on the lightest CTAs
-    const int tile = gridDim.y - 1 - blockIdx.y;
+    int tile = gridDim.y - 1 - blockIdx.y, start = 0, len = S;
+    if constexpr (VARLEN) {
+        if ((int)blockIdx.y >= *vl.count) return;
+        const int4 it = vl.items[blockIdx.y];
+        start = it.x, len = it.y, tile = it.z;
+    }
     const int b = blockIdx.x;
     const int m0 = tile * BM;
-    const int n_tiles = (m0 + BM) / BN;                // key tiles 0 .. (causal)
-    const int hn = b / H, hh = b % H;
+    const int n_tiles = VARLEN ? (min(m0 + BM, len) + BN - 1) / BN : (m0 + BM) / BN;   // key tiles 0 .. (causal)
+    const int hn = VARLEN ? 0 : b / H, hh = VARLEN ? b : b % H;
 
     if (threadIdx.x == 0) {
         mbar_init(q_full, 1);
@@ -107,16 +115,16 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_const
         // ===== TMA producer =====
         if (lane == 0) {
             mbar_expect_tx(q_full, OWN_BYTES);
-            tma_owner<D>(s_q, &map_q, q_full, hh, m0, hn);
+            tma_owner<D>(s_q, &map_q, q_full, hh, start + m0, hn);
             for (int j = 0; j < n_tiles; ++j) {
                 const int st = j % STAGES;
                 const uint32_t ph = (j / STAGES) & 1;
                 mbar_wait(k_empty(st), ph ^ 1);
                 mbar_expect_tx(k_full(st), T_BYTES);
-                tma_other<D>(s_k + st * T_BYTES, &map_k, k_full(st), hh, j * BN, hn);
+                tma_other<D>(s_k + st * T_BYTES, &map_k, k_full(st), hh, start + j * BN, hn);
                 mbar_wait(v_empty(st), ph ^ 1);
                 mbar_expect_tx(v_full(st), T_BYTES);
-                tma_other<D>(s_v + st * T_BYTES, &map_v, v_full(st), hh, j * BN, hn);
+                tma_other<D>(s_v + st * T_BYTES, &map_v, v_full(st), hh, start + j * BN, hn);
             }
         }
     } else if (warp == 9) {
@@ -183,9 +191,10 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_const
         const int quarter = warp & 3, half = warp >> 2;
         const int rt = quarter * 32 + lane;               // row inside the tile
         const int row = m0 + rt;
-        const size_t grow = (size_t)b * S + row;
-        const uint4 *mrow = reinterpret_cast<const uint4 *>(mask + grow * (S / 32));
-        const float ex0 = (float)extra0[grow];
+        const bool live = !VARLEN || row < len;           // warp-uniform (len is a multiple of 32)
+        const size_t grow = (size_t)b * S + start + row;
+        const uint4 *mrow = reinterpret_cast<const uint4 *>(mask + grow * (VARLEN ? vl.mwords : S / 32));
+        const float ex0 = live ? (float)extra0[grow] : 0.0f;
         const uint32_t lane_base = tmem_base + ((uint32_t)(quarter * 32) << 16);
         // Ping-pong: warpgroup `half` (warps 4 half .. 4 half + 3, one per scheduler) owns the key tiles j = half (mod 2) and
         // score buffer `half`; a thread processes ALL 64 columns of its row as two 32-column chunks.  The two groups of a
@@ -195,14 +204,14 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_const
         // warp of the CTA on every tile).
         uint64_t sum2 = pk2(0.0f, 0.0f);
         const MathK mk = make_math(scale_log2, clamp_log2);
-        uint4 mw = __ldg(mrow);
+        uint4 mw = live ? __ldg(mrow) : make_uint4(0, 0, 0, 0);
         float nofs = 0.0f;                                // fp16: -o of this row
         if constexpr (is_f16<T>) {
             // o = max(floor(c log2 e) - 15, floor(log2 t0) - 14), t0 = (1 + ex0) exp(clamp(scale q.k_0)) the key-0 term:
             // t0 2^-o < 2^15 and e^c 2^-o < 2^16, so no element can overflow, and a row whose scores are all low keeps
             // normal fp16 values.  q.k_0 in fp32 from the row's Q in shared memory and key row 0 of the head.
             mbar_wait(q_full, 0);
-            const T *k0 = kg + ((size_t)hn * S * H + hh) * D;
+            const T *k0 = VARLEN ? kg + ((size_t)start * H + hh) * D : kg + ((size_t)hn * S * H + hh) * D;   // the sequence's key 0
             float dot = 0.0f;
 #pragma unroll
             for (int c = 0; c < D / 8; ++c) {              // 16-byte chunk c: sub-tile c / 8, 128-byte swizzled by the row
@@ -223,7 +232,7 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_const
         PROF(Prof pf; pf.start(); const long long t0 = pf.last; pf.t[6] = t0 - t_entry;)
         for (int j = half, it = 0; j < n_tiles; j += 2, ++it) {
             // tile j = keys 64 j .. 64 j + 63 = bits 16 half .. 16 half + 15 of the lane-major words of key group it = j >> 1
-            const uint4 mw_next = (j + 2 < n_tiles) ? __ldg(mrow + it + 1) : mw;
+            const uint4 mw_next = (j + 2 < n_tiles && live) ? __ldg(mrow + it + 1) : mw;
             const uint32_t buf = lane_base + COL_S + (uint32_t)(j % NBUF) * BN;
             mbar_wait(s_full(j % NBUF), (j / NBUF) & 1);
             PROF(pf.lap(0);)
@@ -265,17 +274,18 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_const
         if constexpr (is_f16<T>) {                        // sum of e 2^-o; Z = sum 2^o (exact)
             const float rs = __uint_as_float((uint32_t)(127 + (int)nofs) << 23);     // 2^-o
             sum = fmaxf(s_part[rt] + s_part[BM + rt], 1e-9f * rs);
-            if (half == 0) zsum[grow] = sum * __uint_as_float((uint32_t)(127 - (int)nofs) << 23);
+            if (half == 0 && live) zsum[grow] = sum * __uint_as_float((uint32_t)(127 - (int)nofs) << 23);
             inv = 1.0f / sum;
         } else {
             sum = fmaxf(s_part[rt] + s_part[BM + rt], 1e-9f);
-            if (half == 0) zsum[grow] = sum;
+            if (half == 0 && live) zsum[grow] = sum;
             inv = 1.0f / sum;
         }
         mbar_wait(o_full, 0);
         fence_after_sync();
-        if (!y_transposed) {
-            T *dst = y + (((size_t)hn * S + row) * H + hh) * D;
+        if (!live) {
+        } else if (!y_transposed) {
+            T *dst = y + (((size_t)hn * S + start + row) * H + hh) * D;
             out_chunks<D>(half, [&](int col, auto w) {
                 uint32_t r[32];
                 tmem_ld32(lane_base + COL_O + col, r);
@@ -284,12 +294,14 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_const
         } else {
             // the shipped reference layer's output layout (attention.py:139-142): y^T [B, D, S] memory; a warp's 32
             // consecutive rows of one feature are 64 contiguous bytes
+            // (VARLEN: each sequence's own y^T [H, D, len], at token offset start)
             out_chunks<D>(half, [&](int col, auto w) {
-                T *dst = y + ((size_t)b * D + col) * S + row;
+                T *dst = VARLEN ? y + (size_t)start * H * D + ((size_t)b * D + col) * len + row : y + ((size_t)b * D + col) * S + row;
+                const size_t stride = VARLEN ? len : S;
                 uint32_t r[32];
                 tmem_ld32(lane_base + COL_O + col, r);
 #pragma unroll
-                for (int i = 0; i < decltype(w)::value; ++i) dst[(size_t)i * S] = out_elem(__uint_as_float(r[i]) * inv, dst);
+                for (int i = 0; i < decltype(w)::value; ++i) dst[(size_t)i * stride] = out_elem(__uint_as_float(r[i]) * inv, dst);
             });
         }
         PROF(pf.t[7] = clock64() - t_loop_end; pf.flush(0, 0, threadIdx.x == 0);)
@@ -347,24 +359,34 @@ attn_bwd_prep_kernel(const T *__restrict__ dy, const T *__restrict__ y,
 
 // The same for dO and y in the reference layer's output layout (y^T, dO^T: [B, D, S] memory): a block transposes a
 // [D] x [64 rows] tile of each through shared memory; dO' is written in the standard [N, S, H, D] layout the TMA maps read.
-template <int D, typename T>
+// VARLEN: block x = one 64-row half of a work-list item; a sequence's y^T / dO^T is [H, D, len] at token offset start.
+template <int D, typename T, bool VARLEN = false>
 __global__ void __launch_bounds__(256)
 attn_bwd_prep_t_kernel(const T *__restrict__ dyt, const T *__restrict__ yt,
                        const float *__restrict__ zsum, float *__restrict__ delta, T *__restrict__ dys, int S,
-                       int H) {
+                       int H, const Varlen vl = {}) {
     constexpr int TR = 64, LD = TR + 8;
     __shared__ __align__(16) T s_dy[D][LD];
     __shared__ __align__(16) T s_y[D][LD];
-    const int b = blockIdx.y, r0 = blockIdx.x * TR;
-    const size_t base = (size_t)b * D * S + r0;
+    int r0 = blockIdx.x * TR, start = 0, len = S;
+    if constexpr (VARLEN) {
+        if ((int)(blockIdx.x >> 1) >= *vl.count) return;
+        const int4 it = vl.items[blockIdx.x >> 1];
+        start = it.x, len = it.y, r0 = it.z * 128 + (blockIdx.x & 1) * TR;
+        if (r0 >= len) return;
+    }
+    const int b = blockIdx.y;
+    const size_t base = VARLEN ? (size_t)start * H * D + (size_t)b * D * len + r0 : (size_t)b * D * S + r0;
+    const size_t ld = VARLEN ? len : S;
     constexpr int EPT = D / 4;                       // features per thread
     // the 16-byte row chunks of feature e sit at chunk index (c / 8) ^ (e / EPT): the four threads of a row read the
     // same column of four features 16 * LD elements apart (the same bank without the swizzle: 4-way conflicts on
     // every one of the 2 * EPT reads)
     for (int id = threadIdx.x; id < D * (TR / 8); id += 256) {
         const int e = id / (TR / 8), c = (id % (TR / 8)) * 8, cs = (((id % (TR / 8)) ^ (e / EPT)) & (TR / 8 - 1)) * 8;
-        *reinterpret_cast<uint4 *>(&s_dy[e][cs]) = *reinterpret_cast<const uint4 *>(dyt + base + (size_t)e * S + c);
-        *reinterpret_cast<uint4 *>(&s_y[e][cs]) = *reinterpret_cast<const uint4 *>(yt + base + (size_t)e * S + c);
+        if (VARLEN && r0 + c >= len) continue;       // rows past the sequence end (the rows of those threads store nothing)
+        *reinterpret_cast<uint4 *>(&s_dy[e][cs]) = *reinterpret_cast<const uint4 *>(dyt + base + (size_t)e * ld + c);
+        *reinterpret_cast<uint4 *>(&s_y[e][cs]) = *reinterpret_cast<const uint4 *>(yt + base + (size_t)e * ld + c);
     }
     __syncthreads();
     const int r = threadIdx.x >> 2, qd = threadIdx.x & 3;
@@ -377,10 +399,11 @@ attn_bwd_prep_t_kernel(const T *__restrict__ dyt, const T *__restrict__ yt,
         acc = fmaf(a[i], to_f32(s_y[qd * EPT + i][rs]), acc);
     }
     acc = group_sum<4>(acc);
-    const size_t grow = (size_t)b * S + r0 + r;
+    if (VARLEN && r0 + r >= len) return;
+    const size_t grow = (size_t)b * S + start + r0 + r;
     const float inv = prep_inv(zsum[grow], is_f16<T>);
-    const int hn = b / H, hh = b % H;
-    T *dst = dys + (((size_t)hn * S + r0 + r) * H + hh) * D + qd * EPT;
+    const int hn = VARLEN ? 0 : b / H, hh = VARLEN ? b : b % H;
+    T *dst = dys + (((size_t)hn * S + start + r0 + r) * H + hh) * D + qd * EPT;
     if constexpr (EPT % 8 == 0) {
 #pragma unroll
         for (int i = 0; i < EPT; i += 8) {
@@ -406,14 +429,14 @@ attn_bwd_prep_t_kernel(const T *__restrict__ dyt, const T *__restrict__ yt,
 // registers, so the tensor core computes the next tile's scores under this tile's exp math.
 // ---------------------------------------------------------------------------------------------------
 
-// fp16: zsum gives the row scales (read by the fp16 instantiations only)
-template <int D, typename T>
+// fp16: zsum gives the row scales (read by the fp16 instantiations only).  VARLEN: see the forward.
+template <int D, typename T, bool VARLEN = false>
 __global__ void __launch_bounds__(THREADS, Dim<D>::CTAS)
 attn_bwd_q_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_k,
                      const __grid_constant__ CUtensorMap map_v, const __grid_constant__ CUtensorMap map_dys,
                      const uint32_t *__restrict__ mask, const int32_t *__restrict__ extra0,
                      const float *__restrict__ delta, T *__restrict__ dq, int S, int H, float scale,
-                     float scale_log2, float clamp_log2, const float *__restrict__ zsum) {
+                     float scale_log2, float clamp_log2, const float *__restrict__ zsum, const Varlen vl = {}) {
     constexpr int OWN_BYTES = Dim<D>::OWN_BYTES, T_BYTES = Dim<D>::T_BYTES, OWN_SUB = Dim<D>::OWN_SUB, T_SUB = Dim<D>::T_SUB,
                   TMEM_COLS = Dim<D>::TMEM_COLS, DP = Dim<D>::DP;
     extern __shared__ unsigned char smem_raw[];
@@ -431,11 +454,16 @@ attn_bwd_q_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
     uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(bars + 7 + 2 * STAGES);
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int tile = gridDim.y - 1 - blockIdx.y;      // grid (heads, tiles): every head's heaviest tile first (see the forward)
+    int tile = gridDim.y - 1 - blockIdx.y, start = 0, len = S;   // grid (heads, tiles): every head's heaviest tile first (see the forward)
+    if constexpr (VARLEN) {
+        if ((int)blockIdx.y >= *vl.count) return;
+        const int4 it = vl.items[blockIdx.y];
+        start = it.x, len = it.y, tile = it.z;
+    }
     const int b = blockIdx.x;
     const int m0 = tile * BM;
-    const int n_tiles = (m0 + BM) / BN;
-    const int hn = b / H, hh = b % H;
+    const int n_tiles = VARLEN ? (min(m0 + BM, len) + BN - 1) / BN : (m0 + BM) / BN;
+    const int hn = VARLEN ? 0 : b / H, hh = VARLEN ? b : b % H;
 
     if (threadIdx.x == 0) {
         mbar_init(own_full, 1);
@@ -461,14 +489,14 @@ attn_bwd_q_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
     if (warp == 8) {
         if (lane == 0) {
             mbar_expect_tx(own_full, 2 * OWN_BYTES);
-            tma_owner<D>(s_q, &map_q, own_full, hh, m0, hn);
-            tma_owner<D>(s_dy, &map_dys, own_full, hh, m0, hn);
+            tma_owner<D>(s_q, &map_q, own_full, hh, start + m0, hn);
+            tma_owner<D>(s_dy, &map_dys, own_full, hh, start + m0, hn);
             for (int j = 0; j < n_tiles; ++j) {
                 const int st = j % STAGES;
                 mbar_wait(kv_empty(st), ((j / STAGES) & 1) ^ 1);
                 mbar_expect_tx(kv_full(st), 2 * T_BYTES);
-                tma_other<D>(s_k + st * T_BYTES, &map_k, kv_full(st), hh, j * BN, hn);
-                tma_other<D>(s_v + st * T_BYTES, &map_v, kv_full(st), hh, j * BN, hn);
+                tma_other<D>(s_k + st * T_BYTES, &map_k, kv_full(st), hh, start + j * BN, hn);
+                tma_other<D>(s_v + st * T_BYTES, &map_v, kv_full(st), hh, start + j * BN, hn);
             }
         }
     } else if (warp == 9) {
@@ -525,20 +553,21 @@ attn_bwd_q_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
     } else {
         const int quarter = warp & 3, half = warp >> 2;
         const int row = m0 + quarter * 32 + lane;
-        const size_t grow = (size_t)b * S + row;
-        const uint4 *mrow = reinterpret_cast<const uint4 *>(mask + grow * (S / 32));
-        const float ex0 = (float)extra0[grow];
-        const float dl = delta[grow];
-        const float nofs = is_f16<T> ? f16_bwd_nofs(zsum[grow]) : 0.0f;
+        const bool live = !VARLEN || row < len;           // warp-uniform (len is a multiple of 32)
+        const size_t grow = (size_t)b * S + start + row;
+        const uint4 *mrow = reinterpret_cast<const uint4 *>(mask + grow * (VARLEN ? vl.mwords : S / 32));
+        const float ex0 = live ? (float)extra0[grow] : 0.0f;
+        const float dl = live ? delta[grow] : 0.0f;
+        const float nofs = (is_f16<T> && live) ? f16_bwd_nofs(zsum[grow]) : 0.0f;
         const uint32_t lane_base = tmem_base + ((uint32_t)(quarter * 32) << 16);
         const MathK mk = make_math(scale_log2, clamp_log2);
-        uint4 mw = __ldg(mrow);
+        uint4 mw = live ? __ldg(mrow) : make_uint4(0, 0, 0, 0);
         PROF(Prof pf; pf.start(); const long long t0 = pf.last;)
         // Ping-pong (see the forward kernel): warpgroup `half` owns the key tiles j = half (mod 2) and dS buffer `half`; a
         // thread processes all 64 columns of its row as two 32-column chunks, and releases the (single) score buffer as
         // soon as the second chunk is in registers.
         for (int j = half, it = 0; j < n_tiles; j += 2, ++it) {
-            const uint4 mw_next = (j + 2 < n_tiles) ? __ldg(mrow + it + 1) : mw;
+            const uint4 mw_next = (j + 2 < n_tiles && live) ? __ldg(mrow + it + 1) : mw;
             mbar_wait(sc_full(half), it & 1);
             PROF(pf.lap(0);)
             fence_after_sync();
@@ -575,12 +604,13 @@ attn_bwd_q_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
         PROF(pf.t[5] = clock64() - t0; pf.t[4] = n_tiles / 2; pf.flush(1, 0, threadIdx.x == 0);)
         mbar_wait(acc_full, 0);
         fence_after_sync();
-        T *dst = dq + (((size_t)hn * S + row) * H + hh) * D;
-        out_chunks<D>(half, [&](int col, auto w) {
-            uint32_t r[32];
-            tmem_ld32(lane_base + COL_DQ + col, r);
-            store_row_n<decltype(w)::value>(dst + col, r, scale);
-        });
+        T *dst = dq + (((size_t)hn * S + start + row) * H + hh) * D;
+        if (live)
+            out_chunks<D>(half, [&](int col, auto w) {
+                uint32_t r[32];
+                tmem_ld32(lane_base + COL_DQ + col, r);
+                store_row_n<decltype(w)::value>(dst + col, r, scale);
+            });
     }
     fence_before_sync();
     __syncthreads();
@@ -598,13 +628,15 @@ attn_bwd_q_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
 // Per-row quantities of the 64 query rows (mask words of this key group, delta', extra0) are staged in
 // shared memory by the producer warp, one slot per pipeline stage (fp16: also the rows' -o, from zsum).
 // ---------------------------------------------------------------------------------------------------
-template <int D, typename T>
+// VARLEN: see the forward.
+template <int D, typename T, bool VARLEN = false>
 __global__ void __launch_bounds__(THREADS, Dim<D>::CTAS)
 attn_bwd_kv_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_k,
                       const __grid_constant__ CUtensorMap map_v, const __grid_constant__ CUtensorMap map_dys,
                       const uint32_t *__restrict__ mask, const int32_t *__restrict__ extra0,
                       const float *__restrict__ delta, T *__restrict__ dk, T *__restrict__ dv,
-                      int S, int H, float scale, float scale_log2, float clamp_log2, const float *__restrict__ zsum) {
+                      int S, int H, float scale, float scale_log2, float clamp_log2, const float *__restrict__ zsum,
+                      const Varlen vl = {}) {
     constexpr int OWN_BYTES = Dim<D>::OWN_BYTES, T_BYTES = Dim<D>::T_BYTES, OWN_SUB = Dim<D>::OWN_SUB, T_SUB = Dim<D>::T_SUB,
                   TMEM_COLS = Dim<D>::TMEM_COLS, DP = Dim<D>::DP;
     extern __shared__ unsigned char smem_raw[];
@@ -623,14 +655,21 @@ attn_bwd_kv_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_co
     uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(bars + 6 + 2 * STAGES);
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int kt = blockIdx.y;                         // key tile (early key tiles are the heaviest); grid (heads, tiles):
-    const int b = blockIdx.x;                          // every head's heaviest tile first (see the forward)
+    int kt = blockIdx.y, start = 0, len = S;           // key tile (early key tiles are the heaviest); grid (heads, tiles):
+    if constexpr (VARLEN) {                            // every head's heaviest tile first (see the forward)
+        if ((int)blockIdx.y >= *vl.count) return;
+        const int4 it = vl.items[blockIdx.y];
+        // the work list puts the query tiles with the most keys first; mirrored inside each sequence, its first items are
+        // the key tiles with the most query rows at and below them
+        start = it.x, len = it.y, kt = (len + BM - 1) / BM - 1 - it.z;
+    }
+    const int b = blockIdx.x;
     const int n0 = kt * BM;
     const int j0 = n0 / BN;                            // first query tile that can see these keys
-    const int n_tiles = S / BN - j0;
-    const int hn = b / H, hh = b % H;
-    const size_t head = (size_t)b * S;
-    const int words = S / 32;
+    const int n_tiles = (VARLEN ? (len + BN - 1) / BN : S / BN) - j0;
+    const int hn = VARLEN ? 0 : b / H, hh = VARLEN ? b : b % H;
+    const size_t head = (size_t)b * S + start;
+    const int words = VARLEN ? vl.mwords : S / 32;
 
     if (threadIdx.x == 0) {
         mbar_init(own_full, 1);
@@ -657,8 +696,8 @@ attn_bwd_kv_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_co
     if (warp == 8) {
         if (lane == 0) {
             mbar_expect_tx(own_full, 2 * OWN_BYTES);
-            tma_owner<D>(s_k, &map_k, own_full, hh, n0, hn);
-            tma_owner<D>(s_v, &map_v, own_full, hh, n0, hn);
+            tma_owner<D>(s_k, &map_k, own_full, hh, start + n0, hn);
+            tma_owner<D>(s_v, &map_v, own_full, hh, start + n0, hn);
         }
         for (int j = 0; j < n_tiles; ++j) {
             const int st = j % STAGES;
@@ -666,23 +705,24 @@ attn_bwd_kv_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_co
             mbar_wait(qd_empty(st), ((j / STAGES) & 1) ^ 1);
             if (lane == 0) {
                 mbar_expect_tx(qd_full(st), 2 * T_BYTES);
-                tma_other<D>(s_q + st * T_BYTES, &map_q, qd_full(st), hh, r0, hn);
-                tma_other<D>(s_dy + st * T_BYTES, &map_dys, qd_full(st), hh, r0, hn);
+                tma_other<D>(s_q + st * T_BYTES, &map_q, qd_full(st), hh, start + r0, hn);
+                tma_other<D>(s_dy + st * T_BYTES, &map_dys, qd_full(st), hh, start + r0, hn);
             }
             unsigned char *slot = rowq + st * ROWQ_BYTES;
 #pragma unroll
             for (int u = 0; u < 2; ++u) {
                 const int rr = lane + 32 * u;
                 const size_t gr = head + r0 + rr;
-                const uint4 mw = __ldg(reinterpret_cast<const uint4 *>(mask + gr * words) + kt);
+                const bool live = !VARLEN || r0 + rr < len;   // rows past the sequence end: no key, neutral row data
+                const uint4 mw = live ? __ldg(reinterpret_cast<const uint4 *>(mask + gr * words) + kt) : make_uint4(0, 0, 0, 0);
                 uint32_t *mt = reinterpret_cast<uint32_t *>(slot);        // transposed: [word t][row], rows padded to MT
                 mt[rr] = mw.x;
                 mt[MT + rr] = mw.y;
                 mt[2 * MT + rr] = mw.z;
                 mt[3 * MT + rr] = mw.w;
-                reinterpret_cast<float *>(slot + MT * 16)[rr] = delta[gr];      // -delta' (the math adds it: dp - delta')
-                reinterpret_cast<float *>(slot + MT * 16 + BN * 4)[rr] = (float)extra0[gr];
-                if constexpr (is_f16<T>) reinterpret_cast<float *>(slot + MT * 16 + 2 * BN * 4)[rr] = f16_bwd_nofs(zsum[gr]);
+                reinterpret_cast<float *>(slot + MT * 16)[rr] = live ? delta[gr] : 0.0f;      // -delta' (the math adds it: dp - delta')
+                reinterpret_cast<float *>(slot + MT * 16 + BN * 4)[rr] = live ? (float)extra0[gr] : 0.0f;
+                if constexpr (is_f16<T>) reinterpret_cast<float *>(slot + MT * 16 + 2 * BN * 4)[rr] = live ? f16_bwd_nofs(zsum[gr]) : 0.0f;
             }
             mbar_arrive(qd_full(st));
         }
@@ -793,14 +833,15 @@ attn_bwd_kv_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_co
         PROF(pf.t[5] = clock64() - t0; pf.t[4] = n_tiles; pf.flush(2, 0, threadIdx.x == 0);)
         mbar_wait(acc_full, 0);
         fence_after_sync();
-        const size_t off = (((size_t)hn * S + n0 + kk) * H + hh) * D;
-        out_chunks<D>(half, [&](int col, auto w) {
-            uint32_t r[32];
-            tmem_ld32(lane_base + COL_DV + col, r);
-            store_row_n<decltype(w)::value>(dv + off + col, r, 1.0f);
-            tmem_ld32(lane_base + COL_DK + col, r);
-            store_row_n<decltype(w)::value>(dk + off + col, r, scale);
-        });
+        const size_t off = (((size_t)hn * S + start + n0 + kk) * H + hh) * D;
+        if (!VARLEN || n0 + kk < len)                  // warp-uniform
+            out_chunks<D>(half, [&](int col, auto w) {
+                uint32_t r[32];
+                tmem_ld32(lane_base + COL_DV + col, r);
+                store_row_n<decltype(w)::value>(dv + off + col, r, 1.0f);
+                tmem_ld32(lane_base + COL_DK + col, r);
+                store_row_n<decltype(w)::value>(dk + off + col, r, scale);
+            });
     }
     fence_before_sync();
     __syncthreads();
@@ -942,18 +983,60 @@ static int launch_bwd(const CUtensorMap &mq, const CUtensorMap &mk, const CUtens
     return SPT_OK;
 }
 
+// ---- packed variable-length sequences: q, k, v [1, T, H, D]; grids (H, work-list capacity) -----------------------------
+// Every head dim runs the 128 x 64 kernels (the persistent 128 x 128 kernels of attn_tc128.cu have no varlen form).
+template <int D, typename T>
+static int launch_fwd_varlen(const CUtensorMap &mq, const CUtensorMap &mk, const CUtensorMap &mv, const uint32_t *mask,
+                             const int32_t *extra0, T *y, float *zsum, const Varlen &vl, int cap, int S, int H, float scale,
+                             float clamp, int y_transposed, const T *k, cudaStream_t st) {
+    cudaFuncSetAttribute(attn_fwd_tc_kernel<D, T, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, Dim<D>::FWD_SMEM);
+    attn_fwd_tc_kernel<D, T, true><<<dim3(H, cap), THREADS, Dim<D>::FWD_SMEM, st>>>(
+        mq, mk, mv, mask, extra0, y, zsum, S, H, scale * LOG2E, clamp * LOG2E, y_transposed, k, vl);
+    return after_launch("attn_fwd_tc_kernel(varlen)");
+}
+
+template <int D, typename T>
+static int launch_prep_varlen(const T *y, const T *grad_y, const float *zsum, float *delta, T *dys, const Varlen &vl, int cap,
+                              int S, int H, int y_transposed, cudaStream_t st) {
+    if (!y_transposed) return launch_prep<D, T>(y, grad_y, zsum, delta, dys, H, S, H, 0, st);   // row-wise: N = 1, S = T
+    attn_bwd_prep_t_kernel<D, T, true><<<dim3(2 * cap, H), 256, 0, st>>>(grad_y, y, zsum, delta, dys, S, H, vl);
+    return after_launch("attn_bwd_prep_t_kernel(varlen)");
+}
+
+template <int D, typename T>
+static int launch_bwd_varlen(const CUtensorMap &mq, const CUtensorMap &mk, const CUtensorMap &mv, const CUtensorMap &md,
+                             const uint32_t *mask, const int32_t *extra0, const float *delta, const float *zsum, T *gq, T *gk,
+                             T *gv, const Varlen &vl, int cap, int S, int H, float scale, float clamp, cudaStream_t st) {
+    constexpr int kv_smem = Dim<D>::BWD_SMEM + (is_f16<T> ? STAGES * BN * 4 : 0);      // fp16: the rows' -o per stage
+    cudaFuncSetAttribute(attn_bwd_kv_tc_kernel<D, T, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kv_smem);
+    attn_bwd_kv_tc_kernel<D, T, true><<<dim3(H, cap), THREADS, kv_smem, st>>>(
+        mq, mk, mv, md, mask, extra0, delta, gk, gv, S, H, scale, scale * LOG2E, clamp * LOG2E, zsum, vl);
+    SPT_LAUNCH_CHECK("attn_bwd_kv_tc_kernel(varlen)");
+    cudaFuncSetAttribute(attn_bwd_q_tc_kernel<D, T, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, Dim<D>::BWD_SMEM);
+    attn_bwd_q_tc_kernel<D, T, true><<<dim3(H, cap), THREADS, Dim<D>::BWD_SMEM, st>>>(
+        mq, mk, mv, md, mask, extra0, delta, gq, S, H, scale, scale * LOG2E, clamp * LOG2E, zsum, vl);
+    SPT_LAUNCH_CHECK("attn_bwd_q_tc_kernel(varlen)");
+    return SPT_OK;
+}
+
 }  // namespace attn_tc
 }  // namespace spt
 
 using namespace spt;
 
-static int check_attn_args(const char *what, int B, int S, int d, int H, int dtype, float clamp) {
+static int check_attn_type(const char *what, int d, int dtype, float clamp) {
     if (dtype != SPT_BF16 && dtype != SPT_F16)
         return fail(SPT_ERR_UNSUPPORTED, "%s: only bf16 and fp16 are supported on the fused path", what);
     if (dtype == SPT_F16 && !(clamp >= 0.0f && clamp <= attn_tc::F16_MAX_CLAMP))
         return fail(SPT_ERR_UNSUPPORTED, "%s: fp16 needs 0 <= clamp <= %g (got %g)", what, (double)attn_tc::F16_MAX_CLAMP, (double)clamp);
     if (d != 64 && d != 80 && d != 128)
         return fail(SPT_ERR_UNSUPPORTED, "%s: head dim %d not supported (64, 80 or 128)", what, d);
+    return SPT_OK;
+}
+
+static int check_attn_args(const char *what, int B, int S, int d, int H, int dtype, float clamp) {
+    const int rc = check_attn_type(what, d, dtype, clamp);
+    if (rc != SPT_OK) return rc;
     if (B < 1 || B > 65535 || S < 128 || S % 128 != 0)
         return fail(SPT_ERR_INVALID_ARGUMENT, "%s: need 1 <= B <= 65535 and S a positive multiple of 128 (B=%d S=%d)", what, B, S);
     if (H < 1 || B % H != 0)
@@ -1072,4 +1155,104 @@ extern "C" int spt_sparse_attn_bwd_ex(const void *q, const void *k, const void *
                                       scale, clamp, yt, as_stream(stream));
     return attn_bwd_typed<__nv_bfloat16>(q, k, v, y, grad_y, mask, extra0, zsum, grad_q, grad_k, grad_v, workspace, B, S, d,
                                          H, scale, clamp, yt, as_stream(stream));
+}
+
+// ---- packed variable-length sequences ----------------------------------------------------------------------------------
+static attn_tc::Varlen varlen_of(const void *work, int max_seqlen) {
+    const int32_t *w = (const int32_t *)work;
+    return {reinterpret_cast<const int4 *>(w + 4), w, 4 * ((max_seqlen + 127) / 128)};
+}
+
+template <typename T>
+static int attn_varlen_fwd_typed(const CUtensorMap &mq, const CUtensorMap &mk, const CUtensorMap &mv, const uint32_t *mask,
+                                 const int32_t *extra0, void *y, float *zsum, const attn_tc::Varlen &vl, int cap, int S, int d,
+                                 int H, float scale, float clamp, int yt, const void *k, cudaStream_t st) {
+    T *yy = (T *)y;
+    const T *kk = (const T *)k;
+    if (d == 64) return attn_tc::launch_fwd_varlen<64, T>(mq, mk, mv, mask, extra0, yy, zsum, vl, cap, S, H, scale, clamp, yt, kk, st);
+    if (d == 80) return attn_tc::launch_fwd_varlen<80, T>(mq, mk, mv, mask, extra0, yy, zsum, vl, cap, S, H, scale, clamp, yt, kk, st);
+    return attn_tc::launch_fwd_varlen<128, T>(mq, mk, mv, mask, extra0, yy, zsum, vl, cap, S, H, scale, clamp, yt, kk, st);
+}
+
+extern "C" int spt_sparse_attn_varlen_fwd(const void *q, const void *k, const void *v, const uint32_t *mask,
+                                          const int32_t *extra0, void *y, float *zsum, const void *work, int n_seq, int T,
+                                          int max_seqlen, int d, int H, float scale, float clamp, int dtype, int flags,
+                                          spt_stream_t stream) {
+    const char *what = "sparse_attn_varlen_fwd";
+    SPT_REQUIRE(q && k && v && mask && extra0 && y && zsum && work, "%s: null pointer", what);
+    int rc = check_attn_type(what, d, dtype, clamp);
+    if (rc != SPT_OK) return rc;
+    if ((rc = check_varlen(what, n_seq, T, max_seqlen, H)) != SPT_OK) return rc;
+    SPT_REQUIRE(((uintptr_t)q | (uintptr_t)k | (uintptr_t)v | (uintptr_t)y | (uintptr_t)mask | (uintptr_t)work) % 16 == 0,
+                "%s: operands must be 16-byte aligned", what);
+    const int yt = (flags & SPT_ATTN_Y_TRANSPOSED) ? 1 : 0;
+    const bool f16 = dtype == SPT_F16;
+    CUtensorMap mq, mk, mv;
+    if ((rc = attn_tc::make_map(&mq, q, 1, T, H, d, f16)) != SPT_OK) return rc;
+    if ((rc = attn_tc::make_map(&mk, k, 1, T, H, d, f16)) != SPT_OK) return rc;
+    if ((rc = attn_tc::make_map(&mv, v, 1, T, H, d, f16)) != SPT_OK) return rc;
+    const attn_tc::Varlen vl = varlen_of(work, max_seqlen);
+    const int cap = (int)varlen_capacity(n_seq, T);
+    return f16 ? attn_varlen_fwd_typed<__half>(mq, mk, mv, mask, extra0, y, zsum, vl, cap, T, d, H, scale, clamp, yt, k, as_stream(stream))
+               : attn_varlen_fwd_typed<__nv_bfloat16>(mq, mk, mv, mask, extra0, y, zsum, vl, cap, T, d, H, scale, clamp, yt, k,
+                                                      as_stream(stream));
+}
+
+// workspace: delta' [H, T] fp32, then (16-byte aligned) dO' [T, H, d] (sized for the largest head dim)
+static size_t varlen_delta_bytes(int T, int H) { return ((size_t)H * T * sizeof(float) + 15) & ~(size_t)15; }
+
+extern "C" size_t spt_sparse_attn_varlen_bwd_workspace_bytes(int T, int H) {
+    if (T < 1 || H < 1) return 16;
+    return varlen_delta_bytes(T, H) + (size_t)H * T * 128 * 2;
+}
+
+template <typename T>
+static int attn_varlen_bwd_typed(const void *q, const void *k, const void *v, const void *y, const void *grad_y,
+                                 const uint32_t *mask, const int32_t *extra0, const float *zsum, void *grad_q, void *grad_k,
+                                 void *grad_v, void *workspace, const attn_tc::Varlen &vl, int cap, int S, int d, int H,
+                                 float scale, float clamp, int yt, cudaStream_t st) {
+    constexpr bool f16 = attn_tc::is_f16<T>;
+    float *delta = (float *)workspace;
+    T *dys = (T *)((char *)workspace + varlen_delta_bytes(S, H));
+    const T *yy = (const T *)y, *dy = (const T *)grad_y;
+    // the row kernel goes first (it binds the primary context before the tensor-map encoder runs; see attn_bwd_typed)
+    int rc = d == 64   ? attn_tc::launch_prep_varlen<64, T>(yy, dy, zsum, delta, dys, vl, cap, S, H, yt, st)
+             : d == 80 ? attn_tc::launch_prep_varlen<80, T>(yy, dy, zsum, delta, dys, vl, cap, S, H, yt, st)
+                       : attn_tc::launch_prep_varlen<128, T>(yy, dy, zsum, delta, dys, vl, cap, S, H, yt, st);
+    if (rc != SPT_OK) return rc;
+    CUtensorMap mq, mk, mv, md;
+    if ((rc = attn_tc::make_map(&mq, q, 1, S, H, d, f16)) != SPT_OK) return rc;
+    if ((rc = attn_tc::make_map(&mk, k, 1, S, H, d, f16)) != SPT_OK) return rc;
+    if ((rc = attn_tc::make_map(&mv, v, 1, S, H, d, f16)) != SPT_OK) return rc;
+    if ((rc = attn_tc::make_map(&md, dys, 1, S, H, d, f16)) != SPT_OK) return rc;
+    T *gq = (T *)grad_q, *gk = (T *)grad_k, *gv = (T *)grad_v;
+    if (d == 64)
+        return attn_tc::launch_bwd_varlen<64, T>(mq, mk, mv, md, mask, extra0, delta, zsum, gq, gk, gv, vl, cap, S, H, scale, clamp, st);
+    if (d == 80)
+        return attn_tc::launch_bwd_varlen<80, T>(mq, mk, mv, md, mask, extra0, delta, zsum, gq, gk, gv, vl, cap, S, H, scale, clamp, st);
+    return attn_tc::launch_bwd_varlen<128, T>(mq, mk, mv, md, mask, extra0, delta, zsum, gq, gk, gv, vl, cap, S, H, scale, clamp, st);
+}
+
+extern "C" int spt_sparse_attn_varlen_bwd(const void *q, const void *k, const void *v, const void *y, const void *grad_y,
+                                          const uint32_t *mask, const int32_t *extra0, const float *zsum, void *grad_q,
+                                          void *grad_k, void *grad_v, void *workspace, const void *work, int n_seq, int T,
+                                          int max_seqlen, int d, int H, float scale, float clamp, int dtype, int flags,
+                                          spt_stream_t stream) {
+    const char *what = "sparse_attn_varlen_bwd";
+    SPT_REQUIRE(q && k && v && y && grad_y && mask && extra0 && zsum && grad_q && grad_k && grad_v && workspace && work,
+                "%s: null pointer", what);
+    int rc = check_attn_type(what, d, dtype, clamp);
+    if (rc != SPT_OK) return rc;
+    if ((rc = check_varlen(what, n_seq, T, max_seqlen, H)) != SPT_OK) return rc;
+    SPT_REQUIRE(((uintptr_t)q | (uintptr_t)k | (uintptr_t)v | (uintptr_t)y | (uintptr_t)grad_y | (uintptr_t)mask |
+                 (uintptr_t)workspace | (uintptr_t)work | (uintptr_t)grad_q | (uintptr_t)grad_k | (uintptr_t)grad_v) % 16 == 0,
+                "%s: operands must be 16-byte aligned", what);
+    const int yt = (flags & SPT_ATTN_Y_TRANSPOSED) ? 1 : 0;
+    const attn_tc::Varlen vl = varlen_of(work, max_seqlen);
+    const int cap = (int)varlen_capacity(n_seq, T);
+    if (dtype == SPT_F16)
+        return attn_varlen_bwd_typed<__half>(q, k, v, y, grad_y, mask, extra0, zsum, grad_q, grad_k, grad_v, workspace, vl, cap, T, d,
+                                             H, scale, clamp, yt, as_stream(stream));
+    return attn_varlen_bwd_typed<__nv_bfloat16>(q, k, v, y, grad_y, mask, extra0, zsum, grad_q, grad_k, grad_v, workspace, vl, cap,
+                                                T, d, H, scale, clamp, yt, as_stream(stream));
 }

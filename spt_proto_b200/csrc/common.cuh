@@ -58,6 +58,24 @@ inline int num_sms() {   // of the CURRENT device (one process may drive several
     return n;
 }
 
+// ---- packed variable-length sequences (varlen.cu) ----------------------------------------------
+// Work list: int32 [0] = item count, [4 ..) int4 items {first token, length, 128-row tile, bitmap word offset} in
+// descending tile order, then int4 per sequence (scratch of the builder).  sum ceil(S_i / 128) <= ceil(T / 128) + n_seq.
+__host__ __device__ inline int64_t varlen_capacity(int n_seq, int T) { return ((int64_t)T + 127) / 128 + n_seq; }
+constexpr int VARLEN_MAX_SEQLEN = 65536;
+// argument checks shared by every varlen entry point; they come before any CUDA call
+inline int check_varlen(const char *what, int n_seq, int T, int max_seqlen, int H) {
+    if (n_seq < 1) return fail(SPT_ERR_INVALID_ARGUMENT, "%s: need n_seq >= 1 (got %d)", what, n_seq);
+    if (T < 1) return fail(SPT_ERR_INVALID_ARGUMENT, "%s: need T >= 1 tokens (got %d)", what, T);
+    if (H < 1) return fail(SPT_ERR_INVALID_ARGUMENT, "%s: need H >= 1 heads (got %d)", what, H);
+    if (max_seqlen < 1 || max_seqlen > VARLEN_MAX_SEQLEN)
+        return fail(SPT_ERR_INVALID_ARGUMENT, "%s: max_seqlen %d outside [1, %d]", what, max_seqlen, VARLEN_MAX_SEQLEN);
+    if (varlen_capacity(n_seq, T) > 65535)
+        return fail(SPT_ERR_INVALID_ARGUMENT, "%s: ceil(T / 128) + n_seq = %lld work items exceed the grid limit 65535", what,
+                    (long long)varlen_capacity(n_seq, T));
+    return SPT_OK;
+}
+
 // ---- device helpers -----------------------------------------------------------------------
 constexpr unsigned FULL = 0xffffffffu;
 

@@ -33,24 +33,43 @@ constexpr int LK_THREADS = LK_ROWS * 4;      // one thread per (row, lane t)
 constexpr int LK_CV = 16;                    // code values covered by the bitmap path
 constexpr int LK_WORD_U32 = LK_CV * 4;       // u32 per (subspace, 128-key word): [v][t]
 
+// Packed variable-length batches (the VARLEN instantiations, spt_lookup_mask_varlen_fwd): codes are [1, T, H, m] (S = T),
+// blocks take items of the work list (varlen.cu: {first token, length, 128-row tile, bitmap word offset}) and exit past
+// *count.  Keys are relative to the sequence start; a sequence's key bitmaps are words [offset, offset + tiles) of the
+// head's bitmap row; mask rows are 4 `groups` words wide; nnz = length / coeff per sequence.
+struct LkVarlen {
+    const int4 *items;
+    const int *count;
+    int groups;
+    int coeff;
+};
+
 // ------------------------------------------------------------------------------------------
 // Pre-pass: key codes [B, S, m] -> bitmaps KB[b][s][w][v][t], overflow flag if any code >= 16.
 // grid (W, B), block 128: warp = lane t, lane = bit i  (key j = 128 w + 4 i + t).
 // ------------------------------------------------------------------------------------------
+// VARLEN: grid (work-list capacity, H); item = one 128-key group of one sequence, keys past its end match nothing.
+template <bool VARLEN = false>
 __global__ void __launch_bounds__(128)
 lookup_pack_kernel(const int32_t *__restrict__ key_codes, uint32_t *__restrict__ kb, int *__restrict__ flag,
-                   int S, int m, int W, int H) {
-    const int w = blockIdx.x, b = blockIdx.y;
+                   int S, int m, int W, int H, const LkVarlen vl = {}) {
+    int w = blockIdx.x, wo = blockIdx.x, start = 0, len = S;      // wo: the group's word in the bitmaps
+    if constexpr (VARLEN) {
+        if ((int)blockIdx.x >= *vl.count) return;
+        const int4 it = vl.items[blockIdx.x];
+        start = it.x, len = it.y, w = it.z, wo = it.w + it.z;
+    }
+    const int b = blockIdx.y;
     const int t = threadIdx.x >> 5, i = threadIdx.x & 31;
     const int j = 128 * w + 4 * i + t;
     // codes are [N, S, H, m] (heads interleaved; H = 1: [B, S, m])
-    const int32_t *kp = key_codes + (((size_t)(b / H) * S + j) * H + (b % H)) * m;
+    const int32_t *kp = key_codes + (((size_t)(b / H) * S + start + j) * H + (b % H)) * m;
     bool overflow = false;
     // m = 8 / 16 (the PQ shapes of the layer): the key's codes are fetched with 16-byte loads up front — the loop below
     // would otherwise issue one dependent 4-byte load per subspace between its ballots (a latency chain per block)
     int32_t pre[16];
     const bool fast = (m == 8 || m == 16) && (reinterpret_cast<uintptr_t>(key_codes) % 16 == 0);
-    if (fast && j < S) {
+    if (fast && j < len) {
 #pragma unroll
         for (int q = 0; q < 4; ++q)
             if (q * 4 < m) {
@@ -64,8 +83,8 @@ lookup_pack_kernel(const int32_t *__restrict__ key_codes, uint32_t *__restrict__
       for (int ss = 0; ss < 8; ++ss) {
         const int s = s0 + ss;
         if (s >= m) break;
-        const unsigned code = (j < S) ? ((unsigned)(fast ? pre[s0 == 0 ? ss : ss + 8] : kp[s]) & 0xffffu) : 0xffffu;
-        overflow |= (j < S) && (code >= (unsigned)LK_CV);
+        const unsigned code = (j < len) ? ((unsigned)(fast ? pre[s0 == 0 ? ss : ss + 8] : kp[s]) & 0xffffu) : 0xffffu;
+        overflow |= (j < len) && (code >= (unsigned)LK_CV);
         // lane v (< 16) wants the mask of keys whose code is v: four ballots over the code's bits, each lane keeps or
         // complements them according to its own index (16 compare + ballot + select rounds took 770 instructions per warp)
         static_assert(LK_CV == 16, "four code bits");
@@ -75,7 +94,7 @@ lookup_pack_kernel(const int32_t *__restrict__ key_codes, uint32_t *__restrict__
             const unsigned bk = __ballot_sync(FULL, (code >> k) & 1u);
             mine &= ((i >> k) & 1) ? bk : ~bk;
         }
-        if (i < LK_CV) kb[(((size_t)b * m + s) * W + w) * LK_WORD_U32 + i * 4 + t] = mine;
+        if (i < LK_CV) kb[(((size_t)b * m + s) * W + wo) * LK_WORD_U32 + i * 4 + t] = mine;
       }
     }
     if (__any_sync(FULL, overflow) && i == 0) atomicOr(flag, 1);
@@ -283,6 +302,11 @@ __device__ __forceinline__ void flush_mask(const uint32_t *s_bits, uint32_t *mas
     const int words = S / 32;
     const int rows = min(LK_ROWS, S - r0);
     uint32_t *dst = mask_out + ((size_t)b * S + r0) * words;
+    for (int i = threadIdx.x; i < rows * words; i += blockDim.x) dst[i] = s_bits[i];
+}
+
+// the same for a packed sequence: `rows` live rows of `words` words from dst on
+__device__ __forceinline__ void flush_mask_rows(const uint32_t *s_bits, uint32_t *dst, int rows, int words) {
     for (int i = threadIdx.x; i < rows * words; i += blockDim.x) dst[i] = s_bits[i];
 }
 
@@ -601,24 +625,32 @@ __device__ __forceinline__ void lkm2_select(uint32_t *s_pl, int tw, int tid, uin
     }
 }
 
-template <int M>
+// VARLEN: grid (H, work-list capacity); rows past the sequence end (whole warps: lengths are multiples of 32) select
+// nothing and store nothing.
+template <int M, bool VARLEN = false>
 __global__ void __launch_bounds__(LKM_THREADS)
 lookup_maskonly2_kernel(const int32_t *__restrict__ query_codes, const uint32_t *__restrict__ kb,
                         const int *__restrict__ flag, uint32_t *__restrict__ mask_out,
-                        int32_t *__restrict__ extra0_out, int S, int nnz, int W, int H) {
+                        int32_t *__restrict__ extra0_out, int S, int nnz, int W, int H, const LkVarlen vl = {}) {
     if (*flag) return;  // some key code >= 16: the generic kernel handles this call
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int b = blockIdx.x;                      // grid (heads, row groups): every head's heaviest (last) row group first
-    const int tile = gridDim.y - 1 - blockIdx.y;
+    int tile = gridDim.y - 1 - blockIdx.y, start = 0, len = S, woff = 0, groups = W;
+    if constexpr (VARLEN) {
+        if ((int)blockIdx.y >= *vl.count) return;
+        const int4 it = vl.items[blockIdx.y];
+        start = it.x, len = it.y, tile = it.z, woff = it.w, groups = vl.groups, nnz = it.y / vl.coeff;
+    }
     const int tw = tile + 1;                       // 128-key words a row of this group can see
     uint32_t *s_kb = reinterpret_cast<uint32_t *>(smem_raw);                 // [M][tw][16][4]
     uint32_t *s_pl = s_kb + (size_t)M * tw * LK_WORD_U32;                    // [2 tw][LKM_THREADS]
     const int tid = threadIdx.x;
     const int rl = tid >> 2, t = tid & 3;
-    const int r = tile * LKM_ROWS + rl;            // S % 128 == 0: every row is live
+    const int r = tile * LKM_ROWS + rl;
+    const bool live = !VARLEN || r < len;          // fixed length: S % 128 == 0, every row is live
     const int quarter = nnz / 4;
-    const int nkeys = r >= t ? (r - t) / 4 + 1 : 0;
-    const int lim = min(r + 1, nnz);
+    const int nkeys = (live && r >= t) ? (r - t) / 4 + 1 : 0;
+    const int lim = live ? min(r + 1, nnz) : 0;
     const int n_t = lim > t ? (lim - t + 3) / 4 : 0;
     const uint32_t last_valid = valid_mask(tw - 1, nkeys);   // words 0 .. tw - 2 are fully valid for every row of the group
 
@@ -627,7 +659,7 @@ lookup_maskonly2_kernel(const int32_t *__restrict__ query_codes, const uint32_t 
         const int per_s = tw * LK_WORD_U32 / 4;  // uint4 per subspace
         for (int i = tid; i < M * per_s; i += LKM_THREADS) {
             const int s = i / per_s, o = i - s * per_s;
-            reinterpret_cast<uint4 *>(s_kb)[i] = reinterpret_cast<const uint4 *>(kb_head + (size_t)s * W * LK_WORD_U32)[o];
+            reinterpret_cast<uint4 *>(s_kb)[i] = reinterpret_cast<const uint4 *>(kb_head + ((size_t)s * W + woff) * LK_WORD_U32)[o];
         }
     }
     // this row's bitmap column of every subspace: s_kb[s][w][q_s][t] = s_kb[koff[s] + 64 w]; a query code the bitmaps do
@@ -635,10 +667,10 @@ lookup_maskonly2_kernel(const int32_t *__restrict__ query_codes, const uint32_t 
     uint32_t koff[M];
     uint32_t badq = 0;
     {
-        const int32_t *qp = query_codes + (((size_t)(b / H) * S + r) * H + (b % H)) * M;
+        const int32_t *qp = query_codes + (((size_t)(b / H) * S + start + r) * H + (b % H)) * M;
 #pragma unroll
         for (int s = 0; s < M; ++s) {
-            const unsigned qc = (unsigned)qp[s] & 0xffffu;
+            const unsigned qc = live ? (unsigned)qp[s] & 0xffffu : 0xffffu;
             badq |= (qc >= (unsigned)LK_CV) ? (1u << s) : 0u;
             koff[s] = (uint32_t)((s * tw * LK_CV + (qc & (LK_CV - 1))) * 4 + t);
         }
@@ -687,16 +719,17 @@ lookup_maskonly2_kernel(const int32_t *__restrict__ query_codes, const uint32_t 
     const int partner_swapped = __shfl_xor_sync(FULL, swap_old >= 0 ? 1 : 0, 3);
     if (swap_old >= 0) s_pl[(2 * (swap_old >> 7)) * LKM_THREADS + tid] &= ~(1u << mask_bit(swap_old));
     if (partner_swapped && last_j >= 0) s_pl[(2 * (last_j >> 7)) * LKM_THREADS + tid] |= 1u << mask_bit(last_j);
-    store_extra0(st, extra0_out, b, r, S, nnz, true, t);
+    store_extra0(st, extra0_out, b, start + r, S, nnz, live, t);
     __syncthreads();
 
     // flush: thread -> (row, word w): 16 B = the four lane words; words the group cannot see are zero
-    uint4 *dst = reinterpret_cast<uint4 *>(mask_out + ((size_t)b * S + (size_t)tile * LKM_ROWS) * (S / 32));
-    for (int i = tid; i < LKM_ROWS * W; i += LKM_THREADS) {
+    uint4 *dst = reinterpret_cast<uint4 *>(mask_out + ((size_t)b * S + start + (size_t)tile * LKM_ROWS) * (VARLEN ? 4 * groups : S / 32));
+    for (int i = tid; i < LKM_ROWS * groups; i += LKM_THREADS) {
         const int w = i / LKM_ROWS, row = i - w * LKM_ROWS;
+        if (VARLEN && tile * LKM_ROWS + row >= len) continue;
         uint4 v = make_uint4(0, 0, 0, 0);
         if (w < tw) v = *reinterpret_cast<const uint4 *>(s_pl + (size_t)(2 * w) * LKM_THREADS + row * 4);
-        dst[(size_t)row * W + w] = v;
+        dst[(size_t)row * groups + w] = v;
     }
 }
 
@@ -728,24 +761,32 @@ __device__ __forceinline__ void lkb_planes(const uint32_t *pw, const uint32_t (&
     g3o = g3;
 }
 
-template <int M>
+// VARLEN: as lookup_maskonly2_kernel
+template <int M, bool VARLEN = false>
 __global__ void __launch_bounds__(LKM_THREADS)
 lookup_maskonly_big_kernel(const int32_t *__restrict__ query_codes, const uint32_t *__restrict__ kb,
                            const int *__restrict__ flag, uint32_t *__restrict__ mask_out,
-                           int32_t *__restrict__ extra0_out, int S, int nnz, int W, int H) {
+                           int32_t *__restrict__ extra0_out, int S, int nnz, int W, int H, const LkVarlen vl = {}) {
     if (*flag) return;  // some key code >= 16: the generic kernel handles this call
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int b = blockIdx.x;                      // grid (heads, row groups): every head's heaviest (last) row group first
-    const int tile = gridDim.y - 1 - blockIdx.y;
+    int tile = gridDim.y - 1 - blockIdx.y, start = 0, len = S, woff = 0, groups = W;
+    if constexpr (VARLEN) {
+        if ((int)blockIdx.y >= *vl.count) return;
+        const int4 it = vl.items[blockIdx.y];
+        start = it.x, len = it.y, tile = it.z, woff = it.w, groups = vl.groups, nnz = it.y / vl.coeff;
+    }
     const int tw = tile + 1;                       // 128-key words a row of this group can see
     uint32_t *s_kb = reinterpret_cast<uint32_t *>(smem_raw);                 // [M][tw][16][4]
     uint32_t *s_out = s_kb + (size_t)M * tw * LK_WORD_U32;                   // [LKB_CHUNK][LKM_THREADS]
     const int tid = threadIdx.x;
     const int rl = tid >> 2, t = tid & 3;
     const int r = tile * LKM_ROWS + rl;
+    const bool live = !VARLEN || r < len;
+    const int live_rows = VARLEN ? min(LKM_ROWS, len - tile * LKM_ROWS) : LKM_ROWS;
     const int quarter = nnz / 4;
-    const int nkeys = r >= t ? (r - t) / 4 + 1 : 0;
-    const int lim = min(r + 1, nnz);
+    const int nkeys = (live && r >= t) ? (r - t) / 4 + 1 : 0;
+    const int lim = live ? min(r + 1, nnz) : 0;
     const int n_t = lim > t ? (lim - t + 3) / 4 : 0;
     const uint32_t last_valid = valid_mask(tw - 1, nkeys);
     {
@@ -753,16 +794,16 @@ lookup_maskonly_big_kernel(const int32_t *__restrict__ query_codes, const uint32
         const int per_s = tw * LK_WORD_U32 / 4;  // uint4 per subspace
         for (int i = tid; i < M * per_s; i += LKM_THREADS) {
             const int s = i / per_s, o = i - s * per_s;
-            reinterpret_cast<uint4 *>(s_kb)[i] = reinterpret_cast<const uint4 *>(kb_head + (size_t)s * W * LK_WORD_U32)[o];
+            reinterpret_cast<uint4 *>(s_kb)[i] = reinterpret_cast<const uint4 *>(kb_head + ((size_t)s * W + woff) * LK_WORD_U32)[o];
         }
     }
     uint32_t koff[M];
     uint32_t badq = 0;
     {
-        const int32_t *qp = query_codes + (((size_t)(b / H) * S + r) * H + (b % H)) * M;
+        const int32_t *qp = query_codes + (((size_t)(b / H) * S + start + r) * H + (b % H)) * M;
 #pragma unroll
         for (int s = 0; s < M; ++s) {
-            const unsigned qc = (unsigned)qp[s] & 0xffffu;
+            const unsigned qc = live ? (unsigned)qp[s] & 0xffffu : 0xffffu;
             badq |= (qc >= (unsigned)LK_CV) ? (1u << s) : 0u;
             koff[s] = (uint32_t)((s * tw * LK_CV + (qc & (LK_CV - 1))) * 4 + t);
         }
@@ -803,7 +844,8 @@ lookup_maskonly_big_kernel(const int32_t *__restrict__ query_codes, const uint32
     }
     const bool track = __any_sync(FULL, st.s_need >= 0 || st.track >= 0);
     int j_old = -1, last_j = -1;
-    uint4 *dst = reinterpret_cast<uint4 *>(mask_out + ((size_t)b * S + (size_t)tile * LKM_ROWS) * (S / 32));
+    const int row_words = VARLEN ? 4 * groups : S / 32;
+    uint4 *dst = reinterpret_cast<uint4 *>(mask_out + ((size_t)b * S + start + (size_t)tile * LKM_ROWS) * row_words);
     for (int c0 = 0; c0 < tw; c0 += LKB_CHUNK) {
         const int c1 = min(tw, c0 + LKB_CHUNK);
         const uint32_t *pw = s_kb + (size_t)c0 * LK_WORD_U32;
@@ -843,49 +885,59 @@ lookup_maskonly_big_kernel(const int32_t *__restrict__ query_codes, const uint32
         __syncthreads();
         for (int i = tid; i < LKM_ROWS * (c1 - c0); i += LKM_THREADS) {
             const int w = i / LKM_ROWS, row = i - w * LKM_ROWS;
-            dst[(size_t)row * W + c0 + w] = *reinterpret_cast<const uint4 *>(s_out + (size_t)w * LKM_THREADS + row * 4);
+            if (!VARLEN || row < live_rows) dst[(size_t)row * groups + c0 + w] = *reinterpret_cast<const uint4 *>(s_out + (size_t)w * LKM_THREADS + row * 4);
         }
         __syncthreads();
     }
     // words the group cannot see are zero
-    for (int i = tid; i < LKM_ROWS * (W - tw); i += LKM_THREADS) {
+    for (int i = tid; i < LKM_ROWS * (groups - tw); i += LKM_THREADS) {
         const int w = i / LKM_ROWS, row = i - w * LKM_ROWS;
-        dst[(size_t)row * W + tw + w] = make_uint4(0, 0, 0, 0);
+        if (!VARLEN || row < live_rows) dst[(size_t)row * groups + tw + w] = make_uint4(0, 0, 0, 0);
     }
     // clobber fix-up (see lookup_maskonly_kernel) on the flushed words: this thread's word of key j is mask word
     // 4 (j >> 7) + t of its row (every flush above is ordered before by the __syncthreads)
     const int recv = __shfl_xor_sync(FULL, last_j, 3);
     const int swap_old = (st.s_need >= 0 && recv >= 0 && j_old >= 0 && (recv >> 2) > (j_old >> 2)) ? j_old : -1;
     const int partner_swapped = __shfl_xor_sync(FULL, swap_old >= 0 ? 1 : 0, 3);
-    uint32_t *my_row = mask_out + ((size_t)b * S + r) * (S / 32);
+    uint32_t *my_row = mask_out + ((size_t)b * S + start + r) * row_words;   // (rows past a sequence end change nothing)
     if (swap_old >= 0) my_row[4 * (swap_old >> 7) + t] &= ~(1u << mask_bit(swap_old));
     if (partner_swapped && last_j >= 0) my_row[4 * (last_j >> 7) + t] |= 1u << mask_bit(last_j);
-    store_extra0(st, extra0_out, b, r, S, nnz, true, t);
+    store_extra0(st, extra0_out, b, start + r, S, nnz, live, t);
 }
 
 // ---- generic path ----------------------------------------------------------------------------
 // smem: [ out image ][ query codes LK_ROWS * m u16 ]
+// VARLEN (mask only): nnz is the largest per-sequence nnz (it sizes the image); items = (head, 32-row quarter of a
+// work-list item), in work-list order.
+template <bool VARLEN = false>
 __global__ void __launch_bounds__(LK_THREADS)
 lookup_generic_kernel(const int32_t *__restrict__ query_codes, const int32_t *__restrict__ key_codes,
                       const int *__restrict__ flag, int flag_expect, int32_t *__restrict__ out,
                       uint32_t *__restrict__ mask_out, int32_t *__restrict__ extra0_out, int S, int m, int nnz, int H,
-                      int tiles, int nb) {
+                      int tiles, int nb, const LkVarlen vl = {}) {
     if (flag && (*flag != 0) != (flag_expect != 0)) return;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     uint16_t *s_out = reinterpret_cast<uint16_t *>(smem_raw);
+    const int words = VARLEN ? 4 * vl.groups : S / 32;        // mask words per row
     const size_t img_bytes = ((size_t)LK_ROWS * nnz * 2 + 15) & ~(size_t)15;
-    const size_t bits_bytes = mask_out ? (size_t)LK_ROWS * (S / 32) * 4 : 0;
+    const size_t bits_bytes = mask_out ? (size_t)LK_ROWS * words * 4 : 0;
     uint32_t *s_bits = mask_out ? reinterpret_cast<uint32_t *>(smem_raw + img_bytes) : nullptr;
     uint16_t *s_q = reinterpret_cast<uint16_t *>(smem_raw + img_bytes + bits_bytes);
+    if constexpr (VARLEN) tiles = 4 * *vl.count;
     // items = (head, row tile), the block strides over them: as the flag-guarded fallback behind the bitmap kernels it is
     // launched with a few hundred blocks (an early exit of one block per item cost 6 us per lookup at 128 heads)
     for (int item = blockIdx.x; item < tiles * nb; item += gridDim.x) {
     const int b = item / tiles;
-    const int tile = tiles - 1 - item % tiles;
+    int tile = tiles - 1 - item % tiles, start = 0, len = S;
+    if constexpr (VARLEN) {
+        const int4 it = vl.items[(item % tiles) >> 2];
+        start = it.x, len = it.y, tile = 4 * it.z + (item % tiles & 3), nnz = it.y / vl.coeff;
+        if (tile * LK_ROWS >= len) continue;     // block-uniform
+    }
     const int r0 = tile * LK_ROWS;
     const int rl = threadIdx.x >> 2, t = threadIdx.x & 3;
     const int r = r0 + rl;
-    const bool live = r < S;
+    const bool live = r < len;
     const int quarter = nnz / 4;
     const int nkeys = (live && r >= t) ? (r - t) / 4 + 1 : 0;
     const int lim = live ? min(r + 1, nnz) : 0;
@@ -893,16 +945,16 @@ lookup_generic_kernel(const int32_t *__restrict__ query_codes, const int32_t *__
 
     for (int i = threadIdx.x; i < LK_ROWS * nnz / 2; i += blockDim.x) reinterpret_cast<uint32_t *>(s_out)[i] = 0;
     if (s_bits)
-        for (int i = threadIdx.x; i < LK_ROWS * (S / 32); i += blockDim.x) s_bits[i] = 0;
-    uint32_t *row_bits = s_bits ? s_bits + rl * (S / 32) : nullptr;
+        for (int i = threadIdx.x; i < LK_ROWS * words; i += blockDim.x) s_bits[i] = 0;
+    uint32_t *row_bits = s_bits ? s_bits + rl * words : nullptr;
     for (int i = threadIdx.x; i < LK_ROWS * m; i += blockDim.x) {
         const int rr = r0 + i / m;
-        s_q[i] = rr < S ? (uint16_t)((unsigned)query_codes[(((size_t)(b / H) * S + rr) * H + (b % H)) * m + i % m] & 0xffffu) : 0;
+        s_q[i] = rr < len ? (uint16_t)((unsigned)query_codes[(((size_t)(b / H) * S + start + rr) * H + (b % H)) * m + i % m] & 0xffffu) : 0;
     }
     __syncthreads();
 
     GenericMatcher mt;
-    mt.kc = key_codes + ((size_t)(b / H) * S * H + (b % H)) * m;
+    mt.kc = key_codes + ((size_t)(b / H) * S * H + (b % H)) * m + (size_t)start * H * m;
     mt.kstride = H * m;
     mt.s_q = s_q + rl * m;
     mt.m = m;
@@ -925,10 +977,14 @@ lookup_generic_kernel(const int32_t *__restrict__ query_codes, const int32_t *__
         place_word(st, mask, w, t, s_out + rl * nnz, row_bits);
     }
     fix_clobber(st, t, quarter, s_out + rl * nnz, row_bits);
-    store_extra0(st, extra0_out, b, r, S, nnz, live, t);
+    store_extra0(st, extra0_out, b, start + r, S, nnz, live, t);
     __syncthreads();
-    flush_rows(s_out, out, b, r0, S, nnz);
-    if (s_bits) flush_mask(s_bits, mask_out, b, r0, S);
+    if constexpr (VARLEN) {
+        flush_mask_rows(s_bits, mask_out + ((size_t)b * S + start + r0) * words, min(LK_ROWS, len - r0), words);
+    } else {
+        flush_rows(s_out, out, b, r0, S, nnz);
+        if (s_bits) flush_mask(s_bits, mask_out, b, r0, S);
+    }
     __syncthreads();
     }
 }
@@ -967,7 +1023,7 @@ static int lookup_impl(const int32_t *query_codes, const int32_t *key_codes, int
     const size_t gen_smem = img + (size_t)LK_ROWS * m * 2;
     SPT_REQUIRE(gen_smem <= 200 * 1024, "lookup_fwd: nnz=%d / S=%d too large for the shared-memory row images", nnz, S);
     if (gen_smem > 48 * 1024)
-        cudaFuncSetAttribute(lookup_generic_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)gen_smem);
+        cudaFuncSetAttribute(lookup_generic_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)gen_smem);
 
     if (!bitmap_m_supported(m)) {
         lookup_generic_kernel<<<grid, LK_THREADS, gen_smem, st>>>(query_codes, key_codes, nullptr, 0, output, mask_out,
@@ -1074,4 +1130,76 @@ extern "C" int spt_lookup_mask_fwd(const int32_t *query_codes, const int32_t *ke
                                    int H, spt_stream_t stream) {
     SPT_REQUIRE(mask && extra0, "lookup_mask_fwd: null mask / extra0");
     return lookup_impl(query_codes, key_codes, output, mask, extra0, workspace, B, S, m, nnz, H, stream);
+}
+
+// ---- packed variable-length sequences ----------------------------------------------------------------------------------
+// shared memory of the varlen kernels at `groups` 128-key groups per row: plane kernel, plane-free kernel, generic fallback
+static size_t lkv_plane_smem(int m, int groups) { return ((size_t)m * LK_WORD_U32 * 4 + 2 * LKM_THREADS * 4) * groups; }
+static size_t lkv_big_smem(int m, int groups) { return (size_t)m * LK_WORD_U32 * 4 * groups + (size_t)LKB_CHUNK * LKM_THREADS * 4; }
+static size_t lkv_generic_smem(int m, int groups, int nnz_max) {
+    return out_image_bytes(nnz_max) + (size_t)LK_ROWS * 4 * groups * 4 + (size_t)LK_ROWS * m * 2;
+}
+constexpr size_t LKV_SMEM_MAX = 200 * 1024;
+
+extern "C" size_t spt_lookup_mask_varlen_workspace_bytes(int n_seq, int T, int H, int m) {
+    if (n_seq < 1 || T < 1 || H < 1 || m < 1) return 16;
+    return 16 + (size_t)H * m * varlen_capacity(n_seq, T) * LK_WORD_U32 * sizeof(uint32_t);
+}
+
+extern "C" int spt_lookup_mask_varlen_max_seqlen(int m) {
+    if (m != 8 && m != 10 && m != 16) return 0;
+    int groups = VARLEN_MAX_SEQLEN / 128;
+    while (groups > 0 && (lkv_big_smem(m, groups) > LKV_SMEM_MAX || lkv_generic_smem(m, groups, groups * 128 / 8) > LKV_SMEM_MAX))
+        --groups;
+    return groups * 128;
+}
+
+template <int M>
+static int lookup_varlen_launch(const int32_t *qc, const int32_t *kc, const uint32_t *kb, const int *flag, uint32_t *mask,
+                                int32_t *extra0, const LkVarlen &vl, int cap, int T, int H, cudaStream_t st) {
+    const size_t psmem = lkv_plane_smem(M, vl.groups), bsmem = lkv_big_smem(M, vl.groups);
+    if (psmem <= LKV_SMEM_MAX) {
+        cudaFuncSetAttribute(lookup_maskonly2_kernel<M, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)psmem);
+        lookup_maskonly2_kernel<M, true><<<dim3(H, cap), LKM_THREADS, psmem, st>>>(qc, kb, flag, mask, extra0, T, 0, cap, H, vl);
+        return after_launch("lookup_maskonly2_kernel(varlen)");
+    }
+    cudaFuncSetAttribute(lookup_maskonly_big_kernel<M, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bsmem);
+    lookup_maskonly_big_kernel<M, true><<<dim3(H, cap), LKM_THREADS, bsmem, st>>>(qc, kb, flag, mask, extra0, T, 0, cap, H, vl);
+    return after_launch("lookup_maskonly_big_kernel(varlen)");
+}
+
+extern "C" int spt_lookup_mask_varlen_fwd(const int32_t *query_codes, const int32_t *key_codes, const void *work,
+                                          uint32_t *mask, int32_t *extra0, void *workspace, int n_seq, int T,
+                                          int max_seqlen, int H, int m, int sparse_coeff, spt_stream_t stream) {
+    const char *what = "lookup_mask_varlen_fwd";
+    SPT_REQUIRE(query_codes && key_codes && work && mask && extra0 && workspace, "%s: null pointer", what);
+    int rc = check_varlen(what, n_seq, T, max_seqlen, H);
+    if (rc != SPT_OK) return rc;
+    SPT_REQUIRE(m == 8 || m == 10 || m == 16, "%s: n_subspaces must be 8, 10 or 16 (got %d)", what, m);
+    SPT_REQUIRE(sparse_coeff >= 1, "%s: sparse_coeff must be >= 1 (got %d)", what, sparse_coeff);
+    const int limit = spt_lookup_mask_varlen_max_seqlen(m);
+    SPT_REQUIRE(max_seqlen <= limit, "%s: max_seqlen %d beyond the mask-only lookup at m = %d (at most %d)", what, max_seqlen, m, limit);
+    SPT_REQUIRE(((uintptr_t)work | (uintptr_t)mask | (uintptr_t)workspace) % 16 == 0, "%s: work, mask and workspace must be 16-byte aligned", what);
+    const int nnz_max = (max_seqlen / sparse_coeff + 3) & ~3;       // sizes the generic fallback's row images
+    const size_t gsmem = lkv_generic_smem(m, (max_seqlen + 127) / 128, nnz_max);
+    SPT_REQUIRE(gsmem <= LKV_SMEM_MAX, "%s: max_seqlen %d / sparse_coeff %d too large for the row images", what, max_seqlen, sparse_coeff);
+    cudaStream_t st = as_stream(stream);
+    const int cap = (int)varlen_capacity(n_seq, T);
+    const int32_t *w = (const int32_t *)work;
+    const LkVarlen vl{reinterpret_cast<const int4 *>(w + 4), w, (max_seqlen + 127) / 128, sparse_coeff};
+    int *flag = reinterpret_cast<int *>(workspace);
+    uint32_t *kb = reinterpret_cast<uint32_t *>(reinterpret_cast<char *>(workspace) + 16);
+    cudaError_t e = cudaMemsetAsync(flag, 0, 16, st);
+    if (e != cudaSuccess) return fail(SPT_ERR_CUDA, "%s: memset: %s", what, cudaGetErrorString(e));
+    lookup_pack_kernel<true><<<dim3(cap, H), 128, 0, st>>>(key_codes, kb, flag, T, m, cap, H, vl);
+    SPT_LAUNCH_CHECK("lookup_pack_kernel(varlen)");
+    rc = m == 8    ? lookup_varlen_launch<8>(query_codes, key_codes, kb, flag, mask, extra0, vl, cap, T, H, st)
+         : m == 10 ? lookup_varlen_launch<10>(query_codes, key_codes, kb, flag, mask, extra0, vl, cap, T, H, st)
+                   : lookup_varlen_launch<16>(query_codes, key_codes, kb, flag, mask, extra0, vl, cap, T, H, st);
+    if (rc != SPT_OK) return rc;
+    // codes >= 16 somewhere: the generic kernel redoes the call (flag-guarded, decided on the device)
+    cudaFuncSetAttribute(lookup_generic_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)gsmem);
+    lookup_generic_kernel<true><<<2 * num_sms(), LK_THREADS, gsmem, st>>>(query_codes, key_codes, flag, 1, nullptr, mask, extra0,
+                                                                         T, m, nnz_max, H, 0, H, vl);
+    return after_launch("lookup_generic_kernel(varlen fallback)");
 }

@@ -546,6 +546,129 @@ def sparse_attn_bwd(q, k, v, y, grad_y, mask, extra0, zsum, scale: float, clamp:
     return gq, gk, gv
 
 
+# ---- packed variable-length sequences (include/spt_b200.h, DESIGN.md section 4.5) ------------------------------
+def check_cu_seqlens(cu_seqlens, T: int, sparse_coeff: int, max_seqlen=None) -> int:
+    """Validate host-side sequence offsets of a packed batch of T tokens; returns the longest length.
+    Raises ValueError naming the broken rule."""
+    cu = [int(x) for x in (cu_seqlens.tolist() if isinstance(cu_seqlens, torch.Tensor) else cu_seqlens)]
+    if len(cu) < 2 or cu[0] != 0:
+        raise ValueError("cu_seqlens must start with 0 and hold at least one sequence")
+    lengths = [b - a for a, b in zip(cu[:-1], cu[1:])]
+    if any(n <= 0 for n in lengths):
+        raise ValueError("cu_seqlens must be strictly increasing (non-monotonic offsets)")
+    if cu[-1] != T:
+        raise ValueError(f"the last offset of cu_seqlens ({cu[-1]}) must equal the token count T = {T}")
+    step = 4 * sparse_coeff
+    for i, n in enumerate(lengths):
+        if n % step or n % 32:
+            raise ValueError(f"sequence {i} has length {n}: lengths must be multiples of 4 * sparse_coeff = {step} and of 32")
+        if n < 8 * sparse_coeff:
+            raise ValueError(f"sequence {i} has length {n}: lengths must be at least 8 * sparse_coeff = {8 * sparse_coeff}")
+    longest = max(lengths)
+    if max_seqlen is not None and int(max_seqlen) < longest:
+        raise ValueError(f"max_seqlen {max_seqlen} is smaller than the longest sequence ({longest})")
+    return longest
+
+
+def _tokens(t: torch.Tensor, name: str):
+    """(T, H) of a packed [T, H, *] or [1, T, H, *] tensor."""
+    if t.dim() == 4 and t.size(0) == 1:
+        return t.size(1), t.size(2)
+    if t.dim() == 3:
+        return t.size(0), t.size(1)
+    raise RuntimeError(f"{name} must be [T, H, *] or [1, T, H, *]")
+
+
+def _cu_device(cu_seqlens, like: torch.Tensor) -> torch.Tensor:
+    if not (isinstance(cu_seqlens, torch.Tensor) and cu_seqlens.is_cuda and cu_seqlens.dtype == torch.int32
+            and cu_seqlens.dim() == 1 and cu_seqlens.is_contiguous()):
+        raise RuntimeError("cu_seqlens must be a contiguous 1-D int32 CUDA tensor")
+    if cu_seqlens.device != like.device:
+        raise RuntimeError("cu_seqlens must be on the operands' device")
+    return cu_seqlens
+
+
+def varlen_worklist(cu_seqlens: torch.Tensor, T: int, max_seqlen: int) -> torch.Tensor:
+    """Work list of a packed batch (one item per sequence and 128-row tile, heaviest first), built on the device from
+    cu_seqlens without a host synchronisation; pass it to lookup_mask_varlen / sparse_attn_varlen_*."""
+    n_seq = cu_seqlens.numel() - 1
+    work = torch.empty(max(int(lib.spt_varlen_worklist_bytes(n_seq, T)), 16) // 4, dtype=torch.int32,
+                       device=cu_seqlens.device)
+    with _on_device(cu_seqlens):
+        check(lib.spt_varlen_worklist(_p(cu_seqlens), n_seq, T, int(max_seqlen), _p(work), _stream(cu_seqlens)))
+    return work
+
+
+def lookup_mask_varlen_max_seqlen(m: int) -> int:
+    """Longest max_seqlen lookup_mask_varlen takes at m subspaces (0: m not supported)."""
+    return int(lib.spt_lookup_mask_varlen_max_seqlen(m))
+
+
+def lookup_mask_varlen(query: torch.Tensor, key: torch.Tensor, cu_seqlens: torch.Tensor, max_seqlen: int,
+                       sparse_coeff: int, work=None):
+    """lookup_mask of every sequence of a packed batch alone, in one launch per kernel.  Codes [T, H, m] or [1, T, H, m]
+    int32; cu_seqlens int32 [n + 1] on the device -> (mask [H, T, 4 ceil(max_seqlen / 128)] int32 lane-major words
+    relative to each sequence's start, extra0 [H, T] int32)."""
+    _check_type(query, torch.int32, "query")
+    _check_type(key, torch.int32, "key")
+    if query.shape != key.shape or not query.is_cuda or not query.is_contiguous() or not key.is_contiguous():
+        raise RuntimeError("query and key must be contiguous CUDA tensors of the same shape")
+    T, H = _tokens(query, "query")
+    m = query.size(-1)
+    cu = _cu_device(cu_seqlens, query)
+    n_seq = cu.numel() - 1
+    if work is None:
+        work = varlen_worklist(cu, T, max_seqlen)
+    words = 4 * ((int(max_seqlen) + 127) // 128)
+    mask = torch.empty((H, T, words), dtype=torch.int32, device=query.device)
+    extra0 = torch.empty((H, T), dtype=torch.int32, device=query.device)
+    ws = _workspace(lib.spt_lookup_mask_varlen_workspace_bytes(n_seq, T, H, m), query)
+    with _on_device(query):
+        check(lib.spt_lookup_mask_varlen_fwd(_p(query), _p(key), _p(work), _p(mask), _p(extra0), _p(ws), n_seq, T,
+                                             int(max_seqlen), H, m, int(sparse_coeff), _stream(query)))
+    return mask, extra0
+
+
+def sparse_attn_varlen_fwd(q, k, v, mask, extra0, cu_seqlens, max_seqlen: int, scale: float, clamp: float = 10.0,
+                           reference_layout: bool = False, work=None):
+    """sparse_attn_fwd of every sequence of a packed batch: q, k, v [T, H, d] or [1, T, H, d] -> (y like q, zsum [H, T]).
+    reference_layout: sequence i's y memory is its own y_i^T [H, d, S_i] at token offset cu[i]."""
+    _B, _S, d, _H, code = _check_attn(q, k, v)
+    T, H = _tokens(q, "q")
+    cu = _cu_device(cu_seqlens, q)
+    if work is None:
+        work = varlen_worklist(cu, T, max_seqlen)
+    y = torch.empty_like(q)
+    zsum = torch.empty((H, T), dtype=torch.float32, device=q.device)
+    with _on_device(q):
+        check(lib.spt_sparse_attn_varlen_fwd(_p(q), _p(k), _p(v), _p(mask), _p(extra0), _p(y), _p(zsum), _p(work),
+                                             cu.numel() - 1, T, int(max_seqlen), d, H, float(scale), float(clamp), code,
+                                             SPT_ATTN_Y_TRANSPOSED if reference_layout else 0, _stream(q)))
+    return y, zsum
+
+
+def sparse_attn_varlen_bwd(q, k, v, y, grad_y, mask, extra0, zsum, cu_seqlens, max_seqlen: int, scale: float,
+                           clamp: float = 10.0, reference_layout: bool = False, work=None):
+    """-> (grad_q, grad_k, grad_v) of sparse_attn_varlen_fwd."""
+    _B, _S, d, _H, code = _check_attn(q, k, v)
+    T, H = _tokens(q, "q")
+    _check_type(grad_y, q.dtype, "grad_y")
+    _check_type(y, q.dtype, "y")
+    if grad_y.shape != q.shape or not grad_y.is_contiguous():
+        raise RuntimeError("grad_y must be contiguous with q's shape")
+    cu = _cu_device(cu_seqlens, q)
+    if work is None:
+        work = varlen_worklist(cu, T, max_seqlen)
+    gq, gk, gv = torch.empty_like(q), torch.empty_like(k), torch.empty_like(v)
+    ws = _workspace(lib.spt_sparse_attn_varlen_bwd_workspace_bytes(T, H), q)
+    with _on_device(q):
+        check(lib.spt_sparse_attn_varlen_bwd(_p(q), _p(k), _p(v), _p(y), _p(grad_y), _p(mask), _p(extra0), _p(zsum),
+                                             _p(gq), _p(gk), _p(gv), _p(ws), _p(work), cu.numel() - 1, T, int(max_seqlen),
+                                             d, H, float(scale), float(clamp), code,
+                                             SPT_ATTN_Y_TRANSPOSED if reference_layout else 0, _stream(q)))
+    return gq, gk, gv
+
+
 # ---- (6) routed FFN: grouped GEMM on tcgen05 ------------------------------------------------------------
 def grouped_gemm(mode: int, A: torch.Tensor, a_mn_major: bool, B: torch.Tensor, b_mn_major: bool, *,
                  tile_group=None, group_ptr=None, M: int = 0, N: int, K: int = 0,

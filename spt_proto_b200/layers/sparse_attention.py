@@ -72,7 +72,9 @@ class _SparseV2Mixin:
     # 71-78).  Setting host_trigger to a bool makes the decision on the host, with no synchronisation:
     # True = compute the PQ loss on the next forward (then resets to False), False = skip it.
     host_trigger = None
-    last_path = None      # "fused" | "stage": which implementation the last forward() used (diagnostics / benches)
+    # "fused" | "stage": which implementation the last forward() used; forward_packed: "fused_packed" | "per_sequence"
+    # (diagnostics / benches)
+    last_path = None
 
     def _init_v2(self, d_head, d_codeword, n_codewords):
         self.quantizer = PQV2(d_codeword=d_codeword, n_codewords=n_codewords, n_subspaces=d_head // d_codeword)
@@ -130,6 +132,52 @@ class _SparseV2Mixin:
         # [N*H, E, S] memory itself (forward epilogue / backward row prologue): no permute pass either way
         return kernels.sparse_attention(q, k, v, mask, extra0, self.scaling,
                                         reference_layout=self.reference_output_layout)
+
+    def _packed_fused_ok(self, q, max_seqlen: int) -> bool:
+        m = self.quantizer.weight.size(0)
+        return (self.use_fused and q.is_cuda and q.dtype in (torch.bfloat16, torch.float16) and q.size(-1) in (64, 80, 128)
+                and max_seqlen <= ext.lookup_mask_varlen_max_seqlen(m))
+
+    def _rotate_packed(self, x, cu):      # the rotary layer restarts positions at every sequence start
+        return x
+
+    def forward_packed(self, q, k, v, cu_seqlens, max_seqlen=None):
+        """Packed variable-length sequences (INTEGRATION.md, "Packed sequences"): q, k, v [T, H, E] or [1, T, H, E] hold
+        n sequences concatenated along the token axis; cu_seqlens [n + 1] their offsets (cu[0] = 0, cu[n] = T).  Sequence
+        i (rows cu[i] .. cu[i+1]) gets exactly what forward() gives for it alone as a batch of one, in the same output
+        layout; y has q's shape.
+        cu_seqlens is a host list / CPU tensor (validated, then copied to the device: not capturable), or an int32 CUDA
+        tensor together with max_seqlen (trusted, never synchronised on: capturable).  Lengths must be multiples of
+        4 * sparse_coeff and of 32, and at least 8 * sparse_coeff.  Outside the fused envelope (or with use_fused =
+        False) every sequence runs forward() on its own, after one synchronisation to read the offsets."""
+        squeeze = q.dim() == 3
+        q, k, v = (t.unsqueeze(0) if squeeze else t for t in (q, k, v))
+        if q.dim() != 4 or q.size(0) != 1 or q.shape != k.shape or q.shape != v.shape:
+            raise ValueError("forward_packed: q, k, v must all be [T, H, E] or [1, T, H, E]")
+        T = q.size(1)
+        if isinstance(cu_seqlens, torch.Tensor) and cu_seqlens.is_cuda:
+            if max_seqlen is None:
+                raise ValueError("forward_packed: a device cu_seqlens needs max_seqlen")
+            cu, max_seqlen = cu_seqlens, int(max_seqlen)
+        else:
+            longest = ext.check_cu_seqlens(cu_seqlens, T, self.sparse_coeff, max_seqlen)
+            max_seqlen = longest if max_seqlen is None else int(max_seqlen)
+            host = cu_seqlens.tolist() if isinstance(cu_seqlens, torch.Tensor) else list(cu_seqlens)
+            cu = torch.tensor([int(x) for x in host], dtype=torch.int32, device=q.device)
+        if self._packed_fused_ok(q, max_seqlen):
+            self.last_path = "fused_packed"
+            q, k, v = self._rotate_packed(q, cu), self._rotate_packed(k, cu), v.contiguous()
+            q, k = q.contiguous(), k.contiguous()
+            self._maybe_train_loss(q, k)      # over all T rows
+            q_c, k_c = ext.pq_encode_pair(q, k, self.quantizer.weight)
+            mask, extra0 = ext.lookup_mask_varlen(q_c, k_c, cu, max_seqlen, self.sparse_coeff)
+            y = kernels.sparse_attention_varlen(q, k, v, mask, extra0, cu, max_seqlen, self.scaling,
+                                                reference_layout=self.reference_output_layout)
+        else:
+            offs = [int(x) for x in cu.tolist()]
+            y = torch.cat([self.forward(q[:, a:b], k[:, a:b], v[:, a:b]) for a, b in zip(offs[:-1], offs[1:])], dim=1)
+            self.last_path = "per_sequence"
+        return y.squeeze(0) if squeeze else y
 
     def _sparse_get_attn(self, q, k):
         assert q.size() == k.size()
@@ -197,6 +245,12 @@ class SparseRotaryAttentionV2(_SparseV2Mixin, RotaryAttention):
 
     def _get_attn(self, q, k, attn_mask):
         return self._sparse_get_attn(self._rotate(q), self._rotate(k))
+
+    def _rotate_packed(self, x, cu):
+        # position of token t = t - cu[sequence of t], built on the device (no host synchronisation)
+        t = torch.arange(x.size(1), dtype=torch.int32, device=x.device)
+        ids = (t - cu[torch.searchsorted(cu, t, right=True) - 1]).long()
+        return self.embedding(x, ids=ids).to(x.dtype)
 
     def forward(self, q, k, v, attn_mask=None):
         if self._fused_ok(q):
