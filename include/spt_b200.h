@@ -41,8 +41,11 @@ typedef enum {
     SPT_ERR_CUDA = 3              /* launch or runtime error (cudaGetLastError)                    */
 } spt_status;
 
-/* SPT_F16 is accepted by spt_pq_encode, spt_pq_encode_pair, spt_pq_train_fwd / _bwd and the fused attention
- * (spt_sparse_attn_fwd / _bwd and their _ex variants); every other entry point takes SPT_F32 / SPT_BF16 only. */
+/* SPT_F16 is accepted by spt_pq_encode, spt_pq_encode_pair, spt_pq_train_fwd / _bwd, the fused attention
+ * (spt_sparse_attn_fwd / _bwd, their _ex and _varlen variants) and the routed FFN: spt_grouped_gemm,
+ * spt_gather_rows_bf16 (a 16-bit row copy), spt_ffn_combine, spt_group_colsum, spt_scale_add_fwd / _bwd,
+ * spt_lora_glu_fwd_ex / _bwd_ex and spt_silu_mul_fwd_ex / _bwd_ex.  Every other entry point takes SPT_F32 /
+ * SPT_BF16 only.  bf16 and fp16 never mix in one call. */
 typedef enum { SPT_F32 = 0, SPT_BF16 = 1, SPT_F16 = 2 } spt_dtype;
 
 #define SPT_ABI_VERSION 1
@@ -327,21 +330,26 @@ int spt_route_bucket(const float *prob, int32_t *bucket_ptr, int32_t *bucket_row
 int spt_row_coeff_bwd(const float *grad_coeff, const int32_t *row_token, const int32_t *tile_group,
                       float *grad_prob, int64_t R, int64_t T, int nb, spt_stream_t stream);
 
-/* dst[r, :] = src[row_token[r], :] for r < R, zeros where row_token[r] < 0 (bf16, C % 8 == 0). */
+/* dst[r, :] = src[row_token[r], :] for r < R, zeros where row_token[r] < 0 (any 16-bit elements, bf16 or fp16:
+ * the copy does not look at the values; C % 8 == 0). */
 int spt_gather_rows_bf16(const void *src, const int32_t *row_token, void *dst, int64_t R, int C,
                          spt_stream_t stream);
 
 /* Deterministic combine: y[t, :] = bias + sum_j partial[token_rows[t, j], :], j ascending (= block
- * order); fp32 accumulation; partial / y are fp32 or bf16; bias may be NULL. */
+ * order); fp32 accumulation; bias may be NULL.  (partial, y) dtypes: fp32 with fp32, bf16 or fp16; a
+ * 16-bit type with itself or fp32.  Any other pair is SPT_ERR_INVALID_ARGUMENT. */
 int spt_ffn_combine(const void *partial, const int32_t *token_rows, const float *bias, void *y, int64_t T,
                     int C, int k_active, int partial_dtype, int y_dtype, spt_stream_t stream);
 
-/* out[g, c] = sum of x[row, c] over the (padded) rows of bucket g — bias gradients; x bf16 [R, C]. */
+/* out[g, c] = sum of x[row, c] over the (padded) rows of bucket g — bias gradients; x [R, C] of `dtype`
+ * (SPT_BF16 or SPT_F16), out fp32.  spt_group_colsum_bf16 is spt_group_colsum with dtype = SPT_BF16. */
 size_t spt_group_colsum_workspace_bytes(int n_groups, int C);
+int spt_group_colsum(const void *x, const int32_t *bucket_ptr, float *out, void *workspace,
+                     int n_groups, int C, int dtype, spt_stream_t stream);
 int spt_group_colsum_bf16(const void *x, const int32_t *bucket_ptr, float *out, void *workspace,
                           int n_groups, int C, spt_stream_t stream);
 
-/* Grouped GEMM on the tcgen05 tensor cores (bf16 operands, fp32 accumulation in TMEM, TMA-fed).
+/* Grouped GEMM on the tcgen05 tensor cores (bf16 or fp16 operands, fp32 accumulation in TMEM, TMA-fed).
  * Operands are described as STORED: a row-major matrix [rows, cols] with leading dimension ld.
  *   K-major operand  (x_mn_major = 0): stored [MN, K]  (reduction dim contiguous)
  *   MN-major operand (x_mn_major = 1): stored [K, MN]  (consumed in place through an MN-major UMMA
@@ -350,11 +358,22 @@ int spt_group_colsum_bf16(const void *x, const int32_t *bucket_ptr, float *out, 
  *   g = tile_group[i / 128] (-1: skip).  B_g is addressed by the per-group coordinate offsets
  *   b_k_off (along K) and b_mn_off (along N), both multiplied by g.  A must be K-major.
  *   epi: + bias[g * bias_stride + n], activation (0 none, 1 relu, 2 silu), * row_scale[i]; then, if `gate`
- *   (bf16 [rows of C, N], leading dimension ldg) is given, the result is zeroed wherever gate <= 0 — the
- *   ReLU backward mask applied to dH in the epilogue of the GEMM that produces it.
+ *   (operand type [rows of C, N], leading dimension ldg) is given, the result is zeroed wherever gate <= 0 —
+ *   the ReLU backward mask applied to dH in the epilogue of the GEMM that produces it.
  * mode 1 (K-grouped; weight gradients): for every group g, C_g[0:M, 0:N] = A_g . B_g^T reduced over
  *   rows group_ptr[g] .. group_ptr[g+1] (multiples of 64); C_g origin = (g*c_row_off, g*c_col_off).
- * C is fp32 or bf16 with leading dimension ldc. */
+ * ab_dtype: the type of A, B and gate, SPT_BF16 or SPT_F16.  C is fp32 or of type ab_dtype, with leading
+ * dimension ldc; bias and row_scale are fp32.  A 16-bit C takes one round-to-nearest of the fp32 result, with no
+ * saturation: an fp16 C holds inf where |result| rounds above 65504, as torch's fp16 matmul does.  Any other
+ * ab_dtype or c_dtype is rejected before any CUDA call.  spt_grouped_gemm_bf16 is spt_grouped_gemm with
+ * ab_dtype = SPT_BF16. */
+int spt_grouped_gemm(int mode, const void *A, long long a_rows, long long a_cols, long long lda,
+                     int a_mn_major, const void *B, long long b_rows, long long b_cols, long long ldb,
+                     int b_mn_major, const int32_t *tile_group, int n_m_tiles, const int32_t *group_ptr,
+                     int n_groups, int M, int N, int K, int a_k_off, int a_mn_off, int b_k_off, int b_mn_off,
+                     long long c_row_off, long long c_col_off, void *C, long long ldc, int c_dtype,
+                     const float *bias, int bias_stride, const float *row_scale, int act, const void *gate,
+                     long long ldg, int ab_dtype, spt_stream_t stream);
 int spt_grouped_gemm_bf16(int mode, const void *A, long long a_rows, long long a_cols, long long lda,
                           int a_mn_major, const void *B, long long b_rows, long long b_cols,
                           long long ldb, int b_mn_major, const int32_t *tile_group, int n_m_tiles,
@@ -392,17 +411,22 @@ int spt_transpose_last2(const void *in, void *out, int64_t batch, int R, int C, 
 int spt_grouped_gemm_plan(const int32_t *tile_group, int n_m_tiles, int tiles_n, int32_t *out, int cap);
 
 /* Gated unit of the plain RoutedLLaMaFFN: h = silu(gate) * side (layers/sparse/feedforward.py:172-176 with the LLaMA
- * activation), bf16 in / out with fp32 math, and its backward (both gradients in one pass).  n elements, multiple of 8,
- * 16-byte aligned. */
+ * activation), 16-bit in / out with fp32 math, and its backward (both gradients in one pass).  n elements, multiple of 8,
+ * 16-byte aligned.  _ex: every operand is of `dtype` (SPT_BF16 or SPT_F16); the plain names are bf16. */
 int spt_silu_mul_fwd(const void *gate, const void *side, void *h, int64_t n, spt_stream_t stream);
 int spt_silu_mul_bwd(const void *gate, const void *side, const void *grad_h, void *grad_gate, void *grad_side, int64_t n,
                      spt_stream_t stream);
+int spt_silu_mul_fwd_ex(const void *gate, const void *side, void *h, int64_t n, int dtype, spt_stream_t stream);
+int spt_silu_mul_bwd_ex(const void *gate, const void *side, const void *grad_h, void *grad_gate, void *grad_side,
+                        int64_t n, int dtype, spt_stream_t stream);
 
 /* Fused elementwise stages of the LoRA-routed FFN (naive_gpt/layers/tuning/lora_ffn.py:87-115,201-222).
- * coeff [R] fp32 = 2 * router probability of the bucket row.  dtypes: SPT_F32 / SPT_BF16.  C % 4 == 0.
+ * coeff [R] fp32 = 2 * router probability of the bucket row.  C % 4 == 0.
  *   scale_add: out = coeff[r] * a + b;   bwd: da = coeff[r] * dout (a's dtype), dcoeff[r] = sum_c dout * a.
- *   lora_glu : h (bf16) = silu(coeff*bg + lg) * (coeff*bs + ls), all inputs fp32 [R, C];
- *              bwd: gradients of the four inputs (fp32) and dcoeff[r]. */
+ *              a, b, out (and dout) are each SPT_F32 or one 16-bit type, SPT_BF16 or SPT_F16.
+ *   lora_glu : h = silu(coeff*bg + lg) * (coeff*bs + ls), all inputs fp32 [R, C];
+ *              bwd: gradients of the four inputs (fp32) and dcoeff[r].  h and grad_h are bf16 in the plain
+ *              names; the _ex names take their type (h_dtype / dh_dtype: SPT_BF16 or SPT_F16). */
 int spt_scale_add_fwd(const float *coeff, const void *a, int a_dtype, const void *b, int b_dtype, void *out,
                       int o_dtype, int64_t R, int C, spt_stream_t stream);
 int spt_scale_add_bwd(const float *coeff, const void *a, int a_dtype, const void *dout, int g_dtype, void *da,
@@ -412,6 +436,11 @@ int spt_lora_glu_fwd(const float *coeff, const float *bg, const float *lg, const
 int spt_lora_glu_bwd(const float *coeff, const float *bg, const float *lg, const float *bs, const float *ls,
                      const void *dh, float *d_bg, float *d_lg, float *d_bs, float *d_ls, float *dcoeff,
                      int64_t R, int C, spt_stream_t stream);
+int spt_lora_glu_fwd_ex(const float *coeff, const float *bg, const float *lg, const float *bs, const float *ls,
+                        void *h, int64_t R, int C, int h_dtype, spt_stream_t stream);
+int spt_lora_glu_bwd_ex(const float *coeff, const float *bg, const float *lg, const float *bs, const float *ls,
+                        const void *dh, float *d_bg, float *d_lg, float *d_bs, float *d_ls, float *dcoeff,
+                        int64_t R, int C, int dh_dtype, spt_stream_t stream);
 
 #ifdef __cplusplus
 }

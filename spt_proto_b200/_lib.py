@@ -11,7 +11,7 @@ LIB_PATH = os.path.join(_HERE, "lib", "libspt_b200.so")
 SPT_OK = 0
 SPT_F32 = 0
 SPT_BF16 = 1
-SPT_F16 = 2          # PQ encode / train and the fused attention only (include/spt_b200.h)
+SPT_F16 = 2          # PQ encode / train, the fused attention and the routed FFN only (include/spt_b200.h)
 SPT_ATTN_Y_TRANSPOSED = 1
 
 
@@ -67,6 +67,7 @@ def _load() -> ctypes.CDLL:
     ll = c.c_longlong
     sig["spt_grouped_gemm_bf16"] = (i32, [i32, vp, ll, ll, ll, i32, vp, ll, ll, ll, i32, vp, i32, vp, i32, i32, i32, i32,
                                           i32, i32, i32, i32, ll, ll, vp, ll, i32, vp, i32, vp, i32, vp, ll, vp])
+    sig["spt_grouped_gemm"] = (i32, sig["spt_grouped_gemm_bf16"][1][:-1] + [i32, vp])
     sig["spt_rmsnorm_bwd_blocks"] = (i32, [i64])
     sig["spt_rmsnorm_fwd_bf16"] = (i32, [vp, vp, vp, vp, i64, i32, f32, vp])
     sig["spt_rmsnorm_bwd_bf16"] = (i32, [vp, vp, vp, vp, vp, vp, i64, i32, vp])
@@ -78,12 +79,17 @@ def _load() -> ctypes.CDLL:
     sig["spt_silu_mul_fwd"] = (i32, [vp] * 3 + [i64, vp])
     sig["spt_silu_mul_bwd"] = (i32, [vp] * 5 + [i64, vp])
     sig["spt_lora_glu_bwd"] = (i32, [vp] * 11 + [i64, i32, vp])
+    sig["spt_lora_glu_fwd_ex"] = (i32, [vp] * 6 + [i64, i32, i32, vp])
+    sig["spt_lora_glu_bwd_ex"] = (i32, [vp] * 11 + [i64, i32, i32, vp])
+    sig["spt_silu_mul_fwd_ex"] = (i32, [vp] * 3 + [i64, i32, vp])
+    sig["spt_silu_mul_bwd_ex"] = (i32, [vp] * 5 + [i64, i32, vp])
     sig["spt_route_bucket_workspace_bytes"] = (sz, [i64, i32])
     sig["spt_route_bucket"] = (i32, [vp] * 8 + [i64, i32, i32, i64, vp])
     sig["spt_gather_rows_bf16"] = (i32, [vp, vp, vp, i64, i32, vp])
     sig["spt_ffn_combine"] = (i32, [vp, vp, vp, vp, i64, i32, i32, i32, i32, vp])
     sig["spt_group_colsum_workspace_bytes"] = (sz, [i32, i32])
     sig["spt_group_colsum_bf16"] = (i32, [vp, vp, vp, vp, i32, i32, vp])
+    sig["spt_group_colsum"] = (i32, [vp, vp, vp, vp, i32, i32, i32, vp])
     sig["spt_row_coeff_bwd"] = (i32, [vp, vp, vp, vp, i64, i64, i32, vp])
     sig["spt_softmax_clamp_bwd"] = (i32, [vp] * 6 + [i32, i32, i64, f32, f32, i32, vp])
     sig["spt_swap_dims12"] = (i32, [vp, vp, i64, i64, i64, i64, vp])

@@ -1,5 +1,5 @@
-// (6) Routed-FFN grouped GEMM on the 5th-generation tensor cores (tcgen05 + TMEM + TMA), bf16 in,
-// fp32 accumulate.
+// (6) Routed-FFN grouped GEMM on the 5th-generation tensor cores (tcgen05 + TMEM + TMA), bf16 or fp16 in
+// (A and B of one type T, a template parameter of both kernels), fp32 accumulate.
 //
 // The reference ships the routed FFN as a Python loop over weight blocks — boolean mask, gather,
 // addmm, activation, matmul, scatter-add per block (naive_gpt/layers/sparse/feedforward.py:47-85);
@@ -31,6 +31,7 @@
 //   between MMA and epilogue.
 #include <algorithm>
 #include <cstdlib>
+#include <type_traits>
 
 #include "tc.cuh"
 
@@ -70,12 +71,12 @@ struct Params {
     long long c_row_off, c_col_off;  // mode 1: C_g origin = (g * c_row_off, g * c_col_off)
     void *C;
     long long ldc;
-    int c_dtype;                   // SPT_F32 / SPT_BF16
+    int c_dtype;                   // SPT_F32 or the operand type
     const float *bias;             // optional, bias[g * bias_stride + n]
     int bias_stride;
     const float *row_scale;        // optional, one factor per C row (mode 0)
     int act;                       // 0 none, 1 relu, 2 silu
-    const __nv_bfloat16 *gate;     // optional (mode 0): zero C where gate <= 0, gate[row * ldg + col]
+    const void *gate;              // optional (mode 0, operand type): zero C where gate <= 0, gate[row * ldg + col]
     long long ldg;
 };
 
@@ -125,6 +126,14 @@ __device__ __forceinline__ Tile get_tile(const Params &p, int t) {
     return ti;
 }
 
+// kind::f16 instruction descriptor bits of the operand type: A / B format fields (bits 7-9, 10-12) = 1 for bf16,
+// 0 for fp16 (tc.cuh idesc_fp16)
+template <typename T>
+constexpr uint32_t ab_format_bits() { return std::is_same<T, __half>::value ? 0u : (1u << 7) | (1u << 10); }
+template <typename T>
+constexpr int c16_dtype() { return std::is_same<T, __half>::value ? SPT_F16 : SPT_BF16; }
+
+template <typename T>
 __global__ void __launch_bounds__(THREADS, 1)
 grouped_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_b,
                     const Params p) {
@@ -197,9 +206,9 @@ grouped_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
     } else if (warp == 1) {
         // ===== MMA issuer: the whole warp runs the (uniform) loops, one elected lane issues; descriptors of a
         // stage's k-slices are a base (computed once) plus small adds =====
-        // instruction descriptor: D = f32 (bits 4-5 = 1), A = B = bf16 (bits 7-9, 10-12 = 1),
+        // instruction descriptor: D = f32 (bits 4-5 = 1), A / B format (bits 7-9, 10-12: 1 = bf16, 0 = fp16),
         // a_major bit 15, b_major bit 16, N >> 3 at bit 17, M >> 4 at bit 24
-        const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)p.a_mn_major << 15) |
+        const uint32_t idesc = (1u << 4) | ab_format_bits<T>() | ((uint32_t)p.a_mn_major << 15) |
                                ((uint32_t)p.b_mn_major << 16) | ((uint32_t)((BN / 2) >> 3) << 17) |
                                ((uint32_t)(BM >> 4) << 24);
         const uint64_t da0 = operand_desc(s_a, p.a_mn_major, 0), db0 = operand_desc(s_b, p.b_mn_major, 0);
@@ -243,8 +252,8 @@ grouped_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
         const int quarter = warp & 3, chalf = (warp - 2) >> 2;
         const int row_in_tile = quarter * 32 + lane;
         unsigned char *stage = s_stage + (warp - 2) * 32 * STG_PITCH;
-        const bool out_bf16 = p.c_dtype == SPT_BF16;
-        const int esz = out_bf16 ? 2 : 4;
+        const bool out16 = p.c_dtype == c16_dtype<T>();
+        const int esz = out16 ? 2 : 4;
         uint32_t n_acc = 0;
         for (int t = blockIdx.x; t < p.n_tiles; t += gridDim.x) {
             const Tile ti = get_tile(p, t);
@@ -254,7 +263,7 @@ grouped_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
                 // consumers of the whole [R, N] buffer never see uninitialised memory
                 for (int i = threadIdx.x - 64; i < BM * n_valid; i += EPI_WARPS * 32) {
                     const long long off = ((long long)ti.m0 + i / n_valid) * p.ldc + ti.n0 + i % n_valid;
-                    if (out_bf16) reinterpret_cast<__nv_bfloat16 *>(p.C)[off] = __float2bfloat16_rn(0.0f);
+                    if (out16) reinterpret_cast<T *>(p.C)[off] = from_f32<T>(0.0f);
                     else reinterpret_cast<float *>(p.C)[off] = 0.0f;
                 }
                 continue;
@@ -297,12 +306,12 @@ grouped_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
 #pragma unroll
                 for (int i = 0; i < 32; ++i) v[i] *= rs;
                 if (p.gate && row_in_tile < rows_ok) {   // ReLU backward mask of the tensor this GEMM differentiates through
-                    const __nv_bfloat16 *gp = p.gate + c_row * p.ldg + ti.c_col0 + c0;
+                    const T *gp = static_cast<const T *>(p.gate) + c_row * p.ldg + ti.c_col0 + c0;
                     if (full && (reinterpret_cast<uintptr_t>(gp) % 16 == 0)) {
 #pragma unroll
                         for (int i = 0; i < 32; i += 8) {
                             float gv[8];
-                            Vec16<__nv_bfloat16>::load(gp + i, gv);
+                            Vec16<T>::load(gp + i, gv);
 #pragma unroll
                             for (int u = 0; u < 8; ++u)
                                 if (!(gv[u] > 0.0f)) v[i + u] = 0.0f;
@@ -310,17 +319,17 @@ grouped_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
                     } else {
 #pragma unroll
                         for (int i = 0; i < 32; ++i)
-                            if (c0 + i < n_valid && !(__bfloat162float(gp[i]) > 0.0f)) v[i] = 0.0f;
+                            if (c0 + i < n_valid && !(to_f32(gp[i]) > 0.0f)) v[i] = 0.0f;
                     }
                 }
                 if (full && aligned) {
                     // registers -> staging tile (thread = row) -> coalesced global stores (lane = 16-byte segment)
                     unsigned char *srow = stage + lane * STG_PITCH;
-                    if (out_bf16) {
+                    if (out16) {
 #pragma unroll
                         for (int i = 0; i < 32; i += 8) {
                             float t8[8] = {v[i], v[i + 1], v[i + 2], v[i + 3], v[i + 4], v[i + 5], v[i + 6], v[i + 7]};
-                            Vec16<__nv_bfloat16>::store(reinterpret_cast<__nv_bfloat16 *>(srow) + i, t8);
+                            Vec16<T>::store(reinterpret_cast<T *>(srow) + i, t8);
                         }
                     } else {
 #pragma unroll
@@ -328,7 +337,7 @@ grouped_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
                             *reinterpret_cast<float4 *>(srow + i * 4) = make_float4(v[i], v[i + 1], v[i + 2], v[i + 3]);
                     }
                     __syncwarp();
-                    const int segs = out_bf16 ? 4 : 8;                 // 16-byte segments per row of the chunk
+                    const int segs = out16 ? 4 : 8;                 // 16-byte segments per row of the chunk
                     const int rows_per = 32 / segs;
                     const int seg = lane % segs, rsub = lane / segs;
                     for (int r0 = 0; r0 < 32; r0 += rows_per) {
@@ -340,11 +349,11 @@ grouped_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
                         }
                     }
                 } else if (row_in_tile < rows_ok) {
-                    if (out_bf16) {
-                        __nv_bfloat16 *dst = reinterpret_cast<__nv_bfloat16 *>(p.C) + c_row * p.ldc + ti.c_col0 + c0;
+                    if (out16) {
+                        T *dst = reinterpret_cast<T *>(p.C) + c_row * p.ldc + ti.c_col0 + c0;
 #pragma unroll
                         for (int i = 0; i < 32; ++i)      // static indices: a run-time bound would put v[] in local memory
-                            if (c0 + i < n_valid) dst[i] = __float2bfloat16_rn(v[i]);
+                            if (c0 + i < n_valid) dst[i] = from_f32<T>(v[i]);
                     } else {
                         float *dst = reinterpret_cast<float *>(p.C) + c_row * p.ldc + ti.c_col0 + c0;
 #pragma unroll
@@ -439,6 +448,7 @@ __host__ __device__ inline Unit get_unit(const Params &p, int u, const uint16_t 
     return un;
 }
 
+template <typename T>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(THREADS, 1)
 grouped_gemm_pair_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_b,
                          const Params p, const int n_units_mode1) {
@@ -536,7 +546,7 @@ grouped_gemm_pair_kernel(const __grid_constant__ CUtensorMap map_a, const __grid
     } else if (warp == 1) {
         if (rank == 0) {
             // ===== MMA issuer (leader only): M = 256 over both CTAs, N = 256, K = 16 per instruction =====
-            const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)p.a_mn_major << 15) |
+            const uint32_t idesc = (1u << 4) | ab_format_bits<T>() | ((uint32_t)p.a_mn_major << 15) |
                                    ((uint32_t)p.b_mn_major << 16) | ((uint32_t)(BN >> 3) << 17) |
                                    ((uint32_t)((2 * BM) >> 4) << 24);
             const uint64_t da0 = operand_desc(s_a, p.a_mn_major, 0), db0 = operand_desc(s_b, p.b_mn_major, 0);
@@ -571,8 +581,8 @@ grouped_gemm_pair_kernel(const __grid_constant__ CUtensorMap map_a, const __grid
         const int quarter = warp & 3, chalf = (warp - 2) >> 2;
         const int row_in_tile = quarter * 32 + lane;
         unsigned char *stage = s_stage + (warp - 2) * 32 * STG_PITCH;
-        const bool out_bf16 = p.c_dtype == SPT_BF16;
-        const int esz = out_bf16 ? 2 : 4;
+        const bool out16 = p.c_dtype == c16_dtype<T>();
+        const int esz = out16 ? 2 : 4;
         uint32_t n_acc = 0;
         for (int u = cluster_id; u < n_units; u += n_clusters) {
             const Unit un = get_unit(p, u, s_list, rank);
@@ -581,7 +591,7 @@ grouped_gemm_pair_kernel(const __grid_constant__ CUtensorMap map_a, const __grid
                 // tail tile beyond the bucketed rows: define its output (zeros)
                 for (int i = threadIdx.x - 64; i < BM * n_valid; i += EPI_WARPS * 32) {
                     const long long off = (un.c_row0 + i / n_valid) * p.ldc + un.c_col0 + i % n_valid;
-                    if (out_bf16) reinterpret_cast<__nv_bfloat16 *>(p.C)[off] = __float2bfloat16_rn(0.0f);
+                    if (out16) reinterpret_cast<T *>(p.C)[off] = from_f32<T>(0.0f);
                     else reinterpret_cast<float *>(p.C)[off] = 0.0f;
                 }
             }
@@ -635,12 +645,12 @@ grouped_gemm_pair_kernel(const __grid_constant__ CUtensorMap map_a, const __grid
 #pragma unroll
                     for (int i = 0; i < 32; ++i) v[i] *= rs;
                     if (p.gate && row_in_tile < rows_ok) {
-                        const __nv_bfloat16 *gp = p.gate + c_row * p.ldg + un.c_col0 + c0;
+                        const T *gp = static_cast<const T *>(p.gate) + c_row * p.ldg + un.c_col0 + c0;
                         if (full && (reinterpret_cast<uintptr_t>(gp) % 16 == 0)) {
 #pragma unroll
                             for (int i = 0; i < 32; i += 8) {
                                 float gv[8];
-                                Vec16<__nv_bfloat16>::load(gp + i, gv);
+                                Vec16<T>::load(gp + i, gv);
 #pragma unroll
                                 for (int q = 0; q < 8; ++q)
                                     if (!(gv[q] > 0.0f)) v[i + q] = 0.0f;
@@ -648,16 +658,16 @@ grouped_gemm_pair_kernel(const __grid_constant__ CUtensorMap map_a, const __grid
                         } else {
 #pragma unroll
                             for (int i = 0; i < 32; ++i)
-                                if (c0 + i < n_valid && !(__bfloat162float(gp[i]) > 0.0f)) v[i] = 0.0f;
+                                if (c0 + i < n_valid && !(to_f32(gp[i]) > 0.0f)) v[i] = 0.0f;
                         }
                     }
                     if (full && aligned) {
                         unsigned char *srow = stage + lane * STG_PITCH;
-                        if (out_bf16) {
+                        if (out16) {
 #pragma unroll
                             for (int i = 0; i < 32; i += 8) {
                                 float t8[8] = {v[i], v[i + 1], v[i + 2], v[i + 3], v[i + 4], v[i + 5], v[i + 6], v[i + 7]};
-                                Vec16<__nv_bfloat16>::store(reinterpret_cast<__nv_bfloat16 *>(srow) + i, t8);
+                                Vec16<T>::store(reinterpret_cast<T *>(srow) + i, t8);
                             }
                         } else {
 #pragma unroll
@@ -665,7 +675,7 @@ grouped_gemm_pair_kernel(const __grid_constant__ CUtensorMap map_a, const __grid
                                 *reinterpret_cast<float4 *>(srow + i * 4) = make_float4(v[i], v[i + 1], v[i + 2], v[i + 3]);
                         }
                         __syncwarp();
-                        const int segs = out_bf16 ? 4 : 8;
+                        const int segs = out16 ? 4 : 8;
                         const int rows_per = 32 / segs;
                         const int seg = lane % segs, rsub = lane / segs;
                         for (int r0 = 0; r0 < 32; r0 += rows_per) {
@@ -677,11 +687,11 @@ grouped_gemm_pair_kernel(const __grid_constant__ CUtensorMap map_a, const __grid
                             }
                         }
                     } else if (row_in_tile < rows_ok) {
-                        if (out_bf16) {
-                            __nv_bfloat16 *dst = reinterpret_cast<__nv_bfloat16 *>(p.C) + c_row * p.ldc + un.c_col0 + c0;
+                        if (out16) {
+                            T *dst = reinterpret_cast<T *>(p.C) + c_row * p.ldc + un.c_col0 + c0;
     #pragma unroll
                         for (int i = 0; i < 32; ++i)      // static indices: a run-time bound would put v[] in local memory
-                            if (c0 + i < n_valid) dst[i] = __float2bfloat16_rn(v[i]);
+                            if (c0 + i < n_valid) dst[i] = from_f32<T>(v[i]);
                         } else {
                             float *dst = reinterpret_cast<float *>(p.C) + c_row * p.ldc + un.c_col0 + c0;
     #pragma unroll
@@ -704,19 +714,46 @@ grouped_gemm_pair_kernel(const __grid_constant__ CUtensorMap map_a, const __grid
 }
 
 // ---- host: tensor maps ---------------------------------------------------------------------------
-// 2-D bf16 tensor map: `inner` contiguous elements per row, `outer` rows of `ld` elements; box = (64, box_outer)
-static int make_map(CUtensorMap *map, const void *base, uint64_t inner, uint64_t outer, uint64_t ld, uint32_t box_outer) {
+// 2-D 16-bit tensor map (bf16 or fp16): `inner` contiguous elements per row, `outer` rows of `ld` elements;
+// box = (64, box_outer)
+static int make_map(CUtensorMap *map, const void *base, uint64_t inner, uint64_t outer, uint64_t ld, uint32_t box_outer,
+                    CUtensorMapDataType type) {
     EncodeTiledFn fn = encode_fn();
     if (!fn) return fail(SPT_ERR_CUDA, "grouped_gemm: cuTensorMapEncodeTiled entry point not available");
     cuuint64_t dims[2] = {inner, outer};
     cuuint64_t strides[1] = {ld * 2};
     cuuint32_t box[2] = {64, box_outer};
     cuuint32_t estr[2] = {1, 1};
-    CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void *>(base), dims, strides, box, estr,
+    CUresult r = fn(map, type, 2, const_cast<void *>(base), dims, strides, box, estr,
                     CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) return fail(SPT_ERR_CUDA, "grouped_gemm: cuTensorMapEncodeTiled failed (%d)", (int)r);
     return SPT_OK;
+}
+
+template <typename T>
+static int launch(const CUtensorMap &map_a, const CUtensorMap &map_b, const Params &p, int mode, int n_groups,
+                  spt_stream_t stream) {
+    static const bool use_pair = [] {
+        const char *e = getenv("SPT_GEMM_CTA_PAIR");       // "0": keep the single-CTA kernel (A/B measurements)
+        return !(e && e[0] == '0');
+    }();
+    if (use_pair && (mode == 1 || p.tiles_m <= MAX_LIST)) {
+        const int pairs_m = (p.tiles_m + 1) / 2;
+        const long long units_cap = (long long)p.tiles_n * (mode == 0 ? 2ll * pairs_m : (long long)pairs_m * n_groups);
+        SPT_REQUIRE(units_cap < (1ll << 31), "grouped_gemm: too many tiles");
+        const int n_units1 = mode == 1 ? (int)units_cap : 0;    // mode 0 counts its units on the device
+        const int n_clusters = (int)std::min<long long>(mode == 1 ? units_cap : (long long)p.tiles_n * pairs_m, num_sms() / 2);
+        // the attribute is per DEVICE and ext._on_device lets one process drive several GPUs: set it on every call
+        // (cheap, and what attn_tc.cu / lookup.cu do) instead of caching a process-wide flag
+        cudaFuncSetAttribute(grouped_gemm_pair_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM2_BYTES);
+        grouped_gemm_pair_kernel<T><<<2 * n_clusters, THREADS, SMEM2_BYTES, as_stream(stream)>>>(map_a, map_b, p, n_units1);
+        return after_launch("grouped_gemm_pair_kernel");
+    }
+    const int n_ctas = (int)std::min<long long>(p.n_tiles, num_sms());
+    cudaFuncSetAttribute(grouped_gemm_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
+    grouped_gemm_kernel<T><<<n_ctas, THREADS, SMEM_BYTES, as_stream(stream)>>>(map_a, map_b, p);
+    return after_launch("grouped_gemm_kernel");
 }
 
 }  // namespace gemm
@@ -726,14 +763,14 @@ using namespace spt;
 
 // See include/spt_b200.h.  A: rows x cols as stored (row-major, leading dim lda); for a K-major operand
 // the stored matrix is [MN, K], for an MN-major operand it is [K, MN].
-extern "C" int spt_grouped_gemm_bf16(int mode, const void *A, long long a_rows, long long a_cols, long long lda,
-                                     int a_mn_major, const void *B, long long b_rows, long long b_cols, long long ldb,
-                                     int b_mn_major, const int32_t *tile_group, int n_m_tiles,
-                                     const int32_t *group_ptr, int n_groups, int M, int N, int K, int a_k_off,
-                                     int a_mn_off, int b_k_off, int b_mn_off, long long c_row_off, long long c_col_off,
-                                     void *C, long long ldc, int c_dtype, const float *bias, int bias_stride,
-                                     const float *row_scale, int act, const void *gate, long long ldg,
-                                     spt_stream_t stream) {
+extern "C" int spt_grouped_gemm(int mode, const void *A, long long a_rows, long long a_cols, long long lda,
+                                int a_mn_major, const void *B, long long b_rows, long long b_cols, long long ldb,
+                                int b_mn_major, const int32_t *tile_group, int n_m_tiles,
+                                const int32_t *group_ptr, int n_groups, int M, int N, int K, int a_k_off,
+                                int a_mn_off, int b_k_off, int b_mn_off, long long c_row_off, long long c_col_off,
+                                void *C, long long ldc, int c_dtype, const float *bias, int bias_stride,
+                                const float *row_scale, int act, const void *gate, long long ldg, int ab_dtype,
+                                spt_stream_t stream) {
     SPT_REQUIRE(A && B && C, "grouped_gemm: null pointer");
     SPT_REQUIRE(mode == 0 || mode == 1, "grouped_gemm: bad mode %d", mode);
     SPT_REQUIRE(mode == 1 || (tile_group && n_m_tiles >= 1 && K >= 1 && !a_mn_major),
@@ -742,11 +779,15 @@ extern "C" int spt_grouped_gemm_bf16(int mode, const void *A, long long a_rows, 
     SPT_REQUIRE(N >= 1, "grouped_gemm: bad N");
     SPT_REQUIRE(lda % 8 == 0 && ldb % 8 == 0 && ((uintptr_t)A % 16 == 0) && ((uintptr_t)B % 16 == 0),
                 "grouped_gemm: operands must be 16-byte aligned with leading dims multiple of 8");
-    SPT_REQUIRE(c_dtype == SPT_F32 || c_dtype == SPT_BF16, "grouped_gemm: bad c_dtype");
+    SPT_REQUIRE(ab_dtype == SPT_BF16 || ab_dtype == SPT_F16,
+                "grouped_gemm: ab_dtype %d unknown: the operands A and B are SPT_BF16 (1) or SPT_F16 (2)", ab_dtype);
+    SPT_REQUIRE(c_dtype == SPT_F32 || c_dtype == ab_dtype,
+                "grouped_gemm: c_dtype %d not allowed: C is SPT_F32 (0) or the operand type ab_dtype (%d)", c_dtype, ab_dtype);
+    const CUtensorMapDataType map_type = ab_dtype == SPT_F16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
     CUtensorMap map_a, map_b;
-    int rc = gemm::make_map(&map_a, A, (uint64_t)a_cols, (uint64_t)a_rows, (uint64_t)lda, a_mn_major ? 64 : 128);
+    int rc = gemm::make_map(&map_a, A, (uint64_t)a_cols, (uint64_t)a_rows, (uint64_t)lda, a_mn_major ? 64 : 128, map_type);
     if (rc != SPT_OK) return rc;
-    rc = gemm::make_map(&map_b, B, (uint64_t)b_cols, (uint64_t)b_rows, (uint64_t)ldb, b_mn_major ? 64 : 128);
+    rc = gemm::make_map(&map_b, B, (uint64_t)b_cols, (uint64_t)b_rows, (uint64_t)ldb, b_mn_major ? 64 : 128, map_type);
     if (rc != SPT_OK) return rc;
     gemm::Params p;
     p.mode = mode; p.tile_group = tile_group; p.group_ptr = group_ptr; p.K = K; p.M = M; p.N = N;
@@ -754,33 +795,28 @@ extern "C" int spt_grouped_gemm_bf16(int mode, const void *A, long long a_rows, 
     p.a_k_off = a_k_off; p.a_mn_off = a_mn_off; p.b_k_off = b_k_off; p.b_mn_off = b_mn_off;
     p.c_row_off = c_row_off; p.c_col_off = c_col_off; p.C = C; p.ldc = ldc; p.c_dtype = c_dtype;
     p.bias = bias; p.bias_stride = bias_stride; p.row_scale = row_scale; p.act = act;
-    p.gate = (const __nv_bfloat16 *)gate; p.ldg = ldg;
+    p.gate = gate; p.ldg = ldg;
     SPT_REQUIRE(!gate || mode == 0, "grouped_gemm: gate is a mode-0 epilogue");
     p.tiles_n = (N + gemm::BN - 1) / gemm::BN;
     p.tiles_m = mode == 0 ? n_m_tiles : (M + gemm::BM - 1) / gemm::BM;
     const long long n_tiles = (long long)p.tiles_n * p.tiles_m * (mode == 0 ? 1 : n_groups);
     SPT_REQUIRE(n_tiles < (1ll << 31), "grouped_gemm: too many tiles");
     p.n_tiles = (int)n_tiles;
-    static const bool use_pair = [] {
-        const char *e = getenv("SPT_GEMM_CTA_PAIR");       // "0": keep the single-CTA kernel (A/B measurements)
-        return !(e && e[0] == '0');
-    }();
-    if (use_pair && (mode == 1 || p.tiles_m <= gemm::MAX_LIST)) {
-        const int pairs_m = (p.tiles_m + 1) / 2;
-        const long long units_cap = (long long)p.tiles_n * (mode == 0 ? 2ll * pairs_m : (long long)pairs_m * n_groups);
-        SPT_REQUIRE(units_cap < (1ll << 31), "grouped_gemm: too many tiles");
-        const int n_units1 = mode == 1 ? (int)units_cap : 0;    // mode 0 counts its units on the device
-        const int n_clusters = (int)std::min<long long>(mode == 1 ? units_cap : (long long)p.tiles_n * pairs_m, num_sms() / 2);
-        // the attribute is per DEVICE and ext._on_device lets one process drive several GPUs: set it on every call
-        // (cheap, and what attn_tc.cu / lookup.cu do) instead of caching a process-wide flag
-        cudaFuncSetAttribute(gemm::grouped_gemm_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, gemm::SMEM2_BYTES);
-        gemm::grouped_gemm_pair_kernel<<<2 * n_clusters, gemm::THREADS, gemm::SMEM2_BYTES, as_stream(stream)>>>(map_a, map_b, p, n_units1);
-        return after_launch("grouped_gemm_pair_kernel");
-    }
-    const int n_ctas = (int)std::min<long long>(n_tiles, num_sms());
-    cudaFuncSetAttribute(gemm::grouped_gemm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, gemm::SMEM_BYTES);
-    gemm::grouped_gemm_kernel<<<n_ctas, gemm::THREADS, gemm::SMEM_BYTES, as_stream(stream)>>>(map_a, map_b, p);
-    return after_launch("grouped_gemm_kernel");
+    return ab_dtype == SPT_F16 ? gemm::launch<__half>(map_a, map_b, p, mode, n_groups, stream)
+                               : gemm::launch<__nv_bfloat16>(map_a, map_b, p, mode, n_groups, stream);
+}
+
+extern "C" int spt_grouped_gemm_bf16(int mode, const void *A, long long a_rows, long long a_cols, long long lda,
+                                     int a_mn_major, const void *B, long long b_rows, long long b_cols, long long ldb,
+                                     int b_mn_major, const int32_t *tile_group, int n_m_tiles,
+                                     const int32_t *group_ptr, int n_groups, int M, int N, int K, int a_k_off,
+                                     int a_mn_off, int b_k_off, int b_mn_off, long long c_row_off, long long c_col_off,
+                                     void *C, long long ldc, int c_dtype, const float *bias, int bias_stride,
+                                     const float *row_scale, int act, const void *gate, long long ldg,
+                                     spt_stream_t stream) {
+    return spt_grouped_gemm(mode, A, a_rows, a_cols, lda, a_mn_major, B, b_rows, b_cols, ldb, b_mn_major, tile_group,
+                            n_m_tiles, group_ptr, n_groups, M, N, K, a_k_off, a_mn_off, b_k_off, b_mn_off, c_row_off,
+                            c_col_off, C, ldc, c_dtype, bias, bias_stride, row_scale, act, gate, ldg, SPT_BF16, stream);
 }
 
 // Host-side replay of the CTA-pair kernel's mode-0 schedule (same unit_exists / get_unit code as the device), for

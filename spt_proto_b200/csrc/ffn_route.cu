@@ -123,7 +123,8 @@ place_kernel(const float *__restrict__ prob, const unsigned long long *__restric
     }
 }
 
-// dst[r, :] = src[row_token[r], :] (zeros for padding rows); 16-byte chunks, C % 8 == 0 (bf16).
+// dst[r, :] = src[row_token[r], :] (zeros for padding rows); 16-byte chunks, C % 8 == 0 (any 16-bit type: bf16 or fp16,
+// the copy never looks at the values).
 // One warp per (row, 2 KB span): every lane moves four 16-byte chunks, all four loads in flight before the stores.
 constexpr int GR_UNROLL = 4;
 __global__ void __launch_bounds__(256)
@@ -194,8 +195,9 @@ constexpr int CS_SPLIT = 64;
 // load per thread and 128 blocks the kernel ran at a quarter of the HBM rate); the eight warps' sums meet in shared memory
 // in warp order, so the result is deterministic.
 constexpr int CS_WARPS = 8;
+template <typename T>   // bf16 or fp16
 __global__ void __launch_bounds__(32 * CS_WARPS)
-colsum_stage1(const __nv_bfloat16 *__restrict__ x, const int32_t *__restrict__ bucket_ptr, float *__restrict__ partial,
+colsum_stage1(const T *__restrict__ x, const int32_t *__restrict__ bucket_ptr, float *__restrict__ partial,
               int C) {
     __shared__ float red[CS_WARPS][256 + 8];
     const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
@@ -206,12 +208,12 @@ colsum_stage1(const __nv_bfloat16 *__restrict__ x, const int32_t *__restrict__ b
     const int a = r0 + part * per, b = min(r1, a + per);
     float acc[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
     if (c + 8 <= C && (C % 8 == 0) && (reinterpret_cast<uintptr_t>(x) % 16 == 0)) {
-        const __nv_bfloat16 *px = x + c;
+        const T *px = x + c;
         int r = a + w;
         for (; r + 3 * CS_WARPS < b; r += 4 * CS_WARPS) {
             float v[4][8];
 #pragma unroll
-            for (int u = 0; u < 4; ++u) Vec16<__nv_bfloat16>::load(px + (long long)(r + u * CS_WARPS) * C, v[u]);
+            for (int u = 0; u < 4; ++u) Vec16<T>::load(px + (long long)(r + u * CS_WARPS) * C, v[u]);
 #pragma unroll
             for (int u = 0; u < 4; ++u)
 #pragma unroll
@@ -219,13 +221,13 @@ colsum_stage1(const __nv_bfloat16 *__restrict__ x, const int32_t *__restrict__ b
         }
         for (; r < b; r += CS_WARPS) {
             float v[8];
-            Vec16<__nv_bfloat16>::load(px + (long long)r * C, v);
+            Vec16<T>::load(px + (long long)r * C, v);
 #pragma unroll
             for (int i = 0; i < 8; ++i) acc[i] += v[i];
         }
     } else {
         for (int i = 0; i < 8 && c + i < C; ++i)
-            for (int r = a + w; r < b; r += CS_WARPS) acc[i] += __bfloat162float(x[(long long)r * C + c + i]);
+            for (int r = a + w; r < b; r += CS_WARPS) acc[i] += to_f32(x[(long long)r * C + c + i]);
     }
 #pragma unroll
     for (int i = 0; i < 8; ++i) red[w][lane * 8 + i] = acc[i];
@@ -321,8 +323,9 @@ extern "C" int spt_ffn_combine(const void *partial, const int32_t *token_rows, c
     SPT_REQUIRE(partial && token_rows && y, "ffn_combine: null pointer");
     SPT_REQUIRE(T >= 1 && C >= 8 && C % 8 == 0 && k_active >= 1, "ffn_combine: bad sizes");
     using bf = __nv_bfloat16;
+    using hf = __half;
     cudaStream_t st = as_stream(stream);
-    const int V = partial_dtype == SPT_BF16 ? 8 : 4;
+    const int V = partial_dtype == SPT_F32 ? 4 : 8;
     const long long n = (long long)T * (C / V);
     const unsigned grid = (unsigned)((n + 255) / 256);
     if (partial_dtype == SPT_BF16 && y_dtype == SPT_BF16)
@@ -333,8 +336,16 @@ extern "C" int spt_ffn_combine(const void *partial, const int32_t *token_rows, c
         route::combine_kernel<float, float><<<grid, 256, 0, st>>>((const float *)partial, token_rows, bias, (float *)y, T, C, k_active);
     else if (partial_dtype == SPT_F32 && y_dtype == SPT_BF16)
         route::combine_kernel<float, bf><<<grid, 256, 0, st>>>((const float *)partial, token_rows, bias, (bf *)y, T, C, k_active);
+    else if (partial_dtype == SPT_F16 && y_dtype == SPT_F16)
+        route::combine_kernel<hf, hf><<<grid, 256, 0, st>>>((const hf *)partial, token_rows, bias, (hf *)y, T, C, k_active);
+    else if (partial_dtype == SPT_F16 && y_dtype == SPT_F32)
+        route::combine_kernel<hf, float><<<grid, 256, 0, st>>>((const hf *)partial, token_rows, bias, (float *)y, T, C, k_active);
+    else if (partial_dtype == SPT_F32 && y_dtype == SPT_F16)
+        route::combine_kernel<float, hf><<<grid, 256, 0, st>>>((const float *)partial, token_rows, bias, (hf *)y, T, C, k_active);
     else
-        return fail(SPT_ERR_INVALID_ARGUMENT, "ffn_combine: bad dtypes");
+        return fail(SPT_ERR_INVALID_ARGUMENT,
+                    "ffn_combine: dtype pair (partial %d, y %d) not supported: fp32 pairs with fp32, bf16 or fp16, and a "
+                    "16-bit type with itself or fp32 (bf16 and fp16 do not mix)", partial_dtype, y_dtype);
     return after_launch("combine_kernel");
 }
 
@@ -342,14 +353,24 @@ extern "C" size_t spt_group_colsum_workspace_bytes(int n_groups, int C) {
     return (size_t)n_groups * route::CS_SPLIT * C * sizeof(float);
 }
 
-extern "C" int spt_group_colsum_bf16(const void *x, const int32_t *bucket_ptr, float *out, void *workspace, int n_groups,
-                                     int C, spt_stream_t stream) {
+extern "C" int spt_group_colsum(const void *x, const int32_t *bucket_ptr, float *out, void *workspace, int n_groups, int C,
+                                int dtype, spt_stream_t stream) {
     SPT_REQUIRE(x && bucket_ptr && out && workspace, "group_colsum: null pointer");
     SPT_REQUIRE(n_groups >= 1 && n_groups <= 65535 && C >= 1, "group_colsum: bad sizes");
+    SPT_REQUIRE(dtype == SPT_BF16 || dtype == SPT_F16, "group_colsum: dtype %d unknown: x is SPT_BF16 (1) or SPT_F16 (2)", dtype);
     cudaStream_t st = as_stream(stream);
     dim3 g1((C + 255) / 256, route::CS_SPLIT, n_groups);
-    route::colsum_stage1<<<g1, 32 * route::CS_WARPS, 0, st>>>((const __nv_bfloat16 *)x, bucket_ptr, (float *)workspace, C);
+    if (dtype == SPT_F16)
+        route::colsum_stage1<__half><<<g1, 32 * route::CS_WARPS, 0, st>>>((const __half *)x, bucket_ptr, (float *)workspace, C);
+    else
+        route::colsum_stage1<__nv_bfloat16><<<g1, 32 * route::CS_WARPS, 0, st>>>((const __nv_bfloat16 *)x, bucket_ptr,
+                                                                                 (float *)workspace, C);
     SPT_LAUNCH_CHECK("colsum_stage1");
     route::colsum_stage2<<<dim3((C + 127) / 128, n_groups), 128, 0, st>>>((const float *)workspace, out, C);
     return after_launch("colsum_stage2");
+}
+
+extern "C" int spt_group_colsum_bf16(const void *x, const int32_t *bucket_ptr, float *out, void *workspace, int n_groups,
+                                     int C, spt_stream_t stream) {
+    return spt_group_colsum(x, bucket_ptr, out, workspace, n_groups, C, SPT_BF16, stream);
 }

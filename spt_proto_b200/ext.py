@@ -22,9 +22,12 @@ import torch
 from ._lib import SPT_ATTN_Y_TRANSPOSED, SPT_BF16, SPT_F16, SPT_F32, check, lib
 
 _DTYPES = {torch.float32: SPT_F32, torch.bfloat16: SPT_BF16}
-# fp16 is taken by the PQ encode / train kernels and the fused attention only (not by the stage entry points)
+# fp16 is taken by the PQ encode / train kernels, the fused attention and the routed-FFN entry points (grouped_gemm,
+# gather_rows, ffn_combine, group_colsum, scale_add_*, silu_mul_*, lora_glu_*), not by the stage entry points
 _PQ_DTYPES = {**_DTYPES, torch.float16: SPT_F16}
 _ATTN_DTYPES = {torch.bfloat16: SPT_BF16, torch.float16: SPT_F16}
+_FFN_DTYPES = {**_DTYPES, torch.float16: SPT_F16}          # fp32 or a 16-bit type (bf16 and fp16 never mix in one call)
+_HALF_DTYPES = {torch.bfloat16: SPT_BF16, torch.float16: SPT_F16}   # grouped GEMM operands, gathered rows, ...
 
 # softmax_backward_cuda computes the TRUE softmax gradient.  The shipped reference kernel clamps the row
 # dot product sum(y * dy) to >= 1e-9 (extension/softmax.cu:69), which is wrong whenever that sum is
@@ -64,6 +67,20 @@ def _pq_code(x: torch.Tensor, name: str) -> int:
     code = _PQ_DTYPES.get(x.dtype)
     if code is None:
         raise RuntimeError(f"{name} must be type of torch.float32, torch.bfloat16 or torch.float16")
+    return code
+
+
+def _ffn_code(x: torch.Tensor, name: str) -> int:
+    code = _FFN_DTYPES.get(x.dtype)
+    if code is None:
+        raise RuntimeError(f"{name} must be type of torch.float32, torch.bfloat16 or torch.float16 (got {x.dtype})")
+    return code
+
+
+def _half_code(x: torch.Tensor, name: str) -> int:
+    code = _HALF_DTYPES.get(x.dtype)
+    if code is None:
+        raise RuntimeError(f"{name} must be type of torch.bfloat16 or torch.float16 (got {x.dtype})")
     return code
 
 
@@ -675,21 +692,28 @@ def grouped_gemm(mode: int, A: torch.Tensor, a_mn_major: bool, B: torch.Tensor, 
                  a_k_off: int = 0, a_mn_off: int = 0, b_k_off: int = 0, b_mn_off: int = 0,
                  c_row_off: int = 0, c_col_off: int = 0, out: torch.Tensor, bias=None, bias_stride: int = 0,
                  row_scale=None, act: int = 0, gate=None) -> torch.Tensor:
-    """Thin binding of spt_grouped_gemm_bf16 (see include/spt_b200.h).  A, B: 2-D bf16 tensors as
-    stored (row-major, possibly with a row stride); `out`: 2-D fp32/bf16 tensor written in place."""
+    """Thin binding of spt_grouped_gemm (see include/spt_b200.h).  A, B: 2-D tensors as stored (row-major, possibly
+    with a row stride), both bf16 or both fp16; `gate` of the same type; `out`: 2-D fp32 tensor or one of the operand
+    type, written in place."""
     for name, t in (("A", A), ("B", B)):
-        if not (t.is_cuda and t.dim() == 2 and t.dtype == torch.bfloat16 and t.stride(1) == 1):
-            raise RuntimeError(f"{name} must be a 2-D bf16 CUDA tensor with unit inner stride")
-    if not (out.is_cuda and out.dim() == 2 and out.stride(1) == 1 and out.dtype in _DTYPES):
-        raise RuntimeError("out must be a 2-D fp32/bf16 CUDA tensor with unit inner stride")
+        if not (t.is_cuda and t.dim() == 2 and t.dtype in _HALF_DTYPES and t.stride(1) == 1):
+            raise RuntimeError(f"{name} must be a 2-D bf16 or fp16 CUDA tensor with unit inner stride")
+    if A.dtype != B.dtype:
+        raise RuntimeError(f"A and B must have the same dtype (A is {A.dtype}, B is {B.dtype})")
+    if gate is not None and gate.dtype != A.dtype:
+        raise RuntimeError(f"gate must have the operands' dtype {A.dtype} (got {gate.dtype})")
+    if not (out.is_cuda and out.dim() == 2 and out.stride(1) == 1):
+        raise RuntimeError("out must be a 2-D CUDA tensor with unit inner stride")
+    if out.dtype not in (torch.float32, A.dtype):
+        raise RuntimeError(f"out must be torch.float32 or the operand type {A.dtype} (got {out.dtype})")
     n_groups = 0 if group_ptr is None else group_ptr.numel() - 1
     n_m_tiles = 0 if tile_group is None else tile_group.numel()
     with _on_device(A):
-        check(lib.spt_grouped_gemm_bf16(
+        check(lib.spt_grouped_gemm(
             mode, _p(A), A.size(0), A.size(1), A.stride(0), int(a_mn_major), _p(B), B.size(0), B.size(1), B.stride(0),
             int(b_mn_major), _p(tile_group), n_m_tiles, _p(group_ptr), n_groups, M, N, K, a_k_off, a_mn_off, b_k_off,
-            b_mn_off, c_row_off, c_col_off, _p(out), out.stride(0), _DTYPES[out.dtype], _p(bias), bias_stride,
-            _p(row_scale), act, _p(gate), 0 if gate is None else gate.stride(0), _stream(A)))
+            b_mn_off, c_row_off, c_col_off, _p(out), out.stride(0), _FFN_DTYPES[out.dtype], _p(bias), bias_stride,
+            _p(row_scale), act, _p(gate), 0 if gate is None else gate.stride(0), _HALF_DTYPES[A.dtype], _stream(A)))
     return out
 
 
@@ -735,38 +759,39 @@ def row_coeff_bwd(grad_coeff: torch.Tensor, bucket: "Bucket") -> torch.Tensor:
 
 
 def gather_rows(src: torch.Tensor, row_token: torch.Tensor) -> torch.Tensor:
-    """dst[r] = src[row_token[r]] (zeros for padding rows); src [T, C] bf16."""
+    """dst[r] = src[row_token[r]] (zeros for padding rows); src [T, C] bf16 or fp16, dst of the same type."""
     _check_dim(src, 2, "src")
-    _check_type(src, torch.bfloat16, "src")
+    _half_code(src, "src")
     R, C = row_token.numel(), src.size(1)
-    dst = torch.empty(R, C, dtype=torch.bfloat16, device=src.device)
+    dst = torch.empty(R, C, dtype=src.dtype, device=src.device)
     with _on_device(src):
         check(lib.spt_gather_rows_bf16(_p(src), _p(row_token), _p(dst), R, C, _stream(src)))
     return dst
 
 
 def ffn_combine(partial: torch.Tensor, token_rows: torch.Tensor, bias, out_dtype) -> torch.Tensor:
-    """y[t] = bias + sum_j partial[token_rows[t, j]] in ascending block order (fp32 accumulation)."""
+    """y[t] = bias + sum_j partial[token_rows[t, j]] in ascending block order (fp32 accumulation).  partial and y are
+    fp32, bf16 or fp16; a 16-bit partial goes with its own type or fp32, bf16 and fp16 do not mix."""
     _check_dim(partial, 2, "partial")
     T, k = token_rows.shape
     C = partial.size(1)
     y = torch.empty(T, C, dtype=out_dtype, device=partial.device)
     bias32 = None if bias is None else bias.float().contiguous()
     with _on_device(partial):
-        check(lib.spt_ffn_combine(_p(partial), _p(token_rows), _p(bias32), _p(y), T, C, k, _DTYPES[partial.dtype],
-                                  _DTYPES[out_dtype], _stream(partial)))
+        check(lib.spt_ffn_combine(_p(partial), _p(token_rows), _p(bias32), _p(y), T, C, k, _ffn_code(partial, "partial"),
+                                  _ffn_code(y, "out"), _stream(partial)))
     return y
 
 
 def group_colsum(x: torch.Tensor, bucket_ptr: torch.Tensor) -> torch.Tensor:
-    """out[g, c] = sum of x[row, c] over bucket g's rows; x [R, C] bf16 -> [G, C] fp32."""
+    """out[g, c] = sum of x[row, c] over bucket g's rows; x [R, C] bf16 or fp16 -> [G, C] fp32."""
     _check_dim(x, 2, "x")
-    _check_type(x, torch.bfloat16, "x")
+    code = _half_code(x, "x")
     G, C = bucket_ptr.numel() - 1, x.size(1)
     out = torch.empty(G, C, dtype=torch.float32, device=x.device)
     ws = _workspace(lib.spt_group_colsum_workspace_bytes(G, C), x)
     with _on_device(x):
-        check(lib.spt_group_colsum_bf16(_p(x), _p(bucket_ptr), _p(out), _p(ws), G, C, _stream(x)))
+        check(lib.spt_group_colsum(_p(x), _p(bucket_ptr), _p(out), _p(ws), G, C, code, _stream(x)))
     return out
 
 
@@ -779,15 +804,16 @@ def _rows_cols(a: torch.Tensor, name: str):
 
 
 def scale_add_fwd(coeff: torch.Tensor, a: torch.Tensor, b: torch.Tensor, out_dtype) -> torch.Tensor:
-    """out[r, :] = coeff[r] * a[r, :] + b[r, :];  coeff [R] fp32, a / b / out fp32 or bf16."""
+    """out[r, :] = coeff[r] * a[r, :] + b[r, :];  coeff [R] fp32, a / b / out each fp32 or one 16-bit type (bf16 or
+    fp16: the two do not mix)."""
     R, C = _rows_cols(a, "a")
     _check_type(coeff, torch.float32, "coeff")
     if b.shape != a.shape or coeff.numel() != R or not b.is_contiguous() or not coeff.is_contiguous():
         raise RuntimeError("scale_add: shape mismatch")
     out = torch.empty(R, C, dtype=out_dtype, device=a.device)
     with _on_device(a):
-        check(lib.spt_scale_add_fwd(_p(coeff), _p(a), _float_code(a, "a"), _p(b), _float_code(b, "b"), _p(out),
-                                    _float_code(out, "out"), R, C, _stream(a)))
+        check(lib.spt_scale_add_fwd(_p(coeff), _p(a), _ffn_code(a, "a"), _p(b), _ffn_code(b, "b"), _p(out),
+                                    _ffn_code(out, "out"), R, C, _stream(a)))
     return out
 
 
@@ -799,58 +825,61 @@ def scale_add_bwd(coeff: torch.Tensor, a: torch.Tensor, grad: torch.Tensor):
     da = torch.empty_like(a)
     dcoeff = torch.empty(R, dtype=torch.float32, device=a.device)
     with _on_device(a):
-        check(lib.spt_scale_add_bwd(_p(coeff), _p(a), _float_code(a, "a"), _p(grad), _float_code(grad, "grad"), _p(da),
+        check(lib.spt_scale_add_bwd(_p(coeff), _p(a), _ffn_code(a, "a"), _p(grad), _ffn_code(grad, "grad"), _p(da),
                                     _p(dcoeff), R, C, _stream(a)))
     return da, dcoeff
 
 
 def silu_mul_fwd(gate: torch.Tensor, side: torch.Tensor) -> torch.Tensor:
-    """h = silu(gate) * side, bf16 tensors of the same shape (fp32 math, one rounding)."""
-    for t, n in ((gate, "gate"), (side, "side")):
-        _check_type(t, torch.bfloat16, n)
+    """h = silu(gate) * side, tensors of the same shape and type, bf16 or fp16 (fp32 math, one rounding)."""
+    code = _half_code(gate, "gate")
+    _check_type(side, gate.dtype, "side")
     if gate.shape != side.shape or not gate.is_contiguous() or not side.is_contiguous() or gate.numel() % 8:
         raise RuntimeError("silu_mul: gate / side must be contiguous, equal-shaped, with a multiple of 8 elements")
     h = torch.empty_like(gate)
     with _on_device(gate):
-        check(lib.spt_silu_mul_fwd(_p(gate), _p(side), _p(h), gate.numel(), _stream(gate)))
+        check(lib.spt_silu_mul_fwd_ex(_p(gate), _p(side), _p(h), gate.numel(), code, _stream(gate)))
     return h
 
 
 def silu_mul_bwd(gate: torch.Tensor, side: torch.Tensor, grad_h: torch.Tensor):
-    """-> (grad_gate, grad_side) bf16."""
-    _check_type(grad_h, torch.bfloat16, "grad_h")
+    """-> (grad_gate, grad_side) in gate's type."""
+    code = _half_code(gate, "gate")
+    for t, n in ((side, "side"), (grad_h, "grad_h")):
+        _check_type(t, gate.dtype, n)
     if grad_h.shape != gate.shape or not grad_h.is_contiguous():
         raise RuntimeError("silu_mul_bwd: shape mismatch")
     dg, ds = torch.empty_like(gate), torch.empty_like(side)
     with _on_device(gate):
-        check(lib.spt_silu_mul_bwd(_p(gate), _p(side), _p(grad_h), _p(dg), _p(ds), gate.numel(), _stream(gate)))
+        check(lib.spt_silu_mul_bwd_ex(_p(gate), _p(side), _p(grad_h), _p(dg), _p(ds), gate.numel(), code, _stream(gate)))
     return dg, ds
 
 
-def lora_glu_fwd(coeff, bg, lg, bs, ls) -> torch.Tensor:
-    """h (bf16) = silu(coeff * bg + lg) * (coeff * bs + ls); all inputs fp32 [R, C], coeff [R]."""
+def lora_glu_fwd(coeff, bg, lg, bs, ls, out_dtype=torch.bfloat16) -> torch.Tensor:
+    """h (out_dtype: bf16 or fp16) = silu(coeff * bg + lg) * (coeff * bs + ls); all inputs fp32 [R, C], coeff [R]."""
     R, C = _rows_cols(bg, "bg")
     for t, n in ((bg, "bg"), (lg, "lg"), (bs, "bs"), (ls, "ls"), (coeff, "coeff")):
         _check_type(t, torch.float32, n)
         if n != "coeff" and (t.shape != bg.shape or not t.is_contiguous()):
             raise RuntimeError("lora_glu: shape mismatch")
-    h = torch.empty(R, C, dtype=torch.bfloat16, device=bg.device)
+    h = torch.empty(R, C, dtype=out_dtype, device=bg.device)
+    code = _half_code(h, "h")
     with _on_device(bg):
-        check(lib.spt_lora_glu_fwd(_p(coeff), _p(bg), _p(lg), _p(bs), _p(ls), _p(h), R, C, _stream(bg)))
+        check(lib.spt_lora_glu_fwd_ex(_p(coeff), _p(bg), _p(lg), _p(bs), _p(ls), _p(h), R, C, code, _stream(bg)))
     return h
 
 
 def lora_glu_bwd(coeff, bg, lg, bs, ls, grad_h):
-    """-> (d_bg, d_lg, d_bs, d_ls fp32 [R, C], dcoeff [R] fp32); grad_h bf16."""
+    """-> (d_bg, d_lg, d_bs, d_ls fp32 [R, C], dcoeff [R] fp32); grad_h bf16 or fp16."""
     R, C = _rows_cols(bg, "bg")
-    _check_type(grad_h, torch.bfloat16, "grad_h")
+    code = _half_code(grad_h, "grad_h")
     if grad_h.shape != bg.shape or not grad_h.is_contiguous():
         raise RuntimeError("lora_glu_bwd: shape mismatch")
     outs = [torch.empty_like(bg) for _ in range(4)]
     dcoeff = torch.empty(R, dtype=torch.float32, device=bg.device)
     with _on_device(bg):
-        check(lib.spt_lora_glu_bwd(_p(coeff), _p(bg), _p(lg), _p(bs), _p(ls), _p(grad_h), *[_p(o) for o in outs],
-                                   _p(dcoeff), R, C, _stream(bg)))
+        check(lib.spt_lora_glu_bwd_ex(_p(coeff), _p(bg), _p(lg), _p(bs), _p(ls), _p(grad_h), *[_p(o) for o in outs],
+                                      _p(dcoeff), R, C, code, _stream(bg)))
     return (*outs, dcoeff)
 
 

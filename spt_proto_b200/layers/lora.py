@@ -99,12 +99,9 @@ def _row_coeff(prob: torch.Tensor, bucket) -> torch.Tensor:
     return _RowCoeff.apply(prob, bucket)
 
 
-def _bf16(t: torch.Tensor) -> torch.Tensor:
-    return t if t.dtype == torch.bfloat16 else t.to(torch.bfloat16)
-
-
 class _MmF32(torch.autograd.Function):
-    """bf16 x bf16 -> fp32 thin matmul (torch.mm(out_dtype=fp32) has no autograd formula)."""
+    """16-bit x 16-bit -> fp32 thin matmul, both operands of one type (torch.mm(out_dtype=fp32) has no autograd
+    formula)."""
 
     @staticmethod
     def forward(ctx, a, b):
@@ -114,20 +111,20 @@ class _MmF32(torch.autograd.Function):
     @staticmethod
     def backward(ctx, g):
         a, b = ctx.saved_tensors
-        g16 = g.to(torch.bfloat16)
+        g16 = g.to(a.dtype)
         da = torch.mm(g16, b.t()) if ctx.needs_input_grad[0] else None
         db = torch.mm(a.t(), g16, out_dtype=torch.float32).to(b.dtype) if ctx.needs_input_grad[1] else None
         return da, db
 
 
 def _down_proj_split(xp: torch.Tensor, left: torch.Tensor) -> torch.Tensor:
-    """t = xp @ left (rank-r, fp32 accumulate) returned as [hi | lo] bf16 halves, hi + lo ~ t to 16
-    mantissa bits.  Fed to the grouped GEMM against [R | R], this keeps the LoRA pre-activation at fp32
-    quality: a single bf16 rounding of t flips ReLU gates when the LoRA term dominates (measured:
-    3 % gradient error vs 0.3 %).  Autograd through hi/lo is exact (d(hi + lo)/dt = 1)."""
-    t = _MmF32.apply(xp, _bf16(left))
-    hi = t.to(torch.bfloat16)
-    lo = (t - hi.float()).to(torch.bfloat16)
+    """t = xp @ left (rank-r, fp32 accumulate) returned as [hi | lo] halves in xp's 16-bit type, hi + lo ~ t
+    to 16 mantissa bits in bf16 (about 22 in fp16).  Fed to the grouped GEMM against [R | R], this keeps the
+    LoRA pre-activation at fp32 quality: a single bf16 rounding of t flips ReLU gates when the LoRA term
+    dominates (measured: 3 % gradient error vs 0.3 %).  Autograd through hi/lo is exact (d(hi + lo)/dt = 1)."""
+    t = _MmF32.apply(xp, left.to(xp.dtype))
+    hi = t.to(xp.dtype)
+    lo = (t - hi.float()).to(xp.dtype)
     return torch.cat([hi, lo], dim=1)
 
 
@@ -169,17 +166,18 @@ class LoRARoutedFFN(RoutedFFN):
         x2 = x.reshape(-1, self.d_model)
         prob, bucket = _route(self.router, x2, self.k_active)
         coeff = _row_coeff(prob.float(), bucket)                               # [R] fp32
-        xp = F.gather(_bf16(x2).contiguous(), bucket)                           # [R, d]
+        cdt = F.compute_dtype(x)                                                # bf16, or fp16 for fp16 x
+        xp = F.gather(x2.to(cdt).contiguous(), bucket)                          # [R, d]
         f32 = torch.float32   # pre-activations stay fp32 so that activation gates are decided as in the reference
         base = F.blocked_linear_rows(xp, self.fc1.weight, self.fc1.bias, bucket, bs, out_dtype=f32)   # x W1_i^T + b1_i
         t1 = _down_proj_split(xp, _pad8(self.fc1.lora.left.weight))             # [R, 2r] = [hi | lo]
         lora = F.blocked_linear_rows(t1, _twice(_pad8(self.fc1.lora.right.weight)), None, bucket, bs,
                                      out_dtype=f32)                             # (x L1) R1_i^T
-        h = self.activation(F.scale_add(coeff, base, lora, f32)).to(torch.bfloat16)
+        h = self.activation(F.scale_add(coeff, base, lora, f32)).to(cdt)
         y_base = F.blocked_linear_cols(h, self.fc2.weight, bucket, bs)          # h W2_i
         t2 = F.blocked_linear_cols_t(h, _pad8(self.fc2.lora.left.weight), bucket, bs)   # h L2_i   [R, r]
-        y_lora = t2 @ _bf16(_pad8(self.fc2.lora.right.weight)).t()              # (h L2_i) R2^T
-        yp = F.scale_add(coeff, y_base, y_lora, torch.bfloat16)
+        y_lora = t2 @ _pad8(self.fc2.lora.right.weight).to(cdt).t()             # (h L2_i) R2^T
+        yp = F.scale_add(coeff, y_base, y_lora, cdt)
         y = F.combine(yp, bucket, self.fc2.bias, x.dtype)
         return y.view(x_size)
 
@@ -220,16 +218,17 @@ class LoRARoutedLLaMaFFN(RoutedLLaMaFFN):
         x2 = x.reshape(-1, self.d_model)
         prob, bucket = _route(self.router, x2, self.k_active)
         coeff = _row_coeff(prob.float(), bucket)
-        xp = F.gather(_bf16(x2).contiguous(), bucket)
+        cdt = F.compute_dtype(x)
+        xp = F.gather(x2.to(cdt).contiguous(), bucket)
         bg, lg = self._proj(self.gate, xp, bucket)
         bsd, lsd = self._proj(self.side, xp, bucket)
         if isinstance(self.activation, nn.SiLU):       # the LLaMA case: one fused kernel per direction
-            h = F.lora_glu(coeff, bg, lg, bsd, lsd)
+            h = F.lora_glu(coeff, bg, lg, bsd, lsd, cdt)
         else:
             h = (self.activation(F.scale_add(coeff, bg, lg, torch.float32))
-                 * F.scale_add(coeff, bsd, lsd, torch.float32)).to(torch.bfloat16)
+                 * F.scale_add(coeff, bsd, lsd, torch.float32)).to(cdt)
         y_base = F.blocked_linear_cols(h, self.down.weight, bucket, bs)
         t2 = F.blocked_linear_cols_t(h, _pad8(self.down.lora.left.weight), bucket, bs)
-        yp = F.scale_add(coeff, y_base, t2 @ _bf16(_pad8(self.down.lora.right.weight)).t(), torch.bfloat16)
+        yp = F.scale_add(coeff, y_base, t2 @ _pad8(self.down.lora.right.weight).to(cdt).t(), cdt)
         y = F.combine(yp, bucket, None, x.dtype)
         return y.view(x_size)

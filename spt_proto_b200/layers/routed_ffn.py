@@ -55,7 +55,7 @@ class RoutedFFN(Feedforward):
         x_size = x.size()
         x2 = x.reshape(-1, self.d_model)
         _, bucket = _route(self.router, x2, self.k_active)
-        xp = F.gather(x2.to(torch.bfloat16).contiguous(), bucket)
+        xp = F.gather(x2.to(F.compute_dtype(x)).contiguous(), bucket)
         relu = isinstance(self.activation, nn.ReLU)
         # ReLU: applied in the fc1 epilogue, its backward mask in the epilogue of the GEMM that produces dH
         h = F.blocked_linear_rows(xp, self.fc1.weight, self.fc1.bias, bucket, self.block_size,
@@ -95,10 +95,10 @@ class RoutedLLaMaFFN(LLaMaFeedforward):
         x_size = x.size()
         x2 = x.reshape(-1, self.d_model)
         _, bucket = _route(self.router, x2, self.k_active)
-        xp = F.gather(x2.to(torch.bfloat16).contiguous(), bucket)
+        xp = F.gather(x2.to(F.compute_dtype(x)).contiguous(), bucket)
         g = F.blocked_linear_rows(xp, self.gate.weight, None, bucket, self.block_size)
         s = F.blocked_linear_rows(xp, self.side.weight, None, bucket, self.block_size)
-        if isinstance(self.activation, nn.SiLU) and g.dtype == torch.bfloat16 and g.numel() % 8 == 0:
+        if isinstance(self.activation, nn.SiLU) and g.numel() % 8 == 0:
             h = F.silu_mul(g, s)                      # one kernel each way instead of the eager act(g) * s chain
         else:
             h = self.activation(g) * s
