@@ -230,7 +230,8 @@ int spt_softmax_clamp_bwd(const int32_t *indptr, const int32_t *indices, const f
  *   y and in the gradients (DESIGN.md section 4.1); it needs clamp <= 10 (SPT_ERR_UNSUPPORTED beyond).
  * spt_sparse_attn_bwd: grad_y -> grad_q, grad_k, grad_v [B, S, d] (dtype).  Recomputes p from q, k
  *   (nothing of size S x k is read or written); deterministic (no atomics).
- *   workspace: spt_sparse_attn_bwd_workspace_bytes(B, S).
+ *   workspace: spt_sparse_attn_bwd_workspace_bytes(B, S) = B*S*4 + B*S*128*2 bytes (delta' fp32 and
+ *   dO', sized for d = 128).
  * Layout: H = 1 means head-major [B, S, *] operands (the reference's layout after its transposes);
  * H > 1 means the layer's native [N, S, H, *] layout with B = N*H heads interleaved (codes
  * [N, S, H, m]; q/k/v/y and their gradients [N, S, H, d]) — the kernels stride over it directly, so

@@ -29,14 +29,11 @@ ext.sparse_attn_fwd(q, k, v, mask, extra0, d ** -0.5)
 ext.sparse_attn_bwd(q, k, v, y, dy, mask, extra0, z, d ** -0.5)
 torch.cuda.synchronize()
 if lib.spt_debug_attn_prof(buf, 2):
-    names = ["fwd128", "bwd_q128", "bwd_kv128"]
-    mlab = ["wait_scores", "tmem_ld", "math", "st+arrive", "iters", "epilogue", "total", "dq_flush"]
+    mlab = ["wait_scores", "tmem_ld", "math", "st+arrive", "iters", "epilogue", "total"]
     ilab = ["issue_scores", "wait_math", "issue_acc", "total", "iters", "wait_k_full", "wait_s_read", "other"]
-    for kidx, name in enumerate(names):
+    for kidx, name in ((1, "bwd_q128"), (2, "bwd_kv128")):
         r = [buf[kidx * 16 + i] for i in range(16)]
         if r[4] == 0: continue
         it_m, it_i = max(r[4], 1), max(r[12], 1)
-        print(name, "math thread, clk per tile:", {mlab[i]: round(r[i] / it_m, 1) for i in (0, 1, 2, 3, 5, 6, 7)}, "tiles", r[4])
-        if name == "bwd_kv128" and r[13]:
-            print("  fused: slot3 = e_free wait, epilogue = st+arrive, dq_flush parts: wait_read %.1f, ld16+arrive %.1f" % (r[13] / it_m, r[14] / it_m))
+        print(name, "math thread, clk per tile:", {mlab[i]: round(r[i] / it_m, 1) for i in (0, 1, 2, 3, 5, 6)}, "tiles", r[4])
         print(name, "issuer, clk per tile:", {ilab[i]: round(r[8 + i] / it_i, 1) for i in (0, 1, 2, 3, 5, 6, 7)}, "tiles", r[12])

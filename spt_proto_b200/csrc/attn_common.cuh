@@ -112,9 +112,7 @@ __device__ __forceinline__ float f16_bwd_zs(float z) { return __uint_as_float((_
 //     zero-gradient indicator.  Otherwise clamp(x) = x and the indicator is 1 — bit-identical results either way;
 //   * the selection mask is applied to the PACKED bf16 pair with one LOP3: the mask bits of four columns are moved to
 //     the sign bits of the four bytes of a register (one shift per four elements), and PRMT's sign-replicate mode
-//     expands two of them into a 0xFFFF / 0x0000 pair mask (one PRMT per two elements);
-//   * a fraction of the exp2 (the XU pipe, 16 / clk / SM, is the floor once the rest is this cheap) is evaluated on the
-//     FMA pipe: Cody-Waite range reduction + a cubic (max relative error 7.5e-5, bf16 keeps 3.9e-3).
+//     expands two of them into a 0xFFFF / 0x0000 pair mask (one PRMT per two elements).
 __device__ __forceinline__ uint64_t pk2(float lo, float hi) {
     uint64_t d;
     asm("mov.b64 %0, {%1, %2};" : "=l"(d) : "f"(lo), "f"(hi));
@@ -161,41 +159,9 @@ __device__ __forceinline__ bool warp_needs_clamp(const uint32_t (&r)[N], float t
     for (int i = 0; i < N; i += 2) mx = max3abs(mx, __uint_as_float(r[i]), __uint_as_float(r[i + 1]));
     return __any_sync(0xffffffffu, mx > thr);
 }
-// exp2 of a pair.  POLY: on the FMA pipe.  r = a + 1.5 * 2^23 holds round(a) in its low mantissa bits; f = a - round(a)
-// in [-0.5, 0.5]; 2^f by a cubic; 2^round(a) by adding round(a) << 23 to the exponent field.
-template <bool POLY>
-__device__ __forceinline__ void ex2_pair(uint64_t a, float &e0, float &e1) {
-    if constexpr (!POLY) {
-        float a0, a1;
-        up2(a, a0, a1);
-        e0 = ex2(a0);
-        e1 = ex2(a1);
-    } else {
-        const uint64_t magic = pk2(12582912.0f, 12582912.0f), nmagic = pk2(-12582912.0f, -12582912.0f);
-        const uint64_t r = add2(a, magic);
-        const uint64_t f = fma2(add2(r, nmagic), pk2(-1.0f, -1.0f), a);
-        uint64_t p = fma2(pk2(0.0551716685295105f, 0.0551716685295105f), f, pk2(0.2426111251115799f, 0.2426111251115799f));
-        p = fma2(p, f, pk2(0.6932609677314758f, 0.6932609677314758f));
-        p = fma2(p, f, pk2(0.9999280571937561f, 0.9999280571937561f));
-        float r0, r1, p0, p1;
-        up2(r, r0, r1);
-        up2(p, p0, p1);
-        e0 = __int_as_float(__float_as_int(p0) + (__float_as_int(r0) << 23));
-        e1 = __int_as_float(__float_as_int(p1) + (__float_as_int(r1) << 23));
-    }
-}
-// which pairs of a chunk go to the FMA pipe: pair index p (0 .. N/2-1); POLY_MOD = 0: none, else every POLY_MOD-th
-#ifndef SPT_ATTN_POLY_MOD
-#define SPT_ATTN_POLY_MOD 0
-#endif
-__device__ __forceinline__ constexpr bool poly_pair(int p) {
-    constexpr int mod = SPT_ATTN_POLY_MOD > 0 ? SPT_ATTN_POLY_MOD : 1;
-    return SPT_ATTN_POLY_MOD > 0 && (p % mod) == mod - 1;
-}
-
 // e of one pair of raw scores: exp2(clamp(s c)); CLAMP: exact path, also returns the per-element gradient indicators.
 // OFS (fp16): exp2(clamp(s c) + nofs), nofs = -o of the pair's rows (one FFMA2 instead of the FMUL2 when unclamped).
-template <bool CLAMP, bool POLY, bool OFS = false>
+template <bool CLAMP, bool OFS = false>
 __device__ __forceinline__ void exp_pair(float s0, float s1, const MathK mk, float &e0, float &e1, bool &in0, bool &in1,
                                          uint64_t nofs = 0) {
     uint64_t a = (OFS && !CLAMP) ? fma2(pk2(s0, s1), pk2(mk.c, mk.c), nofs) : mul2(pk2(s0, s1), pk2(mk.c, mk.c));
@@ -207,7 +173,10 @@ __device__ __forceinline__ void exp_pair(float s0, float s1, const MathK mk, flo
         a = pk2(fminf(fmaxf(a0, -mk.L), mk.L), fminf(fmaxf(a1, -mk.L), mk.L));
         if constexpr (OFS) a = add2(a, nofs);
     }
-    ex2_pair<POLY>(a, e0, e1);
+    float a0, a1;
+    up2(a, a0, a1);
+    e0 = ex2(a0);
+    e1 = ex2(a1);
 }
 
 // The 32 score columns [32 half, 32 half + 32) of key tile j of one query row: gathers, from the row's four lane-major
@@ -257,8 +226,7 @@ __device__ __forceinline__ void fwd_chunk32(const uint32_t (&r)[32], uint32_t X,
             const int i = 4 * n + 2 * h;
             float e0, e1;
             bool in0, in1;
-            if (poly_pair(i >> 1)) exp_pair<CLAMP, true, OFS>(__uint_as_float(r[i]), __uint_as_float(r[i + 1]), mk, e0, e1, in0, in1, no2);
-            else exp_pair<CLAMP, false, OFS>(__uint_as_float(r[i]), __uint_as_float(r[i + 1]), mk, e0, e1, in0, in1, no2);
+            exp_pair<CLAMP, OFS>(__uint_as_float(r[i]), __uint_as_float(r[i + 1]), mk, e0, e1, in0, in1, no2);
             if (FIRST && i == 0) e0 *= mult0;
             const uint32_t p = pack2<T>(e0, e1) & (h ? m23 : m01);
             sum2 = add2(sum2, unpack2<T>(p));
@@ -290,8 +258,7 @@ __device__ __forceinline__ void bwdq_chunk32(const uint32_t (&r)[32], const uint
             const int i = 4 * n + 2 * h;
             float e0, e1;
             bool in0 = true, in1 = true;
-            if (poly_pair(i >> 1)) exp_pair<CLAMP, true, OFS>(__uint_as_float(r[i]), __uint_as_float(r[i + 1]), mk, e0, e1, in0, in1, no2);
-            else exp_pair<CLAMP, false, OFS>(__uint_as_float(r[i]), __uint_as_float(r[i + 1]), mk, e0, e1, in0, in1, no2);
+            exp_pair<CLAMP, OFS>(__uint_as_float(r[i]), __uint_as_float(r[i + 1]), mk, e0, e1, in0, in1, no2);
             if (FIRST && i == 0) e0 *= mult0;
             float d0, d1;
             up2(mul2(pk2(e0, e1), add2(pk2(__uint_as_float(g[i]), __uint_as_float(g[i + 1])), nd2)), d0, d1);
@@ -334,8 +301,7 @@ __device__ __forceinline__ void bwdkv_chunk16(const uint32_t (&rr)[NR], const ui
             const int i = q4 + 2 * h;
             float e0, e1;
             bool in0 = true, in1 = true;
-            if (poly_pair(i >> 1)) exp_pair<CLAMP, true, OFS>(__uint_as_float(r[i]), __uint_as_float(r[i + 1]), mk, e0, e1, in0, in1, nov[h]);
-            else exp_pair<CLAMP, false, OFS>(__uint_as_float(r[i]), __uint_as_float(r[i + 1]), mk, e0, e1, in0, in1, nov[h]);
+            exp_pair<CLAMP, OFS>(__uint_as_float(r[i]), __uint_as_float(r[i + 1]), mk, e0, e1, in0, in1, nov[h]);
             uint32_t ma = mwv[2 * h], mb = mwv[2 * h + 1];
             if (KEY0) {     // key 0: weight = bit + zero-padding multiplicity of the row
                 const float w0 = (float)(ma >> 31) + (float)s_ex0[c0 + i], w1 = (float)(mb >> 31) + (float)s_ex0[c0 + i + 1];
@@ -455,13 +421,6 @@ template <typename T>
 int launch_bwd_q128(const CUtensorMap &mq, const CUtensorMap &mk, const CUtensorMap &mv, const CUtensorMap &md,
                     const uint32_t *mask, const int32_t *extra0, const float *ndelta, const float *zsum, T *gq, int B,
                     int S, int H, float scale, float clamp, cudaStream_t st);
-int launch_bwd_fused128(const CUtensorMap &mq, const CUtensorMap &mk, const CUtensorMap &mv, const CUtensorMap &md,
-                        const uint32_t *mask, const int32_t *extra0, const float *ndelta, float *dq_acc,
-                        __nv_bfloat16 *gq, __nv_bfloat16 *gk, __nv_bfloat16 *gv, int B, int S, int H, float scale,
-                        float clamp, cudaStream_t st);
-int launch_fwd128(const CUtensorMap &mq, const CUtensorMap &mk, const CUtensorMap &mv, const uint32_t *mask,
-                  const int32_t *extra0, __nv_bfloat16 *y, float *zsum, int B, int S, int H, float scale, float clamp,
-                  int y_transposed, cudaStream_t st);
 int read_prof(unsigned long long *out48, int reset);
 }  // namespace attn_tc128
 }  // namespace spt

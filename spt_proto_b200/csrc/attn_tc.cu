@@ -866,20 +866,10 @@ static int make_map(CUtensorMap *map, const void *base, int N, int S, int H, int
 }
 
 // head dim 64: the backward runs on the 128 x 128-tile kernels of attn_tc128.cu unless SPT_ATTN_TILE=64 (A/B switch); the
-// forward stays on the 128 x 64 two-CTAs-per-SM kernel, which is as fast (0.145 vs 0.151 ms at the bench shape: it is
-// bound by the exp unit, not by the tensor pipe) unless SPT_ATTN_FWD128=1
+// forward stays on the 128 x 64 two-CTAs-per-SM kernel: it is bound by the exp unit, not by the tensor pipe, and a
+// 128 x 128 forward measured slower (DESIGN.md section 4.1)
 static bool tile128() {
     static const bool on = [] { const char *e = getenv("SPT_ATTN_TILE"); return !(e && atoi(e) == 64); }();
-    return on;
-}
-// one-pass backward (dK, dV and dQ from the same score tiles, attn_bwd_fused128_kernel): opt-in, SPT_ATTN_BWD_FUSED=1
-static bool bwd_fused() {
-    static const bool on = [] { const char *e = getenv("SPT_ATTN_BWD_FUSED"); return e && atoi(e) == 1; }();
-    return on;
-}
-// dK/dV and dQ kernels on two streams (SPT_ATTN_BWD_STREAMS=0: one after the other on the caller's stream)
-static bool bwd_two_streams() {
-    static const bool on = [] { const char *e = getenv("SPT_ATTN_BWD_STREAMS"); return !(e && atoi(e) == 0); }();
     return on;
 }
 struct SideStream {
@@ -907,21 +897,14 @@ static SideStream *side_stream(cudaStream_t caller) {   // g_side_mu held
     }
     return &s;
 }
-static bool fwd128() {
-    static const bool on = [] { const char *e = getenv("SPT_ATTN_FWD128"); return e && atoi(e) == 1; }();
-    return on;
-}
 
-// k: the key tensor (read by the fp16 forward only, for its row scales).  fp16 always runs the 128 x 64 forward.
+// k: the key tensor (read by the fp16 forward only, for its row scales)
 template <int D, typename T>
 static int launch_fwd(const CUtensorMap &mq, const CUtensorMap &mk, const CUtensorMap &mv, const uint32_t *mask,
                       const int32_t *extra0, T *y, float *zsum, int B, int S, int H, float scale, float clamp,
                       int y_transposed, const T *k, cudaStream_t st) {
-    if constexpr (!is_f16<T>)
-        if (D == 64 && fwd128()) return attn_tc128::launch_fwd128(mq, mk, mv, mask, extra0, y, zsum, B, S, H, scale, clamp, y_transposed, st);
-    static const int extra_smem = [] { const char *e = getenv("SPT_ATTN_EXTRA_SMEM"); return e ? atoi(e) : 0; }();   // diagnostics: forces 1 CTA / SM
-    cudaFuncSetAttribute(attn_fwd_tc_kernel<D, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, Dim<D>::FWD_SMEM + extra_smem);
-    attn_fwd_tc_kernel<D, T><<<dim3(B, S / BM), THREADS, Dim<D>::FWD_SMEM + extra_smem, st>>>(mq, mk, mv, mask, extra0, y, zsum, S, H,
+    cudaFuncSetAttribute(attn_fwd_tc_kernel<D, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, Dim<D>::FWD_SMEM);
+    attn_fwd_tc_kernel<D, T><<<dim3(B, S / BM), THREADS, Dim<D>::FWD_SMEM, st>>>(mq, mk, mv, mask, extra0, y, zsum, S, H,
                                                                                  scale * LOG2E, clamp * LOG2E, y_transposed, k);
     return after_launch("attn_fwd_tc_kernel");
 }
@@ -939,43 +922,40 @@ static int launch_prep(const T *y, const T *grad_y, const float *zsum, float *de
     return after_launch("attn_bwd_prep_kernel");
 }
 
-// fp16 never takes the one-pass backward (SPT_ATTN_BWD_FUSED=1 leaves it on the dK/dV + dQ kernels)
 template <int D, typename T>
 static int launch_bwd(const CUtensorMap &mq, const CUtensorMap &mk, const CUtensorMap &mv, const CUtensorMap &md,
-                      const uint32_t *mask, const int32_t *extra0, const float *delta, const float *zsum, float *dq_acc,
-                      T *gq, T *gk, T *gv, int B, int S, int H, float scale, float clamp, cudaStream_t st) {
-    if constexpr (!is_f16<T>)
-        if (D == 64 && tile128() && bwd_fused())
-            return attn_tc128::launch_bwd_fused128(mq, mk, mv, md, mask, extra0, delta, dq_acc, gq, gk, gv, B, S, H, scale, clamp, st);
-    if (D == 64 && tile128() && bwd_two_streams()) {
-        // The dK/dV and the dQ kernel are independent: the dQ kernel goes to a side stream (fork / join with events, which
-        // a stream capture records as graph edges), so its CTAs start on each SM as that SM's dK/dV CTA retires instead of
-        // after the whole grid has drained (both are one-CTA-per-SM persistent grids: they never share an SM).
-        std::lock_guard<std::mutex> lock(g_side_mu);
-        SideStream *ss = side_stream(st);
-        if (ss) {
-            if (cudaEventRecord(ss->fork, st) != cudaSuccess || cudaStreamWaitEvent(ss->stream, ss->fork, 0) != cudaSuccess)
-                return fail(SPT_ERR_CUDA, "sparse_attn_bwd: fork to the side stream failed");
-            int rc = attn_tc128::launch_bwd_kv128(mq, mk, mv, md, mask, extra0, delta, zsum, gk, gv, B, S, H, scale, clamp, st);
-            if (rc != SPT_OK) return rc;
-            rc = attn_tc128::launch_bwd_q128(mq, mk, mv, md, mask, extra0, delta, zsum, gq, B, S, H, scale, clamp, ss->stream);
-            if (rc != SPT_OK) return rc;
-            if (cudaEventRecord(ss->join, ss->stream) != cudaSuccess || cudaStreamWaitEvent(st, ss->join, 0) != cudaSuccess)
-                return fail(SPT_ERR_CUDA, "sparse_attn_bwd: join of the side stream failed");
-            return SPT_OK;
-        }
-    }
+                      const uint32_t *mask, const int32_t *extra0, const float *delta, const float *zsum, T *gq, T *gk,
+                      T *gv, int B, int S, int H, float scale, float clamp, cudaStream_t st) {
     if (D == 64 && tile128()) {
+        {
+            // The dK/dV and the dQ kernel are independent: the dQ kernel goes to a side stream (fork / join with events,
+            // which a stream capture records as graph edges), so its CTAs start on each SM as that SM's dK/dV CTA retires
+            // instead of after the whole grid has drained (both are one-CTA-per-SM persistent grids: they never share an SM).
+            std::lock_guard<std::mutex> lock(g_side_mu);
+            SideStream *ss = side_stream(st);
+            if (ss) {
+                if (cudaEventRecord(ss->fork, st) != cudaSuccess || cudaStreamWaitEvent(ss->stream, ss->fork, 0) != cudaSuccess)
+                    return fail(SPT_ERR_CUDA, "sparse_attn_bwd: fork to the side stream failed");
+                int rc = attn_tc128::launch_bwd_kv128(mq, mk, mv, md, mask, extra0, delta, zsum, gk, gv, B, S, H, scale, clamp, st);
+                if (rc != SPT_OK) return rc;
+                rc = attn_tc128::launch_bwd_q128(mq, mk, mv, md, mask, extra0, delta, zsum, gq, B, S, H, scale, clamp, ss->stream);
+                if (rc != SPT_OK) return rc;
+                if (cudaEventRecord(ss->join, ss->stream) != cudaSuccess || cudaStreamWaitEvent(st, ss->join, 0) != cudaSuccess)
+                    return fail(SPT_ERR_CUDA, "sparse_attn_bwd: join of the side stream failed");
+                return SPT_OK;
+            }
+        }
+        // no side stream (it is never created during a capture, so a process whose first backward is captured gets
+        // here): one kernel after the other on the caller's stream
         const int rc = attn_tc128::launch_bwd_kv128(mq, mk, mv, md, mask, extra0, delta, zsum, gk, gv, B, S, H, scale, clamp, st);
         if (rc != SPT_OK) return rc;
-    } else {
-        constexpr int kv_smem = Dim<D>::BWD_SMEM + (is_f16<T> ? STAGES * BN * 4 : 0);      // fp16: the rows' -o per stage
-        cudaFuncSetAttribute(attn_bwd_kv_tc_kernel<D, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, kv_smem);
-        attn_bwd_kv_tc_kernel<D, T><<<dim3(B, S / BM), THREADS, kv_smem, st>>>(
-            mq, mk, mv, md, mask, extra0, delta, gk, gv, S, H, scale, scale * LOG2E, clamp * LOG2E, zsum);
-        SPT_LAUNCH_CHECK("attn_bwd_kv_tc_kernel");
+        return attn_tc128::launch_bwd_q128(mq, mk, mv, md, mask, extra0, delta, zsum, gq, B, S, H, scale, clamp, st);
     }
-    if (D == 64 && tile128()) return attn_tc128::launch_bwd_q128(mq, mk, mv, md, mask, extra0, delta, zsum, gq, B, S, H, scale, clamp, st);
+    constexpr int kv_smem = Dim<D>::BWD_SMEM + (is_f16<T> ? STAGES * BN * 4 : 0);      // fp16: the rows' -o per stage
+    cudaFuncSetAttribute(attn_bwd_kv_tc_kernel<D, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, kv_smem);
+    attn_bwd_kv_tc_kernel<D, T><<<dim3(B, S / BM), THREADS, kv_smem, st>>>(
+        mq, mk, mv, md, mask, extra0, delta, gk, gv, S, H, scale, scale * LOG2E, clamp * LOG2E, zsum);
+    SPT_LAUNCH_CHECK("attn_bwd_kv_tc_kernel");
     cudaFuncSetAttribute(attn_bwd_q_tc_kernel<D, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, Dim<D>::BWD_SMEM);
     attn_bwd_q_tc_kernel<D, T><<<dim3(B, S / BM), THREADS, Dim<D>::BWD_SMEM, st>>>(
         mq, mk, mv, md, mask, extra0, delta, gq, S, H, scale, scale * LOG2E, clamp * LOG2E, zsum);
@@ -1064,7 +1044,6 @@ static int attn_bwd_typed(const void *q, const void *k, const void *v, const voi
     constexpr bool f16 = attn_tc::is_f16<T>;
     float *delta = (float *)workspace;
     T *dys = (T *)((char *)workspace + (size_t)B * S * sizeof(float));
-    float *dq_acc = (float *)((char *)workspace + (size_t)B * S * sizeof(float) + (size_t)B * S * 128 * 2);
     // the row kernel goes first: besides producing dO' and delta' it is a runtime-API launch, which binds the
     // device's primary context to this (autograd worker) thread before the driver-API tensor-map encoder runs
     int rc = d == 64   ? attn_tc::launch_prep<64, T>((const T *)y, (const T *)grad_y, zsum, delta, dys, B, S, H, yt, st)
@@ -1078,10 +1057,10 @@ static int attn_bwd_typed(const void *q, const void *k, const void *v, const voi
     if ((rc = attn_tc::make_map(&md, dys, B / H, S, H, d, f16)) != SPT_OK) return rc;
     T *gq = (T *)grad_q, *gk = (T *)grad_k, *gv = (T *)grad_v;
     if (d == 64)
-        return attn_tc::launch_bwd<64, T>(mq, mk, mv, md, mask, extra0, delta, zsum, dq_acc, gq, gk, gv, B, S, H, scale, clamp, st);
+        return attn_tc::launch_bwd<64, T>(mq, mk, mv, md, mask, extra0, delta, zsum, gq, gk, gv, B, S, H, scale, clamp, st);
     if (d == 80)
-        return attn_tc::launch_bwd<80, T>(mq, mk, mv, md, mask, extra0, delta, zsum, dq_acc, gq, gk, gv, B, S, H, scale, clamp, st);
-    return attn_tc::launch_bwd<128, T>(mq, mk, mv, md, mask, extra0, delta, zsum, dq_acc, gq, gk, gv, B, S, H, scale, clamp, st);
+        return attn_tc::launch_bwd<80, T>(mq, mk, mv, md, mask, extra0, delta, zsum, gq, gk, gv, B, S, H, scale, clamp, st);
+    return attn_tc::launch_bwd<128, T>(mq, mk, mv, md, mask, extra0, delta, zsum, gq, gk, gv, B, S, H, scale, clamp, st);
 }
 
 extern "C" int spt_sparse_attn_fwd(const void *q, const void *k, const void *v, const uint32_t *mask,
@@ -1125,10 +1104,9 @@ extern "C" int spt_debug_attn_prof(unsigned long long *out48, int reset) {
 #endif
 }
 
-// workspace: delta' [B, S] fp32, then dO' (bf16, same shape as grad_y; sized for the largest head dim), then the fp32
-// dQ scratch of the one-pass backward (head dim 64)
+// workspace: delta' [B, S] fp32, then dO' (bf16 / fp16, same shape as grad_y; sized for the largest head dim)
 extern "C" size_t spt_sparse_attn_bwd_workspace_bytes(int B, int S) {
-    return (size_t)B * S * sizeof(float) + (size_t)B * S * 128 * 2 + (size_t)B * S * 64 * sizeof(float);
+    return (size_t)B * S * sizeof(float) + (size_t)B * S * 128 * 2;
 }
 
 extern "C" int spt_sparse_attn_bwd(const void *q, const void *k, const void *v, const void *y, const void *grad_y,

@@ -1,4 +1,4 @@
-// Fused PQ-sparse attention on 128 x 128 score tiles, ONE persistent CTA per SM (head dim 64).
+// Backward of the fused PQ-sparse attention on 128 x 128 score tiles, ONE persistent CTA per SM (head dim 64).
 //
 // Same mathematics, mask format and C ABI as attn_tc.cu (see its header); what changes is the shape of the work:
 //   * every tcgen05.mma is M128 x N128 (score products, operands in shared memory: 64 clk = the tensor pipe's peak) or
@@ -30,14 +30,10 @@ constexpr int ST = 3;                        // pipeline stages of the "other" t
 
 // Static schedule: items are ordered heaviest first; round w hands items [w G, (w + 1) G) to the G CTAs, in reversed CTA
 // order on odd rounds so that no CTA collects the heaviest item of every round (backward 0.393 -> 0.380 ms against plain
-// round-robin; -DSPT_SCHED_PLAIN restores that).  -1 = done.
+// round-robin).  -1 = done.
 __device__ __forceinline__ int sched_item(int round, int n_items) {
     const int G = gridDim.x;
-#ifdef SPT_SCHED_PLAIN
-    const int item = round * G + (int)blockIdx.x;
-#else
     const int item = round * G + ((round & 1) ? G - 1 - (int)blockIdx.x : (int)blockIdx.x);
-#endif
     return item < n_items ? item : -1;
 }
 
@@ -346,367 +342,6 @@ __device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&r)[16]) {
     tmem_ld16_nowait(taddr, r);
     tmem_ld_wait();
 }
-__device__ __forceinline__ void math_sync() { asm volatile("bar.sync 1, %0;" ::"n"(MATH_WARPS * 32) : "memory"); }
-
-// ---------------------------------------------------------------------------------------------------------------------
-// Backward, all three gradients in ONE pass over the score tiles.  OPT-IN (SPT_ATTN_BWD_FUSED=1): parity-green, but
-// measured no faster than the dK/dV + dQ kernel pair at the bench shape (0.383 vs 0.378 ms for the whole backward): the
-// math of the dQ kernel disappears (0.154 ms), and comes back as shared-memory traffic — the SS products (dK, dQ) fetch
-// their A tile at the full 128 B/clk of shared memory (48 clk per K16 step = 6 KB), next to the dS^T / staging stores
-// and the TMA reduction's reads — plus the reduction itself (0.043 ms) and the scratch clear / convert (0.03 ms).
-// Switch-by-switch timings in DESIGN.md section 4.1.  Owner / loop / element math are those of attn_bwd_kv128_kernel; what changes:
-//   * dS^T leaves the math warps as bf16 in SHARED memory: rows = keys, 64 queries per 128-byte row, 128-byte swizzle,
-//     two 64-query panels 16 KB apart.  That one buffer is the K-major A operand of dK += dS^T Q_j (M = keys,
-//     K = queries) and the MN-major A operand of dQ_j|kt = dS K (M = queries, K = keys; B = the own K tile, MN-major),
-//     so the element math of the separate dQ kernel (a second exp / mask / dS pass over every tile) disappears;
-//   * the partial dQ tile of every (key tile, query tile) pair is added into an fp32 scratch by the TMA unit: each math
-//     warp stages its 32 rows x 16 columns (2 KB) and issues one cp.reduce.async.bulk (.add.f32) — full-line
-//     reductions in L2, no per-lane atomics (REDG costs ~1.3 clk per LANE on this part).  The scratch is laid out as the
-//     staging blocks are ([head][query tile][warp][32 rows][64 B, chunk-swizzled]); dq_convert_kernel scales it into
-//     the bf16 gradient.  fp32 adds commute only approximately: dQ can differ in the last fp32 bit from run to run.
-// TMEM columns: S^T 0, dP'^T 128, E^T 256, dQ 320, dV 384, dK 448.  The own V tile is single-buffered (it is free as
-// soon as the item's last dP'^T product has been issued), which pays for the dS^T and staging buffers.
-// ---------------------------------------------------------------------------------------------------------------------
-constexpr int FUSED_SMEM = 3 * TILE + 2 * ST * TILE + 2 * TILE + 2 * TILE + ST * ROWQ + 256 + 1024;
-static_assert(FUSED_SMEM <= 227 * 1024, "fused backward: shared memory budget");
-
-__global__ void __launch_bounds__(THREADS, 1)
-attn_bwd_fused128_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_k,
-                         const __grid_constant__ CUtensorMap map_v, const __grid_constant__ CUtensorMap map_dys,
-                         const uint32_t *__restrict__ mask, const int32_t *__restrict__ extra0,
-                         const float *__restrict__ ndelta, float *__restrict__ dq_acc, __nv_bfloat16 *__restrict__ dk,
-                         __nv_bfloat16 *__restrict__ dv, int S, int H, int B, float scale, float scale_log2,
-                         float clamp_log2) {
-    extern __shared__ unsigned char smem_raw[];
-    const Smem sm = align_smem(smem_raw);
-    const uint32_t s_k = sm.base, s_v = s_k + 2 * TILE, s_q = s_v + TILE, s_dy = s_q + ST * TILE, s_ds = s_dy + ST * TILE,
-                   s_st = s_ds + 2 * TILE;
-    unsigned char *rowq = sm.ptr + (7 + 2 * ST) * TILE;
-    uint64_t *bars = reinterpret_cast<uint64_t *>(rowq + ST * ROWQ);
-    const uint32_t bar0 = smem_u32(bars);
-    auto own_full = [&](int i) { return bar0 + i * 8; };
-    auto own_empty = [&](int i) { return bar0 + 16 + i * 8; };
-    auto qd_full = [&](int s) { return bar0 + 32 + s * 8; };
-    auto qd_empty = [&](int s) { return bar0 + 32 + (ST + s) * 8; };
-    const uint32_t sc_full = bar0 + 32 + 2 * ST * 8, s_read = sc_full + 8, p_full = sc_full + 16, e_free = sc_full + 24,
-                   acc_full = sc_full + 32, acc_empty = sc_full + 40, v_full = sc_full + 48, v_empty = sc_full + 56,
-                   dq_empty = sc_full + 64;
-    uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(bars + 4 + 2 * ST + 9);
-
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int n_own = S / T;
-    const int n_items = n_own * B;
-    const int words = S / 32;
-
-    if (threadIdx.x == 0) {
-        for (int i = 0; i < 2; ++i) {
-            mbar_init(own_full(i), 1);
-            mbar_init(own_empty(i), 1);
-        }
-        for (int s = 0; s < ST; ++s) {
-            mbar_init(qd_full(s), 2);                  // expect_tx arrive + the producer warp's row data
-            mbar_init(qd_empty(s), 1);
-        }
-        mbar_init(sc_full, 1);
-        mbar_init(s_read, MATH_WARPS);
-        mbar_init(p_full, MATH_WARPS);
-        mbar_init(e_free, 1);
-        mbar_init(acc_full, 1);
-        mbar_init(acc_empty, MATH_WARPS);
-        mbar_init(v_full, 1);
-        mbar_init(v_empty, 1);
-        mbar_init(dq_empty, MATH_WARPS);
-        mbar_fence_init();
-    }
-    if (warp == W_MMA) tmem_alloc<512>(smem_u32(tmem_slot));
-    fence_before_sync();
-    __syncthreads();
-    fence_after_sync();
-    const uint32_t tmem_base = *tmem_slot;
-    constexpr uint32_t COL_S = 0, COL_DP = 128, COL_E = 256, COL_DQ = 320, COL_DV = 384, COL_DK = 448;
-
-    if (warp == W_TMA) {
-        // ===== producer: own K (double-buffered) and V (single) of the next item, query-side tiles + row data per stage =====
-        int g = 0, w = 0;
-        for (int item; (item = sched_item(w, n_items)) >= 0; ++w) {
-            const int kt = item / B, b = item % B;
-            const int hn = b / H, hh = b % H, n0 = kt * T, n_tiles = n_own - kt;
-            const size_t head = (size_t)b * S;
-            const int buf = w & 1;
-            if (lane == 0) {
-                mbar_wait(own_empty(buf), ((w >> 1) & 1) ^ 1);
-                mbar_expect_tx(own_full(buf), TILE);
-                tma_owner<D>(s_k + buf * TILE, &map_k, own_full(buf), hh, n0, hn);
-                mbar_wait(v_empty, (w & 1) ^ 1);       // the previous item's last dP'^T product has read V
-                mbar_expect_tx(v_full, TILE);
-                tma_owner<D>(s_v, &map_v, v_full, hh, n0, hn);
-            }
-            uint4 mw[4];
-#pragma unroll
-            for (int u = 0; u < 4; ++u)
-                mw[u] = __ldg(reinterpret_cast<const uint4 *>(mask + (head + n0 + lane + 32 * u) * words) + kt);
-            for (int j = 0; j < n_tiles; ++j, ++g) {
-                const int st = g % ST;
-                const int r0 = (kt + j) * T;
-                unsigned char *slot = rowq + st * ROWQ;
-                mbar_wait(qd_empty(st), ((g / ST) & 1) ^ 1);
-                if (lane == 0) {
-                    mbar_expect_tx(qd_full(st), 2 * TILE + 2 * T * 4);
-                    tma_owner<D>(s_q + st * TILE, &map_q, qd_full(st), hh, r0, hn);
-                    tma_owner<D>(s_dy + st * TILE, &map_dys, qd_full(st), hh, r0, hn);
-                    bulk_load_1d(smem_u32(slot + MT * 16), ndelta + head + r0, T * 4, qd_full(st));
-                    bulk_load_1d(smem_u32(slot + MT * 16 + T * 4), extra0 + head + r0, T * 4, qd_full(st));
-                }
-                uint32_t *mt = reinterpret_cast<uint32_t *>(slot);        // transposed: [word t][row], rows padded to MT
-#pragma unroll
-                for (int u = 0; u < 4; ++u) {
-                    const int rr = lane + 32 * u;
-                    mt[rr] = mw[u].x;
-                    mt[MT + rr] = mw[u].y;
-                    mt[2 * MT + rr] = mw[u].z;
-                    mt[3 * MT + rr] = mw[u].w;
-                }
-                if (j + 1 < n_tiles) {
-#pragma unroll
-                    for (int u = 0; u < 4; ++u)
-                        mw[u] = __ldg(reinterpret_cast<const uint4 *>(mask + (head + r0 + T + lane + 32 * u) * words) + kt);
-                }
-                __syncwarp();
-                if (lane == 0) mbar_arrive(qd_full(st));
-            }
-        }
-    } else if (warp == W_MMA) {
-        // ===== MMA issuer =====
-        constexpr uint32_t id_s = idesc_bf16(T, T, 0, 0);     // S^T = K Q^T, dP'^T = V dO'^T
-        constexpr uint32_t id_a = idesc_bf16(T, D, 0, 1);     // dV += E^T dO' (A in TMEM), dK += dS^T Q (A K-major); B MN-major
-        constexpr uint32_t id_q = idesc_bf16(T, D, 1, 1);     // dQ = dS K: A = the dS^T buffer read MN-major, B = K MN-major
-        const uint64_t dk0 = desc_kmajor(s_k, 0), dv0 = desc_kmajor(s_v, 0), dq0 = desc_kmajor(s_q, 0),
-                       ddy0 = desc_kmajor(s_dy, 0), dqt0 = desc_mnmajor(s_q, 0, TILE), ddyt0 = desc_mnmajor(s_dy, 0, TILE),
-                       dkt0 = desc_mnmajor(s_k, 0, TILE), dds_k0 = desc_kmajor(s_ds, 0), dds_m0 = desc_mnmajor(s_ds, 0, TILE);
-        int g = 0, w = 0;
-        PROF(Prof pf; pf.start(); const long long t0 = pf.last;)
-        for (int item; (item = sched_item(w, n_items)) >= 0; ++w) {
-            const int kt = item / B, n_tiles = n_own - kt;
-            const int buf = w & 1;
-            const uint64_t own_off = (uint64_t)((buf * TILE) >> 4);
-            auto issue_scores = [&](int gg, bool last) {       // tile with running index gg; last: of this item
-                const int st = gg % ST;
-                mbar_wait(qd_full(st), (gg / ST) & 1);
-                if (gg > 0) mbar_wait(s_read, (gg - 1) & 1);   // the previous tile's scores are in registers
-                fence_after_sync();
-                if (elect_one()) {
-                    const uint64_t off = (uint64_t)((st * TILE) >> 4);
-#pragma unroll
-                    for (int k = 0; k < D / 16; ++k) {
-                        umma_bf16(tmem_base + COL_S, dk0 + own_off + k * KMAJOR_K16, dq0 + off + k * KMAJOR_K16, id_s, k != 0);
-                        umma_bf16(tmem_base + COL_DP, dv0 + k * KMAJOR_K16, ddy0 + off + k * KMAJOR_K16, id_s, k != 0);
-                    }
-                    umma_commit(sc_full);
-                    if (last) umma_commit(v_empty);
-                }
-                __syncwarp();
-            };
-            mbar_wait(own_full(buf), (w >> 1) & 1);
-            mbar_wait(v_full, w & 1);
-            issue_scores(g, n_tiles == 1);
-            for (int j = 0; j < n_tiles; ++j, ++g) {
-                PROF(pf.lap(2);)
-                if (j + 1 < n_tiles) issue_scores(g + 1, j + 2 == n_tiles);
-                PROF(pf.lap(0);)
-                const int st = g % ST;
-                const uint64_t off = (uint64_t)((st * TILE) >> 4);
-                mbar_wait(p_full, g & 1);
-                if (j == 0 && w > 0) mbar_wait(acc_empty, (w - 1) & 1);     // the previous item's dV / dK have been read
-                PROF(pf.lap(1);)
-                fence_after_sync();
-                if (elect_one()) {
-#pragma unroll
-                    for (int k = 0; k < T / 16; ++k) {         // query rows 16 k .. 16 k + 15
-                        umma_bf16_ts(tmem_base + COL_DV, tmem_base + COL_E + k * 8, ddyt0 + off + k * MNMAJOR_K16, id_a, (j | k) != 0);
-                        umma_bf16(tmem_base + COL_DK, dds_k0 + (uint64_t)((k >> 2) * (TILE >> 4)) + (k & 3) * KMAJOR_K16,
-                                  dqt0 + off + k * MNMAJOR_K16, id_a, (j | k) != 0);
-                    }
-                }
-                __syncwarp();
-                if (g > 0) mbar_wait(dq_empty, (g - 1) & 1);   // the previous partial dQ tile has been read out of TMEM
-                fence_after_sync();
-                if (elect_one()) {
-#pragma unroll
-                    for (int k = 0; k < T / 16; ++k)           // keys 16 k .. 16 k + 15
-                        umma_bf16(tmem_base + COL_DQ, dds_m0 + k * MNMAJOR_K16, dkt0 + own_off + k * MNMAJOR_K16, id_q, k != 0);
-                    umma_commit(qd_empty(st));
-                    umma_commit(e_free);
-                    if (j + 1 == n_tiles) {
-                        umma_commit(acc_full);
-                        umma_commit(own_empty(buf));
-                    }
-                }
-                __syncwarp();
-            }
-        }
-        PROF(pf.t[3] = clock64() - t0; pf.t[4] = g; pf.flush(2, 8, lane == 0);)
-    } else {
-        // ===== math warps: thread = (key = TMEM lane, 32 query columns) =====
-        const int quarter = warp & 3, cg = warp >> 2;
-        const int kk = quarter * 32 + lane;
-        const int wsel = kk & 3;
-        const int shl = 31 - (kk >> 2);                 // moves this key's bit of a lane-major word to the sign bit
-        const MathK mk = make_math(scale_log2, clamp_log2);
-        const uint32_t lane_base = tmem_base + ((uint32_t)(quarter * 32) << 16);
-        const int c0 = cg * 32;                         // query rows c0 .. c0 + 31 of every tile
-        // this key's row of the dS^T buffer: panel (c0 / 64), 16-byte chunks 4 (cg & 1) .. + 3, XOR-swizzled by the row
-        const uint32_t ds_row = s_ds + (cg >> 1) * TILE + kk * 128;
-        const int ds_ch = (cg & 1) * 4, ds_sw = kk & 7;
-        // dQ staging block of this warp: 32 rows (queries quarter * 32 + lane) x 64 bytes (columns 16 cg .. + 15)
-        const uint32_t st_blk = s_st + warp * 2048, st_row = st_blk + lane * 64;
-        const int st_sw = (lane >> 1) & 3;
-        int g = 0, w = 0;
-        PROF(long long fx[2] = {0, 0};)
-        PROF(Prof pf; pf.start(); const long long t0 = pf.last;)
-        for (int item; (item = sched_item(w, n_items)) >= 0; ++w) {
-            const int kt = item / B, b = item % B;
-            const int hn = b / H, hh = b % H, n0 = kt * T, n_tiles = n_own - kt;
-            const bool key0 = (n0 + kk) == 0;
-            // partial dQ of query tile qt: TMEM -> staging block -> bulk add-reduction into the scratch
-            auto dq_flush = [&](int qt) {
-                PROF(const long long f0 = clock64();)
-                if (lane == 0) bulk_wait_read0();       // this warp's previous reduction has read the staging block
-                __syncwarp();
-                PROF(const long long f1 = clock64(); fx[0] += f1 - f0;)
-                uint32_t o[16];
-                tmem_ld16(lane_base + COL_DQ + cg * 16, o);
-                warp_arrive(dq_empty, lane);
-                PROF(fx[1] += clock64() - f1;)
-#pragma unroll
-                for (int c = 0; c < 4; ++c)
-                    st_shared_v4(st_row + ((c ^ st_sw) << 4), o[4 * c], o[4 * c + 1], o[4 * c + 2], o[4 * c + 3]);
-                fence_proxy_async();
-                __syncwarp();
-                if (lane == 0) {
-                    bulk_reduce_add_f32(dq_acc + (((size_t)b * n_own + qt) * MATH_WARPS + warp) * 512, st_blk, 2048);
-                    bulk_commit();
-                }
-            };
-            for (int j = 0; j < n_tiles; ++j, ++g) {
-                const int st = g % ST;
-                const unsigned char *slot = rowq + st * ROWQ;
-                const uint32_t *mrow = reinterpret_cast<const uint32_t *>(slot) + wsel * MT;   // this key's word of every row
-                const float *s_nd = reinterpret_cast<const float *>(slot + MT * 16);
-                const int32_t *s_ex0 = reinterpret_cast<const int32_t *>(slot + MT * 16 + T * 4);
-                mbar_wait(qd_full(st), (g / ST) & 1);
-                mbar_wait(sc_full, g & 1);
-                PROF(pf.lap(0);)
-                fence_after_sync();
-                uint32_t r[32], gr[32];
-                tmem_ld32_nowait(lane_base + COL_S + c0, r);
-                tmem_ld32_nowait(lane_base + COL_DP + c0, gr);
-                tmem_ld_wait();
-                warp_arrive(s_read, lane);
-                PROF(pf.lap(1);)
-                const bool clamp = warp_needs_clamp(r, mk.thr);
-                bool pad = false;                       // see attn_bwd_kv128_kernel
-                if (key0) {
-#pragma unroll
-                    for (int i = 0; i < 32; i += 4) {
-                        const int4 e4 = *reinterpret_cast<const int4 *>(s_ex0 + c0 + i);
-                        pad |= (e4.x | e4.y | e4.z | e4.w) != 0;
-                    }
-                }
-                uint32_t pe0[8], pd0[8], pe1[8], pd1[8];
-#define SPT_KV_HALF(OFF, PE, PD)                                                                                           \
-                if (pad) {                                                                                                \
-                    if (clamp) bwdkv_chunk16<true, true, OFF, 32>(r, gr, mrow, s_nd, s_ex0, c0 + OFF, shl, mk, PE, PD);    \
-                    else bwdkv_chunk16<true, false, OFF, 32>(r, gr, mrow, s_nd, s_ex0, c0 + OFF, shl, mk, PE, PD);         \
-                } else {                                                                                                   \
-                    if (clamp) bwdkv_chunk16<false, true, OFF, 32>(r, gr, mrow, s_nd, s_ex0, c0 + OFF, shl, mk, PE, PD);   \
-                    else bwdkv_chunk16<false, false, OFF, 32>(r, gr, mrow, s_nd, s_ex0, c0 + OFF, shl, mk, PE, PD);        \
-                }
-                SPT_KV_HALF(0, pe0, pd0)
-                SPT_KV_HALF(16, pe1, pd1)
-#undef SPT_KV_HALF
-                PROF(pf.lap(2);)
-                if (g > 0) {                            // the previous tile's E^T / dS^T have been consumed (and its dQ is complete)
-                    mbar_wait(e_free, (g - 1) & 1);
-                    fence_after_sync();
-                }
-                PROF(pf.lap(3);)
-                tmem_st8(lane_base + COL_E + c0 / 2, pe0);
-                tmem_st8(lane_base + COL_E + c0 / 2 + 8, pe1);
-                st_shared_v4(ds_row + (((ds_ch + 0) ^ ds_sw) << 4), pd0[0], pd0[1], pd0[2], pd0[3]);
-                st_shared_v4(ds_row + (((ds_ch + 1) ^ ds_sw) << 4), pd0[4], pd0[5], pd0[6], pd0[7]);
-                st_shared_v4(ds_row + (((ds_ch + 2) ^ ds_sw) << 4), pd1[0], pd1[1], pd1[2], pd1[3]);
-                st_shared_v4(ds_row + (((ds_ch + 3) ^ ds_sw) << 4), pd1[4], pd1[5], pd1[6], pd1[7]);
-                fence_proxy_async();
-                tmem_st_wait();
-                warp_arrive(p_full, lane);
-                PROF(pf.lap(5);)
-                if (j > 0) dq_flush(kt + j - 1);        // complete since e_free(g - 1)
-                PROF(pf.lap(7);)
-            }
-            // epilogue: the last partial dQ, then column group 0, 1 -> dV halves, 2, 3 -> dK halves (dK follows dV in TMEM)
-            mbar_wait(acc_full, w & 1);
-            fence_after_sync();
-            dq_flush(kt + n_tiles - 1);
-            {
-                uint32_t o[32];
-                tmem_ld32(lane_base + COL_DV + c0, o);
-                warp_arrive(acc_empty, lane);
-                const size_t off = (((size_t)hn * S + n0 + kk) * H + hh) * D + (cg & 1) * 32;
-                store_row32((cg < 2 ? dv : dk) + off, o, cg < 2 ? 1.0f : scale);
-            }
-            PROF(pf.last = clock64();)
-        }
-        if (lane == 0) bulk_wait0();                    // every reduction of this warp has landed
-        PROF(pf.t[6] = clock64() - t0; pf.t[4] = g; pf.flush(2, 0, threadIdx.x == 0);)
-        PROF(if (threadIdx.x == 0) { atomicAdd(&g_prof[2][13], (unsigned long long)fx[0]); atomicAdd(&g_prof[2][14], (unsigned long long)fx[1]); })
-    }
-    fence_before_sync();
-    __syncthreads();
-    if (warp == W_MMA) tmem_dealloc<512>(tmem_base);
-}
-
-// fp32 scratch ([head][query tile][warp = 4 cg + quarter][32 rows][4 chunks of 16 B, chunk c at c ^ ((row >> 1) & 3)])
-// -> bf16 dQ in the layer layout, scaled.  One thread per (row, 16 columns).
-__global__ void __launch_bounds__(256)
-dq_convert_kernel(const float *__restrict__ acc, __nv_bfloat16 *__restrict__ dq, int S, int H, int n_own, float scale,
-                  long long n_threads) {
-    const long long t = (long long)blockIdx.x * 256 + threadIdx.x;
-    if (t >= n_threads) return;
-    const int lane = (int)(t & 31);
-    const long long blk = t >> 5;
-    const int wv = (int)(blk % MATH_WARPS);
-    const long long bq = blk / MATH_WARPS;
-    const int qt = (int)(bq % n_own), b = (int)(bq / n_own);
-    const int quarter = wv & 3, cg = wv >> 2;
-    const int row = qt * T + quarter * 32 + lane;
-    const float4 *src = reinterpret_cast<const float4 *>(acc + blk * 512 + lane * 16);
-    const int sw = (lane >> 1) & 3;
-    __nv_bfloat16 *dst = dq + (((size_t)(b / H) * S + row) * H + (b % H)) * D + cg * 16;
-#pragma unroll
-    for (int h = 0; h < 2; ++h) {
-        const float4 x = src[(2 * h) ^ sw], y = src[(2 * h + 1) ^ sw];
-        float v[8] = {x.x * scale, x.y * scale, x.z * scale, x.w * scale, y.x * scale, y.y * scale, y.z * scale, y.w * scale};
-        Vec16<__nv_bfloat16>::store(dst + 8 * h, v);
-    }
-}
-
-int launch_bwd_fused128(const CUtensorMap &mq, const CUtensorMap &mk, const CUtensorMap &mv, const CUtensorMap &md,
-                        const uint32_t *mask, const int32_t *extra0, const float *ndelta, float *dq_acc,
-                        __nv_bfloat16 *gq, __nv_bfloat16 *gk, __nv_bfloat16 *gv, int B, int S, int H, float scale,
-                        float clamp, cudaStream_t st) {
-    cudaFuncSetAttribute(attn_bwd_fused128_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, FUSED_SMEM);
-    if (cudaMemsetAsync(dq_acc, 0, (size_t)B * S * D * sizeof(float), st) != cudaSuccess)
-        return fail(SPT_ERR_CUDA, "sparse_attn_bwd: clearing the dQ scratch failed");
-    const int n_items = (S / T) * B;
-    const int grid = n_items < num_sms() ? n_items : num_sms();
-    attn_bwd_fused128_kernel<<<grid, THREADS, FUSED_SMEM, st>>>(mq, mk, mv, md, mask, extra0, ndelta, dq_acc, gk, gv, S, H,
-                                                               B, scale, scale * LOG2E, clamp * LOG2E);
-    SPT_LAUNCH_CHECK("attn_bwd_fused128_kernel");
-    const long long n_threads = (long long)B * S * (D / 16);
-    dq_convert_kernel<<<(unsigned)((n_threads + 255) / 256), 256, 0, st>>>(dq_acc, gq, S, H, S / T, scale, n_threads);
-    return after_launch("dq_convert_kernel");
-}
-
 
 // ---------------------------------------------------------------------------------------------------------------------
 // Backward, dQ.  Owner = 128 query rows (Q, dO'), loop over the 128-key tiles 0 .. diagonal (K_j, V_j).
@@ -907,221 +542,6 @@ attn_bwd_q128_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
     if (warp == W_MMA) tmem_dealloc<512>(tmem_base);
 }
 
-// ---------------------------------------------------------------------------------------------------------------------
-// Forward.  Owner = 128 query rows (Q), loop over the 128-key tiles 0 .. diagonal (K_j, V_j).
-//   S = Q K_j^T,  P = w exp(clamp(scale S)) as a bf16 TMEM A-operand,  O += P V_j;  y = O / Z, Z = max(1e-9, row sum of P).
-// TMEM columns: S 0, P[2] 128 / 192, O 256.
-// ---------------------------------------------------------------------------------------------------------------------
-constexpr int F_SMEM = 2 * TILE + 2 * ST * TILE + 4 * T * 4 + 256 + 1024;
-
-__global__ void __launch_bounds__(THREADS, 1)
-attn_fwd128_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_k,
-                   const __grid_constant__ CUtensorMap map_v, const uint32_t *__restrict__ mask,
-                   const int32_t *__restrict__ extra0, __nv_bfloat16 *__restrict__ y, float *__restrict__ zsum, int S,
-                   int H, int B, float scale_log2, float clamp_log2, int y_transposed) {
-    extern __shared__ unsigned char smem_raw[];
-    const Smem sm = align_smem(smem_raw);
-    const uint32_t s_q = sm.base, s_k = s_q + 2 * TILE, s_v = s_k + ST * TILE;
-    float *s_part = reinterpret_cast<float *>(sm.ptr + 2 * TILE + 2 * ST * TILE);      // [4][128] partial row sums
-    uint64_t *bars = reinterpret_cast<uint64_t *>(sm.ptr + 2 * TILE + 2 * ST * TILE + 4 * T * 4);
-    const uint32_t bar0 = smem_u32(bars);
-    auto own_full = [&](int i) { return bar0 + i * 8; };
-    auto own_empty = [&](int i) { return bar0 + 16 + i * 8; };
-    auto k_full = [&](int s) { return bar0 + 32 + s * 8; };
-    auto k_empty = [&](int s) { return bar0 + 32 + (ST + s) * 8; };
-    auto v_full = [&](int s) { return bar0 + 32 + (2 * ST + s) * 8; };
-    auto v_empty = [&](int s) { return bar0 + 32 + (3 * ST + s) * 8; };
-    const uint32_t sc_full = bar0 + 32 + 4 * ST * 8, s_read = sc_full + 8, acc_full = sc_full + 16, acc_empty = sc_full + 24;
-    auto p_full = [&](int i) { return sc_full + 32 + i * 8; };
-    auto e_free = [&](int i) { return sc_full + 48 + i * 8; };
-    uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(bars + 4 + 4 * ST + 8);
-
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int n_own = S / T;
-    const int n_items = n_own * B;
-
-    if (threadIdx.x == 0) {
-        for (int i = 0; i < 2; ++i) {
-            mbar_init(own_full(i), 1);
-            mbar_init(own_empty(i), 1);
-            mbar_init(p_full(i), MATH_WARPS);
-            mbar_init(e_free(i), 1);
-        }
-        for (int s = 0; s < ST; ++s) {
-            mbar_init(k_full(s), 1);
-            mbar_init(k_empty(s), 1);
-            mbar_init(v_full(s), 1);
-            mbar_init(v_empty(s), 1);
-        }
-        mbar_init(sc_full, 1);
-        mbar_init(s_read, MATH_WARPS);
-        mbar_init(acc_full, 1);
-        mbar_init(acc_empty, MATH_WARPS);
-        mbar_fence_init();
-    }
-    if (warp == W_MMA) tmem_alloc<512>(smem_u32(tmem_slot));
-    fence_before_sync();
-    __syncthreads();
-    fence_after_sync();
-    const uint32_t tmem_base = *tmem_slot;
-    constexpr uint32_t COL_S = 0, COL_P = 128, COL_O = 256;
-
-    if (warp == W_TMA) {
-        if (lane == 0) {
-            int g = 0, w = 0;
-            for (int item; (item = sched_item(w, n_items)) >= 0; ++w) {
-                const int qt = n_own - 1 - item / B, b = item % B;
-                const int hn = b / H, hh = b % H, n_tiles = qt + 1;
-                const int buf = w & 1;
-                mbar_wait(own_empty(buf), ((w >> 1) & 1) ^ 1);
-                mbar_expect_tx(own_full(buf), TILE);
-                tma_owner<D>(s_q + buf * TILE, &map_q, own_full(buf), hh, qt * T, hn);
-                for (int j = 0; j < n_tiles; ++j, ++g) {
-                    const int st = g % ST;
-                    const uint32_t ph = ((g / ST) & 1) ^ 1;
-                    mbar_wait(k_empty(st), ph);
-                    mbar_expect_tx(k_full(st), TILE);
-                    tma_owner<D>(s_k + st * TILE, &map_k, k_full(st), hh, j * T, hn);
-                    mbar_wait(v_empty(st), ph);
-                    mbar_expect_tx(v_full(st), TILE);
-                    tma_owner<D>(s_v + st * TILE, &map_v, v_full(st), hh, j * T, hn);
-                }
-            }
-        }
-    } else if (warp == W_MMA) {
-        constexpr uint32_t id_s = idesc_bf16(T, T, 0, 0);     // S = Q K^T
-        constexpr uint32_t id_o = idesc_bf16(T, D, 0, 1);     // O += P V   (A in TMEM, V MN-major)
-        const uint64_t dq0 = desc_kmajor(s_q, 0), dk0 = desc_kmajor(s_k, 0), dvt0 = desc_mnmajor(s_v, 0, TILE);
-        int g = 0, w = 0;
-        PROF(Prof pf; pf.start(); const long long t0 = pf.last;)
-        for (int item; (item = sched_item(w, n_items)) >= 0; ++w) {
-            const int n_tiles = n_own - item / B;
-            const int buf = w & 1;
-            const uint64_t own_off = (uint64_t)((buf * TILE) >> 4);
-            auto issue_scores = [&](int gg) {
-                const int st = gg % ST;
-                mbar_wait(k_full(st), (gg / ST) & 1);
-                if (gg > 0) mbar_wait(s_read, (gg - 1) & 1);
-                fence_after_sync();
-                if (elect_one()) {
-                    const uint64_t off = (uint64_t)((st * TILE) >> 4);
-#pragma unroll
-                    for (int k = 0; k < D / 16; ++k)
-                        umma_bf16(tmem_base + COL_S, dq0 + own_off + k * KMAJOR_K16, dk0 + off + k * KMAJOR_K16, id_s, k != 0);
-                    umma_commit(sc_full);
-                    umma_commit(k_empty(st));
-                }
-                __syncwarp();
-            };
-            mbar_wait(own_full(buf), (w >> 1) & 1);
-            issue_scores(g);
-            for (int j = 0; j < n_tiles; ++j, ++g) {
-                PROF(pf.lap(2);)
-                if (j + 1 < n_tiles) issue_scores(g + 1);
-                PROF(pf.lap(0);)
-                const int st = g % ST;
-                mbar_wait(p_full(g & 1), (g >> 1) & 1);
-                mbar_wait(v_full(st), (g / ST) & 1);
-                if (j == 0 && w > 0) mbar_wait(acc_empty, (w - 1) & 1);
-                PROF(pf.lap(1);)
-                fence_after_sync();
-                if (elect_one()) {
-                    const uint64_t off = (uint64_t)((st * TILE) >> 4);
-#pragma unroll
-                    for (int k = 0; k < T / 16; ++k)
-                        umma_bf16_ts(tmem_base + COL_O, tmem_base + COL_P + (g & 1) * 64 + k * 8, dvt0 + off + k * MNMAJOR_K16, id_o,
-                                     (j | k) != 0);
-                    umma_commit(v_empty(st));
-                    umma_commit(e_free(g & 1));
-                    if (j + 1 == n_tiles) {
-                        umma_commit(acc_full);
-                        umma_commit(own_empty(buf));
-                    }
-                }
-                __syncwarp();
-            }
-        }
-        PROF(pf.t[3] = clock64() - t0; pf.t[4] = g; pf.flush(0, 8, lane == 0);)
-    } else {
-        // ===== math warps: thread = (query row = TMEM lane, 32 key columns) =====
-        const int quarter = warp & 3, cg = warp >> 2;
-        const int rt = quarter * 32 + lane;
-        const MathK mk = make_math(scale_log2, clamp_log2);
-        const uint32_t lane_base = tmem_base + ((uint32_t)(quarter * 32) << 16);
-        int g = 0, w = 0;
-        PROF(Prof pf; pf.start(); const long long t0 = pf.last;)
-        for (int item; (item = sched_item(w, n_items)) >= 0; ++w) {
-            const int qt = n_own - 1 - item / B, b = item % B;
-            const int hn = b / H, hh = b % H, n_tiles = qt + 1;
-            const int row = qt * T + rt;
-            const size_t grow = (size_t)b * S + row;
-            const uint4 *mrow = reinterpret_cast<const uint4 *>(mask + grow * (S / 32));
-            const float ex0 = (float)extra0[grow];
-            uint64_t sum2 = pk2(0.0f, 0.0f);
-            uint4 mw = __ldg(mrow);
-            for (int j = 0; j < n_tiles; ++j, ++g) {
-                const uint4 mw_next = (j + 1 < n_tiles) ? __ldg(mrow + j + 1) : mw;
-                mbar_wait(sc_full, g & 1);
-                PROF(pf.lap(0);)
-                fence_after_sync();
-                uint32_t r[32];
-                tmem_ld32(lane_base + COL_S + cg * 32, r);
-                warp_arrive(s_read, lane);
-                PROF(pf.lap(1);)
-                const uint32_t X = chunk_mask_bytes(mw, cg);
-                uint32_t pk[16];
-                const bool first = (j == 0 && cg == 0);
-                if (!warp_needs_clamp(r, mk.thr)) {
-                    if (first) fwd_chunk32<true, false>(r, X, mk, ex0, sum2, pk);
-                    else fwd_chunk32<false, false>(r, X, mk, ex0, sum2, pk);
-                } else {
-                    if (first) fwd_chunk32<true, true>(r, X, mk, ex0, sum2, pk);
-                    else fwd_chunk32<false, true>(r, X, mk, ex0, sum2, pk);
-                }
-                PROF(pf.lap(2);)
-                if (g >= 2) {
-                    mbar_wait(e_free(g & 1), ((g >> 1) - 1) & 1);
-                    fence_after_sync();
-                }
-                tmem_st16(lane_base + COL_P + (g & 1) * 64 + cg * 16, pk);
-                tmem_st_wait();
-                warp_arrive(p_full(g & 1), lane);
-                PROF(pf.lap(3);)
-                mw = mw_next;
-            }
-            float sum;
-            {
-                float lo, hi;
-                up2(sum2, lo, hi);
-                sum = lo + hi;
-            }
-            s_part[cg * T + rt] = sum;
-            math_sync();
-            sum = fmaxf((s_part[rt] + s_part[T + rt]) + (s_part[2 * T + rt] + s_part[3 * T + rt]), 1e-9f);
-            if (cg == 0) zsum[grow] = sum;
-            const float inv = 1.0f / sum;
-            mbar_wait(acc_full, w & 1);
-            fence_after_sync();
-            uint32_t o[16];
-            tmem_ld16(lane_base + COL_O + cg * 16, o);
-            warp_arrive(acc_empty, lane);
-            if (!y_transposed) {
-                store_row16(y + (((size_t)hn * S + row) * H + hh) * D + cg * 16, o, inv);
-            } else {
-                // the shipped reference layer's output layout (attention.py:139-142): y^T [B, D, S] memory
-                __nv_bfloat16 *dst = y + ((size_t)b * D + cg * 16) * S + row;
-#pragma unroll
-                for (int i = 0; i < 16; ++i) dst[(size_t)i * S] = __float2bfloat16(__uint_as_float(o[i]) * inv);
-            }
-            PROF(pf.lap(5);)
-        }
-        PROF(pf.t[6] = clock64() - t0; pf.t[4] = g; pf.flush(0, 0, threadIdx.x == 0);)
-    }
-    fence_before_sync();
-    __syncthreads();
-    if (warp == W_MMA) tmem_dealloc<512>(tmem_base);
-}
-
 static int grid_for(int n_items) { return n_items < num_sms() ? n_items : num_sms(); }
 
 template <typename E>
@@ -1139,15 +559,6 @@ template int launch_bwd_q128<__nv_bfloat16>(const CUtensorMap &, const CUtensorM
 template int launch_bwd_q128<__half>(const CUtensorMap &, const CUtensorMap &, const CUtensorMap &, const CUtensorMap &,
                                      const uint32_t *, const int32_t *, const float *, const float *, __half *, int, int,
                                      int, float, float, cudaStream_t);
-
-int launch_fwd128(const CUtensorMap &mq, const CUtensorMap &mk, const CUtensorMap &mv, const uint32_t *mask,
-                  const int32_t *extra0, __nv_bfloat16 *y, float *zsum, int B, int S, int H, float scale, float clamp,
-                  int y_transposed, cudaStream_t st) {
-    cudaFuncSetAttribute(attn_fwd128_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, F_SMEM);
-    attn_fwd128_kernel<<<grid_for((S / T) * B), THREADS, F_SMEM, st>>>(mq, mk, mv, mask, extra0, y, zsum, S, H, B,
-                                                                      scale * LOG2E, clamp * LOG2E, y_transposed);
-    return after_launch("attn_fwd128_kernel");
-}
 
 }  // namespace attn_tc128
 }  // namespace spt

@@ -52,22 +52,6 @@ __device__ __forceinline__ void bulk_load_1d(uint32_t dst, const void *src, uint
                  ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
 }
 
-// 1-D bulk reduction shared -> global: global[i] += shared[i] (fp32), performed by the TMA unit in L2 (full lines, no
-// per-lane atomics).  Bulk-group completion: commit, then wait_group.read before the shared source is overwritten and
-// wait_group before relying on the global result / leaving the kernel.
-__device__ __forceinline__ void bulk_reduce_add_f32(const void *dst_global, uint32_t src_smem, uint32_t bytes) {
-    asm volatile("cp.reduce.async.bulk.global.shared::cta.bulk_group.add.f32 [%0], [%1], %2;"
-                 ::"l"(dst_global), "r"(src_smem), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-__device__ __forceinline__ void bulk_wait_read0() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
-__device__ __forceinline__ void bulk_wait0() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
-// generic-proxy shared-memory writes -> visible to the async proxy (UMMA operand reads, bulk copies out of shared memory)
-__device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-__device__ __forceinline__ void st_shared_v4(uint32_t addr, uint32_t a, uint32_t b, uint32_t c, uint32_t d) {
-    asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "r"(a), "r"(b), "r"(c), "r"(d) : "memory");
-}
-
 // One lane of a converged warp (warp-uniform control flow around it keeps operands in uniform registers).
 __device__ __forceinline__ bool elect_one() {
     uint32_t pred;

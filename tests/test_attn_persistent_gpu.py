@@ -403,57 +403,32 @@ def _child_pytest(env_extra, expr):
 
 
 @gpu
-@pytest.mark.parametrize("switch", ["SPT_ATTN_TILE=64", "SPT_ATTN_FWD128=1"])
+@pytest.mark.parametrize("switch", ["SPT_ATTN_TILE=64"])
 def test_switch_parity_and_batch_invariance(switch):
-    """SPT_ATTN_TILE=64 (128 x 64-tile backward) and SPT_ATTN_FWD128=1 (persistent 128 x 128 forward) are documented to
-    give the same results: the multi-round parity and the bit-exact batch invariance hold under each."""
+    """SPT_ATTN_TILE=64 (128 x 64-tile backward) is documented to give the same results: the multi-round parity and the
+    bit-exact batch invariance hold under it."""
     name, value = switch.split("=")
     _child_pytest({name: value}, "test_multi_round_parity or test_batch_invariance")
-
-
-@gpu
-def test_switch_one_pass_backward_parity():
-    """SPT_ATTN_BWD_FUSED=1: the one-pass backward against the reference at every multi-round case.  Its dQ goes through
-    add-reductions in an order that is not fixed, so only the tolerance checks apply (no batch invariance)."""
-    _child_pytest({"SPT_ATTN_BWD_FUSED": "1"}, "test_multi_round_parity")
-
-
-def _streams_case_outputs():
-    """y, zsum, dq, dk, dv of the s2048_5rounds case (interleaved layout), on the CPU."""
-    q, k, v, dy, mask, extra0 = _lookup_case("s2048_5rounds")
-    out = _run(q.to(DEV), k.to(DEV), v.to(DEV), dy.to(DEV), mask, extra0, 64 ** -0.5, False)
-    return [t.cpu() for t in out]
-
-
-@gpu
-def test_switch_one_stream_backward_equals_two_streams(tmp_path):
-    """SPT_ATTN_BWD_STREAMS=0 launches the dK/dV and dQ kernels one after the other on the caller's stream instead of
-    forking dQ onto a side stream: the same kernels, so the outputs are equal bit for bit."""
-    path = str(tmp_path / "one_stream.pt")
-    code = ("import sys, torch; sys.path[:0] = [%r, %r]; import test_attn_persistent_gpu as t; "
-            "torch.save(t._streams_case_outputs(), %r)" % (ROOT, os.path.dirname(os.path.abspath(__file__)), path))
-    res = subprocess.run([sys.executable, "-c", code], cwd=ROOT, env=dict(os.environ, SPT_ATTN_BWD_STREAMS="0"),
-                         capture_output=True, text=True, timeout=600)
-    assert res.returncode == 0, res.stdout[-3000:] + res.stderr[-3000:]
-    for name, a, b in zip(("y", "zsum", "dq", "dk", "dv"), torch.load(path), _streams_case_outputs()):
-        assert torch.equal(a, b), name
 
 
 # ---------------------------------------------------------------------------------------------------------------------
 # CUDA graph capture of the d 64 layer
 # ---------------------------------------------------------------------------------------------------------------------
-def _graph_replay_equals_eager(first_backward_in_capture=False):
+def _graph_replay_equals_eager(first_backward_in_capture=False, dtype=torch.bfloat16, seed=17):
     """SparseVanillaAttentionV2 (d 64, fused, N 1, S 2048, G / 16 + 2 heads: two rounds) captured forward + backward
     with torch.cuda.graph; two replays give y and the three gradients of the eager step bit for bit.
     first_backward_in_capture: the capture holds the process's first backward, so the launcher cannot create its side
-    stream (no stream or event creation during a capture) and runs the dK/dV and dQ kernels one after the other."""
+    stream (no stream or event creation during a capture) and runs the dK/dV and dQ kernels one after the other.
+    dtype: of q, k, v; float16 also converts the layer with .half()."""
     from spt_proto_b200 import layers
-    torch.manual_seed(17)
+    torch.manual_seed(seed)
     N, S, H, E = 1, 2048, _num_sms() // 16 + 2, 64
     attn = layers.SparseVanillaAttentionV2(d_head=E, d_codeword=8, n_codewords=16, p_dropout=0.0).to(DEV)
+    if dtype == torch.float16:
+        attn = attn.half()
     attn.host_trigger = False                          # no device -> host read of the PQ-loss trigger inside the capture
-    q, k, v = (torch.randn(N, S, H, E, device=DEV).bfloat16().requires_grad_() for _ in range(3))
-    dy = torch.randn(N, S, H, E, device=DEV).bfloat16()
+    q, k, v = (torch.randn(N, S, H, E, device=DEV).to(dtype).requires_grad_() for _ in range(3))
+    dy = torch.randn(N, S, H, E, device=DEV).to(dtype)
 
     def step():
         q.grad = k.grad = v.grad = None

@@ -14,8 +14,9 @@ import pytest
 import torch
 
 from oracle import spt_oracle as O
-from test_attn_persistent_gpu import (_assert_batch_invariant, _case_shape, _dy_memory, _edge_heads, _heads,
-                                      _mask_from_indices, _num_sms, _pack, _reference, _run, _split, _unpack, _y_heads)
+from test_attn_persistent_gpu import (_assert_batch_invariant, _case_shape, _dy_memory, _edge_heads,
+                                      _graph_replay_equals_eager, _heads, _mask_from_indices, _num_sms, _pack, _reference,
+                                      _run, _split, _unpack, _y_heads)
 
 DEV = "cuda"
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -304,31 +305,6 @@ def test_fp16_batch_invariance(case, reference_layout):
                             _dy_memory(dy, reference_layout).half().to(DEV), mask, extra0, d ** -0.5, reference_layout)
 
 
-def _switch_case_outputs():
-    """y, zsum, dq, dk, dv of an fp16 case on the persistent grids (S 2048, 2G / 16 + 1 heads), on the CPU."""
-    G = _num_sms()
-    N, S, H, d = 1, 2048, G // 8 + 1, 64
-    q, k, v, dy, w = _inputs16(N, S, H, d, 31)
-    mask, extra0 = _lookup(q, k, w)
-    return [t.cpu() for t in _run_dtype(torch.float16, q, k, v, dy, mask, extra0, d ** -0.5, False)]
-
-
-@gpu
-@pytest.mark.parametrize("switch", ["SPT_ATTN_BWD_STREAMS=0", "SPT_ATTN_FWD128=1", "SPT_ATTN_BWD_FUSED=1"])
-def test_fp16_switch_equals_default(switch, tmp_path):
-    """SPT_ATTN_BWD_STREAMS=0 runs the same kernels one after the other; SPT_ATTN_FWD128=1 and SPT_ATTN_BWD_FUSED=1 are
-    bf16-only kernels, so fp16 keeps the default ones.  Each gives the default outputs bit for bit."""
-    name, value = switch.split("=")
-    path = str(tmp_path / "switch.pt")
-    code = ("import sys, torch; sys.path[:0] = [%r, %r]; import test_fp16_gpu as t; "
-            "torch.save(t._switch_case_outputs(), %r)" % (ROOT, HERE, path))
-    res = subprocess.run([sys.executable, "-c", code], cwd=ROOT, env=dict(os.environ, **{name: value}),
-                         capture_output=True, text=True, timeout=600)
-    assert res.returncode == 0, res.stdout[-3000:] + res.stderr[-3000:]
-    for what, a, b in zip(("y", "zsum", "dq", "dk", "dv"), torch.load(path), _switch_case_outputs()):
-        assert torch.equal(a, b), what
-
-
 @gpu
 def test_fp16_switch_tile64_parity():
     """SPT_ATTN_TILE=64 (the 128 x 64 backward at d 64), in a child process: the parity tests at d 64, including the
@@ -344,38 +320,18 @@ def test_fp16_switch_tile64_parity():
 def test_fp16_graph_capture_layer():
     """The fp16 SparseVanillaAttentionV2 (d 64, fused, two rounds) captured forward + backward with torch.cuda.graph:
     two replays give y and the three gradients of the eager step bit for bit."""
-    from spt_proto_b200 import layers
-    torch.manual_seed(19)
-    N, S, H, E = 1, 2048, _num_sms() // 16 + 2, 64
-    attn = layers.SparseVanillaAttentionV2(d_head=E, d_codeword=8, n_codewords=16, p_dropout=0.0).to(DEV).half()
-    attn.host_trigger = False
-    q, k, v = (torch.randn(N, S, H, E, device=DEV).half().requires_grad_() for _ in range(3))
-    dy = torch.randn(N, S, H, E, device=DEV).half()
+    _graph_replay_equals_eager(dtype=torch.float16, seed=19)
 
-    def step():
-        q.grad = k.grad = v.grad = None
-        y = attn(q, k, v)
-        y.backward(dy)
-        return [y, q.grad, k.grad, v.grad]
 
-    want = [t.detach().clone() for t in step()]
-    side = torch.cuda.Stream()
-    side.wait_stream(torch.cuda.current_stream())
-    with torch.cuda.stream(side):
-        for _ in range(2):
-            step()
-    torch.cuda.current_stream().wait_stream(side)
-    graph = torch.cuda.CUDAGraph()
-    with torch.cuda.graph(graph):
-        outs = step()
-    assert attn.last_path == "fused"
-    for _ in range(2):
-        for t in outs:
-            t.detach().zero_()
-        graph.replay()
-        torch.cuda.synchronize()
-        for name, a, b in zip(("y", "dq", "dk", "dv"), outs, want):
-            assert torch.equal(a.detach(), b), name
+@gpu
+def test_fp16_graph_capture_first_backward_in_capture():
+    """As test_fp16_graph_capture_layer in a fresh process whose first backward is captured: the replays run the dK/dV
+    and dQ kernels one after the other (the launcher's fall-back without a side stream) and equal the eager step, which
+    forks dQ onto the side stream, bit for bit."""
+    code = ("import sys, torch; sys.path[:0] = [%r, %r]; import test_attn_persistent_gpu as t; "
+            "t._graph_replay_equals_eager(first_backward_in_capture=True, dtype=torch.float16, seed=19)" % (ROOT, HERE))
+    res = subprocess.run([sys.executable, "-c", code], cwd=ROOT, capture_output=True, text=True, timeout=600)
+    assert res.returncode == 0, res.stdout[-3000:] + res.stderr[-3000:]
 
 
 @gpu
