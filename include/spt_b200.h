@@ -220,6 +220,16 @@ int spt_softmax_clamp_bwd(const int32_t *indptr, const int32_t *indices, const f
  *   mask [B, S, S/32] uint32, lane-major: bit i of word 4 g + t <=> key 128 g + 4 i + t selected, and
  *   extra0 [B, S] int32 = number of zero-padding slots of the row (multiplicity of key 0 beyond its
  *   own bit).  `output` (the int32 index tensor) may be NULL on this path.  Needs S % 128 == 0.
+ *   S <= 65536.  Mask-only calls (output NULL) at m = 8, 10 or 16 take no more shared memory than a
+ *   fixed amount at any S (DESIGN.md section 4.1).  Codes >= 16 are handled by a fallback kernel,
+ *   decided on the device; its row images (32 nnz 2 + S 4 + 32 m 2 bytes) must fit 200 KB, i.e.
+ *   S up to about 16 k at sparse_coeff 8.  Beyond that spt_lookup_mask_fwd fails.
+ * spt_lookup_mask_fwd_ex: the same, with the caller's promise that every code is < n_codewords.
+ *   Where the fallback fits, it launches exactly what spt_lookup_mask_fwd launches.  Where it does
+ *   not: n_codewords > 16 returns SPT_ERR_UNSUPPORTED before any CUDA call; n_codewords <= 16 runs
+ *   without the fallback (mask-only calls at m 8, 10, 16 only), and a code >= 16 that arrives all
+ *   the same matches no key: the result stays deterministic and nothing is written outside mask and
+ *   extra0.
  *
  * spt_sparse_attn_fwd: q, k, v [B, S, d] bf16 or fp16 (dtype SPT_BF16 / SPT_F16) ->
  *   y [B, S, d] (same type) = sum_j p_rj v_j,  p = w * exp(clamp(scale * q.k, -clamp, clamp)) / Z,
@@ -247,6 +257,9 @@ int spt_softmax_clamp_bwd(const int32_t *indptr, const int32_t *indices, const f
 int spt_lookup_mask_fwd(const int32_t *query_codes, const int32_t *key_codes, int32_t *output,
                         uint32_t *mask, int32_t *extra0, void *workspace, int B, int S, int m, int nnz,
                         int H, spt_stream_t stream);
+int spt_lookup_mask_fwd_ex(const int32_t *query_codes, const int32_t *key_codes, int32_t *output,
+                           uint32_t *mask, int32_t *extra0, void *workspace, int B, int S, int m, int nnz,
+                           int H, int n_codewords, spt_stream_t stream);
 int spt_sparse_attn_fwd(const void *q, const void *k, const void *v, const uint32_t *mask,
                         const int32_t *extra0, void *y, float *zsum, int B, int S, int d, int H,
                         float scale, float clamp, int dtype, spt_stream_t stream);
@@ -276,7 +289,10 @@ int spt_sparse_attn_bwd(const void *q, const void *k, const void *v, const void 
  *   Wm = 4 ceil(max_seqlen / 128), lane-major words relative to the sequence start (words past a
  *   row's sequence are zero), extra0 [H, T]; nnz_i = S_i / sparse_coeff.  workspace:
  *   spt_lookup_mask_varlen_workspace_bytes.  spt_lookup_mask_varlen_max_seqlen(m) is the longest
- *   max_seqlen the mask-only kernels take at m (0: m not supported).
+ *   max_seqlen the mask-only kernels take at m: 65536 at m 8, 10 and 16, 0 otherwise.  The codes
+ *   >= 16 fallback needs its row images (32 nnz_max 2 + 32 Wm 4 + 32 m 2 bytes, nnz_max =
+ *   max_seqlen / sparse_coeff) within 200 KB; beyond that spt_lookup_mask_varlen_fwd fails.
+ * spt_lookup_mask_varlen_fwd_ex: as spt_lookup_mask_fwd_ex for the packed call (codes < n_codewords).
  * spt_sparse_attn_varlen_fwd / _bwd: as the _ex calls on q, k, v [T, H, d]; zsum [H, T].
  *   SPT_ATTN_Y_TRANSPOSED: sequence i's y (and grad_y) memory is its own y_i^T [H, d, S_i] at
  *   token offset cu[i] — the reference layer's layout for that sequence alone.
@@ -289,6 +305,10 @@ int spt_lookup_mask_varlen_max_seqlen(int m);
 int spt_lookup_mask_varlen_fwd(const int32_t *query_codes, const int32_t *key_codes, const void *work,
                                uint32_t *mask, int32_t *extra0, void *workspace, int n_seq, int T,
                                int max_seqlen, int H, int m, int sparse_coeff, spt_stream_t stream);
+int spt_lookup_mask_varlen_fwd_ex(const int32_t *query_codes, const int32_t *key_codes, const void *work,
+                                  uint32_t *mask, int32_t *extra0, void *workspace, int n_seq, int T,
+                                  int max_seqlen, int H, int m, int sparse_coeff, int n_codewords,
+                                  spt_stream_t stream);
 int spt_sparse_attn_varlen_fwd(const void *q, const void *k, const void *v, const uint32_t *mask,
                                const int32_t *extra0, void *y, float *zsum, const void *work, int n_seq,
                                int T, int max_seqlen, int d, int H, float scale, float clamp, int dtype,

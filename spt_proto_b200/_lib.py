@@ -57,6 +57,7 @@ def _load() -> ctypes.CDLL:
         "spt_softmax_bwd": (i32, [vp, vp, vp, vp, vp, i32, i32, i64, vp]),
         "spt_softmax_bwd_ex": (i32, [vp, vp, vp, vp, vp, i32, i32, i64, i32, vp]),
         "spt_lookup_mask_fwd": (i32, [vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, i32, vp]),
+        "spt_lookup_mask_fwd_ex": (i32, [vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, i32, i32, vp]),
         "spt_sparse_attn_fwd": (i32, [vp, vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, f32, f32, i32, vp]),
         "spt_sparse_attn_fwd_ex": (i32, [vp, vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, f32, f32, i32, i32, vp]),
         "spt_sparse_attn_bwd_ex": (i32, [vp] * 12 + [i32, i32, i32, i32, f32, f32, i32, i32, vp]),
@@ -100,6 +101,7 @@ def _load() -> ctypes.CDLL:
     sig["spt_lookup_mask_varlen_workspace_bytes"] = (sz, [i32, i32, i32, i32])
     sig["spt_lookup_mask_varlen_max_seqlen"] = (i32, [i32])
     sig["spt_lookup_mask_varlen_fwd"] = (i32, [vp] * 6 + [i32] * 6 + [vp])
+    sig["spt_lookup_mask_varlen_fwd_ex"] = (i32, [vp] * 6 + [i32] * 7 + [vp])
     sig["spt_sparse_attn_varlen_fwd"] = (i32, [vp] * 8 + [i32, i32, i32, i32, i32, f32, f32, i32, i32, vp])
     sig["spt_sparse_attn_varlen_bwd_workspace_bytes"] = (sz, [i32, i32])
     sig["spt_sparse_attn_varlen_bwd"] = (i32, [vp] * 13 + [i32, i32, i32, i32, i32, f32, f32, i32, i32, vp])

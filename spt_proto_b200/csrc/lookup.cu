@@ -761,9 +761,37 @@ __device__ __forceinline__ void lkb_planes(const uint32_t *pw, const uint32_t (&
     g3o = g3;
 }
 
-// VARLEN: as lookup_maskonly2_kernel
-template <int M, bool VARLEN = false>
-__global__ void __launch_bounds__(LKM_THREADS)
+// ---- streaming: no length cap ------------------------------------------------------------------------
+// STREAM keeps a head's bitmaps in global memory (L2 serves them: m * 256 B per 128-key word, 2 MiB per head at S 65536,
+// m 16) and moves them through two shared-memory buffers of LKB_CHUNK words each, in both passes: chunk k + 1 is copied
+// (cp.async) while chunk k is evaluated.  The chunks of pass 1 and pass 2 form one sequence 0 .. 2 nc - 1 (nc chunks per
+// pass), chunk i in buffer i & 1.  Shared memory: (2 m LKB_CHUNK 256 + LKB_CHUNK LKM_THREADS 4) B whatever S is.
+__device__ __forceinline__ void cp_async16(void *smem, const void *gmem) {
+    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;\n" ::"r"((unsigned)__cvta_generic_to_shared(smem)), "l"(gmem));
+}
+__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;\n" ::); }
+__device__ __forceinline__ void cp_async_wait1() { asm volatile("cp.async.wait_group 1;\n" ::: "memory"); }
+
+// issue chunk i of the sequence (an empty group past its end, so that wait_group 1 always means "chunk i - 1 landed")
+template <int M>
+__device__ __forceinline__ void lks_load(uint32_t *s_kb, const uint32_t *kb_head, int i, int nc, int tw, int W, int woff) {
+    if (i < 2 * nc) {
+        const int c0 = (i % nc) * LKB_CHUNK, cw = min(LKB_CHUNK, tw - c0);
+        uint32_t *buf = s_kb + (size_t)(i & 1) * M * LKB_CHUNK * LK_WORD_U32;
+        const int per_s = cw * LK_WORD_U32 / 4;  // uint4 per subspace
+        for (int k = threadIdx.x; k < M * per_s; k += LKM_THREADS) {
+            const int s = k / per_s, o = k - s * per_s;
+            cp_async16(reinterpret_cast<uint4 *>(buf + (size_t)s * LKB_CHUNK * LK_WORD_U32) + o,
+                       reinterpret_cast<const uint4 *>(kb_head + ((size_t)s * W + woff + c0) * LK_WORD_U32) + o);
+        }
+    }
+    cp_async_commit();
+}
+
+// VARLEN: as lookup_maskonly2_kernel.  STREAM: two blocks per SM at m 8 / 10 (96 / 112 KB of shared memory each), one
+// at m 16 (160 KB), which then needs more than 64 registers to keep from spilling.
+template <int M, bool VARLEN = false, bool STREAM = false>
+__global__ void __launch_bounds__(LKM_THREADS, STREAM ? (M == 16 ? 1 : 2) : 0)
 lookup_maskonly_big_kernel(const int32_t *__restrict__ query_codes, const uint32_t *__restrict__ kb,
                            const int *__restrict__ flag, uint32_t *__restrict__ mask_out,
                            int32_t *__restrict__ extra0_out, int S, int nnz, int W, int H, const LkVarlen vl = {}) {
@@ -777,8 +805,9 @@ lookup_maskonly_big_kernel(const int32_t *__restrict__ query_codes, const uint32
         start = it.x, len = it.y, tile = it.z, woff = it.w, groups = vl.groups, nnz = it.y / vl.coeff;
     }
     const int tw = tile + 1;                       // 128-key words a row of this group can see
-    uint32_t *s_kb = reinterpret_cast<uint32_t *>(smem_raw);                 // [M][tw][16][4]
-    uint32_t *s_out = s_kb + (size_t)M * tw * LK_WORD_U32;                   // [LKB_CHUNK][LKM_THREADS]
+    const int kw = STREAM ? LKB_CHUNK : tw;        // words per subspace in shared memory
+    uint32_t *s_kb = reinterpret_cast<uint32_t *>(smem_raw);                 // [M][kw][16][4] (STREAM: two of them)
+    uint32_t *s_out = s_kb + (size_t)(STREAM ? 2 : 1) * M * kw * LK_WORD_U32;  // [LKB_CHUNK][LKM_THREADS]
     const int tid = threadIdx.x;
     const int rl = tid >> 2, t = tid & 3;
     const int r = tile * LKM_ROWS + rl;
@@ -789,7 +818,10 @@ lookup_maskonly_big_kernel(const int32_t *__restrict__ query_codes, const uint32
     const int lim = live ? min(r + 1, nnz) : 0;
     const int n_t = lim > t ? (lim - t + 3) / 4 : 0;
     const uint32_t last_valid = valid_mask(tw - 1, nkeys);
-    {
+    const int nc = (tw + LKB_CHUNK - 1) / LKB_CHUNK;   // STREAM: chunks per pass
+    if constexpr (STREAM) {
+        lks_load<M>(s_kb, kb + (size_t)b * M * W * LK_WORD_U32, 0, nc, tw, W, woff);
+    } else {
         const uint32_t *kb_head = kb + (size_t)b * M * W * LK_WORD_U32;
         const int per_s = tw * LK_WORD_U32 / 4;  // uint4 per subspace
         for (int i = tid; i < M * per_s; i += LKM_THREADS) {
@@ -805,15 +837,33 @@ lookup_maskonly_big_kernel(const int32_t *__restrict__ query_codes, const uint32
         for (int s = 0; s < M; ++s) {
             const unsigned qc = live ? (unsigned)qp[s] & 0xffffu : 0xffffu;
             badq |= (qc >= (unsigned)LK_CV) ? (1u << s) : 0u;
-            koff[s] = (uint32_t)((s * tw * LK_CV + (qc & (LK_CV - 1))) * 4 + t);
+            koff[s] = (uint32_t)((s * kw * LK_CV + (qc & (LK_CV - 1))) * 4 + t);
         }
     }
     const bool any_bad = __any_sync(FULL, badq != 0);
-    __syncthreads();
+    if constexpr (!STREAM) __syncthreads();
 
     // pass 1: bucket sizes
     int len1 = 0, len2 = 0, len3 = 0;
-    {
+    if constexpr (STREAM) {
+        for (int c = 0; c < nc; ++c) {
+            lks_load<M>(s_kb, kb + (size_t)b * M * W * LK_WORD_U32, c + 1, nc, tw, W, woff);
+            cp_async_wait1();
+            __syncthreads();
+            const uint32_t *pw = s_kb + (size_t)(c & 1) * M * LKB_CHUNK * LK_WORD_U32;
+            const int c1 = min(tw, (c + 1) * LKB_CHUNK);
+#pragma unroll 1
+            for (int w = c * LKB_CHUNK; w < c1; ++w, pw += LK_WORD_U32) {
+                uint32_t lo, hi, g1, g3;
+                lkb_planes<M>(pw, koff, any_bad, badq, lo, hi, g1, g3);
+                const uint32_t valid = (w == tw - 1) ? last_valid : 0xffffffffu;
+                len3 += __popc(g3 & valid);
+                len2 += __popc(hi & valid);
+                len1 += __popc(g1 & valid);
+            }
+            __syncthreads();   // buffer c & 1 is refilled by the next iteration's copy
+        }
+    } else {
         const uint32_t *pw = s_kb;
 #pragma unroll 1
         for (int w = 0; w < tw; ++w, pw += LK_WORD_U32) {
@@ -849,6 +899,13 @@ lookup_maskonly_big_kernel(const int32_t *__restrict__ query_codes, const uint32
     for (int c0 = 0; c0 < tw; c0 += LKB_CHUNK) {
         const int c1 = min(tw, c0 + LKB_CHUNK);
         const uint32_t *pw = s_kb + (size_t)c0 * LK_WORD_U32;
+        if constexpr (STREAM) {
+            const int i = nc + c0 / LKB_CHUNK;
+            lks_load<M>(s_kb, kb + (size_t)b * M * W * LK_WORD_U32, i + 1, nc, tw, W, woff);
+            cp_async_wait1();
+            __syncthreads();
+            pw = s_kb + (size_t)(i & 1) * M * LKB_CHUNK * LK_WORD_U32;
+        }
 #pragma unroll 1
         for (int w = c0; w < c1; ++w, pw += LK_WORD_U32) {
             uint32_t lo, hi, g1, g3;
@@ -1006,8 +1063,22 @@ extern "C" size_t spt_lookup_workspace_bytes(int B, int S, int m, int nnz) {
     return 16 + (size_t)B * m * W * LK_WORD_U32 * sizeof(uint32_t);
 }
 
+// shared memory of the streaming mask-only kernel (lookup_maskonly_big_kernel<M, VARLEN, true>), independent of S
+static size_t lks_smem(int m) { return (size_t)2 * m * LKB_CHUNK * LK_WORD_U32 * 4 + (size_t)LKB_CHUNK * LKM_THREADS * 4; }
+
+template <int M, bool VARLEN>
+static void lks_launch(dim3 grid, const int32_t *qc, const uint32_t *kb, const int *flag, uint32_t *mask, int32_t *extra0,
+                       int S, int nnz, int W, int H, cudaStream_t st, const LkVarlen &vl = {}) {
+    const size_t smem = lks_smem(M);
+    cudaFuncSetAttribute(lookup_maskonly_big_kernel<M, VARLEN, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    lookup_maskonly_big_kernel<M, VARLEN, true><<<grid, LKM_THREADS, smem, st>>>(qc, kb, flag, mask, extra0, S, nnz, W, H, vl);
+}
+
+// n_codewords: codes are < n_codewords (the _ex entry points), or -1: unknown.  Where the generic kernel's row images do not
+// fit, only a promise of n_codewords <= 16 lets a call run: the fallback is skipped and a code >= 16 matches no key.
 static int lookup_impl(const int32_t *query_codes, const int32_t *key_codes, int32_t *output, uint32_t *mask_out,
-                       int32_t *extra0_out, void *workspace, int B, int S, int m, int nnz, int H, spt_stream_t stream) {
+                       int32_t *extra0_out, void *workspace, int B, int S, int m, int nnz, int H, int n_codewords,
+                       spt_stream_t stream) {
     SPT_REQUIRE(query_codes && key_codes && (output || mask_out), "lookup_fwd: null pointer");
     SPT_REQUIRE(H >= 1 && B % H == 0, "lookup_fwd: B=%d must be a multiple of the interleaved head count H=%d", B, H);
     SPT_REQUIRE(B >= 1 && S >= 1 && S <= 65536, "lookup_fwd: bad batch/seq (B=%d, S=%d; S must be <= 65536)", B, S);
@@ -1015,14 +1086,30 @@ static int lookup_impl(const int32_t *query_codes, const int32_t *key_codes, int
     SPT_REQUIRE(m >= 4, "lookup_fwd: n_subspaces must be >= 4 (got %d)", m);
     SPT_REQUIRE(nnz >= 8 && nnz % 4 == 0 && nnz <= S, "lookup_fwd: nonzeros per row must be a multiple of 4 in [8, S] (got %d)", nnz);
     SPT_REQUIRE(!mask_out || (S % 128 == 0 && extra0_out), "lookup_fwd: bitmask output needs S %% 128 == 0 and extra0");
-    cudaStream_t st = as_stream(stream);
     const int tiles = (S + LK_ROWS - 1) / LK_ROWS;
-    const unsigned grid = (unsigned)tiles * B;                                            // one block per (head, row tile)
-    const unsigned fb_grid = grid < 2u * num_sms() ? grid : 2u * num_sms();               // the flag-guarded fallback
     const size_t img = out_image_bytes(nnz) + (mask_out ? (size_t)LK_ROWS * (S / 32) * 4 : 0);
     const size_t gen_smem = img + (size_t)LK_ROWS * m * 2;
-    SPT_REQUIRE(gen_smem <= 200 * 1024, "lookup_fwd: nnz=%d / S=%d too large for the shared-memory row images", nnz, S);
-    if (gen_smem > 48 * 1024)
+    const bool fb_fits = gen_smem <= 200 * 1024;
+    // mask-only calls at m 8, 10, 16: the plane kernel, else the plane-free kernel, else the streaming kernel
+    const bool mask_only = mask_out && !output && (m == 8 || m == 10 || m == 16);
+    if (!fb_fits) {
+        SPT_REQUIRE(n_codewords >= 0, "lookup_fwd: nnz=%d / S=%d too large for the shared-memory row images", nnz, S);
+        if (n_codewords > LK_CV || !mask_only)
+            return fail(SPT_ERR_UNSUPPORTED,
+                        "lookup_mask_fwd_ex: S=%d, nnz=%d, m=%d runs only as a mask-only lookup with n_codewords <= %d "
+                        "(got %d): the fallback for codes >= %d needs %zu bytes of row images, beyond its limit of %d",
+                        S, nnz, m, LK_CV, n_codewords, LK_CV, gen_smem, 200 * 1024);
+    }
+    const int W = (S + 127) / 128;
+    const size_t per_word = (size_t)m * LK_WORD_U32 * 4;   // bitmaps per 128-key word: m * 256 B
+    const size_t msmem = (per_word + 2 * LKM_THREADS * 4) * (size_t)W;
+    const size_t bsmem = per_word * (size_t)W + (size_t)LKB_CHUNK * LKM_THREADS * 4;
+    if (bitmap_m_supported(m) && !mask_only)
+        SPT_REQUIRE(img + per_word <= LK_SMEM_BUDGET, "lookup_fwd: nnz=%d / S=%d too large", nnz, S);
+    cudaStream_t st = as_stream(stream);
+    const unsigned grid = (unsigned)tiles * B;                                            // one block per (head, row tile)
+    const unsigned fb_grid = grid < 2u * num_sms() ? grid : 2u * num_sms();               // the flag-guarded fallback
+    if (fb_fits && gen_smem > 48 * 1024)
         cudaFuncSetAttribute(lookup_generic_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)gen_smem);
 
     if (!bitmap_m_supported(m)) {
@@ -1034,61 +1121,64 @@ static int lookup_impl(const int32_t *query_codes, const int32_t *key_codes, int
     SPT_REQUIRE(workspace, "lookup_fwd: workspace required");
     int *flag = reinterpret_cast<int *>(workspace);
     uint32_t *kb = reinterpret_cast<uint32_t *>(reinterpret_cast<char *>(workspace) + 16);
-    const int W = (S + 127) / 128;
     cudaError_t e = cudaMemsetAsync(flag, 0, 16, st);
     if (e != cudaSuccess) return fail(SPT_ERR_CUDA, "lookup_fwd: memset: %s", cudaGetErrorString(e));
     lookup_pack_kernel<<<dim3(W, B), 128, 0, st>>>(key_codes, kb, flag, S, m, W, H);
     SPT_LAUNCH_CHECK("lookup_pack_kernel");
+    // without the fallback the kernels read flag + 1, a word of the zeroed 16 bytes that nothing raises
+    const int *kflag = fb_fits ? flag : flag + 1;
 
-    // bitmaps per 128-key word: m * 256 B; pick the chunk so that images + chunk fit the budget
-    const size_t per_word = (size_t)m * LK_WORD_U32 * 4;
-    SPT_REQUIRE(img + per_word <= LK_SMEM_BUDGET, "lookup_fwd: nnz=%d / S=%d too large", nnz, S);
+    // pick the chunk so that images + chunk fit the budget
     int chunk_words = (int)((LK_SMEM_BUDGET - img) / per_word);
     if (chunk_words > W) chunk_words = W;
     const size_t smem = img + per_word * chunk_words;
-    const size_t msmem = (per_word + 2 * LKM_THREADS * 4) * (size_t)W;
-    if (mask_out && !output && (m == 8 || m == 10 || m == 16) && msmem <= 200 * 1024) {
+    if (mask_only) {
         const dim3 mgrid(B, S / LKM_ROWS);
-        static const bool v1 = [] { const char *e = getenv("SPT_LOOKUP_MASK_V1"); return e && atoi(e) == 1; }();   // A/B switch
-        if (v1 && m != 10) {
-            if (m == 8) {
-                cudaFuncSetAttribute(lookup_maskonly_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)msmem);
-                lookup_maskonly_kernel<8><<<mgrid, LKM_THREADS, msmem, st>>>(query_codes, kb, flag, mask_out, extra0_out, S, nnz, W, H);
+        if (msmem <= 200 * 1024) {
+            static const bool v1 = [] { const char *e = getenv("SPT_LOOKUP_MASK_V1"); return e && atoi(e) == 1; }();   // A/B switch
+            if (v1 && m != 10) {
+                if (m == 8) {
+                    cudaFuncSetAttribute(lookup_maskonly_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)msmem);
+                    lookup_maskonly_kernel<8><<<mgrid, LKM_THREADS, msmem, st>>>(query_codes, kb, kflag, mask_out, extra0_out, S, nnz, W, H);
+                } else {
+                    cudaFuncSetAttribute(lookup_maskonly_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)msmem);
+                    lookup_maskonly_kernel<16><<<mgrid, LKM_THREADS, msmem, st>>>(query_codes, kb, kflag, mask_out, extra0_out, S, nnz, W, H);
+                }
+            } else if (m == 8) {
+                cudaFuncSetAttribute(lookup_maskonly2_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)msmem);
+                lookup_maskonly2_kernel<8><<<mgrid, LKM_THREADS, msmem, st>>>(query_codes, kb, kflag, mask_out, extra0_out, S, nnz, W, H);
+            } else if (m == 10) {       // head dim 80 (OPT-2.7B) at d_codeword 8
+                cudaFuncSetAttribute(lookup_maskonly2_kernel<10>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)msmem);
+                lookup_maskonly2_kernel<10><<<mgrid, LKM_THREADS, msmem, st>>>(query_codes, kb, kflag, mask_out, extra0_out, S, nnz, W, H);
             } else {
-                cudaFuncSetAttribute(lookup_maskonly_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)msmem);
-                lookup_maskonly_kernel<16><<<mgrid, LKM_THREADS, msmem, st>>>(query_codes, kb, flag, mask_out, extra0_out, S, nnz, W, H);
+                cudaFuncSetAttribute(lookup_maskonly2_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)msmem);
+                lookup_maskonly2_kernel<16><<<mgrid, LKM_THREADS, msmem, st>>>(query_codes, kb, kflag, mask_out, extra0_out, S, nnz, W, H);
             }
-        } else if (m == 8) {
-            cudaFuncSetAttribute(lookup_maskonly2_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)msmem);
-            lookup_maskonly2_kernel<8><<<mgrid, LKM_THREADS, msmem, st>>>(query_codes, kb, flag, mask_out, extra0_out, S, nnz, W, H);
-        } else if (m == 10) {       // head dim 80 (OPT-2.7B) at d_codeword 8
-            cudaFuncSetAttribute(lookup_maskonly2_kernel<10>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)msmem);
-            lookup_maskonly2_kernel<10><<<mgrid, LKM_THREADS, msmem, st>>>(query_codes, kb, flag, mask_out, extra0_out, S, nnz, W, H);
+            SPT_LAUNCH_CHECK("lookup_maskonly_kernel");
+        } else if (bsmem <= 200 * 1024) {
+            // long sequences: the plane-free mask-only kernel (S 8192 at m 8)
+            if (m == 8) {
+                cudaFuncSetAttribute(lookup_maskonly_big_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bsmem);
+                lookup_maskonly_big_kernel<8><<<mgrid, LKM_THREADS, bsmem, st>>>(query_codes, kb, kflag, mask_out, extra0_out, S, nnz, W, H);
+            } else if (m == 10) {
+                cudaFuncSetAttribute(lookup_maskonly_big_kernel<10>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bsmem);
+                lookup_maskonly_big_kernel<10><<<mgrid, LKM_THREADS, bsmem, st>>>(query_codes, kb, kflag, mask_out, extra0_out, S, nnz, W, H);
+            } else {
+                cudaFuncSetAttribute(lookup_maskonly_big_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bsmem);
+                lookup_maskonly_big_kernel<16><<<mgrid, LKM_THREADS, bsmem, st>>>(query_codes, kb, kflag, mask_out, extra0_out, S, nnz, W, H);
+            }
+            SPT_LAUNCH_CHECK("lookup_maskonly_big_kernel");
         } else {
-            cudaFuncSetAttribute(lookup_maskonly2_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)msmem);
-            lookup_maskonly2_kernel<16><<<mgrid, LKM_THREADS, msmem, st>>>(query_codes, kb, flag, mask_out, extra0_out, S, nnz, W, H);
+            // longer still: the streaming kernel (its shared memory does not grow with S)
+            if (m == 8)
+                lks_launch<8, false>(mgrid, query_codes, kb, kflag, mask_out, extra0_out, S, nnz, W, H, st);
+            else if (m == 10)
+                lks_launch<10, false>(mgrid, query_codes, kb, kflag, mask_out, extra0_out, S, nnz, W, H, st);
+            else
+                lks_launch<16, false>(mgrid, query_codes, kb, kflag, mask_out, extra0_out, S, nnz, W, H, st);
+            SPT_LAUNCH_CHECK("lookup_maskonly_big_kernel(stream)");
         }
-        SPT_LAUNCH_CHECK("lookup_maskonly_kernel");
-        lookup_generic_kernel<<<fb_grid, LK_THREADS, gen_smem, st>>>(query_codes, key_codes, flag, 1, output, mask_out,
-                                                                  extra0_out, S, m, nnz, H, tiles, B);
-        SPT_LAUNCH_CHECK("lookup_generic_kernel(fallback)");
-        return SPT_OK;
-    }
-    const size_t bsmem = per_word * (size_t)W + (size_t)LKB_CHUNK * LKM_THREADS * 4;
-    if (mask_out && !output && (m == 8 || m == 10 || m == 16) && bsmem <= 200 * 1024) {
-        // long sequences: the plane-free mask-only kernel (S 8192 at m 8)
-        const dim3 mgrid(B, S / LKM_ROWS);
-        if (m == 8) {
-            cudaFuncSetAttribute(lookup_maskonly_big_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bsmem);
-            lookup_maskonly_big_kernel<8><<<mgrid, LKM_THREADS, bsmem, st>>>(query_codes, kb, flag, mask_out, extra0_out, S, nnz, W, H);
-        } else if (m == 10) {
-            cudaFuncSetAttribute(lookup_maskonly_big_kernel<10>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bsmem);
-            lookup_maskonly_big_kernel<10><<<mgrid, LKM_THREADS, bsmem, st>>>(query_codes, kb, flag, mask_out, extra0_out, S, nnz, W, H);
-        } else {
-            cudaFuncSetAttribute(lookup_maskonly_big_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bsmem);
-            lookup_maskonly_big_kernel<16><<<mgrid, LKM_THREADS, bsmem, st>>>(query_codes, kb, flag, mask_out, extra0_out, S, nnz, W, H);
-        }
-        SPT_LAUNCH_CHECK("lookup_maskonly_big_kernel");
+        if (!fb_fits) return SPT_OK;
         lookup_generic_kernel<<<fb_grid, LK_THREADS, gen_smem, st>>>(query_codes, key_codes, flag, 1, output, mask_out,
                                                                   extra0_out, S, m, nnz, H, tiles, B);
         SPT_LAUNCH_CHECK("lookup_generic_kernel(fallback)");
@@ -1122,14 +1212,22 @@ static int lookup_impl(const int32_t *query_codes, const int32_t *key_codes, int
 extern "C" int spt_lookup_fwd(const int32_t *query_codes, const int32_t *key_codes, int32_t *output, void *workspace,
                               int B, int S, int m, int nnz, spt_stream_t stream) {
     SPT_REQUIRE(output, "lookup_fwd: null output");
-    return lookup_impl(query_codes, key_codes, output, nullptr, nullptr, workspace, B, S, m, nnz, 1, stream);
+    return lookup_impl(query_codes, key_codes, output, nullptr, nullptr, workspace, B, S, m, nnz, 1, -1, stream);
 }
 
 extern "C" int spt_lookup_mask_fwd(const int32_t *query_codes, const int32_t *key_codes, int32_t *output,
                                    uint32_t *mask, int32_t *extra0, void *workspace, int B, int S, int m, int nnz,
                                    int H, spt_stream_t stream) {
     SPT_REQUIRE(mask && extra0, "lookup_mask_fwd: null mask / extra0");
-    return lookup_impl(query_codes, key_codes, output, mask, extra0, workspace, B, S, m, nnz, H, stream);
+    return lookup_impl(query_codes, key_codes, output, mask, extra0, workspace, B, S, m, nnz, H, -1, stream);
+}
+
+extern "C" int spt_lookup_mask_fwd_ex(const int32_t *query_codes, const int32_t *key_codes, int32_t *output,
+                                      uint32_t *mask, int32_t *extra0, void *workspace, int B, int S, int m, int nnz,
+                                      int H, int n_codewords, spt_stream_t stream) {
+    SPT_REQUIRE(mask && extra0, "lookup_mask_fwd_ex: null mask / extra0");
+    SPT_REQUIRE(n_codewords >= 1, "lookup_mask_fwd_ex: n_codewords must be >= 1 (got %d)", n_codewords);
+    return lookup_impl(query_codes, key_codes, output, mask, extra0, workspace, B, S, m, nnz, H, n_codewords, stream);
 }
 
 // ---- packed variable-length sequences ----------------------------------------------------------------------------------
@@ -1147,11 +1245,7 @@ extern "C" size_t spt_lookup_mask_varlen_workspace_bytes(int n_seq, int T, int H
 }
 
 extern "C" int spt_lookup_mask_varlen_max_seqlen(int m) {
-    if (m != 8 && m != 10 && m != 16) return 0;
-    int groups = VARLEN_MAX_SEQLEN / 128;
-    while (groups > 0 && (lkv_big_smem(m, groups) > LKV_SMEM_MAX || lkv_generic_smem(m, groups, groups * 128 / 8) > LKV_SMEM_MAX))
-        --groups;
-    return groups * 128;
+    return (m == 8 || m == 10 || m == 16) ? VARLEN_MAX_SEQLEN : 0;    // the streaming kernel has no length cap
 }
 
 template <int M>
@@ -1163,26 +1257,36 @@ static int lookup_varlen_launch(const int32_t *qc, const int32_t *kc, const uint
         lookup_maskonly2_kernel<M, true><<<dim3(H, cap), LKM_THREADS, psmem, st>>>(qc, kb, flag, mask, extra0, T, 0, cap, H, vl);
         return after_launch("lookup_maskonly2_kernel(varlen)");
     }
-    cudaFuncSetAttribute(lookup_maskonly_big_kernel<M, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bsmem);
-    lookup_maskonly_big_kernel<M, true><<<dim3(H, cap), LKM_THREADS, bsmem, st>>>(qc, kb, flag, mask, extra0, T, 0, cap, H, vl);
-    return after_launch("lookup_maskonly_big_kernel(varlen)");
+    if (bsmem <= LKV_SMEM_MAX) {
+        cudaFuncSetAttribute(lookup_maskonly_big_kernel<M, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bsmem);
+        lookup_maskonly_big_kernel<M, true><<<dim3(H, cap), LKM_THREADS, bsmem, st>>>(qc, kb, flag, mask, extra0, T, 0, cap, H, vl);
+        return after_launch("lookup_maskonly_big_kernel(varlen)");
+    }
+    lks_launch<M, true>(dim3(H, cap), qc, kb, flag, mask, extra0, T, 0, cap, H, st, vl);
+    return after_launch("lookup_maskonly_big_kernel(stream, varlen)");
 }
 
-extern "C" int spt_lookup_mask_varlen_fwd(const int32_t *query_codes, const int32_t *key_codes, const void *work,
-                                          uint32_t *mask, int32_t *extra0, void *workspace, int n_seq, int T,
-                                          int max_seqlen, int H, int m, int sparse_coeff, spt_stream_t stream) {
-    const char *what = "lookup_mask_varlen_fwd";
+static int lookup_varlen_impl(const int32_t *query_codes, const int32_t *key_codes, const void *work, uint32_t *mask,
+                              int32_t *extra0, void *workspace, int n_seq, int T, int max_seqlen, int H, int m,
+                              int sparse_coeff, int n_codewords, spt_stream_t stream) {
+    const char *what = n_codewords < 0 ? "lookup_mask_varlen_fwd" : "lookup_mask_varlen_fwd_ex";
     SPT_REQUIRE(query_codes && key_codes && work && mask && extra0 && workspace, "%s: null pointer", what);
     int rc = check_varlen(what, n_seq, T, max_seqlen, H);
     if (rc != SPT_OK) return rc;
     SPT_REQUIRE(m == 8 || m == 10 || m == 16, "%s: n_subspaces must be 8, 10 or 16 (got %d)", what, m);
     SPT_REQUIRE(sparse_coeff >= 1, "%s: sparse_coeff must be >= 1 (got %d)", what, sparse_coeff);
-    const int limit = spt_lookup_mask_varlen_max_seqlen(m);
-    SPT_REQUIRE(max_seqlen <= limit, "%s: max_seqlen %d beyond the mask-only lookup at m = %d (at most %d)", what, max_seqlen, m, limit);
     SPT_REQUIRE(((uintptr_t)work | (uintptr_t)mask | (uintptr_t)workspace) % 16 == 0, "%s: work, mask and workspace must be 16-byte aligned", what);
     const int nnz_max = (max_seqlen / sparse_coeff + 3) & ~3;       // sizes the generic fallback's row images
     const size_t gsmem = lkv_generic_smem(m, (max_seqlen + 127) / 128, nnz_max);
-    SPT_REQUIRE(gsmem <= LKV_SMEM_MAX, "%s: max_seqlen %d / sparse_coeff %d too large for the row images", what, max_seqlen, sparse_coeff);
+    const bool fb_fits = gsmem <= LKV_SMEM_MAX;
+    if (!fb_fits) {
+        SPT_REQUIRE(n_codewords >= 0, "%s: max_seqlen %d / sparse_coeff %d too large for the row images", what, max_seqlen, sparse_coeff);
+        if (n_codewords > LK_CV)
+            return fail(SPT_ERR_UNSUPPORTED,
+                        "%s: max_seqlen %d / sparse_coeff %d needs n_codewords <= %d (got %d): the fallback for codes >= %d "
+                        "needs %zu bytes of row images, beyond its limit of %zu",
+                        what, max_seqlen, sparse_coeff, LK_CV, n_codewords, LK_CV, gsmem, LKV_SMEM_MAX);
+    }
     cudaStream_t st = as_stream(stream);
     const int cap = (int)varlen_capacity(n_seq, T);
     const int32_t *w = (const int32_t *)work;
@@ -1193,13 +1297,30 @@ extern "C" int spt_lookup_mask_varlen_fwd(const int32_t *query_codes, const int3
     if (e != cudaSuccess) return fail(SPT_ERR_CUDA, "%s: memset: %s", what, cudaGetErrorString(e));
     lookup_pack_kernel<true><<<dim3(cap, H), 128, 0, st>>>(key_codes, kb, flag, T, m, cap, H, vl);
     SPT_LAUNCH_CHECK("lookup_pack_kernel(varlen)");
-    rc = m == 8    ? lookup_varlen_launch<8>(query_codes, key_codes, kb, flag, mask, extra0, vl, cap, T, H, st)
-         : m == 10 ? lookup_varlen_launch<10>(query_codes, key_codes, kb, flag, mask, extra0, vl, cap, T, H, st)
-                   : lookup_varlen_launch<16>(query_codes, key_codes, kb, flag, mask, extra0, vl, cap, T, H, st);
-    if (rc != SPT_OK) return rc;
+    const int *kflag = fb_fits ? flag : flag + 1;       // as in lookup_impl: flag + 1 is never raised
+    rc = m == 8    ? lookup_varlen_launch<8>(query_codes, key_codes, kb, kflag, mask, extra0, vl, cap, T, H, st)
+         : m == 10 ? lookup_varlen_launch<10>(query_codes, key_codes, kb, kflag, mask, extra0, vl, cap, T, H, st)
+                   : lookup_varlen_launch<16>(query_codes, key_codes, kb, kflag, mask, extra0, vl, cap, T, H, st);
+    if (rc != SPT_OK || !fb_fits) return rc;
     // codes >= 16 somewhere: the generic kernel redoes the call (flag-guarded, decided on the device)
     cudaFuncSetAttribute(lookup_generic_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)gsmem);
     lookup_generic_kernel<true><<<2 * num_sms(), LK_THREADS, gsmem, st>>>(query_codes, key_codes, flag, 1, nullptr, mask, extra0,
                                                                          T, m, nnz_max, H, 0, H, vl);
     return after_launch("lookup_generic_kernel(varlen fallback)");
+}
+
+extern "C" int spt_lookup_mask_varlen_fwd(const int32_t *query_codes, const int32_t *key_codes, const void *work,
+                                          uint32_t *mask, int32_t *extra0, void *workspace, int n_seq, int T,
+                                          int max_seqlen, int H, int m, int sparse_coeff, spt_stream_t stream) {
+    return lookup_varlen_impl(query_codes, key_codes, work, mask, extra0, workspace, n_seq, T, max_seqlen, H, m, sparse_coeff,
+                              -1, stream);
+}
+
+extern "C" int spt_lookup_mask_varlen_fwd_ex(const int32_t *query_codes, const int32_t *key_codes, const void *work,
+                                             uint32_t *mask, int32_t *extra0, void *workspace, int n_seq, int T,
+                                             int max_seqlen, int H, int m, int sparse_coeff, int n_codewords,
+                                             spt_stream_t stream) {
+    SPT_REQUIRE(n_codewords >= 1, "lookup_mask_varlen_fwd_ex: n_codewords must be >= 1 (got %d)", n_codewords);
+    return lookup_varlen_impl(query_codes, key_codes, work, mask, extra0, workspace, n_seq, T, max_seqlen, H, m, sparse_coeff,
+                              n_codewords, stream);
 }

@@ -493,11 +493,18 @@ def _heads(t: torch.Tensor, name: str):
     raise RuntimeError(f"{name} must be of dim 3 ([B,S,*]) or 4 ([N,S,H,*])")
 
 
-def lookup_mask(query: torch.Tensor, key: torch.Tensor, sparse_coeff: int, want_indices: bool = False):
+LOOKUP_MAX_SEQ = 65536    # longest S of lookup_mask (include/spt_b200.h): the key indices of the reference fit uint16
+
+
+def lookup_mask(query: torch.Tensor, key: torch.Tensor, sparse_coeff: int, want_indices: bool = False,
+                n_codewords=None):
     """Same selection as lookup_forward_cuda, emitted as (mask [B,S,S/32] int32 bit-words in the
     lane-major layout: word 4g+t bit i <=> key 128g+4i+t, extra0 [B,S] int32 zero-padding multiplicity
     of key 0, indices [B,S,nnz] or None).
-    Codes: [B,S,m] head-major or [N,S,H,m] (heads interleaved, B = N*H)."""
+    Codes: [B,S,m] head-major or [N,S,H,m] (heads interleaved, B = N*H).
+    n_codewords: the caller's promise that every code is < n_codewords (the codebook size).  At lengths where
+    the fallback for codes >= 16 cannot run (beyond about 16 k tokens at sparse_coeff 8) only n_codewords <= 16
+    lets the call run; None makes no promise (include/spt_b200.h, spt_lookup_mask_fwd_ex)."""
     _check_dim(key, query.dim(), "key")
     _check_type(key, torch.int32, "key")
     _check_type(query, torch.int32, "query")
@@ -514,8 +521,12 @@ def lookup_mask(query: torch.Tensor, key: torch.Tensor, sparse_coeff: int, want_
     indices = torch.empty((B, S, nnz), dtype=torch.int32, device=dev) if want_indices else None
     ws = _workspace(lib.spt_lookup_workspace_bytes(B, S, m, nnz), query)
     with _on_device(query):
-        check(lib.spt_lookup_mask_fwd(_p(query), _p(key), _p(indices), _p(mask), _p(extra0), _p(ws), B, S, m, nnz, H,
-                                      _stream(query)))
+        if n_codewords is None:
+            check(lib.spt_lookup_mask_fwd(_p(query), _p(key), _p(indices), _p(mask), _p(extra0), _p(ws), B, S, m, nnz, H,
+                                          _stream(query)))
+        else:
+            check(lib.spt_lookup_mask_fwd_ex(_p(query), _p(key), _p(indices), _p(mask), _p(extra0), _p(ws), B, S, m, nnz,
+                                             H, int(n_codewords), _stream(query)))
     return mask, extra0, indices
 
 
@@ -622,10 +633,10 @@ def lookup_mask_varlen_max_seqlen(m: int) -> int:
 
 
 def lookup_mask_varlen(query: torch.Tensor, key: torch.Tensor, cu_seqlens: torch.Tensor, max_seqlen: int,
-                       sparse_coeff: int, work=None):
+                       sparse_coeff: int, work=None, n_codewords=None):
     """lookup_mask of every sequence of a packed batch alone, in one launch per kernel.  Codes [T, H, m] or [1, T, H, m]
     int32; cu_seqlens int32 [n + 1] on the device -> (mask [H, T, 4 ceil(max_seqlen / 128)] int32 lane-major words
-    relative to each sequence's start, extra0 [H, T] int32)."""
+    relative to each sequence's start, extra0 [H, T] int32).  n_codewords: as in lookup_mask."""
     _check_type(query, torch.int32, "query")
     _check_type(key, torch.int32, "key")
     if query.shape != key.shape or not query.is_cuda or not query.is_contiguous() or not key.is_contiguous():
@@ -641,8 +652,13 @@ def lookup_mask_varlen(query: torch.Tensor, key: torch.Tensor, cu_seqlens: torch
     extra0 = torch.empty((H, T), dtype=torch.int32, device=query.device)
     ws = _workspace(lib.spt_lookup_mask_varlen_workspace_bytes(n_seq, T, H, m), query)
     with _on_device(query):
-        check(lib.spt_lookup_mask_varlen_fwd(_p(query), _p(key), _p(work), _p(mask), _p(extra0), _p(ws), n_seq, T,
-                                             int(max_seqlen), H, m, int(sparse_coeff), _stream(query)))
+        if n_codewords is None:
+            check(lib.spt_lookup_mask_varlen_fwd(_p(query), _p(key), _p(work), _p(mask), _p(extra0), _p(ws), n_seq, T,
+                                                 int(max_seqlen), H, m, int(sparse_coeff), _stream(query)))
+        else:
+            check(lib.spt_lookup_mask_varlen_fwd_ex(_p(query), _p(key), _p(work), _p(mask), _p(extra0), _p(ws), n_seq, T,
+                                                    int(max_seqlen), H, m, int(sparse_coeff), int(n_codewords),
+                                                    _stream(query)))
     return mask, extra0
 
 

@@ -5,6 +5,8 @@ from .lookup import lookup
 from .softmax import softmax
 from .sddmm import sddmm, sddmm_scaled, sddmm_softmax
 from .spmm import spmm
-from .fused import sparse_attention, sparse_attention_varlen
+from .fused import (sparse_attention, sparse_attention_recompute, sparse_attention_varlen,
+                    sparse_attention_varlen_recompute)
 
-__all__ = ["cdist", "lookup", "softmax", "sddmm", "sddmm_scaled", "sddmm_softmax", "spmm", "sparse_attention", "sparse_attention_varlen"]
+__all__ = ["cdist", "lookup", "softmax", "sddmm", "sddmm_scaled", "sddmm_softmax", "spmm", "sparse_attention", "sparse_attention_varlen",
+           "sparse_attention_recompute", "sparse_attention_varlen_recompute"]

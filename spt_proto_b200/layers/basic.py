@@ -18,10 +18,32 @@ class RotaryEmbedding(nn.Module):
         super().__init__()
         if d_model % 2:
             raise ValueError("d_model must be even")
-        inv_freq = base ** (-torch.arange(0, d_model, 2) / d_model)
-        angles = torch.outer(torch.arange(n_embeddings), inv_freq).repeat(1, 2)   # [S, E]
-        self.register_buffer("cos_cached", angles.cos())
-        self.register_buffer("sin_cached", angles.sin())
+        self.base, self.d_model = base, d_model
+        cos, sin = self._angles(n_embeddings)
+        self.register_buffer("cos_cached", cos)
+        self.register_buffer("sin_cached", sin)
+        # rows n_embeddings .. of longer tables, per (device, dtype): not buffers, so state_dict keeps the reference's
+        # keys and shapes and reference checkpoints load unchanged
+        self._beyond = {}
+
+    def _angles(self, n: int):
+        inv_freq = self.base ** (-torch.arange(0, self.d_model, 2) / self.d_model)
+        angles = torch.outer(torch.arange(n), inv_freq).repeat(1, 2)   # [S, E]
+        return angles.cos(), angles.sin()
+
+    def tables(self, n: int):
+        """(cos, sin) [n', E] with n' >= n rows: the registered buffers, followed past their length by rows of the same
+        expression (what RotaryEmbedding(n_embeddings=n) holds there)."""
+        L = self.cos_cached.size(0)
+        if n <= L:
+            return self.cos_cached, self.sin_cached
+        key = (self.cos_cached.device, self.cos_cached.dtype)
+        hit = self._beyond.get(key)
+        if hit is None or hit[0].size(0) < n - L:
+            cos, sin = self._angles(n)
+            hit = tuple(t[L:].to(device=key[0], dtype=key[1]) for t in (cos, sin))
+            self._beyond[key] = hit
+        return torch.cat([self.cos_cached, hit[0][: n - L]]), torch.cat([self.sin_cached, hit[1][: n - L]])
 
     @staticmethod
     def rotate_half(x: torch.Tensor) -> torch.Tensor:
@@ -30,9 +52,11 @@ class RotaryEmbedding(nn.Module):
 
     fused = True    # one CUDA kernel per direction for bf16 inputs on the GPU (same roundings as the expression below)
 
-    def forward(self, x: torch.Tensor, ids: torch.Tensor) -> torch.Tensor:
+    def forward(self, x: torch.Tensor, ids: torch.Tensor, n_positions=None) -> torch.Tensor:
+        """n_positions: ids are < n_positions, which may exceed the registered tables (see tables)."""
         assert x.dim() == 4 and ids.dim() == 1
-        cos, sin = self.cos_cached[ids], self.sin_cached[ids]
+        cos_t, sin_t = self.tables(n_positions) if n_positions is not None else (self.cos_cached, self.sin_cached)
+        cos, sin = cos_t[ids], sin_t[ids]
         if self.fused and ids.numel() == x.size(1) and ext.rope_supported(x, cos):
             return norm_rope.rope(x, cos.contiguous(), sin.contiguous())
         cos = cos.view(1, -1, 1, x.size(-1))
@@ -76,7 +100,11 @@ class RotaryAttention(VanillaAttention):
         self.register_buffer("cached_ids", torch.arange(max_length))
 
     def _rotate(self, x):
-        return self.embedding(x, ids=self.cached_ids[: x.size(1)])
+        S = x.size(1)
+        if S <= self.cached_ids.numel():
+            return self.embedding(x, ids=self.cached_ids[:S])
+        # positions >= max_length: the embedding's tables extended by the same expression
+        return self.embedding(x, ids=torch.arange(S, device=self.cached_ids.device), n_positions=S)
 
     def _get_attn(self, q, k, attn_mask):
         return VanillaAttention._get_attn(self, self._rotate(q), self._rotate(k), attn_mask)

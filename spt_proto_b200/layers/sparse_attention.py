@@ -72,6 +72,10 @@ class _SparseV2Mixin:
     # 71-78).  Setting host_trigger to a bool makes the decision on the host, with no synchronisation:
     # True = compute the PQ loss on the next forward (then resets to False), False = skip it.
     host_trigger = None
+    # Above this length (S, or max_seqlen of a packed batch) the fused path keeps the PQ codes (S m 4 bytes per head)
+    # between forward and backward and runs the lookup again in the backward, instead of keeping the bitmask (S^2 / 8
+    # bytes per head: 8 MiB at S 8192, 128 MiB at S 32768).  Same gradients bit for bit.
+    recompute_mask_above: int = 8192
     # "fused" | "stage": which implementation the last forward() used; forward_packed: "fused_packed" | "per_sequence"
     # (diagnostics / benches)
     last_path = None
@@ -107,7 +111,8 @@ class _SparseV2Mixin:
     def _fused_ok(self, q) -> bool:
         return (self.use_fused and q.is_cuda and q.dtype in (torch.bfloat16, torch.float16) and q.size(-1) in (64, 80, 128)
                 and q.size(1) % 128 == 0 and q.size(1) % self.sparse_coeff == 0
-                and (q.size(1) // self.sparse_coeff) % 4 == 0 and q.size(1) // self.sparse_coeff >= 8)
+                and (q.size(1) // self.sparse_coeff) % 4 == 0 and q.size(1) // self.sparse_coeff >= 8
+                and q.size(1) <= ext.LOOKUP_MAX_SEQ)
 
     def _maybe_train_loss(self, q, k):
         if self.host_trigger is not None:
@@ -127,9 +132,14 @@ class _SparseV2Mixin:
         q, k, v = q.contiguous(), k.contiguous(), v.contiguous()
         self._maybe_train_loss(q, k)           # PQ loss is a mean over rows: layout-invariant
         q_c, k_c = ext.pq_encode_pair(q, k, self.quantizer.weight)   # quantizer('encode') of both: [N, S, H, m]
-        mask, extra0, _ = ext.lookup_mask(q_c, k_c, self.sparse_coeff)
+        n_codewords = self.quantizer.weight.size(1)
         # [N, S, H, E]; with reference_output_layout the kernel writes the shipped layer's re-interpretation of
         # [N*H, E, S] memory itself (forward epilogue / backward row prologue): no permute pass either way
+        if q.size(1) > self.recompute_mask_above:
+            return kernels.sparse_attention_recompute(q, k, v, q_c, k_c, self.sparse_coeff, self.scaling,
+                                                      reference_layout=self.reference_output_layout,
+                                                      n_codewords=n_codewords)
+        mask, extra0, _ = ext.lookup_mask(q_c, k_c, self.sparse_coeff, n_codewords=n_codewords)
         return kernels.sparse_attention(q, k, v, mask, extra0, self.scaling,
                                         reference_layout=self.reference_output_layout)
 
@@ -138,7 +148,7 @@ class _SparseV2Mixin:
         return (self.use_fused and q.is_cuda and q.dtype in (torch.bfloat16, torch.float16) and q.size(-1) in (64, 80, 128)
                 and max_seqlen <= ext.lookup_mask_varlen_max_seqlen(m))
 
-    def _rotate_packed(self, x, cu):      # the rotary layer restarts positions at every sequence start
+    def _rotate_packed(self, x, cu, max_seqlen=None):      # the rotary layer restarts positions at every sequence start
         return x
 
     def forward_packed(self, q, k, v, cu_seqlens, max_seqlen=None):
@@ -166,13 +176,19 @@ class _SparseV2Mixin:
             cu = torch.tensor([int(x) for x in host], dtype=torch.int32, device=q.device)
         if self._packed_fused_ok(q, max_seqlen):
             self.last_path = "fused_packed"
-            q, k, v = self._rotate_packed(q, cu), self._rotate_packed(k, cu), v.contiguous()
+            q, k, v = self._rotate_packed(q, cu, max_seqlen), self._rotate_packed(k, cu, max_seqlen), v.contiguous()
             q, k = q.contiguous(), k.contiguous()
             self._maybe_train_loss(q, k)      # over all T rows
             q_c, k_c = ext.pq_encode_pair(q, k, self.quantizer.weight)
-            mask, extra0 = ext.lookup_mask_varlen(q_c, k_c, cu, max_seqlen, self.sparse_coeff)
-            y = kernels.sparse_attention_varlen(q, k, v, mask, extra0, cu, max_seqlen, self.scaling,
-                                                reference_layout=self.reference_output_layout)
+            n_codewords = self.quantizer.weight.size(1)
+            if max_seqlen > self.recompute_mask_above:
+                y = kernels.sparse_attention_varlen_recompute(q, k, v, q_c, k_c, cu, max_seqlen, self.sparse_coeff,
+                                                              self.scaling, reference_layout=self.reference_output_layout,
+                                                              n_codewords=n_codewords)
+            else:
+                mask, extra0 = ext.lookup_mask_varlen(q_c, k_c, cu, max_seqlen, self.sparse_coeff, n_codewords=n_codewords)
+                y = kernels.sparse_attention_varlen(q, k, v, mask, extra0, cu, max_seqlen, self.scaling,
+                                                    reference_layout=self.reference_output_layout)
         else:
             offs = [int(x) for x in cu.tolist()]
             y = torch.cat([self.forward(q[:, a:b], k[:, a:b], v[:, a:b]) for a, b in zip(offs[:-1], offs[1:])], dim=1)
@@ -246,11 +262,12 @@ class SparseRotaryAttentionV2(_SparseV2Mixin, RotaryAttention):
     def _get_attn(self, q, k, attn_mask):
         return self._sparse_get_attn(self._rotate(q), self._rotate(k))
 
-    def _rotate_packed(self, x, cu):
-        # position of token t = t - cu[sequence of t], built on the device (no host synchronisation)
+    def _rotate_packed(self, x, cu, max_seqlen=None):
+        # position of token t = t - cu[sequence of t], built on the device (no host synchronisation); max_seqlen (> every
+        # position) extends the rotation tables where it exceeds them
         t = torch.arange(x.size(1), dtype=torch.int32, device=x.device)
         ids = (t - cu[torch.searchsorted(cu, t, right=True) - 1]).long()
-        return self.embedding(x, ids=ids).to(x.dtype)
+        return self.embedding(x, ids=ids, n_positions=max_seqlen).to(x.dtype)
 
     def forward(self, q, k, v, attn_mask=None):
         if self._fused_ok(q):
