@@ -329,6 +329,51 @@ int spt_sparse_attn_bwd_ex(const void *q, const void *k, const void *v, const vo
                            float scale, float clamp, int dtype, int flags, spt_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------
+ * Grouped-query / multi-query attention (DESIGN.md section 4.6).  H query heads, Hkv key / value heads,
+ * H % Hkv == 0, G = H / Hkv: query head h attends with key / value head h / G (HF LLaMA / Mistral
+ * repeat_kv, i.e. k and v repeated G times along the head axis).  Interleaved layouts only: q, y [N, S, H, d]
+ * with k, v [N, S, Hkv, d] (B = N*H), or packed q [T, H, d] with k, v [T, Hkv, d]; query codes [N, S, H, m]
+ * with key codes [N, S, Hkv, m] (packed: [T, H, m] / [T, Hkv, m]).  mask / extra0 / zsum and grad_q are per
+ * query head as in the multi-head calls; grad_k / grad_v have k's shape.  The result is the multi-head call
+ * on the repeated k and v; grad_k / grad_v are its gradients summed over each group of G heads in fp32,
+ * ascending, rounded once.  Hkv = H is exactly the multi-head call (the plain / _ex entry points are these
+ * with Hkv = H).  Hkv < 1 and H % Hkv != 0 return SPT_ERR_INVALID_ARGUMENT before any CUDA call.
+ *
+ * spt_lookup_mask_gqa_fwd / spt_lookup_mask_varlen_gqa_fwd: the key bitmaps are built once per key head, so
+ *   the workspace is spt_lookup_workspace_bytes(N*Hkv, S, m, nnz) / spt_lookup_mask_varlen_workspace_bytes(n_seq,
+ *   T, Hkv, m).  n_codewords: as in the _ex forms, or -1 for no promise (the plain forms).
+ * spt_sparse_attn_bwd_gqa / spt_sparse_attn_varlen_bwd_gqa: with Hkv < H the dK/dV kernels write every query
+ *   head's dK and dV into partials in the workspace and a reduction kernel sums the groups;
+ *   spt_sparse_attn_bwd_gqa_workspace_bytes / spt_sparse_attn_varlen_bwd_gqa_workspace_bytes are the multi-head
+ *   sizes plus 2 B S d 2 (packed: 2 H T d 2) bytes when Hkv < H.
+ * ------------------------------------------------------------------------------------------ */
+int spt_lookup_mask_gqa_fwd(const int32_t *query_codes, const int32_t *key_codes, int32_t *output,
+                            uint32_t *mask, int32_t *extra0, void *workspace, int B, int S, int m, int nnz,
+                            int H, int Hkv, int n_codewords, spt_stream_t stream);
+int spt_lookup_mask_varlen_gqa_fwd(const int32_t *query_codes, const int32_t *key_codes, const void *work,
+                                   uint32_t *mask, int32_t *extra0, void *workspace, int n_seq, int T,
+                                   int max_seqlen, int H, int Hkv, int m, int sparse_coeff, int n_codewords,
+                                   spt_stream_t stream);
+int spt_sparse_attn_fwd_gqa(const void *q, const void *k, const void *v, const uint32_t *mask,
+                            const int32_t *extra0, void *y, float *zsum, int B, int S, int d, int H, int Hkv,
+                            float scale, float clamp, int dtype, int flags, spt_stream_t stream);
+size_t spt_sparse_attn_bwd_gqa_workspace_bytes(int B, int S, int d, int H, int Hkv);
+int spt_sparse_attn_bwd_gqa(const void *q, const void *k, const void *v, const void *y, const void *grad_y,
+                            const uint32_t *mask, const int32_t *extra0, const float *zsum, void *grad_q,
+                            void *grad_k, void *grad_v, void *workspace, int B, int S, int d, int H, int Hkv,
+                            float scale, float clamp, int dtype, int flags, spt_stream_t stream);
+int spt_sparse_attn_varlen_fwd_gqa(const void *q, const void *k, const void *v, const uint32_t *mask,
+                                   const int32_t *extra0, void *y, float *zsum, const void *work, int n_seq,
+                                   int T, int max_seqlen, int d, int H, int Hkv, float scale, float clamp,
+                                   int dtype, int flags, spt_stream_t stream);
+size_t spt_sparse_attn_varlen_bwd_gqa_workspace_bytes(int T, int d, int H, int Hkv);
+int spt_sparse_attn_varlen_bwd_gqa(const void *q, const void *k, const void *v, const void *y, const void *grad_y,
+                                   const uint32_t *mask, const int32_t *extra0, const float *zsum, void *grad_q,
+                                   void *grad_k, void *grad_v, void *workspace, const void *work, int n_seq,
+                                   int T, int max_seqlen, int d, int H, int Hkv, float scale, float clamp,
+                                   int dtype, int flags, spt_stream_t stream);
+
+/* ------------------------------------------------------------------------------------------
  * (6) routed FFN — the grouped GEMM the reference only sketches (legacy/routed.cpp:10-68,
  * legacy/test_routed.py:9-26) and ships as a Python loop (layers/sparse/feedforward.py:47-85).
  *

@@ -105,6 +105,15 @@ def _load() -> ctypes.CDLL:
     sig["spt_sparse_attn_varlen_fwd"] = (i32, [vp] * 8 + [i32, i32, i32, i32, i32, f32, f32, i32, i32, vp])
     sig["spt_sparse_attn_varlen_bwd_workspace_bytes"] = (sz, [i32, i32])
     sig["spt_sparse_attn_varlen_bwd"] = (i32, [vp] * 13 + [i32, i32, i32, i32, i32, f32, f32, i32, i32, vp])
+    # grouped-query attention: H query heads, Hkv key / value heads
+    sig["spt_lookup_mask_gqa_fwd"] = (i32, [vp] * 6 + [i32] * 7 + [vp])
+    sig["spt_lookup_mask_varlen_gqa_fwd"] = (i32, [vp] * 6 + [i32] * 8 + [vp])
+    sig["spt_sparse_attn_fwd_gqa"] = (i32, [vp] * 7 + [i32, i32, i32, i32, i32, f32, f32, i32, i32, vp])
+    sig["spt_sparse_attn_bwd_gqa_workspace_bytes"] = (sz, [i32] * 5)
+    sig["spt_sparse_attn_bwd_gqa"] = (i32, [vp] * 12 + [i32, i32, i32, i32, i32, f32, f32, i32, i32, vp])
+    sig["spt_sparse_attn_varlen_fwd_gqa"] = (i32, [vp] * 8 + [i32] * 6 + [f32, f32, i32, i32, vp])
+    sig["spt_sparse_attn_varlen_bwd_gqa_workspace_bytes"] = (sz, [i32] * 4)
+    sig["spt_sparse_attn_varlen_bwd_gqa"] = (i32, [vp] * 13 + [i32] * 6 + [f32, f32, i32, i32, vp])
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)  # AttributeError => header/library mismatch, fail loudly
         fn.restype = res

@@ -412,15 +412,15 @@ __device__ __forceinline__ void out_chunks(int half, F &&f) {
 
 // 128 x 128-tile kernels (attn_tc128.cu), head dim 64
 namespace attn_tc128 {
-// T = __nv_bfloat16 or __half; zsum is read by the fp16 kernels only (row scales)
+// T = __nv_bfloat16 or __half; zsum is read by the fp16 kernels only (row scales); G query heads per key / value head
 template <typename T>
 int launch_bwd_kv128(const CUtensorMap &mq, const CUtensorMap &mk, const CUtensorMap &mv, const CUtensorMap &md,
                      const uint32_t *mask, const int32_t *extra0, const float *ndelta, const float *zsum, T *gk, T *gv,
-                     int B, int S, int H, float scale, float clamp, cudaStream_t st);
+                     int B, int S, int H, int G, float scale, float clamp, cudaStream_t st);
 template <typename T>
 int launch_bwd_q128(const CUtensorMap &mq, const CUtensorMap &mk, const CUtensorMap &mv, const CUtensorMap &md,
                     const uint32_t *mask, const int32_t *extra0, const float *ndelta, const float *zsum, T *gq, int B,
-                    int S, int H, float scale, float clamp, cudaStream_t st);
+                    int S, int H, int G, float scale, float clamp, cudaStream_t st);
 int read_prof(unsigned long long *out48, int reset);
 }  // namespace attn_tc128
 }  // namespace spt

@@ -48,12 +48,14 @@ namespace attn_tc {
 // fp16 (T = __half): kg is the key tensor itself (the row scale reads key row 0 of the head); unused in bf16.
 // VARLEN: packed sequences (S = T, H heads, grid (H, work-list capacity)); rows at or past the sequence end read
 // neutral per-row data and store nothing.
+// G: query heads per key / value head (grouped-query attention; 1 = multi-head).  k and v have H / G heads and query head
+// hh reads key / value head hh / G, in every kernel of this file and of attn_tc128.cu.
 template <int D, typename T, bool VARLEN = false>
 __global__ void __launch_bounds__(THREADS, Dim<D>::CTAS)
 attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_k,
                    const __grid_constant__ CUtensorMap map_v, const uint32_t *__restrict__ mask,
                    const int32_t *__restrict__ extra0, T *__restrict__ y, float *__restrict__ zsum, int S,
-                   int H, float scale_log2, float clamp_log2, int y_transposed, const T *__restrict__ kg,
+                   int H, float scale_log2, float clamp_log2, int y_transposed, const T *__restrict__ kg, int G,
                    const Varlen vl = {}) {
     constexpr int OWN_BYTES = Dim<D>::OWN_BYTES, T_BYTES = Dim<D>::T_BYTES, OWN_SUB = Dim<D>::OWN_SUB, T_SUB = Dim<D>::T_SUB,
                   TMEM_COLS = Dim<D>::TMEM_COLS, DP = Dim<D>::DP;
@@ -86,7 +88,7 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_const
     const int b = blockIdx.x;
     const int m0 = tile * BM;
     const int n_tiles = VARLEN ? (min(m0 + BM, len) + BN - 1) / BN : (m0 + BM) / BN;   // key tiles 0 .. (causal)
-    const int hn = VARLEN ? 0 : b / H, hh = VARLEN ? b : b % H;
+    const int hn = VARLEN ? 0 : b / H, hh = VARLEN ? b : b % H, hk = hh / G;
 
     if (threadIdx.x == 0) {
         mbar_init(q_full, 1);
@@ -121,10 +123,10 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_const
                 const uint32_t ph = (j / STAGES) & 1;
                 mbar_wait(k_empty(st), ph ^ 1);
                 mbar_expect_tx(k_full(st), T_BYTES);
-                tma_other<D>(s_k + st * T_BYTES, &map_k, k_full(st), hh, start + j * BN, hn);
+                tma_other<D>(s_k + st * T_BYTES, &map_k, k_full(st), hk, start + j * BN, hn);
                 mbar_wait(v_empty(st), ph ^ 1);
                 mbar_expect_tx(v_full(st), T_BYTES);
-                tma_other<D>(s_v + st * T_BYTES, &map_v, v_full(st), hh, start + j * BN, hn);
+                tma_other<D>(s_v + st * T_BYTES, &map_v, v_full(st), hk, start + j * BN, hn);
             }
         }
     } else if (warp == 9) {
@@ -211,7 +213,8 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_const
             // t0 2^-o < 2^15 and e^c 2^-o < 2^16, so no element can overflow, and a row whose scores are all low keeps
             // normal fp16 values.  q.k_0 in fp32 from the row's Q in shared memory and key row 0 of the head.
             mbar_wait(q_full, 0);
-            const T *k0 = VARLEN ? kg + ((size_t)start * H + hh) * D : kg + ((size_t)hn * S * H + hh) * D;   // the sequence's key 0
+            const int hkv = H / G;
+            const T *k0 = VARLEN ? kg + ((size_t)start * hkv + hk) * D : kg + ((size_t)hn * S * hkv + hk) * D;   // the sequence's key 0
             float dot = 0.0f;
 #pragma unroll
             for (int c = 0; c < D / 8; ++c) {              // 16-byte chunk c: sub-tile c / 8, 128-byte swizzled by the row
@@ -436,7 +439,7 @@ attn_bwd_q_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
                      const __grid_constant__ CUtensorMap map_v, const __grid_constant__ CUtensorMap map_dys,
                      const uint32_t *__restrict__ mask, const int32_t *__restrict__ extra0,
                      const float *__restrict__ delta, T *__restrict__ dq, int S, int H, float scale,
-                     float scale_log2, float clamp_log2, const float *__restrict__ zsum, const Varlen vl = {}) {
+                     float scale_log2, float clamp_log2, const float *__restrict__ zsum, int G, const Varlen vl = {}) {
     constexpr int OWN_BYTES = Dim<D>::OWN_BYTES, T_BYTES = Dim<D>::T_BYTES, OWN_SUB = Dim<D>::OWN_SUB, T_SUB = Dim<D>::T_SUB,
                   TMEM_COLS = Dim<D>::TMEM_COLS, DP = Dim<D>::DP;
     extern __shared__ unsigned char smem_raw[];
@@ -463,7 +466,7 @@ attn_bwd_q_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
     const int b = blockIdx.x;
     const int m0 = tile * BM;
     const int n_tiles = VARLEN ? (min(m0 + BM, len) + BN - 1) / BN : (m0 + BM) / BN;
-    const int hn = VARLEN ? 0 : b / H, hh = VARLEN ? b : b % H;
+    const int hn = VARLEN ? 0 : b / H, hh = VARLEN ? b : b % H, hk = hh / G;
 
     if (threadIdx.x == 0) {
         mbar_init(own_full, 1);
@@ -495,8 +498,8 @@ attn_bwd_q_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
                 const int st = j % STAGES;
                 mbar_wait(kv_empty(st), ((j / STAGES) & 1) ^ 1);
                 mbar_expect_tx(kv_full(st), 2 * T_BYTES);
-                tma_other<D>(s_k + st * T_BYTES, &map_k, kv_full(st), hh, start + j * BN, hn);
-                tma_other<D>(s_v + st * T_BYTES, &map_v, kv_full(st), hh, start + j * BN, hn);
+                tma_other<D>(s_k + st * T_BYTES, &map_k, kv_full(st), hk, start + j * BN, hn);
+                tma_other<D>(s_v + st * T_BYTES, &map_v, kv_full(st), hk, start + j * BN, hn);
             }
         }
     } else if (warp == 9) {
@@ -636,7 +639,7 @@ attn_bwd_kv_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_co
                       const uint32_t *__restrict__ mask, const int32_t *__restrict__ extra0,
                       const float *__restrict__ delta, T *__restrict__ dk, T *__restrict__ dv,
                       int S, int H, float scale, float scale_log2, float clamp_log2, const float *__restrict__ zsum,
-                      const Varlen vl = {}) {
+                      int G, const Varlen vl = {}) {
     constexpr int OWN_BYTES = Dim<D>::OWN_BYTES, T_BYTES = Dim<D>::T_BYTES, OWN_SUB = Dim<D>::OWN_SUB, T_SUB = Dim<D>::T_SUB,
                   TMEM_COLS = Dim<D>::TMEM_COLS, DP = Dim<D>::DP;
     extern __shared__ unsigned char smem_raw[];
@@ -667,7 +670,7 @@ attn_bwd_kv_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_co
     const int n0 = kt * BM;
     const int j0 = n0 / BN;                            // first query tile that can see these keys
     const int n_tiles = (VARLEN ? (len + BN - 1) / BN : S / BN) - j0;
-    const int hn = VARLEN ? 0 : b / H, hh = VARLEN ? b : b % H;
+    const int hn = VARLEN ? 0 : b / H, hh = VARLEN ? b : b % H, hk = hh / G;
     const size_t head = (size_t)b * S + start;
     const int words = VARLEN ? vl.mwords : S / 32;
 
@@ -696,8 +699,8 @@ attn_bwd_kv_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_co
     if (warp == 8) {
         if (lane == 0) {
             mbar_expect_tx(own_full, 2 * OWN_BYTES);
-            tma_owner<D>(s_k, &map_k, own_full, hh, start + n0, hn);
-            tma_owner<D>(s_v, &map_v, own_full, hh, start + n0, hn);
+            tma_owner<D>(s_k, &map_k, own_full, hk, start + n0, hn);
+            tma_owner<D>(s_v, &map_v, own_full, hk, start + n0, hn);
         }
         for (int j = 0; j < n_tiles; ++j) {
             const int st = j % STAGES;
@@ -902,10 +905,10 @@ static SideStream *side_stream(cudaStream_t caller) {   // g_side_mu held
 template <int D, typename T>
 static int launch_fwd(const CUtensorMap &mq, const CUtensorMap &mk, const CUtensorMap &mv, const uint32_t *mask,
                       const int32_t *extra0, T *y, float *zsum, int B, int S, int H, float scale, float clamp,
-                      int y_transposed, const T *k, cudaStream_t st) {
+                      int y_transposed, const T *k, int G, cudaStream_t st) {
     cudaFuncSetAttribute(attn_fwd_tc_kernel<D, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, Dim<D>::FWD_SMEM);
     attn_fwd_tc_kernel<D, T><<<dim3(B, S / BM), THREADS, Dim<D>::FWD_SMEM, st>>>(mq, mk, mv, mask, extra0, y, zsum, S, H,
-                                                                                 scale * LOG2E, clamp * LOG2E, y_transposed, k);
+                                                                                 scale * LOG2E, clamp * LOG2E, y_transposed, k, G);
     return after_launch("attn_fwd_tc_kernel");
 }
 
@@ -925,7 +928,7 @@ static int launch_prep(const T *y, const T *grad_y, const float *zsum, float *de
 template <int D, typename T>
 static int launch_bwd(const CUtensorMap &mq, const CUtensorMap &mk, const CUtensorMap &mv, const CUtensorMap &md,
                       const uint32_t *mask, const int32_t *extra0, const float *delta, const float *zsum, T *gq, T *gk,
-                      T *gv, int B, int S, int H, float scale, float clamp, cudaStream_t st) {
+                      T *gv, int B, int S, int H, int G, float scale, float clamp, cudaStream_t st) {
     if (D == 64 && tile128()) {
         {
             // The dK/dV and the dQ kernel are independent: the dQ kernel goes to a side stream (fork / join with events,
@@ -936,9 +939,9 @@ static int launch_bwd(const CUtensorMap &mq, const CUtensorMap &mk, const CUtens
             if (ss) {
                 if (cudaEventRecord(ss->fork, st) != cudaSuccess || cudaStreamWaitEvent(ss->stream, ss->fork, 0) != cudaSuccess)
                     return fail(SPT_ERR_CUDA, "sparse_attn_bwd: fork to the side stream failed");
-                int rc = attn_tc128::launch_bwd_kv128(mq, mk, mv, md, mask, extra0, delta, zsum, gk, gv, B, S, H, scale, clamp, st);
+                int rc = attn_tc128::launch_bwd_kv128(mq, mk, mv, md, mask, extra0, delta, zsum, gk, gv, B, S, H, G, scale, clamp, st);
                 if (rc != SPT_OK) return rc;
-                rc = attn_tc128::launch_bwd_q128(mq, mk, mv, md, mask, extra0, delta, zsum, gq, B, S, H, scale, clamp, ss->stream);
+                rc = attn_tc128::launch_bwd_q128(mq, mk, mv, md, mask, extra0, delta, zsum, gq, B, S, H, G, scale, clamp, ss->stream);
                 if (rc != SPT_OK) return rc;
                 if (cudaEventRecord(ss->join, ss->stream) != cudaSuccess || cudaStreamWaitEvent(st, ss->join, 0) != cudaSuccess)
                     return fail(SPT_ERR_CUDA, "sparse_attn_bwd: join of the side stream failed");
@@ -947,18 +950,18 @@ static int launch_bwd(const CUtensorMap &mq, const CUtensorMap &mk, const CUtens
         }
         // no side stream (it is never created during a capture, so a process whose first backward is captured gets
         // here): one kernel after the other on the caller's stream
-        const int rc = attn_tc128::launch_bwd_kv128(mq, mk, mv, md, mask, extra0, delta, zsum, gk, gv, B, S, H, scale, clamp, st);
+        const int rc = attn_tc128::launch_bwd_kv128(mq, mk, mv, md, mask, extra0, delta, zsum, gk, gv, B, S, H, G, scale, clamp, st);
         if (rc != SPT_OK) return rc;
-        return attn_tc128::launch_bwd_q128(mq, mk, mv, md, mask, extra0, delta, zsum, gq, B, S, H, scale, clamp, st);
+        return attn_tc128::launch_bwd_q128(mq, mk, mv, md, mask, extra0, delta, zsum, gq, B, S, H, G, scale, clamp, st);
     }
     constexpr int kv_smem = Dim<D>::BWD_SMEM + (is_f16<T> ? STAGES * BN * 4 : 0);      // fp16: the rows' -o per stage
     cudaFuncSetAttribute(attn_bwd_kv_tc_kernel<D, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, kv_smem);
     attn_bwd_kv_tc_kernel<D, T><<<dim3(B, S / BM), THREADS, kv_smem, st>>>(
-        mq, mk, mv, md, mask, extra0, delta, gk, gv, S, H, scale, scale * LOG2E, clamp * LOG2E, zsum);
+        mq, mk, mv, md, mask, extra0, delta, gk, gv, S, H, scale, scale * LOG2E, clamp * LOG2E, zsum, G);
     SPT_LAUNCH_CHECK("attn_bwd_kv_tc_kernel");
     cudaFuncSetAttribute(attn_bwd_q_tc_kernel<D, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, Dim<D>::BWD_SMEM);
     attn_bwd_q_tc_kernel<D, T><<<dim3(B, S / BM), THREADS, Dim<D>::BWD_SMEM, st>>>(
-        mq, mk, mv, md, mask, extra0, delta, gq, S, H, scale, scale * LOG2E, clamp * LOG2E, zsum);
+        mq, mk, mv, md, mask, extra0, delta, gq, S, H, scale, scale * LOG2E, clamp * LOG2E, zsum, G);
     SPT_LAUNCH_CHECK("attn_bwd_q_tc_kernel");
     return SPT_OK;
 }
@@ -968,10 +971,10 @@ static int launch_bwd(const CUtensorMap &mq, const CUtensorMap &mk, const CUtens
 template <int D, typename T>
 static int launch_fwd_varlen(const CUtensorMap &mq, const CUtensorMap &mk, const CUtensorMap &mv, const uint32_t *mask,
                              const int32_t *extra0, T *y, float *zsum, const Varlen &vl, int cap, int S, int H, float scale,
-                             float clamp, int y_transposed, const T *k, cudaStream_t st) {
+                             float clamp, int y_transposed, const T *k, int G, cudaStream_t st) {
     cudaFuncSetAttribute(attn_fwd_tc_kernel<D, T, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, Dim<D>::FWD_SMEM);
     attn_fwd_tc_kernel<D, T, true><<<dim3(H, cap), THREADS, Dim<D>::FWD_SMEM, st>>>(
-        mq, mk, mv, mask, extra0, y, zsum, S, H, scale * LOG2E, clamp * LOG2E, y_transposed, k, vl);
+        mq, mk, mv, mask, extra0, y, zsum, S, H, scale * LOG2E, clamp * LOG2E, y_transposed, k, G, vl);
     return after_launch("attn_fwd_tc_kernel(varlen)");
 }
 
@@ -986,23 +989,62 @@ static int launch_prep_varlen(const T *y, const T *grad_y, const float *zsum, fl
 template <int D, typename T>
 static int launch_bwd_varlen(const CUtensorMap &mq, const CUtensorMap &mk, const CUtensorMap &mv, const CUtensorMap &md,
                              const uint32_t *mask, const int32_t *extra0, const float *delta, const float *zsum, T *gq, T *gk,
-                             T *gv, const Varlen &vl, int cap, int S, int H, float scale, float clamp, cudaStream_t st) {
+                             T *gv, const Varlen &vl, int cap, int S, int H, int G, float scale, float clamp, cudaStream_t st) {
     constexpr int kv_smem = Dim<D>::BWD_SMEM + (is_f16<T> ? STAGES * BN * 4 : 0);      // fp16: the rows' -o per stage
     cudaFuncSetAttribute(attn_bwd_kv_tc_kernel<D, T, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kv_smem);
     attn_bwd_kv_tc_kernel<D, T, true><<<dim3(H, cap), THREADS, kv_smem, st>>>(
-        mq, mk, mv, md, mask, extra0, delta, gk, gv, S, H, scale, scale * LOG2E, clamp * LOG2E, zsum, vl);
+        mq, mk, mv, md, mask, extra0, delta, gk, gv, S, H, scale, scale * LOG2E, clamp * LOG2E, zsum, G, vl);
     SPT_LAUNCH_CHECK("attn_bwd_kv_tc_kernel(varlen)");
     cudaFuncSetAttribute(attn_bwd_q_tc_kernel<D, T, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, Dim<D>::BWD_SMEM);
     attn_bwd_q_tc_kernel<D, T, true><<<dim3(H, cap), THREADS, Dim<D>::BWD_SMEM, st>>>(
-        mq, mk, mv, md, mask, extra0, delta, gq, S, H, scale, scale * LOG2E, clamp * LOG2E, zsum, vl);
+        mq, mk, mv, md, mask, extra0, delta, gq, S, H, scale, scale * LOG2E, clamp * LOG2E, zsum, G, vl);
     SPT_LAUNCH_CHECK("attn_bwd_q_tc_kernel(varlen)");
     return SPT_OK;
+}
+
+// ---- grouped-query attention: the dK / dV group sum --------------------------------------------------------------------
+// With G > 1 query heads per key / value head, the dK/dV kernels write every query head's dK and dV (what they write for
+// k and v repeated G times) into partials [rows, H, D]; key / value head hk of a row is the sum of heads hk G .. hk G + G - 1,
+// added in fp32 in ascending order and rounded once.  One thread per 8 elements (D % 8 == 0).
+template <typename T>
+__global__ void __launch_bounds__(256)
+gqa_group_sum_kernel(const T *__restrict__ part, T *__restrict__ out, int64_t n8, int G, int D) {
+    const int64_t i = (int64_t)blockIdx.x * 256 + threadIdx.x;   // 8-element chunk of out [rows, H / G, D]
+    if (i >= n8) return;
+    const int c8 = D / 8;
+    const int64_t rk = i / c8;                                   // (row, kv head)
+    const int c = (int)(i - rk * c8) * 8;
+    const T *src = part + rk * G * D + c;
+    float acc[8] = {0.0f, 0.0f, 0.0f, 0.0f, 0.0f, 0.0f, 0.0f, 0.0f};
+    for (int g = 0; g < G; ++g) {
+        float x[8];
+        Vec16<T>::load(src + (size_t)g * D, x);
+#pragma unroll
+        for (int u = 0; u < 8; ++u) acc[u] += x[u];
+    }
+    Vec16<T>::store(out + rk * D + c, acc);
+}
+
+template <typename T>
+static int launch_group_sum(const T *part, T *out, int64_t rows_kv, int G, int D, cudaStream_t st) {
+    const int64_t n8 = rows_kv * (D / 8);
+    gqa_group_sum_kernel<T><<<(unsigned)((n8 + 255) / 256), 256, 0, st>>>(part, out, n8, G, D);
+    return after_launch("gqa_group_sum_kernel");
 }
 
 }  // namespace attn_tc
 }  // namespace spt
 
 using namespace spt;
+
+// grouped-query attention: H query heads, Hkv key / value heads
+static int check_gqa(const char *what, int H, int Hkv) {
+    if (Hkv < 1) return fail(SPT_ERR_INVALID_ARGUMENT, "%s: the key / value head count Hkv=%d must be >= 1", what, Hkv);
+    if (H % Hkv != 0)
+        return fail(SPT_ERR_INVALID_ARGUMENT, "%s: the query head count H=%d must be a multiple of the key / value head count Hkv=%d",
+                    what, H, Hkv);
+    return SPT_OK;
+}
 
 static int check_attn_type(const char *what, int d, int dtype, float clamp) {
     if (dtype != SPT_BF16 && dtype != SPT_F16)
@@ -1027,19 +1069,19 @@ static int check_attn_args(const char *what, int B, int S, int d, int H, int dty
 template <typename T>
 static int attn_fwd_typed(const CUtensorMap &mq, const CUtensorMap &mk, const CUtensorMap &mv, const uint32_t *mask,
                           const int32_t *extra0, void *y, float *zsum, int B, int S, int d, int H, float scale, float clamp,
-                          int yt, const void *k, cudaStream_t st) {
+                          int yt, const void *k, int G, cudaStream_t st) {
     T *yy = (T *)y;
     const T *kk = (const T *)k;
-    if (d == 64) return attn_tc::launch_fwd<64, T>(mq, mk, mv, mask, extra0, yy, zsum, B, S, H, scale, clamp, yt, kk, st);
-    if (d == 80) return attn_tc::launch_fwd<80, T>(mq, mk, mv, mask, extra0, yy, zsum, B, S, H, scale, clamp, yt, kk, st);
-    return attn_tc::launch_fwd<128, T>(mq, mk, mv, mask, extra0, yy, zsum, B, S, H, scale, clamp, yt, kk, st);
+    if (d == 64) return attn_tc::launch_fwd<64, T>(mq, mk, mv, mask, extra0, yy, zsum, B, S, H, scale, clamp, yt, kk, G, st);
+    if (d == 80) return attn_tc::launch_fwd<80, T>(mq, mk, mv, mask, extra0, yy, zsum, B, S, H, scale, clamp, yt, kk, G, st);
+    return attn_tc::launch_fwd<128, T>(mq, mk, mv, mask, extra0, yy, zsum, B, S, H, scale, clamp, yt, kk, G, st);
 }
 
-// the backward after the argument checks: row kernel, tensor maps, dK/dV + dQ kernels
+// the backward after the argument checks: row kernel, tensor maps, dK/dV + dQ kernels (+ the group sum when Hkv < H)
 template <typename T>
 static int attn_bwd_typed(const void *q, const void *k, const void *v, const void *y, const void *grad_y,
                           const uint32_t *mask, const int32_t *extra0, const float *zsum, void *grad_q, void *grad_k,
-                          void *grad_v, void *workspace, int B, int S, int d, int H, float scale, float clamp, int yt,
+                          void *grad_v, void *workspace, int B, int S, int d, int H, int Hkv, float scale, float clamp, int yt,
                           cudaStream_t st) {
     constexpr bool f16 = attn_tc::is_f16<T>;
     float *delta = (float *)workspace;
@@ -1052,15 +1094,21 @@ static int attn_bwd_typed(const void *q, const void *k, const void *v, const voi
     if (rc != SPT_OK) return rc;
     CUtensorMap mq, mk, mv, md;
     if ((rc = attn_tc::make_map(&mq, q, B / H, S, H, d, f16)) != SPT_OK) return rc;
-    if ((rc = attn_tc::make_map(&mk, k, B / H, S, H, d, f16)) != SPT_OK) return rc;
-    if ((rc = attn_tc::make_map(&mv, v, B / H, S, H, d, f16)) != SPT_OK) return rc;
+    if ((rc = attn_tc::make_map(&mk, k, B / H, S, Hkv, d, f16)) != SPT_OK) return rc;
+    if ((rc = attn_tc::make_map(&mv, v, B / H, S, Hkv, d, f16)) != SPT_OK) return rc;
     if ((rc = attn_tc::make_map(&md, dys, B / H, S, H, d, f16)) != SPT_OK) return rc;
+    const int G = H / Hkv;
     T *gq = (T *)grad_q, *gk = (T *)grad_k, *gv = (T *)grad_v;
-    if (d == 64)
-        return attn_tc::launch_bwd<64, T>(mq, mk, mv, md, mask, extra0, delta, zsum, gq, gk, gv, B, S, H, scale, clamp, st);
-    if (d == 80)
-        return attn_tc::launch_bwd<80, T>(mq, mk, mv, md, mask, extra0, delta, zsum, gq, gk, gv, B, S, H, scale, clamp, st);
-    return attn_tc::launch_bwd<128, T>(mq, mk, mv, md, mask, extra0, delta, zsum, gq, gk, gv, B, S, H, scale, clamp, st);
+    // G > 1: every query head's dK / dV go to partials [N, S, H, d] after dO' in the workspace, then the group sum
+    T *pk = G > 1 ? (T *)((char *)workspace + spt_sparse_attn_bwd_workspace_bytes(B, S)) : gk;
+    T *pv = G > 1 ? pk + (size_t)B * S * d : gv;
+    rc = d == 64   ? attn_tc::launch_bwd<64, T>(mq, mk, mv, md, mask, extra0, delta, zsum, gq, pk, pv, B, S, H, G, scale, clamp, st)
+         : d == 80 ? attn_tc::launch_bwd<80, T>(mq, mk, mv, md, mask, extra0, delta, zsum, gq, pk, pv, B, S, H, G, scale, clamp, st)
+                   : attn_tc::launch_bwd<128, T>(mq, mk, mv, md, mask, extra0, delta, zsum, gq, pk, pv, B, S, H, G, scale, clamp, st);
+    if (rc != SPT_OK || G == 1) return rc;
+    const int64_t rows_kv = (int64_t)(B / G) * S;
+    if ((rc = attn_tc::launch_group_sum<T>(pk, gk, rows_kv, G, d, st)) != SPT_OK) return rc;
+    return attn_tc::launch_group_sum<T>(pv, gv, rows_kv, G, d, st);
 }
 
 extern "C" int spt_sparse_attn_fwd(const void *q, const void *k, const void *v, const uint32_t *mask,
@@ -1072,18 +1120,27 @@ extern "C" int spt_sparse_attn_fwd(const void *q, const void *k, const void *v, 
 extern "C" int spt_sparse_attn_fwd_ex(const void *q, const void *k, const void *v, const uint32_t *mask,
                                       const int32_t *extra0, void *y, float *zsum, int B, int S, int d, int H,
                                       float scale, float clamp, int dtype, int flags, spt_stream_t stream) {
+    return spt_sparse_attn_fwd_gqa(q, k, v, mask, extra0, y, zsum, B, S, d, H, H, scale, clamp, dtype, flags, stream);
+}
+
+extern "C" int spt_sparse_attn_fwd_gqa(const void *q, const void *k, const void *v, const uint32_t *mask,
+                                       const int32_t *extra0, void *y, float *zsum, int B, int S, int d, int H, int Hkv,
+                                       float scale, float clamp, int dtype, int flags, spt_stream_t stream) {
     SPT_REQUIRE(q && k && v && mask && extra0 && y && zsum, "sparse_attn_fwd: null pointer");
     const int yt = (flags & SPT_ATTN_Y_TRANSPOSED) ? 1 : 0;
     int rc = check_attn_args("sparse_attn_fwd", B, S, d, H, dtype, clamp);
     if (rc != SPT_OK) return rc;
+    if ((rc = check_gqa("sparse_attn_fwd", H, Hkv)) != SPT_OK) return rc;
     SPT_REQUIRE(((uintptr_t)q | (uintptr_t)k | (uintptr_t)v | (uintptr_t)y) % 16 == 0, "sparse_attn_fwd: operands must be 16-byte aligned");
     const bool f16 = dtype == SPT_F16;
     CUtensorMap mq, mk, mv;
     if ((rc = attn_tc::make_map(&mq, q, B / H, S, H, d, f16)) != SPT_OK) return rc;
-    if ((rc = attn_tc::make_map(&mk, k, B / H, S, H, d, f16)) != SPT_OK) return rc;
-    if ((rc = attn_tc::make_map(&mv, v, B / H, S, H, d, f16)) != SPT_OK) return rc;
-    return f16 ? attn_fwd_typed<__half>(mq, mk, mv, mask, extra0, y, zsum, B, S, d, H, scale, clamp, yt, k, as_stream(stream))
-               : attn_fwd_typed<__nv_bfloat16>(mq, mk, mv, mask, extra0, y, zsum, B, S, d, H, scale, clamp, yt, k, as_stream(stream));
+    if ((rc = attn_tc::make_map(&mk, k, B / H, S, Hkv, d, f16)) != SPT_OK) return rc;
+    if ((rc = attn_tc::make_map(&mv, v, B / H, S, Hkv, d, f16)) != SPT_OK) return rc;
+    const int G = H / Hkv;
+    return f16 ? attn_fwd_typed<__half>(mq, mk, mv, mask, extra0, y, zsum, B, S, d, H, scale, clamp, yt, k, G, as_stream(stream))
+               : attn_fwd_typed<__nv_bfloat16>(mq, mk, mv, mask, extra0, y, zsum, B, S, d, H, scale, clamp, yt, k, G,
+                                               as_stream(stream));
 }
 
 // diagnostics: phase timers of the attention kernels (all zeros unless built with -DSPT_ATTN_PROF); reset != 0 clears them
@@ -1109,6 +1166,12 @@ extern "C" size_t spt_sparse_attn_bwd_workspace_bytes(int B, int S) {
     return (size_t)B * S * sizeof(float) + (size_t)B * S * 128 * 2;
 }
 
+// Hkv < H: + the dK and dV partials of every query head, [B, S, d] each (operand type)
+extern "C" size_t spt_sparse_attn_bwd_gqa_workspace_bytes(int B, int S, int d, int H, int Hkv) {
+    const size_t base = spt_sparse_attn_bwd_workspace_bytes(B, S);
+    return Hkv >= 1 && Hkv < H ? base + 2 * (size_t)B * S * d * 2 : base;
+}
+
 extern "C" int spt_sparse_attn_bwd(const void *q, const void *k, const void *v, const void *y, const void *grad_y,
                                    const uint32_t *mask, const int32_t *extra0, const float *zsum, void *grad_q,
                                    void *grad_k, void *grad_v, void *workspace, int B, int S, int d, int H,
@@ -1121,18 +1184,29 @@ extern "C" int spt_sparse_attn_bwd_ex(const void *q, const void *k, const void *
                                       const uint32_t *mask, const int32_t *extra0, const float *zsum, void *grad_q,
                                       void *grad_k, void *grad_v, void *workspace, int B, int S, int d, int H,
                                       float scale, float clamp, int dtype, int flags, spt_stream_t stream) {
+    return spt_sparse_attn_bwd_gqa(q, k, v, y, grad_y, mask, extra0, zsum, grad_q, grad_k, grad_v, workspace, B, S, d, H, H,
+                                   scale, clamp, dtype, flags, stream);
+}
+
+extern "C" int spt_sparse_attn_bwd_gqa(const void *q, const void *k, const void *v, const void *y, const void *grad_y,
+                                       const uint32_t *mask, const int32_t *extra0, const float *zsum, void *grad_q,
+                                       void *grad_k, void *grad_v, void *workspace, int B, int S, int d, int H, int Hkv,
+                                       float scale, float clamp, int dtype, int flags, spt_stream_t stream) {
     const int yt = (flags & SPT_ATTN_Y_TRANSPOSED) ? 1 : 0;
     SPT_REQUIRE(q && k && v && y && grad_y && mask && extra0 && zsum && grad_q && grad_k && grad_v && workspace,
                 "sparse_attn_bwd: null pointer");
     int rc = check_attn_args("sparse_attn_bwd", B, S, d, H, dtype, clamp);
     if (rc != SPT_OK) return rc;
+    if ((rc = check_gqa("sparse_attn_bwd", H, Hkv)) != SPT_OK) return rc;
     SPT_REQUIRE(((uintptr_t)q | (uintptr_t)k | (uintptr_t)v | (uintptr_t)grad_y | (uintptr_t)workspace) % 16 == 0,
                 "sparse_attn_bwd: operands must be 16-byte aligned");
+    SPT_REQUIRE(Hkv == H || ((uintptr_t)grad_k | (uintptr_t)grad_v) % 16 == 0,
+                "sparse_attn_bwd: grad_k and grad_v must be 16-byte aligned");
     if (dtype == SPT_F16)
         return attn_bwd_typed<__half>(q, k, v, y, grad_y, mask, extra0, zsum, grad_q, grad_k, grad_v, workspace, B, S, d, H,
-                                      scale, clamp, yt, as_stream(stream));
+                                      Hkv, scale, clamp, yt, as_stream(stream));
     return attn_bwd_typed<__nv_bfloat16>(q, k, v, y, grad_y, mask, extra0, zsum, grad_q, grad_k, grad_v, workspace, B, S, d,
-                                         H, scale, clamp, yt, as_stream(stream));
+                                         H, Hkv, scale, clamp, yt, as_stream(stream));
 }
 
 // ---- packed variable-length sequences ----------------------------------------------------------------------------------
@@ -1144,35 +1218,46 @@ static attn_tc::Varlen varlen_of(const void *work, int max_seqlen) {
 template <typename T>
 static int attn_varlen_fwd_typed(const CUtensorMap &mq, const CUtensorMap &mk, const CUtensorMap &mv, const uint32_t *mask,
                                  const int32_t *extra0, void *y, float *zsum, const attn_tc::Varlen &vl, int cap, int S, int d,
-                                 int H, float scale, float clamp, int yt, const void *k, cudaStream_t st) {
+                                 int H, float scale, float clamp, int yt, const void *k, int G, cudaStream_t st) {
     T *yy = (T *)y;
     const T *kk = (const T *)k;
-    if (d == 64) return attn_tc::launch_fwd_varlen<64, T>(mq, mk, mv, mask, extra0, yy, zsum, vl, cap, S, H, scale, clamp, yt, kk, st);
-    if (d == 80) return attn_tc::launch_fwd_varlen<80, T>(mq, mk, mv, mask, extra0, yy, zsum, vl, cap, S, H, scale, clamp, yt, kk, st);
-    return attn_tc::launch_fwd_varlen<128, T>(mq, mk, mv, mask, extra0, yy, zsum, vl, cap, S, H, scale, clamp, yt, kk, st);
+    if (d == 64) return attn_tc::launch_fwd_varlen<64, T>(mq, mk, mv, mask, extra0, yy, zsum, vl, cap, S, H, scale, clamp, yt, kk, G, st);
+    if (d == 80) return attn_tc::launch_fwd_varlen<80, T>(mq, mk, mv, mask, extra0, yy, zsum, vl, cap, S, H, scale, clamp, yt, kk, G, st);
+    return attn_tc::launch_fwd_varlen<128, T>(mq, mk, mv, mask, extra0, yy, zsum, vl, cap, S, H, scale, clamp, yt, kk, G, st);
 }
 
 extern "C" int spt_sparse_attn_varlen_fwd(const void *q, const void *k, const void *v, const uint32_t *mask,
                                           const int32_t *extra0, void *y, float *zsum, const void *work, int n_seq, int T,
                                           int max_seqlen, int d, int H, float scale, float clamp, int dtype, int flags,
                                           spt_stream_t stream) {
+    return spt_sparse_attn_varlen_fwd_gqa(q, k, v, mask, extra0, y, zsum, work, n_seq, T, max_seqlen, d, H, H, scale, clamp,
+                                          dtype, flags, stream);
+}
+
+extern "C" int spt_sparse_attn_varlen_fwd_gqa(const void *q, const void *k, const void *v, const uint32_t *mask,
+                                              const int32_t *extra0, void *y, float *zsum, const void *work, int n_seq,
+                                              int T, int max_seqlen, int d, int H, int Hkv, float scale, float clamp,
+                                              int dtype, int flags, spt_stream_t stream) {
     const char *what = "sparse_attn_varlen_fwd";
     SPT_REQUIRE(q && k && v && mask && extra0 && y && zsum && work, "%s: null pointer", what);
     int rc = check_attn_type(what, d, dtype, clamp);
     if (rc != SPT_OK) return rc;
     if ((rc = check_varlen(what, n_seq, T, max_seqlen, H)) != SPT_OK) return rc;
+    if ((rc = check_gqa(what, H, Hkv)) != SPT_OK) return rc;
     SPT_REQUIRE(((uintptr_t)q | (uintptr_t)k | (uintptr_t)v | (uintptr_t)y | (uintptr_t)mask | (uintptr_t)work) % 16 == 0,
                 "%s: operands must be 16-byte aligned", what);
     const int yt = (flags & SPT_ATTN_Y_TRANSPOSED) ? 1 : 0;
     const bool f16 = dtype == SPT_F16;
     CUtensorMap mq, mk, mv;
     if ((rc = attn_tc::make_map(&mq, q, 1, T, H, d, f16)) != SPT_OK) return rc;
-    if ((rc = attn_tc::make_map(&mk, k, 1, T, H, d, f16)) != SPT_OK) return rc;
-    if ((rc = attn_tc::make_map(&mv, v, 1, T, H, d, f16)) != SPT_OK) return rc;
+    if ((rc = attn_tc::make_map(&mk, k, 1, T, Hkv, d, f16)) != SPT_OK) return rc;
+    if ((rc = attn_tc::make_map(&mv, v, 1, T, Hkv, d, f16)) != SPT_OK) return rc;
     const attn_tc::Varlen vl = varlen_of(work, max_seqlen);
     const int cap = (int)varlen_capacity(n_seq, T);
-    return f16 ? attn_varlen_fwd_typed<__half>(mq, mk, mv, mask, extra0, y, zsum, vl, cap, T, d, H, scale, clamp, yt, k, as_stream(stream))
-               : attn_varlen_fwd_typed<__nv_bfloat16>(mq, mk, mv, mask, extra0, y, zsum, vl, cap, T, d, H, scale, clamp, yt, k,
+    const int G = H / Hkv;
+    return f16 ? attn_varlen_fwd_typed<__half>(mq, mk, mv, mask, extra0, y, zsum, vl, cap, T, d, H, scale, clamp, yt, k, G,
+                                               as_stream(stream))
+               : attn_varlen_fwd_typed<__nv_bfloat16>(mq, mk, mv, mask, extra0, y, zsum, vl, cap, T, d, H, scale, clamp, yt, k, G,
                                                       as_stream(stream));
 }
 
@@ -1184,11 +1269,17 @@ extern "C" size_t spt_sparse_attn_varlen_bwd_workspace_bytes(int T, int H) {
     return varlen_delta_bytes(T, H) + (size_t)H * T * 128 * 2;
 }
 
+// Hkv < H: + the dK and dV partials of every query head, [T, H, d] each (operand type)
+extern "C" size_t spt_sparse_attn_varlen_bwd_gqa_workspace_bytes(int T, int d, int H, int Hkv) {
+    const size_t base = spt_sparse_attn_varlen_bwd_workspace_bytes(T, H);
+    return T >= 1 && Hkv >= 1 && Hkv < H ? base + 2 * (size_t)H * T * d * 2 : base;
+}
+
 template <typename T>
 static int attn_varlen_bwd_typed(const void *q, const void *k, const void *v, const void *y, const void *grad_y,
                                  const uint32_t *mask, const int32_t *extra0, const float *zsum, void *grad_q, void *grad_k,
                                  void *grad_v, void *workspace, const attn_tc::Varlen &vl, int cap, int S, int d, int H,
-                                 float scale, float clamp, int yt, cudaStream_t st) {
+                                 int Hkv, float scale, float clamp, int yt, cudaStream_t st) {
     constexpr bool f16 = attn_tc::is_f16<T>;
     float *delta = (float *)workspace;
     T *dys = (T *)((char *)workspace + varlen_delta_bytes(S, H));
@@ -1200,15 +1291,21 @@ static int attn_varlen_bwd_typed(const void *q, const void *k, const void *v, co
     if (rc != SPT_OK) return rc;
     CUtensorMap mq, mk, mv, md;
     if ((rc = attn_tc::make_map(&mq, q, 1, S, H, d, f16)) != SPT_OK) return rc;
-    if ((rc = attn_tc::make_map(&mk, k, 1, S, H, d, f16)) != SPT_OK) return rc;
-    if ((rc = attn_tc::make_map(&mv, v, 1, S, H, d, f16)) != SPT_OK) return rc;
+    if ((rc = attn_tc::make_map(&mk, k, 1, S, Hkv, d, f16)) != SPT_OK) return rc;
+    if ((rc = attn_tc::make_map(&mv, v, 1, S, Hkv, d, f16)) != SPT_OK) return rc;
     if ((rc = attn_tc::make_map(&md, dys, 1, S, H, d, f16)) != SPT_OK) return rc;
+    const int G = H / Hkv;
     T *gq = (T *)grad_q, *gk = (T *)grad_k, *gv = (T *)grad_v;
-    if (d == 64)
-        return attn_tc::launch_bwd_varlen<64, T>(mq, mk, mv, md, mask, extra0, delta, zsum, gq, gk, gv, vl, cap, S, H, scale, clamp, st);
-    if (d == 80)
-        return attn_tc::launch_bwd_varlen<80, T>(mq, mk, mv, md, mask, extra0, delta, zsum, gq, gk, gv, vl, cap, S, H, scale, clamp, st);
-    return attn_tc::launch_bwd_varlen<128, T>(mq, mk, mv, md, mask, extra0, delta, zsum, gq, gk, gv, vl, cap, S, H, scale, clamp, st);
+    // G > 1: per-query-head dK / dV partials [T, H, d] after dO' in the workspace, then the group sum (see attn_bwd_typed)
+    T *pk = G > 1 ? (T *)((char *)workspace + spt_sparse_attn_varlen_bwd_workspace_bytes(S, H)) : gk;
+    T *pv = G > 1 ? pk + (size_t)H * S * d : gv;
+    rc = d == 64   ? attn_tc::launch_bwd_varlen<64, T>(mq, mk, mv, md, mask, extra0, delta, zsum, gq, pk, pv, vl, cap, S, H, G, scale, clamp, st)
+         : d == 80 ? attn_tc::launch_bwd_varlen<80, T>(mq, mk, mv, md, mask, extra0, delta, zsum, gq, pk, pv, vl, cap, S, H, G, scale, clamp, st)
+                   : attn_tc::launch_bwd_varlen<128, T>(mq, mk, mv, md, mask, extra0, delta, zsum, gq, pk, pv, vl, cap, S, H, G, scale, clamp, st);
+    if (rc != SPT_OK || G == 1) return rc;
+    const int64_t rows_kv = (int64_t)S * Hkv;
+    if ((rc = attn_tc::launch_group_sum<T>(pk, gk, rows_kv, G, d, st)) != SPT_OK) return rc;
+    return attn_tc::launch_group_sum<T>(pv, gv, rows_kv, G, d, st);
 }
 
 extern "C" int spt_sparse_attn_varlen_bwd(const void *q, const void *k, const void *v, const void *y, const void *grad_y,
@@ -1216,12 +1313,22 @@ extern "C" int spt_sparse_attn_varlen_bwd(const void *q, const void *k, const vo
                                           void *grad_k, void *grad_v, void *workspace, const void *work, int n_seq, int T,
                                           int max_seqlen, int d, int H, float scale, float clamp, int dtype, int flags,
                                           spt_stream_t stream) {
+    return spt_sparse_attn_varlen_bwd_gqa(q, k, v, y, grad_y, mask, extra0, zsum, grad_q, grad_k, grad_v, workspace, work, n_seq,
+                                          T, max_seqlen, d, H, H, scale, clamp, dtype, flags, stream);
+}
+
+extern "C" int spt_sparse_attn_varlen_bwd_gqa(const void *q, const void *k, const void *v, const void *y, const void *grad_y,
+                                              const uint32_t *mask, const int32_t *extra0, const float *zsum, void *grad_q,
+                                              void *grad_k, void *grad_v, void *workspace, const void *work, int n_seq,
+                                              int T, int max_seqlen, int d, int H, int Hkv, float scale, float clamp,
+                                              int dtype, int flags, spt_stream_t stream) {
     const char *what = "sparse_attn_varlen_bwd";
     SPT_REQUIRE(q && k && v && y && grad_y && mask && extra0 && zsum && grad_q && grad_k && grad_v && workspace && work,
                 "%s: null pointer", what);
     int rc = check_attn_type(what, d, dtype, clamp);
     if (rc != SPT_OK) return rc;
     if ((rc = check_varlen(what, n_seq, T, max_seqlen, H)) != SPT_OK) return rc;
+    if ((rc = check_gqa(what, H, Hkv)) != SPT_OK) return rc;
     SPT_REQUIRE(((uintptr_t)q | (uintptr_t)k | (uintptr_t)v | (uintptr_t)y | (uintptr_t)grad_y | (uintptr_t)mask |
                  (uintptr_t)workspace | (uintptr_t)work | (uintptr_t)grad_q | (uintptr_t)grad_k | (uintptr_t)grad_v) % 16 == 0,
                 "%s: operands must be 16-byte aligned", what);
@@ -1230,7 +1337,7 @@ extern "C" int spt_sparse_attn_varlen_bwd(const void *q, const void *k, const vo
     const int cap = (int)varlen_capacity(n_seq, T);
     if (dtype == SPT_F16)
         return attn_varlen_bwd_typed<__half>(q, k, v, y, grad_y, mask, extra0, zsum, grad_q, grad_k, grad_v, workspace, vl, cap, T, d,
-                                             H, scale, clamp, yt, as_stream(stream));
+                                             H, Hkv, scale, clamp, yt, as_stream(stream));
     return attn_varlen_bwd_typed<__nv_bfloat16>(q, k, v, y, grad_y, mask, extra0, zsum, grad_q, grad_k, grad_v, workspace, vl, cap,
-                                                T, d, H, scale, clamp, yt, as_stream(stream));
+                                                T, d, H, Hkv, scale, clamp, yt, as_stream(stream));
 }

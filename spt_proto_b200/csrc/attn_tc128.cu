@@ -69,7 +69,8 @@ attn_bwd_kv128_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_co
                       const __grid_constant__ CUtensorMap map_v, const __grid_constant__ CUtensorMap map_dys,
                       const uint32_t *__restrict__ mask, const int32_t *__restrict__ extra0,
                       const float *__restrict__ ndelta, E *__restrict__ dk, E *__restrict__ dv,
-                      int S, int H, int B, float scale, float scale_log2, float clamp_log2, const float *__restrict__ zsum) {
+                      int S, int H, int B, float scale, float scale_log2, float clamp_log2, const float *__restrict__ zsum,
+                      int G) {
     constexpr int ROWQ = rowq_bytes<E>;
     extern __shared__ unsigned char smem_raw[];
     const Smem sm = align_smem(smem_raw);
@@ -120,13 +121,14 @@ attn_bwd_kv128_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_co
         for (int item; (item = sched_item(w, n_items)) >= 0; ++w) {
             const int kt = item / B, b = item % B;     // key tile 0 is the heaviest: items are ordered by key tile
             const int hn = b / H, hh = b % H, n0 = kt * T, n_tiles = n_own - kt;
+            const int hk = hh / G;                     // key / value head of query head hh (G > 1: grouped-query attention)
             const size_t head = (size_t)b * S;
             const int buf = w & 1;
             if (lane == 0) {
                 mbar_wait(own_empty(buf), ((w >> 1) & 1) ^ 1);
                 mbar_expect_tx(own_full(buf), 2 * TILE);
-                tma_owner<D>(s_k + buf * TILE, &map_k, own_full(buf), hh, n0, hn);
-                tma_owner<D>(s_v + buf * TILE, &map_v, own_full(buf), hh, n0, hn);
+                tma_owner<D>(s_k + buf * TILE, &map_k, own_full(buf), hk, n0, hn);
+                tma_owner<D>(s_v + buf * TILE, &map_v, own_full(buf), hk, n0, hn);
             }
             uint4 mw[4];
 #pragma unroll
@@ -310,21 +312,21 @@ attn_bwd_kv128_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_co
 template <typename E>
 int launch_bwd_kv128(const CUtensorMap &mq, const CUtensorMap &mk, const CUtensorMap &mv, const CUtensorMap &md,
                      const uint32_t *mask, const int32_t *extra0, const float *ndelta, const float *zsum, E *gk, E *gv,
-                     int B, int S, int H, float scale, float clamp, cudaStream_t st) {
+                     int B, int S, int H, int G, float scale, float clamp, cudaStream_t st) {
     cudaFuncSetAttribute(attn_bwd_kv128_kernel<E>, cudaFuncAttributeMaxDynamicSharedMemorySize, kv_smem<E>);
     const int n_items = (S / T) * B;
     const int grid = n_items < num_sms() ? n_items : num_sms();
     attn_bwd_kv128_kernel<E><<<grid, THREADS, kv_smem<E>, st>>>(mq, mk, mv, md, mask, extra0, ndelta, gk, gv, S, H, B, scale,
-                                                              scale * LOG2E, clamp * LOG2E, zsum);
+                                                              scale * LOG2E, clamp * LOG2E, zsum, G);
     return after_launch("attn_bwd_kv128_kernel");
 }
 template int launch_bwd_kv128<__nv_bfloat16>(const CUtensorMap &, const CUtensorMap &, const CUtensorMap &,
                                              const CUtensorMap &, const uint32_t *, const int32_t *, const float *,
-                                             const float *, __nv_bfloat16 *, __nv_bfloat16 *, int, int, int, float, float,
-                                             cudaStream_t);
+                                             const float *, __nv_bfloat16 *, __nv_bfloat16 *, int, int, int, int, float,
+                                             float, cudaStream_t);
 template int launch_bwd_kv128<__half>(const CUtensorMap &, const CUtensorMap &, const CUtensorMap &, const CUtensorMap &,
                                       const uint32_t *, const int32_t *, const float *, const float *, __half *, __half *,
-                                      int, int, int, float, float, cudaStream_t);
+                                      int, int, int, int, float, float, cudaStream_t);
 
 
 // 16 fp32 accumulator values (scaled) -> 16 bf16 / fp16 = 32 contiguous bytes
@@ -357,7 +359,7 @@ attn_bwd_q128_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
                      const __grid_constant__ CUtensorMap map_v, const __grid_constant__ CUtensorMap map_dys,
                      const uint32_t *__restrict__ mask, const int32_t *__restrict__ extra0,
                      const float *__restrict__ ndelta, E *__restrict__ dq, int S, int H, int B, float scale,
-                     float scale_log2, float clamp_log2, const float *__restrict__ zsum) {
+                     float scale_log2, float clamp_log2, const float *__restrict__ zsum, int G) {
     extern __shared__ unsigned char smem_raw[];
     const Smem sm = align_smem(smem_raw);
     const uint32_t s_q = sm.base, s_dy = s_q + 2 * TILE, s_k = s_dy + 2 * TILE, s_v = s_k + ST * TILE;
@@ -405,7 +407,7 @@ attn_bwd_q128_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
             int g = 0, w = 0;
             for (int item; (item = sched_item(w, n_items)) >= 0; ++w) {
                 const int qt = n_own - 1 - item / B, b = item % B;       // the last query tile sees the most keys
-                const int hn = b / H, hh = b % H, n_tiles = qt + 1;
+                const int hn = b / H, hh = b % H, hk = hh / G, n_tiles = qt + 1;
                 const int buf = w & 1;
                 mbar_wait(own_empty(buf), ((w >> 1) & 1) ^ 1);
                 mbar_expect_tx(own_full(buf), 2 * TILE);
@@ -415,8 +417,8 @@ attn_bwd_q128_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
                     const int st = g % ST;
                     mbar_wait(kv_empty(st), ((g / ST) & 1) ^ 1);
                     mbar_expect_tx(kv_full(st), 2 * TILE);
-                    tma_owner<D>(s_k + st * TILE, &map_k, kv_full(st), hh, j * T, hn);
-                    tma_owner<D>(s_v + st * TILE, &map_v, kv_full(st), hh, j * T, hn);
+                    tma_owner<D>(s_k + st * TILE, &map_k, kv_full(st), hk, j * T, hn);
+                    tma_owner<D>(s_v + st * TILE, &map_v, kv_full(st), hk, j * T, hn);
                 }
             }
         }
@@ -547,18 +549,18 @@ static int grid_for(int n_items) { return n_items < num_sms() ? n_items : num_sm
 template <typename E>
 int launch_bwd_q128(const CUtensorMap &mq, const CUtensorMap &mk, const CUtensorMap &mv, const CUtensorMap &md,
                     const uint32_t *mask, const int32_t *extra0, const float *ndelta, const float *zsum, E *gq, int B,
-                    int S, int H, float scale, float clamp, cudaStream_t st) {
+                    int S, int H, int G, float scale, float clamp, cudaStream_t st) {
     cudaFuncSetAttribute(attn_bwd_q128_kernel<E>, cudaFuncAttributeMaxDynamicSharedMemorySize, Q_SMEM);
     attn_bwd_q128_kernel<E><<<grid_for((S / T) * B), THREADS, Q_SMEM, st>>>(mq, mk, mv, md, mask, extra0, ndelta, gq, S, H, B,
-                                                                           scale, scale * LOG2E, clamp * LOG2E, zsum);
+                                                                           scale, scale * LOG2E, clamp * LOG2E, zsum, G);
     return after_launch("attn_bwd_q128_kernel");
 }
 template int launch_bwd_q128<__nv_bfloat16>(const CUtensorMap &, const CUtensorMap &, const CUtensorMap &,
                                             const CUtensorMap &, const uint32_t *, const int32_t *, const float *,
-                                            const float *, __nv_bfloat16 *, int, int, int, float, float, cudaStream_t);
+                                            const float *, __nv_bfloat16 *, int, int, int, int, float, float, cudaStream_t);
 template int launch_bwd_q128<__half>(const CUtensorMap &, const CUtensorMap &, const CUtensorMap &, const CUtensorMap &,
                                      const uint32_t *, const int32_t *, const float *, const float *, __half *, int, int,
-                                     int, float, float, cudaStream_t);
+                                     int, int, float, float, cudaStream_t);
 
 }  // namespace attn_tc128
 }  // namespace spt

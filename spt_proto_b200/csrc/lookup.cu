@@ -44,6 +44,9 @@ struct LkVarlen {
     int coeff;
 };
 
+// Grouped-query attention: key codes have Hkv = H / G heads, the pre-pass builds the bitmaps once per key head, and the
+// kernels that take G read those of key head b / G for query head b (b = n H + h  ->  n Hkv + h / G).  G = 1: multi-head.
+
 // ------------------------------------------------------------------------------------------
 // Pre-pass: key codes [B, S, m] -> bitmaps KB[b][s][w][v][t], overflow flag if any code >= 16.
 // grid (W, B), block 128: warp = lane t, lane = bit i  (key j = 128 w + 4 i + t).
@@ -446,7 +449,7 @@ template <int M>
 __global__ void __launch_bounds__(LKM_THREADS)
 lookup_maskonly_kernel(const int32_t *__restrict__ query_codes, const uint32_t *__restrict__ kb,
                        const int *__restrict__ flag, uint32_t *__restrict__ mask_out,
-                       int32_t *__restrict__ extra0_out, int S, int nnz, int W, int H) {
+                       int32_t *__restrict__ extra0_out, int S, int nnz, int W, int H, int G) {
     if (*flag) return;  // some key code >= 16: the generic kernel handles this call
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int b = blockIdx.x;                      // grid (heads, row groups): every head's heaviest (last) row group first
@@ -463,7 +466,7 @@ lookup_maskonly_kernel(const int32_t *__restrict__ query_codes, const uint32_t *
     const int n_t = lim > t ? (lim - t + 3) / 4 : 0;
 
     {
-        const uint32_t *kb_head = kb + (size_t)b * M * W * LK_WORD_U32;
+        const uint32_t *kb_head = kb + (size_t)(b / G) * M * W * LK_WORD_U32;
         const int per_s = tw * LK_WORD_U32 / 4;  // uint4 per subspace
         for (int i = tid; i < M * per_s; i += LKM_THREADS) {
             const int s = i / per_s, o = i - s * per_s;
@@ -631,7 +634,7 @@ template <int M, bool VARLEN = false>
 __global__ void __launch_bounds__(LKM_THREADS)
 lookup_maskonly2_kernel(const int32_t *__restrict__ query_codes, const uint32_t *__restrict__ kb,
                         const int *__restrict__ flag, uint32_t *__restrict__ mask_out,
-                        int32_t *__restrict__ extra0_out, int S, int nnz, int W, int H, const LkVarlen vl = {}) {
+                        int32_t *__restrict__ extra0_out, int S, int nnz, int W, int H, int G, const LkVarlen vl = {}) {
     if (*flag) return;  // some key code >= 16: the generic kernel handles this call
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int b = blockIdx.x;                      // grid (heads, row groups): every head's heaviest (last) row group first
@@ -655,7 +658,7 @@ lookup_maskonly2_kernel(const int32_t *__restrict__ query_codes, const uint32_t 
     const uint32_t last_valid = valid_mask(tw - 1, nkeys);   // words 0 .. tw - 2 are fully valid for every row of the group
 
     {
-        const uint32_t *kb_head = kb + (size_t)b * M * W * LK_WORD_U32;
+        const uint32_t *kb_head = kb + (size_t)(b / G) * M * W * LK_WORD_U32;
         const int per_s = tw * LK_WORD_U32 / 4;  // uint4 per subspace
         for (int i = tid; i < M * per_s; i += LKM_THREADS) {
             const int s = i / per_s, o = i - s * per_s;
@@ -794,7 +797,7 @@ template <int M, bool VARLEN = false, bool STREAM = false>
 __global__ void __launch_bounds__(LKM_THREADS, STREAM ? (M == 16 ? 1 : 2) : 0)
 lookup_maskonly_big_kernel(const int32_t *__restrict__ query_codes, const uint32_t *__restrict__ kb,
                            const int *__restrict__ flag, uint32_t *__restrict__ mask_out,
-                           int32_t *__restrict__ extra0_out, int S, int nnz, int W, int H, const LkVarlen vl = {}) {
+                           int32_t *__restrict__ extra0_out, int S, int nnz, int W, int H, int G, const LkVarlen vl = {}) {
     if (*flag) return;  // some key code >= 16: the generic kernel handles this call
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int b = blockIdx.x;                      // grid (heads, row groups): every head's heaviest (last) row group first
@@ -820,9 +823,9 @@ lookup_maskonly_big_kernel(const int32_t *__restrict__ query_codes, const uint32
     const uint32_t last_valid = valid_mask(tw - 1, nkeys);
     const int nc = (tw + LKB_CHUNK - 1) / LKB_CHUNK;   // STREAM: chunks per pass
     if constexpr (STREAM) {
-        lks_load<M>(s_kb, kb + (size_t)b * M * W * LK_WORD_U32, 0, nc, tw, W, woff);
+        lks_load<M>(s_kb, kb + (size_t)(b / G) * M * W * LK_WORD_U32, 0, nc, tw, W, woff);
     } else {
-        const uint32_t *kb_head = kb + (size_t)b * M * W * LK_WORD_U32;
+        const uint32_t *kb_head = kb + (size_t)(b / G) * M * W * LK_WORD_U32;
         const int per_s = tw * LK_WORD_U32 / 4;  // uint4 per subspace
         for (int i = tid; i < M * per_s; i += LKM_THREADS) {
             const int s = i / per_s, o = i - s * per_s;
@@ -847,7 +850,7 @@ lookup_maskonly_big_kernel(const int32_t *__restrict__ query_codes, const uint32
     int len1 = 0, len2 = 0, len3 = 0;
     if constexpr (STREAM) {
         for (int c = 0; c < nc; ++c) {
-            lks_load<M>(s_kb, kb + (size_t)b * M * W * LK_WORD_U32, c + 1, nc, tw, W, woff);
+            lks_load<M>(s_kb, kb + (size_t)(b / G) * M * W * LK_WORD_U32, c + 1, nc, tw, W, woff);
             cp_async_wait1();
             __syncthreads();
             const uint32_t *pw = s_kb + (size_t)(c & 1) * M * LKB_CHUNK * LK_WORD_U32;
@@ -901,7 +904,7 @@ lookup_maskonly_big_kernel(const int32_t *__restrict__ query_codes, const uint32
         const uint32_t *pw = s_kb + (size_t)c0 * LK_WORD_U32;
         if constexpr (STREAM) {
             const int i = nc + c0 / LKB_CHUNK;
-            lks_load<M>(s_kb, kb + (size_t)b * M * W * LK_WORD_U32, i + 1, nc, tw, W, woff);
+            lks_load<M>(s_kb, kb + (size_t)(b / G) * M * W * LK_WORD_U32, i + 1, nc, tw, W, woff);
             cp_async_wait1();
             __syncthreads();
             pw = s_kb + (size_t)(i & 1) * M * LKB_CHUNK * LK_WORD_U32;
@@ -971,7 +974,7 @@ __global__ void __launch_bounds__(LK_THREADS)
 lookup_generic_kernel(const int32_t *__restrict__ query_codes, const int32_t *__restrict__ key_codes,
                       const int *__restrict__ flag, int flag_expect, int32_t *__restrict__ out,
                       uint32_t *__restrict__ mask_out, int32_t *__restrict__ extra0_out, int S, int m, int nnz, int H,
-                      int tiles, int nb, const LkVarlen vl = {}) {
+                      int G, int tiles, int nb, const LkVarlen vl = {}) {
     if (flag && (*flag != 0) != (flag_expect != 0)) return;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     uint16_t *s_out = reinterpret_cast<uint16_t *>(smem_raw);
@@ -1011,8 +1014,9 @@ lookup_generic_kernel(const int32_t *__restrict__ query_codes, const int32_t *__
     __syncthreads();
 
     GenericMatcher mt;
-    mt.kc = key_codes + ((size_t)(b / H) * S * H + (b % H)) * m + (size_t)start * H * m;
-    mt.kstride = H * m;
+    const int hkv = H / G;                        // key codes [N, S, H / G, m]: query head b % H reads kv head (b % H) / G
+    mt.kc = key_codes + ((size_t)(b / H) * S * hkv + (b % H) / G) * m + (size_t)start * hkv * m;
+    mt.kstride = hkv * m;
     mt.s_q = s_q + rl * m;
     mt.m = m;
     mt.div = m / 4;
@@ -1068,19 +1072,23 @@ static size_t lks_smem(int m) { return (size_t)2 * m * LKB_CHUNK * LK_WORD_U32 *
 
 template <int M, bool VARLEN>
 static void lks_launch(dim3 grid, const int32_t *qc, const uint32_t *kb, const int *flag, uint32_t *mask, int32_t *extra0,
-                       int S, int nnz, int W, int H, cudaStream_t st, const LkVarlen &vl = {}) {
+                       int S, int nnz, int W, int H, int G, cudaStream_t st, const LkVarlen &vl = {}) {
     const size_t smem = lks_smem(M);
     cudaFuncSetAttribute(lookup_maskonly_big_kernel<M, VARLEN, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    lookup_maskonly_big_kernel<M, VARLEN, true><<<grid, LKM_THREADS, smem, st>>>(qc, kb, flag, mask, extra0, S, nnz, W, H, vl);
+    lookup_maskonly_big_kernel<M, VARLEN, true><<<grid, LKM_THREADS, smem, st>>>(qc, kb, flag, mask, extra0, S, nnz, W, H, G, vl);
 }
 
 // n_codewords: codes are < n_codewords (the _ex entry points), or -1: unknown.  Where the generic kernel's row images do not
 // fit, only a promise of n_codewords <= 16 lets a call run: the fallback is skipped and a code >= 16 matches no key.
+// Hkv: key heads (grouped-query attention: query head h reads key head h / (H / Hkv)); the key bitmaps are built once per
+// key head.
 static int lookup_impl(const int32_t *query_codes, const int32_t *key_codes, int32_t *output, uint32_t *mask_out,
-                       int32_t *extra0_out, void *workspace, int B, int S, int m, int nnz, int H, int n_codewords,
+                       int32_t *extra0_out, void *workspace, int B, int S, int m, int nnz, int H, int Hkv, int n_codewords,
                        spt_stream_t stream) {
     SPT_REQUIRE(query_codes && key_codes && (output || mask_out), "lookup_fwd: null pointer");
     SPT_REQUIRE(H >= 1 && B % H == 0, "lookup_fwd: B=%d must be a multiple of the interleaved head count H=%d", B, H);
+    SPT_REQUIRE(Hkv >= 1 && H % Hkv == 0, "lookup_fwd: H=%d must be a multiple of the key head count Hkv=%d (Hkv >= 1)", H, Hkv);
+    const int G = H / Hkv;
     SPT_REQUIRE(B >= 1 && S >= 1 && S <= 65536, "lookup_fwd: bad batch/seq (B=%d, S=%d; S must be <= 65536)", B, S);
     SPT_REQUIRE(B <= 65535, "lookup_fwd: batch %d exceeds grid limit", B);
     SPT_REQUIRE(m >= 4, "lookup_fwd: n_subspaces must be >= 4 (got %d)", m);
@@ -1112,9 +1120,10 @@ static int lookup_impl(const int32_t *query_codes, const int32_t *key_codes, int
     if (fb_fits && gen_smem > 48 * 1024)
         cudaFuncSetAttribute(lookup_generic_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)gen_smem);
 
-    if (!bitmap_m_supported(m)) {
+    // grouped-query calls that are not mask-only at m 8, 10, 16 (index output, other m) run the generic kernel alone
+    if (!bitmap_m_supported(m) || (G > 1 && !mask_only)) {
         lookup_generic_kernel<<<grid, LK_THREADS, gen_smem, st>>>(query_codes, key_codes, nullptr, 0, output, mask_out,
-                                                                  extra0_out, S, m, nnz, H, tiles, B);
+                                                                  extra0_out, S, m, nnz, H, G, tiles, B);
         SPT_LAUNCH_CHECK("lookup_generic_kernel");
         return SPT_OK;
     }
@@ -1123,7 +1132,7 @@ static int lookup_impl(const int32_t *query_codes, const int32_t *key_codes, int
     uint32_t *kb = reinterpret_cast<uint32_t *>(reinterpret_cast<char *>(workspace) + 16);
     cudaError_t e = cudaMemsetAsync(flag, 0, 16, st);
     if (e != cudaSuccess) return fail(SPT_ERR_CUDA, "lookup_fwd: memset: %s", cudaGetErrorString(e));
-    lookup_pack_kernel<<<dim3(W, B), 128, 0, st>>>(key_codes, kb, flag, S, m, W, H);
+    lookup_pack_kernel<<<dim3(W, B / G), 128, 0, st>>>(key_codes, kb, flag, S, m, W, Hkv);
     SPT_LAUNCH_CHECK("lookup_pack_kernel");
     // without the fallback the kernels read flag + 1, a word of the zeroed 16 bytes that nothing raises
     const int *kflag = fb_fits ? flag : flag + 1;
@@ -1139,48 +1148,48 @@ static int lookup_impl(const int32_t *query_codes, const int32_t *key_codes, int
             if (v1 && m != 10) {
                 if (m == 8) {
                     cudaFuncSetAttribute(lookup_maskonly_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)msmem);
-                    lookup_maskonly_kernel<8><<<mgrid, LKM_THREADS, msmem, st>>>(query_codes, kb, kflag, mask_out, extra0_out, S, nnz, W, H);
+                    lookup_maskonly_kernel<8><<<mgrid, LKM_THREADS, msmem, st>>>(query_codes, kb, kflag, mask_out, extra0_out, S, nnz, W, H, G);
                 } else {
                     cudaFuncSetAttribute(lookup_maskonly_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)msmem);
-                    lookup_maskonly_kernel<16><<<mgrid, LKM_THREADS, msmem, st>>>(query_codes, kb, kflag, mask_out, extra0_out, S, nnz, W, H);
+                    lookup_maskonly_kernel<16><<<mgrid, LKM_THREADS, msmem, st>>>(query_codes, kb, kflag, mask_out, extra0_out, S, nnz, W, H, G);
                 }
             } else if (m == 8) {
                 cudaFuncSetAttribute(lookup_maskonly2_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)msmem);
-                lookup_maskonly2_kernel<8><<<mgrid, LKM_THREADS, msmem, st>>>(query_codes, kb, kflag, mask_out, extra0_out, S, nnz, W, H);
+                lookup_maskonly2_kernel<8><<<mgrid, LKM_THREADS, msmem, st>>>(query_codes, kb, kflag, mask_out, extra0_out, S, nnz, W, H, G);
             } else if (m == 10) {       // head dim 80 (OPT-2.7B) at d_codeword 8
                 cudaFuncSetAttribute(lookup_maskonly2_kernel<10>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)msmem);
-                lookup_maskonly2_kernel<10><<<mgrid, LKM_THREADS, msmem, st>>>(query_codes, kb, kflag, mask_out, extra0_out, S, nnz, W, H);
+                lookup_maskonly2_kernel<10><<<mgrid, LKM_THREADS, msmem, st>>>(query_codes, kb, kflag, mask_out, extra0_out, S, nnz, W, H, G);
             } else {
                 cudaFuncSetAttribute(lookup_maskonly2_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)msmem);
-                lookup_maskonly2_kernel<16><<<mgrid, LKM_THREADS, msmem, st>>>(query_codes, kb, kflag, mask_out, extra0_out, S, nnz, W, H);
+                lookup_maskonly2_kernel<16><<<mgrid, LKM_THREADS, msmem, st>>>(query_codes, kb, kflag, mask_out, extra0_out, S, nnz, W, H, G);
             }
             SPT_LAUNCH_CHECK("lookup_maskonly_kernel");
         } else if (bsmem <= 200 * 1024) {
             // long sequences: the plane-free mask-only kernel (S 8192 at m 8)
             if (m == 8) {
                 cudaFuncSetAttribute(lookup_maskonly_big_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bsmem);
-                lookup_maskonly_big_kernel<8><<<mgrid, LKM_THREADS, bsmem, st>>>(query_codes, kb, kflag, mask_out, extra0_out, S, nnz, W, H);
+                lookup_maskonly_big_kernel<8><<<mgrid, LKM_THREADS, bsmem, st>>>(query_codes, kb, kflag, mask_out, extra0_out, S, nnz, W, H, G);
             } else if (m == 10) {
                 cudaFuncSetAttribute(lookup_maskonly_big_kernel<10>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bsmem);
-                lookup_maskonly_big_kernel<10><<<mgrid, LKM_THREADS, bsmem, st>>>(query_codes, kb, kflag, mask_out, extra0_out, S, nnz, W, H);
+                lookup_maskonly_big_kernel<10><<<mgrid, LKM_THREADS, bsmem, st>>>(query_codes, kb, kflag, mask_out, extra0_out, S, nnz, W, H, G);
             } else {
                 cudaFuncSetAttribute(lookup_maskonly_big_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bsmem);
-                lookup_maskonly_big_kernel<16><<<mgrid, LKM_THREADS, bsmem, st>>>(query_codes, kb, kflag, mask_out, extra0_out, S, nnz, W, H);
+                lookup_maskonly_big_kernel<16><<<mgrid, LKM_THREADS, bsmem, st>>>(query_codes, kb, kflag, mask_out, extra0_out, S, nnz, W, H, G);
             }
             SPT_LAUNCH_CHECK("lookup_maskonly_big_kernel");
         } else {
             // longer still: the streaming kernel (its shared memory does not grow with S)
             if (m == 8)
-                lks_launch<8, false>(mgrid, query_codes, kb, kflag, mask_out, extra0_out, S, nnz, W, H, st);
+                lks_launch<8, false>(mgrid, query_codes, kb, kflag, mask_out, extra0_out, S, nnz, W, H, G, st);
             else if (m == 10)
-                lks_launch<10, false>(mgrid, query_codes, kb, kflag, mask_out, extra0_out, S, nnz, W, H, st);
+                lks_launch<10, false>(mgrid, query_codes, kb, kflag, mask_out, extra0_out, S, nnz, W, H, G, st);
             else
-                lks_launch<16, false>(mgrid, query_codes, kb, kflag, mask_out, extra0_out, S, nnz, W, H, st);
+                lks_launch<16, false>(mgrid, query_codes, kb, kflag, mask_out, extra0_out, S, nnz, W, H, G, st);
             SPT_LAUNCH_CHECK("lookup_maskonly_big_kernel(stream)");
         }
         if (!fb_fits) return SPT_OK;
         lookup_generic_kernel<<<fb_grid, LK_THREADS, gen_smem, st>>>(query_codes, key_codes, flag, 1, output, mask_out,
-                                                                  extra0_out, S, m, nnz, H, tiles, B);
+                                                                  extra0_out, S, m, nnz, H, G, tiles, B);
         SPT_LAUNCH_CHECK("lookup_generic_kernel(fallback)");
         return SPT_OK;
     }
@@ -1204,7 +1213,7 @@ static int lookup_impl(const int32_t *query_codes, const int32_t *key_codes, int
 #undef SPT_LK_CASE
     SPT_LAUNCH_CHECK("lookup_bitmap_kernel");
     lookup_generic_kernel<<<fb_grid, LK_THREADS, gen_smem, st>>>(query_codes, key_codes, flag, 1, output, mask_out,
-                                                              extra0_out, S, m, nnz, H, tiles, B);
+                                                              extra0_out, S, m, nnz, H, G, tiles, B);
     SPT_LAUNCH_CHECK("lookup_generic_kernel(fallback)");
     return SPT_OK;
 }
@@ -1212,14 +1221,14 @@ static int lookup_impl(const int32_t *query_codes, const int32_t *key_codes, int
 extern "C" int spt_lookup_fwd(const int32_t *query_codes, const int32_t *key_codes, int32_t *output, void *workspace,
                               int B, int S, int m, int nnz, spt_stream_t stream) {
     SPT_REQUIRE(output, "lookup_fwd: null output");
-    return lookup_impl(query_codes, key_codes, output, nullptr, nullptr, workspace, B, S, m, nnz, 1, -1, stream);
+    return lookup_impl(query_codes, key_codes, output, nullptr, nullptr, workspace, B, S, m, nnz, 1, 1, -1, stream);
 }
 
 extern "C" int spt_lookup_mask_fwd(const int32_t *query_codes, const int32_t *key_codes, int32_t *output,
                                    uint32_t *mask, int32_t *extra0, void *workspace, int B, int S, int m, int nnz,
                                    int H, spt_stream_t stream) {
     SPT_REQUIRE(mask && extra0, "lookup_mask_fwd: null mask / extra0");
-    return lookup_impl(query_codes, key_codes, output, mask, extra0, workspace, B, S, m, nnz, H, -1, stream);
+    return lookup_impl(query_codes, key_codes, output, mask, extra0, workspace, B, S, m, nnz, H, H, -1, stream);
 }
 
 extern "C" int spt_lookup_mask_fwd_ex(const int32_t *query_codes, const int32_t *key_codes, int32_t *output,
@@ -1227,7 +1236,17 @@ extern "C" int spt_lookup_mask_fwd_ex(const int32_t *query_codes, const int32_t 
                                       int H, int n_codewords, spt_stream_t stream) {
     SPT_REQUIRE(mask && extra0, "lookup_mask_fwd_ex: null mask / extra0");
     SPT_REQUIRE(n_codewords >= 1, "lookup_mask_fwd_ex: n_codewords must be >= 1 (got %d)", n_codewords);
-    return lookup_impl(query_codes, key_codes, output, mask, extra0, workspace, B, S, m, nnz, H, n_codewords, stream);
+    return spt_lookup_mask_gqa_fwd(query_codes, key_codes, output, mask, extra0, workspace, B, S, m, nnz, H, H, n_codewords,
+                                   stream);
+}
+
+extern "C" int spt_lookup_mask_gqa_fwd(const int32_t *query_codes, const int32_t *key_codes, int32_t *output,
+                                       uint32_t *mask, int32_t *extra0, void *workspace, int B, int S, int m, int nnz,
+                                       int H, int Hkv, int n_codewords, spt_stream_t stream) {
+    SPT_REQUIRE(mask && extra0, "lookup_mask_gqa_fwd: null mask / extra0");
+    SPT_REQUIRE(n_codewords >= 1 || n_codewords == -1, "lookup_mask_gqa_fwd: n_codewords must be >= 1, or -1 (got %d)",
+                n_codewords);
+    return lookup_impl(query_codes, key_codes, output, mask, extra0, workspace, B, S, m, nnz, H, Hkv, n_codewords, stream);
 }
 
 // ---- packed variable-length sequences ----------------------------------------------------------------------------------
@@ -1250,29 +1269,31 @@ extern "C" int spt_lookup_mask_varlen_max_seqlen(int m) {
 
 template <int M>
 static int lookup_varlen_launch(const int32_t *qc, const int32_t *kc, const uint32_t *kb, const int *flag, uint32_t *mask,
-                                int32_t *extra0, const LkVarlen &vl, int cap, int T, int H, cudaStream_t st) {
+                                int32_t *extra0, const LkVarlen &vl, int cap, int T, int H, int G, cudaStream_t st) {
     const size_t psmem = lkv_plane_smem(M, vl.groups), bsmem = lkv_big_smem(M, vl.groups);
     if (psmem <= LKV_SMEM_MAX) {
         cudaFuncSetAttribute(lookup_maskonly2_kernel<M, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)psmem);
-        lookup_maskonly2_kernel<M, true><<<dim3(H, cap), LKM_THREADS, psmem, st>>>(qc, kb, flag, mask, extra0, T, 0, cap, H, vl);
+        lookup_maskonly2_kernel<M, true><<<dim3(H, cap), LKM_THREADS, psmem, st>>>(qc, kb, flag, mask, extra0, T, 0, cap, H, G, vl);
         return after_launch("lookup_maskonly2_kernel(varlen)");
     }
     if (bsmem <= LKV_SMEM_MAX) {
         cudaFuncSetAttribute(lookup_maskonly_big_kernel<M, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bsmem);
-        lookup_maskonly_big_kernel<M, true><<<dim3(H, cap), LKM_THREADS, bsmem, st>>>(qc, kb, flag, mask, extra0, T, 0, cap, H, vl);
+        lookup_maskonly_big_kernel<M, true><<<dim3(H, cap), LKM_THREADS, bsmem, st>>>(qc, kb, flag, mask, extra0, T, 0, cap, H, G, vl);
         return after_launch("lookup_maskonly_big_kernel(varlen)");
     }
-    lks_launch<M, true>(dim3(H, cap), qc, kb, flag, mask, extra0, T, 0, cap, H, st, vl);
+    lks_launch<M, true>(dim3(H, cap), qc, kb, flag, mask, extra0, T, 0, cap, H, G, st, vl);
     return after_launch("lookup_maskonly_big_kernel(stream, varlen)");
 }
 
 static int lookup_varlen_impl(const int32_t *query_codes, const int32_t *key_codes, const void *work, uint32_t *mask,
-                              int32_t *extra0, void *workspace, int n_seq, int T, int max_seqlen, int H, int m,
+                              int32_t *extra0, void *workspace, int n_seq, int T, int max_seqlen, int H, int Hkv, int m,
                               int sparse_coeff, int n_codewords, spt_stream_t stream) {
     const char *what = n_codewords < 0 ? "lookup_mask_varlen_fwd" : "lookup_mask_varlen_fwd_ex";
     SPT_REQUIRE(query_codes && key_codes && work && mask && extra0 && workspace, "%s: null pointer", what);
     int rc = check_varlen(what, n_seq, T, max_seqlen, H);
     if (rc != SPT_OK) return rc;
+    SPT_REQUIRE(Hkv >= 1 && H % Hkv == 0, "%s: H=%d must be a multiple of the key head count Hkv=%d (Hkv >= 1)", what, H, Hkv);
+    const int G = H / Hkv;
     SPT_REQUIRE(m == 8 || m == 10 || m == 16, "%s: n_subspaces must be 8, 10 or 16 (got %d)", what, m);
     SPT_REQUIRE(sparse_coeff >= 1, "%s: sparse_coeff must be >= 1 (got %d)", what, sparse_coeff);
     SPT_REQUIRE(((uintptr_t)work | (uintptr_t)mask | (uintptr_t)workspace) % 16 == 0, "%s: work, mask and workspace must be 16-byte aligned", what);
@@ -1295,24 +1316,24 @@ static int lookup_varlen_impl(const int32_t *query_codes, const int32_t *key_cod
     uint32_t *kb = reinterpret_cast<uint32_t *>(reinterpret_cast<char *>(workspace) + 16);
     cudaError_t e = cudaMemsetAsync(flag, 0, 16, st);
     if (e != cudaSuccess) return fail(SPT_ERR_CUDA, "%s: memset: %s", what, cudaGetErrorString(e));
-    lookup_pack_kernel<true><<<dim3(cap, H), 128, 0, st>>>(key_codes, kb, flag, T, m, cap, H, vl);
+    lookup_pack_kernel<true><<<dim3(cap, Hkv), 128, 0, st>>>(key_codes, kb, flag, T, m, cap, Hkv, vl);
     SPT_LAUNCH_CHECK("lookup_pack_kernel(varlen)");
     const int *kflag = fb_fits ? flag : flag + 1;       // as in lookup_impl: flag + 1 is never raised
-    rc = m == 8    ? lookup_varlen_launch<8>(query_codes, key_codes, kb, kflag, mask, extra0, vl, cap, T, H, st)
-         : m == 10 ? lookup_varlen_launch<10>(query_codes, key_codes, kb, kflag, mask, extra0, vl, cap, T, H, st)
-                   : lookup_varlen_launch<16>(query_codes, key_codes, kb, kflag, mask, extra0, vl, cap, T, H, st);
+    rc = m == 8    ? lookup_varlen_launch<8>(query_codes, key_codes, kb, kflag, mask, extra0, vl, cap, T, H, G, st)
+         : m == 10 ? lookup_varlen_launch<10>(query_codes, key_codes, kb, kflag, mask, extra0, vl, cap, T, H, G, st)
+                   : lookup_varlen_launch<16>(query_codes, key_codes, kb, kflag, mask, extra0, vl, cap, T, H, G, st);
     if (rc != SPT_OK || !fb_fits) return rc;
     // codes >= 16 somewhere: the generic kernel redoes the call (flag-guarded, decided on the device)
     cudaFuncSetAttribute(lookup_generic_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)gsmem);
     lookup_generic_kernel<true><<<2 * num_sms(), LK_THREADS, gsmem, st>>>(query_codes, key_codes, flag, 1, nullptr, mask, extra0,
-                                                                         T, m, nnz_max, H, 0, H, vl);
+                                                                         T, m, nnz_max, H, G, 0, H, vl);
     return after_launch("lookup_generic_kernel(varlen fallback)");
 }
 
 extern "C" int spt_lookup_mask_varlen_fwd(const int32_t *query_codes, const int32_t *key_codes, const void *work,
                                           uint32_t *mask, int32_t *extra0, void *workspace, int n_seq, int T,
                                           int max_seqlen, int H, int m, int sparse_coeff, spt_stream_t stream) {
-    return lookup_varlen_impl(query_codes, key_codes, work, mask, extra0, workspace, n_seq, T, max_seqlen, H, m, sparse_coeff,
+    return lookup_varlen_impl(query_codes, key_codes, work, mask, extra0, workspace, n_seq, T, max_seqlen, H, H, m, sparse_coeff,
                               -1, stream);
 }
 
@@ -1321,6 +1342,16 @@ extern "C" int spt_lookup_mask_varlen_fwd_ex(const int32_t *query_codes, const i
                                              int max_seqlen, int H, int m, int sparse_coeff, int n_codewords,
                                              spt_stream_t stream) {
     SPT_REQUIRE(n_codewords >= 1, "lookup_mask_varlen_fwd_ex: n_codewords must be >= 1 (got %d)", n_codewords);
-    return lookup_varlen_impl(query_codes, key_codes, work, mask, extra0, workspace, n_seq, T, max_seqlen, H, m, sparse_coeff,
-                              n_codewords, stream);
+    return spt_lookup_mask_varlen_gqa_fwd(query_codes, key_codes, work, mask, extra0, workspace, n_seq, T, max_seqlen, H, H, m,
+                                          sparse_coeff, n_codewords, stream);
+}
+
+extern "C" int spt_lookup_mask_varlen_gqa_fwd(const int32_t *query_codes, const int32_t *key_codes, const void *work,
+                                              uint32_t *mask, int32_t *extra0, void *workspace, int n_seq, int T,
+                                              int max_seqlen, int H, int Hkv, int m, int sparse_coeff, int n_codewords,
+                                              spt_stream_t stream) {
+    SPT_REQUIRE(n_codewords >= 1 || n_codewords == -1, "lookup_mask_varlen_gqa_fwd: n_codewords must be >= 1, or -1 (got %d)",
+                n_codewords);
+    return lookup_varlen_impl(query_codes, key_codes, work, mask, extra0, workspace, n_seq, T, max_seqlen, H, Hkv, m,
+                              sparse_coeff, n_codewords, stream);
 }

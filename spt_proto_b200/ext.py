@@ -496,20 +496,36 @@ def _heads(t: torch.Tensor, name: str):
 LOOKUP_MAX_SEQ = 65536    # longest S of lookup_mask (include/spt_b200.h): the key indices of the reference fit uint16
 
 
+def _kv_heads(q: torch.Tensor, k: torch.Tensor, head_dim, what: str) -> int:
+    """Key / value head count of k against q (grouped-query attention): the same shape except along head_dim, where k's
+    count divides q's (query head h reads key head h // (H // Hkv)).  head_dim None: the same shape.  Raises before any
+    CUDA call."""
+    same = k.dim() == q.dim() and (
+        q.shape == k.shape if head_dim is None else
+        (q.shape[:head_dim] == k.shape[:head_dim] and q.shape[head_dim + 1:] == k.shape[head_dim + 1:]
+         and k.size(head_dim) >= 1 and q.size(head_dim) % k.size(head_dim) == 0))
+    if not same:
+        raise RuntimeError(f"{what}: k must have q's shape, except that an [N,S,H,*] / packed [T,H,*] q may come with k "
+                           f"of fewer heads Hkv, H % Hkv == 0 (got q {tuple(q.shape)}, k {tuple(k.shape)})")
+    return 1 if head_dim is None else k.size(head_dim)
+
+
 def lookup_mask(query: torch.Tensor, key: torch.Tensor, sparse_coeff: int, want_indices: bool = False,
                 n_codewords=None):
     """Same selection as lookup_forward_cuda, emitted as (mask [B,S,S/32] int32 bit-words in the
     lane-major layout: word 4g+t bit i <=> key 128g+4i+t, extra0 [B,S] int32 zero-padding multiplicity
     of key 0, indices [B,S,nnz] or None).
-    Codes: [B,S,m] head-major or [N,S,H,m] (heads interleaved, B = N*H).
+    Codes: [B,S,m] head-major or [N,S,H,m] (heads interleaved, B = N*H); 4-D key codes may have Hkv heads with
+    H % Hkv == 0 (grouped-query attention: query head h reads key head h // (H // Hkv)).
     n_codewords: the caller's promise that every code is < n_codewords (the codebook size).  At lengths where
     the fallback for codes >= 16 cannot run (beyond about 16 k tokens at sparse_coeff 8) only n_codewords <= 16
     lets the call run; None makes no promise (include/spt_b200.h, spt_lookup_mask_fwd_ex)."""
     _check_dim(key, query.dim(), "key")
     _check_type(key, torch.int32, "key")
     _check_type(query, torch.int32, "query")
-    if query.shape != key.shape or not query.is_cuda or not query.is_contiguous():
-        raise RuntimeError("query and key must be contiguous CUDA tensors of the same shape")
+    if not query.is_cuda or not query.is_contiguous():
+        raise RuntimeError("query and key must be contiguous CUDA tensors")
+    Hkv = _kv_heads(query, key, 2 if query.dim() == 4 else None, "lookup_mask")
     B, S, H = _heads(query, "query")
     m = query.size(-1)
     if sparse_coeff <= 0 or S % sparse_coeff != 0 or S % 128 != 0:
@@ -519,58 +535,66 @@ def lookup_mask(query: torch.Tensor, key: torch.Tensor, sparse_coeff: int, want_
     mask = torch.empty((B, S, S // 32), dtype=torch.int32, device=dev)
     extra0 = torch.empty((B, S), dtype=torch.int32, device=dev)
     indices = torch.empty((B, S, nnz), dtype=torch.int32, device=dev) if want_indices else None
-    ws = _workspace(lib.spt_lookup_workspace_bytes(B, S, m, nnz), query)
+    ws = _workspace(lib.spt_lookup_workspace_bytes(B // H * Hkv, S, m, nnz), query)   # key bitmaps: one per key head
     with _on_device(query):
-        if n_codewords is None:
-            check(lib.spt_lookup_mask_fwd(_p(query), _p(key), _p(indices), _p(mask), _p(extra0), _p(ws), B, S, m, nnz, H,
-                                          _stream(query)))
-        else:
-            check(lib.spt_lookup_mask_fwd_ex(_p(query), _p(key), _p(indices), _p(mask), _p(extra0), _p(ws), B, S, m, nnz,
-                                             H, int(n_codewords), _stream(query)))
+        check(lib.spt_lookup_mask_gqa_fwd(_p(query), _p(key), _p(indices), _p(mask), _p(extra0), _p(ws), B, S, m, nnz, H,
+                                          Hkv, _codewords(n_codewords, "lookup_mask"), _stream(query)))
     return mask, extra0, indices
 
 
-def _check_attn(q, k, v):
-    """-> (B, S, d, H, dtype code): q, k, v of one shape and one dtype, bf16 or fp16."""
+def _codewords(n_codewords, what: str) -> int:
+    """n_codewords of the lookups: None (no promise) -> -1, else a codebook size >= 1."""
+    if n_codewords is None:
+        return -1
+    if int(n_codewords) < 1:
+        raise RuntimeError(f"{what}: n_codewords must be >= 1 (got {n_codewords})")
+    return int(n_codewords)
+
+
+def _check_attn(q, k, v, packed: bool = False):
+    """-> (B, S, d, H, Hkv, dtype code): q, k, v of one dtype, bf16 or fp16; k and v of one shape, q's or (4-D
+    [N,S,H,d] q, or packed [T,H,d] / [1,T,H,d] q) with Hkv heads, H % Hkv == 0 (grouped-query attention)."""
     if q.dtype not in _ATTN_DTYPES:
         raise RuntimeError("q must be type of torch.bfloat16 or torch.float16")
+    if k.shape != v.shape:
+        raise RuntimeError("k and v must have the same shape (one key / value head count)")
+    Hkv = _kv_heads(q, k, q.dim() - 2 if packed else (2 if q.dim() == 4 else None), "sparse_attn")
     for name, t in (("q", q), ("k", k), ("v", v)):
         _check_dim(t, q.dim(), name)
         _check_type(t, q.dtype, name)
-    if q.shape != k.shape or q.shape != v.shape:
-        raise RuntimeError("q, k, v must have the same shape")
     B, S, H = _heads(q, "q")
-    return B, S, q.size(-1), H, _ATTN_DTYPES[q.dtype]
+    return B, S, q.size(-1), H, Hkv, _ATTN_DTYPES[q.dtype]
 
 
 def sparse_attn_fwd(q, k, v, mask, extra0, scale: float, clamp: float = 10.0, reference_layout: bool = False):
-    """q, k, v: [B,S,d] head-major or [N,S,H,d] (native layer layout, no transposes), all bf16 or all fp16
-    -> (y, same shape and dtype as q; zsum [B,S] fp32).  fp16 needs 0 <= clamp <= 10.  reference_layout: y's MEMORY is the shipped layer's y^T [B, d, S]
+    """q, k, v: [B,S,d] head-major or [N,S,H,d] (native layer layout, no transposes), all bf16 or all fp16; 4-D k and v
+    may have Hkv heads, H % Hkv == 0 (grouped-query attention) -> (y, same shape and dtype as q; zsum [B,S] fp32).
+    fp16 needs 0 <= clamp <= 10.  reference_layout: y's MEMORY is the shipped layer's y^T [B, d, S]
     (attention.py:139-142), returned viewed with q's shape.  See include/spt_b200.h."""
-    B, S, d, H, code = _check_attn(q, k, v)
+    B, S, d, H, Hkv, code = _check_attn(q, k, v)
     y = torch.empty_like(q)
     zsum = torch.empty((B, S), dtype=torch.float32, device=q.device)
     with _on_device(q):
-        check(lib.spt_sparse_attn_fwd_ex(_p(q), _p(k), _p(v), _p(mask), _p(extra0), _p(y), _p(zsum), B, S, d, H,
-                                         float(scale), float(clamp), code,
-                                         SPT_ATTN_Y_TRANSPOSED if reference_layout else 0, _stream(q)))
+        check(lib.spt_sparse_attn_fwd_gqa(_p(q), _p(k), _p(v), _p(mask), _p(extra0), _p(y), _p(zsum), B, S, d, H, Hkv,
+                                          float(scale), float(clamp), code,
+                                          SPT_ATTN_Y_TRANSPOSED if reference_layout else 0, _stream(q)))
     return y, zsum
 
 
 def sparse_attn_bwd(q, k, v, y, grad_y, mask, extra0, zsum, scale: float, clamp: float = 10.0,
                     reference_layout: bool = False):
-    """-> (grad_q, grad_k, grad_v) in q's dtype.  reference_layout: y and grad_y are in the layout
-    sparse_attn_fwd(..., reference_layout=True) returned."""
-    B, S, d, H, code = _check_attn(q, k, v)
+    """-> (grad_q, grad_k, grad_v) in q's dtype, with q's, k's and v's shapes.  reference_layout: y and grad_y are in the
+    layout sparse_attn_fwd(..., reference_layout=True) returned."""
+    B, S, d, H, Hkv, code = _check_attn(q, k, v)
     _check_dim(grad_y, q.dim(), "grad_y")
     _check_type(grad_y, q.dtype, "grad_y")
     _check_type(y, q.dtype, "y")
     gq, gk, gv = torch.empty_like(q), torch.empty_like(k), torch.empty_like(v)
-    ws = _workspace(lib.spt_sparse_attn_bwd_workspace_bytes(B, S), q)
+    ws = _workspace(lib.spt_sparse_attn_bwd_gqa_workspace_bytes(B, S, d, H, Hkv), q)
     with _on_device(q):
-        check(lib.spt_sparse_attn_bwd_ex(_p(q), _p(k), _p(v), _p(y), _p(grad_y), _p(mask), _p(extra0), _p(zsum),
-                                         _p(gq), _p(gk), _p(gv), _p(ws), B, S, d, H, float(scale), float(clamp), code,
-                                         SPT_ATTN_Y_TRANSPOSED if reference_layout else 0, _stream(q)))
+        check(lib.spt_sparse_attn_bwd_gqa(_p(q), _p(k), _p(v), _p(y), _p(grad_y), _p(mask), _p(extra0), _p(zsum),
+                                          _p(gq), _p(gk), _p(gv), _p(ws), B, S, d, H, Hkv, float(scale), float(clamp), code,
+                                          SPT_ATTN_Y_TRANSPOSED if reference_layout else 0, _stream(q)))
     return gq, gk, gv
 
 
@@ -636,11 +660,13 @@ def lookup_mask_varlen(query: torch.Tensor, key: torch.Tensor, cu_seqlens: torch
                        sparse_coeff: int, work=None, n_codewords=None):
     """lookup_mask of every sequence of a packed batch alone, in one launch per kernel.  Codes [T, H, m] or [1, T, H, m]
     int32; cu_seqlens int32 [n + 1] on the device -> (mask [H, T, 4 ceil(max_seqlen / 128)] int32 lane-major words
-    relative to each sequence's start, extra0 [H, T] int32).  n_codewords: as in lookup_mask."""
+    relative to each sequence's start, extra0 [H, T] int32).  Key codes may have Hkv heads, H % Hkv == 0 (grouped-query
+    attention).  n_codewords: as in lookup_mask."""
     _check_type(query, torch.int32, "query")
     _check_type(key, torch.int32, "key")
-    if query.shape != key.shape or not query.is_cuda or not query.is_contiguous() or not key.is_contiguous():
-        raise RuntimeError("query and key must be contiguous CUDA tensors of the same shape")
+    if not query.is_cuda or not query.is_contiguous() or not key.is_contiguous():
+        raise RuntimeError("query and key must be contiguous CUDA tensors")
+    Hkv = _kv_heads(query, key, query.dim() - 2, "lookup_mask_varlen")
     T, H = _tokens(query, "query")
     m = query.size(-1)
     cu = _cu_device(cu_seqlens, query)
@@ -650,23 +676,20 @@ def lookup_mask_varlen(query: torch.Tensor, key: torch.Tensor, cu_seqlens: torch
     words = 4 * ((int(max_seqlen) + 127) // 128)
     mask = torch.empty((H, T, words), dtype=torch.int32, device=query.device)
     extra0 = torch.empty((H, T), dtype=torch.int32, device=query.device)
-    ws = _workspace(lib.spt_lookup_mask_varlen_workspace_bytes(n_seq, T, H, m), query)
+    ws = _workspace(lib.spt_lookup_mask_varlen_workspace_bytes(n_seq, T, Hkv, m), query)   # key bitmaps per key head
     with _on_device(query):
-        if n_codewords is None:
-            check(lib.spt_lookup_mask_varlen_fwd(_p(query), _p(key), _p(work), _p(mask), _p(extra0), _p(ws), n_seq, T,
-                                                 int(max_seqlen), H, m, int(sparse_coeff), _stream(query)))
-        else:
-            check(lib.spt_lookup_mask_varlen_fwd_ex(_p(query), _p(key), _p(work), _p(mask), _p(extra0), _p(ws), n_seq, T,
-                                                    int(max_seqlen), H, m, int(sparse_coeff), int(n_codewords),
-                                                    _stream(query)))
+        check(lib.spt_lookup_mask_varlen_gqa_fwd(_p(query), _p(key), _p(work), _p(mask), _p(extra0), _p(ws), n_seq, T,
+                                                 int(max_seqlen), H, Hkv, m, int(sparse_coeff),
+                                                 _codewords(n_codewords, "lookup_mask_varlen"), _stream(query)))
     return mask, extra0
 
 
 def sparse_attn_varlen_fwd(q, k, v, mask, extra0, cu_seqlens, max_seqlen: int, scale: float, clamp: float = 10.0,
                            reference_layout: bool = False, work=None):
-    """sparse_attn_fwd of every sequence of a packed batch: q, k, v [T, H, d] or [1, T, H, d] -> (y like q, zsum [H, T]).
+    """sparse_attn_fwd of every sequence of a packed batch: q, k, v [T, H, d] or [1, T, H, d] (k, v may have Hkv heads,
+    H % Hkv == 0) -> (y like q, zsum [H, T]).
     reference_layout: sequence i's y memory is its own y_i^T [H, d, S_i] at token offset cu[i]."""
-    _B, _S, d, _H, code = _check_attn(q, k, v)
+    _B, _S, d, _H, Hkv, code = _check_attn(q, k, v, packed=True)
     T, H = _tokens(q, "q")
     cu = _cu_device(cu_seqlens, q)
     if work is None:
@@ -674,16 +697,16 @@ def sparse_attn_varlen_fwd(q, k, v, mask, extra0, cu_seqlens, max_seqlen: int, s
     y = torch.empty_like(q)
     zsum = torch.empty((H, T), dtype=torch.float32, device=q.device)
     with _on_device(q):
-        check(lib.spt_sparse_attn_varlen_fwd(_p(q), _p(k), _p(v), _p(mask), _p(extra0), _p(y), _p(zsum), _p(work),
-                                             cu.numel() - 1, T, int(max_seqlen), d, H, float(scale), float(clamp), code,
-                                             SPT_ATTN_Y_TRANSPOSED if reference_layout else 0, _stream(q)))
+        check(lib.spt_sparse_attn_varlen_fwd_gqa(_p(q), _p(k), _p(v), _p(mask), _p(extra0), _p(y), _p(zsum), _p(work),
+                                                 cu.numel() - 1, T, int(max_seqlen), d, H, Hkv, float(scale), float(clamp), code,
+                                                 SPT_ATTN_Y_TRANSPOSED if reference_layout else 0, _stream(q)))
     return y, zsum
 
 
 def sparse_attn_varlen_bwd(q, k, v, y, grad_y, mask, extra0, zsum, cu_seqlens, max_seqlen: int, scale: float,
                            clamp: float = 10.0, reference_layout: bool = False, work=None):
-    """-> (grad_q, grad_k, grad_v) of sparse_attn_varlen_fwd."""
-    _B, _S, d, _H, code = _check_attn(q, k, v)
+    """-> (grad_q, grad_k, grad_v) of sparse_attn_varlen_fwd, with q's, k's and v's shapes."""
+    _B, _S, d, _H, Hkv, code = _check_attn(q, k, v, packed=True)
     T, H = _tokens(q, "q")
     _check_type(grad_y, q.dtype, "grad_y")
     _check_type(y, q.dtype, "y")
@@ -693,12 +716,12 @@ def sparse_attn_varlen_bwd(q, k, v, y, grad_y, mask, extra0, zsum, cu_seqlens, m
     if work is None:
         work = varlen_worklist(cu, T, max_seqlen)
     gq, gk, gv = torch.empty_like(q), torch.empty_like(k), torch.empty_like(v)
-    ws = _workspace(lib.spt_sparse_attn_varlen_bwd_workspace_bytes(T, H), q)
+    ws = _workspace(lib.spt_sparse_attn_varlen_bwd_gqa_workspace_bytes(T, d, H, Hkv), q)
     with _on_device(q):
-        check(lib.spt_sparse_attn_varlen_bwd(_p(q), _p(k), _p(v), _p(y), _p(grad_y), _p(mask), _p(extra0), _p(zsum),
-                                             _p(gq), _p(gk), _p(gv), _p(ws), _p(work), cu.numel() - 1, T, int(max_seqlen),
-                                             d, H, float(scale), float(clamp), code,
-                                             SPT_ATTN_Y_TRANSPOSED if reference_layout else 0, _stream(q)))
+        check(lib.spt_sparse_attn_varlen_bwd_gqa(_p(q), _p(k), _p(v), _p(y), _p(grad_y), _p(mask), _p(extra0), _p(zsum),
+                                                 _p(gq), _p(gk), _p(gv), _p(ws), _p(work), cu.numel() - 1, T,
+                                                 int(max_seqlen), d, H, Hkv, float(scale), float(clamp), code,
+                                                 SPT_ATTN_Y_TRANSPOSED if reference_layout else 0, _stream(q)))
     return gq, gk, gv
 
 

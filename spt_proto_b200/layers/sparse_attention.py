@@ -114,6 +114,36 @@ class _SparseV2Mixin:
                 and (q.size(1) // self.sparse_coeff) % 4 == 0 and q.size(1) // self.sparse_coeff >= 8
                 and q.size(1) <= ext.LOOKUP_MAX_SEQ)
 
+    @staticmethod
+    def _kv_group(q, k, v) -> int:
+        """G = H // Hkv for grouped-query / multi-query attention: q [N, S, H, E] (packed: [1, T, H, E]) with k, v
+        [N, S, Hkv, E], H % Hkv == 0; query head h attends with key / value head h // G (the contiguous grouping of HF
+        LLaMA / Mistral repeat_kv, i.e. torch.repeat_interleave(k, G, dim=2)).  1 when q, k, v share one shape.
+        Raises ValueError naming the broken rule."""
+        if q.shape == k.shape == v.shape:
+            return 1
+        if k.shape != v.shape:
+            raise ValueError(f"k and v must have the same shape (got k {tuple(k.shape)}, v {tuple(v.shape)})")
+        if q.dim() != 4 or k.dim() != 4 or q.shape[:2] != k.shape[:2] or q.size(3) != k.size(3):
+            raise ValueError(f"grouped-query attention needs q [N, S, H, E] and k, v [N, S, Hkv, E] with the same N, S and "
+                             f"E (got q {tuple(q.shape)}, k {tuple(k.shape)})")
+        if k.size(2) < 1 or q.size(2) % k.size(2):
+            raise ValueError(f"the query head count H = {q.size(2)} must be a multiple of the key / value head count "
+                             f"Hkv = {k.size(2)}")
+        return q.size(2) // k.size(2)
+
+    @staticmethod
+    def _repeat_kv(k, v, G: int):
+        """k, v repeated to H heads (HF repeat_kv): the multi-head input the grouped-query result is defined by."""
+        return (k, v) if G == 1 else (k.repeat_interleave(G, dim=2), v.repeat_interleave(G, dim=2))
+
+    @staticmethod
+    def _encode_qk(q, k, weight):
+        """quantizer('encode') of q and k: one launch for both when they share a shape, else (fewer key heads) one each."""
+        if q.shape == k.shape:
+            return ext.pq_encode_pair(q, k, weight)
+        return ext.pq_encode(q, weight), ext.pq_encode(k, weight)
+
     def _maybe_train_loss(self, q, k):
         if self.host_trigger is not None:
             armed, self.host_trigger = bool(self.host_trigger), False
@@ -130,8 +160,10 @@ class _SparseV2Mixin:
         # the attention kernels stride over the interleaved heads, so none of the reference's
         # transpose(1, 2).contiguous() copies (attention.py:92-95,138-142) is made
         q, k, v = q.contiguous(), k.contiguous(), v.contiguous()
-        self._maybe_train_loss(q, k)           # PQ loss is a mean over rows: layout-invariant
-        q_c, k_c = ext.pq_encode_pair(q, k, self.quantizer.weight)   # quantizer('encode') of both: [N, S, H, m]
+        # PQ loss is a mean over rows: layout-invariant.  With fewer key heads (grouped-query attention) it runs on the
+        # un-repeated k, whose mean equals that of the repeated k: every row appears G times there.
+        self._maybe_train_loss(q, k)
+        q_c, k_c = self._encode_qk(q, k, self.quantizer.weight)   # [N, S, H, m] and [N, S, Hkv, m]
         n_codewords = self.quantizer.weight.size(1)
         # [N, S, H, E]; with reference_output_layout the kernel writes the shipped layer's re-interpretation of
         # [N*H, E, S] memory itself (forward epilogue / backward row prologue): no permute pass either way
@@ -162,8 +194,10 @@ class _SparseV2Mixin:
         False) every sequence runs forward() on its own, after one synchronisation to read the offsets."""
         squeeze = q.dim() == 3
         q, k, v = (t.unsqueeze(0) if squeeze else t for t in (q, k, v))
-        if q.dim() != 4 or q.size(0) != 1 or q.shape != k.shape or q.shape != v.shape:
-            raise ValueError("forward_packed: q, k, v must all be [T, H, E] or [1, T, H, E]")
+        if q.dim() != 4 or q.size(0) != 1 or k.dim() != 4 or v.dim() != 4:
+            raise ValueError("forward_packed: q, k, v must all be [T, H, E] or [1, T, H, E] (k, v: [T, Hkv, E] or "
+                             "[1, T, Hkv, E] with H % Hkv == 0)")
+        self._kv_group(q, k, v)
         T = q.size(1)
         if isinstance(cu_seqlens, torch.Tensor) and cu_seqlens.is_cuda:
             if max_seqlen is None:
@@ -178,8 +212,8 @@ class _SparseV2Mixin:
             self.last_path = "fused_packed"
             q, k, v = self._rotate_packed(q, cu, max_seqlen), self._rotate_packed(k, cu, max_seqlen), v.contiguous()
             q, k = q.contiguous(), k.contiguous()
-            self._maybe_train_loss(q, k)      # over all T rows
-            q_c, k_c = ext.pq_encode_pair(q, k, self.quantizer.weight)
+            self._maybe_train_loss(q, k)      # over all T rows (un-repeated k: see _fused_forward)
+            q_c, k_c = self._encode_qk(q, k, self.quantizer.weight)
             n_codewords = self.quantizer.weight.size(1)
             if max_seqlen > self.recompute_mask_above:
                 y = kernels.sparse_attention_varlen_recompute(q, k, v, q_c, k_c, cu, max_seqlen, self.sparse_coeff,
@@ -241,11 +275,12 @@ class SparseVanillaAttentionV2(_SparseV2Mixin, VanillaAttention):
         return self._sparse_get_attn(q, k)
 
     def forward(self, q, k, v, attn_mask=None):
+        G = self._kv_group(q, k, v)
         if self._fused_ok(q):
             self.last_path = "fused"
             return self._fused_forward(q, k, v)
         self.last_path = "stage"
-        return self._stage_forward(q, k, v, attn_mask)
+        return self._stage_forward(q, *self._repeat_kv(k, v, G), attn_mask)
 
 
 class SparseRotaryAttentionV2(_SparseV2Mixin, RotaryAttention):
@@ -270,10 +305,11 @@ class SparseRotaryAttentionV2(_SparseV2Mixin, RotaryAttention):
         return self.embedding(x, ids=ids, n_positions=max_seqlen).to(x.dtype)
 
     def forward(self, q, k, v, attn_mask=None):
+        G = self._kv_group(q, k, v)
         if self._fused_ok(q):
             self.last_path = "fused"
             # fp32 rotation tables promote a bf16 input to fp32 (as in the reference); the fused kernels take the rotated
-            # operands in the input's own dtype
+            # operands in the input's own dtype (k at its own head count)
             return self._fused_forward(self._rotate(q).to(q.dtype), self._rotate(k).to(k.dtype), v)
         self.last_path = "stage"
-        return self._stage_forward(q, k, v, attn_mask)
+        return self._stage_forward(q, *self._repeat_kv(k, v, G), attn_mask)
